@@ -1,9 +1,13 @@
 #!/usr/bin/env python
 """bench.py - nav-step decisions/sec of the VLN-Imagine hot path on B200 (BASELINE.json's metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload duet_cfg2|hamt_cfg3|duet_cfg5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload duet_cfg2|hamt_cfg3|duet_cfg5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference          # the reference algorithm on the host CPU cores
+
+--dump-outputs DIR writes what the timed path computed in its last timed step (rank 0) as DIR/<name>.npy in float32, so
+that two builds can be compared output for output: the inputs, weights and dropout seeds depend on the arguments only.
+The files hold finite numbers only; where an output has -inf (masked logits), see dump_outputs / load_dump.
 
 One "step" = one navigation decision for every episode of the batch = the two per-step model calls the
 reference agent makes (DUET: 'panorama' + 'navigation', VLN-DUET/map_nav_src/r2r/agent.py:467,500; HAMT:
@@ -25,6 +29,7 @@ import statistics
 import sys
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -147,20 +152,69 @@ DUET_NAV_KEYS = ('txt_masks', 'gmap_img_embeds', 'gmap_step_ids', 'gmap_pos_fts'
                  'gmap_visited_masks', 'vp_img_embeds', 'vp_pos_fts', 'vp_masks', 'vp_nav_masks', 'imagine_masks')
 HAMT_VIS_KEYS = ('txt_masks', 'ob_img_feats', 'ob_ang_feats', 'ob_nav_types', 'ob_masks', 'imagine_masks')
 HAMT_HIST_KEYS = ('hist_img_feats', 'hist_ang_feats', 'hist_pano_img_feats', 'hist_pano_ang_feats')
+LOGITS = {'duet': 'fused_logits', 'hamt': 'act_logits'}
 
 
 def duet_step(model, d, txt, img):
+    """every tensor the two calls of a step hand back, by name"""
     pano, pano_masks = model('panorama', {k: d[k] for k in DUET_PANO_KEYS})
     nav = model('navigation', {**{k: d[k] for k in DUET_NAV_KEYS}, 'txt_embeds': txt, 'imagine_embeds': img,
                                'gmap_vpids': d['gmap_vpids'], 'vp_cand_vpids': d['vp_cand_vpids']})
-    return nav['fused_logits'], pano
+    return {'pano_embeds': pano, 'pano_masks': pano_masks, **{k: v for k, v in nav.items() if v is not None}}
 
 
 def hamt_step(model, d, txt, img):
+    """every tensor the two calls of a step hand back, by name"""
     out = model('visual', txt_embeds=txt, hist_embeds=d['hist_list'], hist_lens=d['hist_lens'], imagine_embeds=img,
                 **{k: d[k] for k in HAMT_VIS_KEYS})
     h = model('history', ob_step=d['ob_step'], **{k: d[k] for k in HAMT_HIST_KEYS})
-    return out[0], h
+    return {'act_logits': out[0], 'hist_embeds': h}
+
+
+DUMP_BYTES = 64 << 20                                   # --dump-outputs writes at most this much in all
+NONFINITE = '_nonfinite'                                # <name>_nonfinite.npy: 0 finite, -1 -inf, 1 +inf, 2 NaN
+
+
+def dump_outputs(directory, outputs):
+    """--dump-outputs: every tensor of ``outputs`` ({name: tensor}) as directory/<name>.npy in float32, every element finite.
+    Masked logits are -inf, so a tensor with non-finite elements is written with 0 in their place, and beside it
+    <name>_nonfinite.npy of the same shape tells which they were (load_dump puts them back).  When together the files would
+    exceed DUMP_BYTES, the smaller tensors are written whole and what is left of the budget is shared evenly by the others,
+    each written as a fixed sample of its elements (flat indices from a generator seeded with the name, in increasing order),
+    so that every run with the same arguments writes the same elements."""
+    os.makedirs(directory, exist_ok=True)
+    left = DUMP_BYTES // 4
+    items = sorted(outputs.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(items):
+        t = t.detach().float()
+        files = 1 if bool(torch.isfinite(t).all()) else 2
+        share = left // (len(items) - i) // files
+        if t.numel() > share:
+            idx = np.unique(np.random.default_rng(zlib.crc32(name.encode())).integers(0, t.numel(), share))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        left -= a.size * files
+        fin = np.isfinite(a)
+        np.save(os.path.join(directory, name + '.npy'), np.where(fin, a, 0).astype(np.float32))
+        if files == 2:
+            code = np.select([fin, np.isnan(a), a > 0], [0, 2, 1], -1).astype(np.float32)
+            np.save(os.path.join(directory, name + NONFINITE + '.npy'), code)
+
+
+def load_dump(directory):
+    """{name: float32 array} of what dump_outputs wrote to ``directory``, the non-finite elements put back"""
+    out = {}
+    for f in sorted(os.listdir(directory)):
+        if not f.endswith('.npy') or f.endswith(NONFINITE + '.npy'):
+            continue
+        name = f[:-4]
+        a = np.load(os.path.join(directory, f))
+        code_file = os.path.join(directory, name + NONFINITE + '.npy')
+        if os.path.exists(code_file):
+            code = np.load(code_file)
+            a = np.where(code == 0, a, np.select([code == -1, code == 1], [-np.inf, np.inf], np.nan)).astype(np.float32)
+        out[name] = a
+    return out
 
 
 def build(model_kind, shape, rank, precision):
@@ -411,19 +465,14 @@ def run_reference_arm(args, model_kind, shape, desc, rank):
     step, kind, note = reference_stepper(model_kind, shape, 'cpu')
     steps, warm = args.steps, args.warmup
     with torch.no_grad():
-        t0 = time.perf_counter()
-        step()
-        t_one = time.perf_counter() - t0
-        budget = float(os.environ.get('VI_REFERENCE_BUDGET_S', '240'))
-        if t_one * (steps + warm) > budget:                 # keep the whole arm within a few minutes, and say so
-            scale = budget / (t_one * (steps + warm))
-            steps, warm = max(int(steps * scale), 3), max(int(warm * scale), 1)
-        for _ in range(max(warm - 1, 0)):
+        for _ in range(warm):
             step()
         t0 = time.perf_counter()
         for _ in range(steps):
-            step()
+            out = step()
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {LOGITS[model_kind]: out})
     B = shape.batch
     val = B * steps / dt
     line = {'impl': 'reference', 'metric': METRIC, 'value': val, 'unit': UNIT, 'n_gpus': args.gpus, 'steps': steps,
@@ -442,9 +491,10 @@ def run_reference_arm(args, model_kind, shape, desc, rank):
 # ----------------------------------------------------------------------------------------------
 # fine-tuning workload (BASELINE.json cfg-4): forward + backward + gradient all-reduce + optimiser step
 # ----------------------------------------------------------------------------------------------
-def train_measure(args, shape, rank, local_rank, world, K, W, detail=True):
+def train_measure(args, shape, rank, local_rank, world, K, W, detail=True, dump_dir=None):
     """Fine-tuning iterations (forward + backward + gradient all-reduce + clipping + AdamW) on this rank's episodes; the
-    process group is the caller's.  Returns the measurements of rank 0's report (every rank must call it)."""
+    process group is the caller's.  Returns the measurements of rank 0's report (every rank must call it).  With dump_dir,
+    rank 0 writes the loss, gradients and updated parameters of the last timed iteration there (dump_outputs)."""
     import torch.distributed as dist
     from vln_imagine_b200 import config, duet, ops, synth, train
     dev = torch.device('cuda', local_rank)
@@ -548,6 +598,9 @@ def train_measure(args, shape, rank, local_rank, world, K, W, detail=True):
         torch.cuda.synchronize()
     barrier()
     ms = e0.elapsed_time(e1)
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {'loss': loss, 'gradients': flat.buffer,
+                                'parameters': torch.cat([p.detach().reshape(-1) for p in flat.params])})
     # e2e: the iteration's inputs come from pinned host memory, the loss is read back
     barrier()
     e0.record()
@@ -623,7 +676,7 @@ def run_train(args, shape, desc, rank, local_rank, world):
     dev = torch.device('cuda', local_rank)
     if world > 1:
         dist.init_process_group('nccl', device_id=dev)
-    r = train_measure(args, shape, rank, local_rank, world, args.steps, args.warmup, detail=True)
+    r = train_measure(args, shape, rank, local_rank, world, args.steps, args.warmup, detail=True, dump_dir=args.dump_outputs)
     ms, ms_e2e, K, W, T, B, h2d, launches, loss_host = (r[k] for k in ('ms', 'ms_e2e', 'K', 'W', 'T', 'B', 'h2d', 'launches', 'loss'))
     gemm_flops, gemm_ms, breakdown = r['gemm_flops'], r['gemm_ms'], r['breakdown']
     if world > 1:
@@ -687,11 +740,16 @@ def main():
     ap.add_argument('--precision', default='bf16', choices=['bf16', 'fp32'])
     ap.add_argument('--no-graph', action='store_true', help='time eager launches instead of a CUDA-graph replay')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed as DIR/<name>.npy '
+                    '(float32, at most 64 MB in all; rank 0)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
+    torch.manual_seed(1234 + rank)                      # the fine-tuning dropout seeds (autograd_ops.dropout_seed) follow it
     model_kind, shape, desc = workload(args.workload)
 
     if args.impl == 'reference':
@@ -750,14 +808,14 @@ def main():
         # ---- leg 1: inputs resident in HBM; the step replayed as a CUDA graph
         model.use_cuda_graphs = False                   # this leg captures the whole step itself
         for _ in range(3):
-            logits, _ = step_fn(model, d, txt, img2)
+            step_fn(model, d, txt, img2)
         torch.cuda.synchronize()
         new_episode()
         n0 = ops._Counters.launches
-        logits, _ = step_fn(model, d, txt, img2)            # first step of an episode
+        step_fn(model, d, txt, img2)                        # first step of an episode
         launches_first = ops._Counters.launches - n0
         n0 = ops._Counters.launches
-        logits, _ = step_fn(model, d, txt, img2)            # a later step
+        logits = step_fn(model, d, txt, img2)[LOGITS[model_kind]]      # a later step
         launches_later = ops._Counters.launches - n0
         state = {'i': 0}
         if not args.no_graph:
@@ -771,10 +829,10 @@ def main():
                     new_episode()                           # the capture then contains the context projections
                 g = torch.cuda.CUDAGraph()
                 with vgraphs.capture(g):
-                    step_fn(model, d, txt, img2)
-                return g
-            g_later = capture(False)
-            g_first = capture(True) if ctx_cache else g_later
+                    out = step_fn(model, d, txt, img2)      # every replay of g writes its results into these tensors
+                return g, out
+            g_later, out_later = capture(False)
+            g_first, out_first = capture(True) if ctx_cache else (g_later, out_later)
 
             def run():
                 (g_first if state['i'] % EP_LEN == 0 else g_later).replay()
@@ -783,7 +841,7 @@ def main():
             def run():
                 if state['i'] % EP_LEN == 0:
                     new_episode()
-                step_fn(model, d, txt, img2)
+                state['out'] = step_fn(model, d, txt, img2)
                 state['i'] += 1
         for _ in range(W):
             run()
@@ -803,6 +861,9 @@ def main():
         launches_per_step = launches_first
         ms = max_over_ranks(e0.elapsed_time(e1))
         value = world * B * K / (ms * 1e-3)
+        if args.dump_outputs and rank == 0:
+            last = state['out'] if args.no_graph else out_first if (K - 1) % EP_LEN == 0 else out_later
+            dump_outputs(args.dump_outputs, last)
 
         # ---- leg 2 (e2e): public module API; every step's inputs that the reference agent builds on the host
         # (r2r/agent.py:57-207: panorama / location features, nav types, graph step ids, position features, pair
@@ -834,7 +895,7 @@ def main():
                 hh = host['hist_embeds'].to(dev, non_blocking=True)
                 dd['hist_list'] = [hh[:, t] for t in range(hh.shape[1])]
                 dd['hist_lens'] = hist_lens_host             # python ints, as the agent passes them
-                lg, _ = step_fn(model, dd, txt, img2)
+                lg = step_fn(model, dd, txt, img2)['act_logits']
             else:
                 pano, _ = model('panorama', {k: dd[k] for k in DUET_PANO_KEYS})
                 dd['vp_img_embeds'] = torch.cat([torch.zeros_like(pano[:, :1]), pano], 1)     # agent.py:173-186
