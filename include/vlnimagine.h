@@ -55,28 +55,15 @@ int vi_init(int device);
  * Grouped form: rows are split into n_groups consecutive row ranges ending at group_row_end[g]
  * (HOST array; every group but the last must end on a multiple of 128 rows); group g uses rows
  * [g*N, (g+1)*N) of W / bias.  n_groups == 1 and group_row_end == NULL is the plain GEMM.
- * vi_gemm_bf16: X, W bf16; fp32 accumulation in TMEM (tcgen05.mma fed by TMA).  K % 64 == 0,
- *               N % 64 == 0, ldx % 8 == 0.  y_dtype selects bf16 or fp32 output.
+ * vi_gemm16   : X, W 16-bit; fp32 accumulation in TMEM (tcgen05.mma fed by TMA).  K % 64 == 0, N % 64 == 0, ldx % 8 == 0.
+ *               y_dtype selects a 16-bit (in_dtype) or an fp32 output.
  * vi_gemm_f32 : the fp32 check mode (FFMA, no tensor cores); X, W, Y fp32.
- * bias / residual may be NULL.  residual is fp32 [M, ldr] and requires an fp32 output in vi_gemm_bf16.
- * ------------------------------------------------------------------------------------------- */
-int vi_gemm_bf16(const void* x, int64_t ldx, const void* w, const float* bias,
-                 const float* residual, int64_t ldr, void* y, int64_t ldy, int y_dtype,
-                 int M, int N, int K, int epilogue,
-                 int n_groups, const int32_t* group_row_end, vi_stream_t stream);
-/* Same as vi_gemm_bf16 with the output-tile shape chosen by the caller: tile = width (64, 96, 128, 192, 256),
- * optionally | VI_TILE_PAIR for the two-CTA (cta_group::2, 256-row) form; 0 = the library's own cost model.
- * Results do not depend on the tile (the K accumulation order is the same). */
-#define VI_TILE_PAIR 0x1000
-int vi_gemm_bf16_tiled(const void* x, int64_t ldx, const void* w, const float* bias,
-                       const float* residual, int64_t ldr, void* y, int64_t ldy, int y_dtype,
-                       int M, int N, int K, int epilogue,
-                       int n_groups, const int32_t* group_row_end, int tile, vi_stream_t stream);
-/* The general form behind vi_gemm_bf16(_tiled): 16-bit operands of either format (bf16, or fp16 for tensors whose range
- * the caller has bounded: LayerNorm outputs, probabilities, their projections - same tensor-core rate, 8x smaller rounding
- * error; 16-bit outputs saturate at +-65504 instead of overflowing), an optional 16-bit copy of an fp32 output, and
- * LayerNorm folded into the neighbouring contractions so that BertSelfOutput / BertOutput (D/models/vilmodel.py:151-155,
- * 190-194) and norm1 / norm2 of the panorama encoder (D/models/transformer.py:171,179) need no pass of their own:
+ * bias / residual may be NULL.  residual is fp32 [M, ldr] and requires an fp32 output in vi_gemm16.
+ * Operands of either 16-bit format: bf16, or fp16 for tensors whose range the caller has bounded (LayerNorm outputs,
+ * probabilities, their projections - same tensor-core rate, 8x smaller rounding error; 16-bit outputs saturate at +-65504
+ * instead of overflowing).  Optionally a 16-bit copy of an fp32 output, and LayerNorm folded into the neighbouring
+ * contractions so that BertSelfOutput / BertOutput (D/models/vilmodel.py:151-155, 190-194) and norm1 / norm2 of the panorama
+ * encoder (D/models/transformer.py:171,179) need no pass of their own:
  *   stats_out  : the producer (dense + residual) writes, for every output row and every 32-column chunk, (mean, M2) of the
  *                chunk: float2 [N / 32][stats_ld].  Its fp32 output is the RAW pre-LayerNorm sum z (plus y16 = z in 16 bits).
  *   VI_LN_FOLD : the consumer computes LayerNorm(z) W^T + b from z itself:  x = z in 16 bits, w = W * gamma (columnwise),
@@ -85,7 +72,13 @@ int vi_gemm_bf16_tiled(const void* x, int64_t ldx, const void* w, const float* b
  *   VI_LN_RESIDUAL : the residual operand is LayerNorm(z) given as the RAW fp32 rows z: the epilogue adds
  *                (z - mu) / sigma * gamma + beta with ln_vec_a = gamma and bias = beta + b ([n_groups * N], N = 32 * ln_chunks;
  *                no activation).
- * Grouped calls index bias / ln_vec_* as [g * N + n]. */
+ * Grouped calls index bias / ln_vec_* as [g * N + n].
+ * tile: 0 = the library's own cost model, or the output-tile shape chosen by the caller: width (64, 96, 128, 192, 256)
+ * dividing N, optionally | VI_TILE_PAIR for the two-CTA (cta_group::2, 256-row) form, which needs width >= 128 and every
+ * group but the last ending on a multiple of 256 rows; any other request is VI_ERR_ARG.  Results do not depend on the tile
+ * (the K accumulation order is the same).
+ * ------------------------------------------------------------------------------------------- */
+#define VI_TILE_PAIR 0x1000
 enum { VI_LN_NONE = 0, VI_LN_FOLD = 1, VI_LN_RESIDUAL = 2 };
 typedef struct {
   const void* x; int64_t ldx;      /* [M, K] 16-bit */
@@ -97,7 +90,7 @@ typedef struct {
   void* y16; int64_t ldy16;        /* optional 16-bit copy (in_dtype) of an fp32 output, or NULL */
   int M, N, K, epilogue;
   int n_groups; const int32_t* group_row_end;   /* HOST array */
-  int tile;                        /* 0 or width | VI_TILE_PAIR */
+  int tile;                        /* 0 (cost model) or width | VI_TILE_PAIR */
   int ln_mode;                     /* VI_LN_* */
   const float* ln_vec_a;
   const float* ln_stats;           /* float2 [ln_chunks][stats_ld] written by the producer of the rows being normalised */
@@ -138,18 +131,10 @@ typedef struct {
   const uint32_t* drop_seed;   /* device pointer to the dropout seed, or NULL */
 } vi_attn_problem;
 /* Several independent attention problems (token streams of one row-stacked activation: DUET global | local,
- * HAMT language | vision) in ONE launch; same arithmetic as vi_attn_fwd per problem. */
+ * HAMT language | vision) in ONE launch; a single problem is n_problems == 1.  16-bit inference shapes (<= 96 keys, no
+ * dropout, no lse) run a single-pass kernel; dropout, lse or more keys run the generic mma.sync kernel. */
 int vi_attn_fwd_multi(const vi_attn_problem* problems, int n_problems, int H, int dtype, int mask_mode,
                       vi_stream_t stream);
-/* The same contraction on the 5th-gen tensor cores (vi_attn_tc.cu: tcgen05.mma M = 64 score tiles of two heads interleaved in
- * the TMEM lanes, TMA-fed operands, V consumed as an MN-major operand, softmax from tcgen05.ld).  Inference shapes only: 16-bit
- * operands, even H, Lk <= 256, no dropout / lse.  vi_attn_fwd_multi routes to it when VI_ATTN_TC=1; at the 30 - 37 query tiles of
- * this path the mma.sync kernel is faster (DESIGN.md), so it is not the default. */
-int vi_attn_fwd_tc(const vi_attn_problem* problems, int n_problems, int H, int dtype, int mask_mode, vi_stream_t stream);
-int vi_attn_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
-                void* o, int64_t ldo, int dtype,
-                const uint8_t* key_mask, const float* pair_dist, const float* bias_affine,
-                float* lse, int B, int H, int Lq, int Lk, int mask_mode, vi_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Row kernels (one warp per 768-wide row, fp32 statistics, 16-byte accesses).
@@ -280,10 +265,11 @@ int vi_copy_rows(const float* src, int64_t src_batch_stride, int64_t src_row_str
                  vi_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
- * Backward pass (fine-tuning).  The dense gradients reuse vi_gemm_* on transposed operands:
- *   dX = dY W  (vi_gemm with the [K, N] transposed weight shadow),  dW = dY^T X  (vi_gemm on vi_transpose'd
- *   dY and X),  db = vi_colsum(dY).  The entry points below are the adjoints of the remaining forward kernels;
- *   each mirrors what torch.autograd computes for the reference ops it cites.
+ * Backward pass (fine-tuning).  The dense gradients of the 16-bit path:
+ *   dX = dY W  (vi_gemm16 with the [K, N] transposed weight shadow),  dW = dY^T X and db = column sums of dY
+ *   (vi_wgrad16, no transposes).  The fp32 check mode computes dW with vi_gemm_f32 on vi_transpose'd dY and X and db with
+ *   vi_colsum.  The other entry points below are the adjoints of the remaining forward kernels; each mirrors what
+ *   torch.autograd computes for the reference ops it cites.
  * ------------------------------------------------------------------------------------------- */
 /* dst[c, r] = src[r, c]; dst is [cols, ldd] with columns rows..pad_rows-1 zero-filled (pad_rows <= ldd) */
 int vi_transpose(const void* src, int64_t ld, void* dst, int64_t ldd, int rows, int cols, int pad_rows, int dtype,
@@ -303,8 +289,7 @@ int vi_wgrad16(const void* dy, int64_t lddy, const void* x, int64_t ldx, int dty
                const int32_t* group_row_end, float* dw, float* db, float* workspace, int64_t workspace_floats, int splits,
                int accumulate, vi_stream_t stream);
 /* Column reductions over rows run in two deterministic stages (128-row chunks -> a caller-provided fp32 scratch ->
- * fixed-order sum).  vi_reduce_scratch_elems gives the scratch size for n_out reduced quantities per column. */
-int64_t vi_reduce_scratch_elems(int64_t rows, int cols, int n_out);
+ * fixed-order sum): n_out * ceil(rows / 128) * cols floats for n_out reduced quantities per column. */
 /* out[c] = sum_r x[r, c] (fp32 accumulation, fixed order); bias gradients of nn.Linear.  scratch: n_out = 1 */
 int vi_colsum(const void* x, int64_t ld, int dtype, float* out, int64_t rows, int cols, float* scratch,
               int64_t scratch_elems, vi_stream_t stream);
@@ -312,22 +297,15 @@ int vi_colsum(const void* x, int64_t ld, int dtype, float* out, int64_t rows, in
  * The training forward keeps the pre-activation, so activations run as their own kernels there. */
 int vi_act_fwd(const void* x, void* y, int64_t n, int act, int dtype, vi_stream_t stream);
 int vi_act_bwd(const void* x, const void* dy, void* dx, int64_t n, int act, int dtype, vi_stream_t stream);
-/* adjoint of vi_add_ln: dy = dy32 (+ dy16); dx (fp32 and/or bf16 copy) is the gradient of both a and b;
- * dgamma / dbeta [n_groups, 768] (16-byte aligned) may be NULL; stats is a [rows, 2] fp32 scratch (mean, rstd).
- * scratch: at least 2 * ceil(rows / 32) * 768 floats; with 2 * ceil(rows / 8) * 768 the kernel may use chunks of 8 or 16 rows
- * (more CTAs for the short streams of this path; the summation order, hence the last bits of dgamma / dbeta, follows the chunk). */
-int vi_add_ln_bwd(const float* a, const float* b, const float* gamma, float eps, const float* dy32, const void* dy16,
-                  float* dx32, void* dx16, float* dgamma, float* dbeta, float* stats, int64_t rows,
-                  int n_groups, const int32_t* group_row_end, float* scratch, int64_t scratch_elems, vi_stream_t stream);
-/* the same with dgamma / dbeta ADDED to (accumulate != 0) instead of overwritten */
-int vi_add_ln_bwd_acc(const float* a, const float* b, const float* gamma, float eps, const float* dy32, const void* dy16,
-                      float* dx32, void* dx16, float* dgamma, float* dbeta, float* stats, int64_t rows,
-                      int n_groups, const int32_t* group_row_end, float* scratch, int64_t scratch_elems, int accumulate,
-                      vi_stream_t stream);
 /* LN(dropout(a) + b) and its adjoint: the hidden dropout of BertSelfOutput / BertOutput (D/models/vilmodel.py:151-155,190-194)
- * applied inside the LayerNorm kernels (mask of vi_dropout for a [rows, 768] tensor at `site`).  Backward: dx32 / dx16 = gradient
- * of b; dxa16 (optional, bf16) = dropout(dx) = gradient of a, the operand of the dense layer's gradient GEMMs - no separate
- * dropout or cast pass.  p == 0: no dropout (dxa16 = the 16-bit copy of dx). */
+ * applied inside the LayerNorm kernels (mask of vi_dropout for a [rows, 768] tensor at `site`).  p == 0: no dropout, and
+ * vi_add_ln_drop_bwd is the adjoint of vi_add_ln.
+ * Backward: dy = dy32 (+ dy16); dx32 / dx16 = gradient of b (and of a when p == 0); dxa16 (optional, bf16) = dropout(dx) =
+ * gradient of a, the operand of the dense layer's gradient GEMMs - no separate dropout or cast pass (p == 0: the 16-bit copy
+ * of dx).  dgamma / dbeta [n_groups, 768] (16-byte aligned) are required; accumulate != 0 adds to them instead of overwriting.
+ * stats is a [rows, 2] fp32 scratch (mean, rstd).  scratch: at least 2 * ceil(rows / 32) * 768 floats; with
+ * 2 * ceil(rows / 8) * 768 the kernel may use chunks of 8 or 16 rows (more CTAs for the short streams of this path; the
+ * summation order, hence the last bits of dgamma / dbeta, follows the chunk). */
 int vi_add_ln_drop(const float* a, const float* b, const float* gamma, const float* beta, float eps, float* y32, void* y16,
                    int y16_dtype, int64_t rows, int n_groups, const int32_t* group_row_end, float p, const uint32_t* seed,
                    uint32_t site, vi_stream_t stream);
@@ -343,7 +321,7 @@ int vi_scatter_add_rows(const float* src, const int64_t* idx, int period, float*
 /* adjoint of the dot-product tail of vi_ln_dot (out[r] = x[r] . w[g] + b[g]) */
 int vi_rowdot_bwd(const float* dout, const float* x, const float* w, float* dx, float* dw, float* db_cols, int64_t rows,
                   int n_groups, const int32_t* group_row_end, float* scratch, int64_t scratch_elems, vi_stream_t stream);
-/* attention backward for one token stream (same operand conventions as vi_attn_fwd); d_affine -> device {dw, db}
+/* attention backward for one token stream (same operand conventions as one vi_attn_problem); d_affine -> device {dw, db}
  * of the GASA affine, accumulated (+=); dq / dk / dv have the dtype of q / k / v. */
 int vi_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
                 const void* dout, int64_t ldo, void* dq, int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv,
@@ -380,9 +358,7 @@ int vi_margin_loss_bwd(const float* proj, const float* tgt, const float* negs, c
  * (D/models/transformer.py:178-181), MLPProjectionHead (:585) and VLNBert.drop_env (D/models/model.py:27). */
 int vi_dropout(const void* x, void* y, int64_t n, float p, const uint32_t* seed, uint32_t site, int dtype, vi_stream_t stream);
 
-/* fp32 -> bf16 shadow copy of a weight or activation */
-int vi_cast_bf16(const float* src, void* dst, int64_t n, vi_stream_t stream);
-/* fp32 -> bf16 or fp16 (saturating at +-65504) */
+/* fp32 -> bf16 or fp16 (saturating at +-65504): 16-bit shadow copies of weights and activations */
 int vi_cast_h16(const float* src, void* dst, int dst_dtype, int64_t n, vi_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------

@@ -176,7 +176,7 @@ def test_duet_infonce_alignment_gradients(env, precision):
 
 def test_fused_gradient_accumulation_matches_autograd(env):
     """train.duet_finetune_iteration(fused_accumulation=True): the per-step parameter gradients summed inside vi_wgrad16 /
-    vi_add_ln_bwd_acc (autograd gets None, one multi-tensor add into .grad at the end of the backward pass) against the plain path
+    vi_add_ln_drop_bwd (autograd gets None, one multi-tensor add into .grad at the end of the backward pass) against the plain path
     where autograd adds one gradient per parameter per step.  Same kernels, same operands: only the order of the fp32 additions
     over the steps differs.  Three navigation steps so that every accumulator sees overwrite + add + add; run twice to check that
     nothing leaks from one backward pass into the next."""

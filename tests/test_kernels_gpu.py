@@ -55,28 +55,32 @@ def test_gemm_bf16(ops, M, N, K, epi):
     assert relerr(y3, ref3) < 1e-2
 
 
+def _tile(ops, name: str) -> int:
+    """'192' -> 192, '256p' -> 256 | TILE_PAIR (the two-CTA form)"""
+    return int(name.rstrip('p')) | (ops.TILE_PAIR if name.endswith('p') else 0)
+
+
 @pytest.mark.parametrize('tile', ['64', '96', '128', '192', '256', '128p', '192p', '256p'])
 @pytest.mark.parametrize('M,N,K', [(1000, 768, 1536), (4416, 2304, 768), (300, 768, 64)])
-def test_gemm_bf16_every_tile_shape(ops, tile, M, N, K, monkeypatch):
+def test_gemm_bf16_every_tile_shape(ops, tile, M, N, K):
     """every tile width of the tcgen05 kernel, single-CTA and CTA-pair ('p', cta_group::2) forms, with and
     without the TMA-fed residual, fp32 and bf16 outputs, GELU epilogue"""
-    monkeypatch.setenv('VI_GEMM_TILE', tile)
+    t = _tile(ops, tile)
     x16, w16 = _rand(M, K, seed=5).bfloat16(), _rand(N, K, scale=0.05, seed=6).bfloat16()
     b, res = _rand(N, scale=0.1, seed=7), _rand(M, N, seed=8)
     ref = F.linear(x16.float(), w16.float(), b)
-    y = ops.gemm(x16, w16, b, out_dtype=torch.float32)
+    y = ops.gemm(x16, w16, b, out_dtype=torch.float32, tile=t)
     assert relerr(y, ref) < 2e-3
-    y = ops.gemm(x16, w16, b, residual=res, out_dtype=torch.float32)
+    y = ops.gemm(x16, w16, b, residual=res, out_dtype=torch.float32, tile=t)
     assert relerr(y, ref + res) < 2e-3
-    y = ops.gemm(x16, w16, b, residual=res, epilogue=1, out_dtype=torch.float32)
+    y = ops.gemm(x16, w16, b, residual=res, epilogue=1, out_dtype=torch.float32, tile=t)
     assert relerr(y, F.gelu(ref) + res) < 2e-3
-    y = ops.gemm(x16, w16, b, epilogue=1, out_dtype=torch.bfloat16)
+    y = ops.gemm(x16, w16, b, epilogue=1, out_dtype=torch.bfloat16, tile=t)
     assert relerr(y, F.gelu(ref)) < 1e-2
 
 
 @pytest.mark.parametrize('tile', ['128', '256p'])
-def test_gemm_grouped_pair_tiles(ops, tile, monkeypatch):
-    monkeypatch.setenv('VI_GEMM_TILE', tile)
+def test_gemm_grouped_pair_tiles(ops, tile):
     rows = [1920, 2368]
     K, N = 768, 768
     M0 = ops.pad_rows(rows[0])
@@ -86,7 +90,7 @@ def test_gemm_grouped_pair_tiles(ops, tile, monkeypatch):
     x[M0:] = _rand(rows[1], K, seed=2)
     w, b = _rand(2 * N, K, scale=0.05, seed=3).bfloat16(), _rand(2 * N, scale=0.1, seed=4)
     xx = x.bfloat16()
-    y = ops.gemm(xx, w, b, out_dtype=torch.float32, group_row_end=[M0, M])
+    y = ops.gemm(xx, w, b, out_dtype=torch.float32, group_row_end=[M0, M], tile=_tile(ops, tile))
     assert relerr(y[:rows[0]], F.linear(xx[:rows[0]].float(), w[:N].float(), b[:N])) < 2e-3
     assert relerr(y[M0:], F.linear(xx[M0:].float(), w[N:].float(), b[N:])) < 2e-3
 
@@ -289,7 +293,7 @@ def test_infonce(ops):
     row_ep = torch.tensor([0, 0, 1, 1, 1, 2, 3, 3, 3], dtype=torch.int32, device='cuda')
     neg_ep = torch.tensor([0, 0, 0, 1, 1, 1, 1, 2, 2, 3, 3, 3, 3, 3], dtype=torch.int32, device='cuda')
     T = 0.07
-    loss = ops.infonce_loss(p, t, negs, row_ep, neg_ep, T, R, Nn, 'cuda')
+    loss, _ = ops.infonce_loss(p, t, negs, row_ep, neg_ep, T, R, Nn, 'cuda')
     ref = []
     for r in range(R):
         keep = negs[neg_ep != row_ep[r]]
@@ -307,7 +311,7 @@ def test_margin_loss(ops):
     row_ep = torch.tensor([0, 0, 1, 1, 1, 2, 3, 3, 3], dtype=torch.int32, device='cuda')
     neg_ep = torch.tensor([0, 0, 0, 1, 1, 1, 1, 2, 2, 3, 3, 3, 3, 3], dtype=torch.int32, device='cuda')
     margin = 0.5
-    loss = ops.margin_loss(p, t, negs, row_ep, neg_ep, margin, R, Nn, 'cuda')
+    loss, _ = ops.margin_loss(p, t, negs, row_ep, neg_ep, margin, R, Nn, 'cuda')
     ref = []
     for r in range(R):
         pos = F.cosine_similarity(p[r:r + 1], t[r:r + 1]).squeeze()
@@ -315,7 +319,7 @@ def test_margin_loss(ops):
         ref.append((1 - pos) + F.relu(margin + neg - pos).mean())
     assert abs(float(loss) - float(torch.stack(ref).mean())) < 1e-5
     same = torch.zeros(Nn, dtype=torch.int32, device='cuda')
-    lone = ops.margin_loss(p[:2], t[:2], negs, torch.zeros(2, dtype=torch.int32, device='cuda'), same, margin, 2, Nn, 'cuda')
+    lone, _ = ops.margin_loss(p[:2], t[:2], negs, torch.zeros(2, dtype=torch.int32, device='cuda'), same, margin, 2, Nn, 'cuda')
     assert torch.isnan(lone)
 
 
@@ -401,7 +405,7 @@ def test_copy_rows(ops):
 
 def test_cast_bf16(ops):
     x = _rand(1003, seed=1)
-    assert torch.equal(ops.cast_bf16(x), x.bfloat16())
+    assert torch.equal(ops.cast_h16(x, dtype=torch.bfloat16), x.bfloat16())
 
 
 def test_argument_errors_are_reported_not_fatal(ops):
@@ -535,79 +539,21 @@ def test_embed_compose_chained_layernorm(ops):
     assert y16.dtype == torch.float16 and relerr(y16, F.layer_norm(r32, (768,), g2, b2, 1e-5)) < 2e-3
 
 
-# ---------------------------------------------------------------------------------------------------------------------
-# vi_attn_tc.cu: the tcgen05 attention kernel, called by name (vi_attn_fwd_tc); the dispatcher uses it only with VI_ATTN_TC=1
-# ---------------------------------------------------------------------------------------------------------------------
-TC_ATTN_CASES = ATTN_CASES + [(64, 30, 85, True, False, False), (3, 64, 256, True, False, False), (2, 65, 17, True, True, False),
-                              (2, 200, 200, True, False, False), (1, 37, 240, False, False, True)]
+# longer, wider and edge-case problems on top of ATTN_CASES (> 96 keys: the generic kernel; 1 key; odd query counts)
+ATTN_EDGE_CASES = ATTN_CASES + [(64, 30, 85, True, False, False), (3, 64, 256, True, False, False), (2, 65, 17, True, True, False),
+                                (2, 200, 200, True, False, False), (1, 37, 240, False, False, True)]
 
 
-@pytest.mark.parametrize('B,Lq,Lk,masked,gasa,neg_inf', [c for c in TC_ATTN_CASES if c[2] <= 256])
-@pytest.mark.parametrize('fmt', [torch.bfloat16, torch.float16])
-def test_attention_tcgen05(ops, B, Lq, Lk, masked, gasa, neg_inf, fmt):
-    qkv_q = _rand(B * Lq, 2304, seed=1).to(fmt)            # strided views, like the fused QKV output
-    qkv_k = _rand(B * Lk, 2304, seed=2).to(fmt)
-    q, k, v = qkv_q[:, :768], qkv_k[:, 768:1536], qkv_k[:, 1536:]
-    key_mask = None
-    if masked:
-        g = torch.Generator().manual_seed(3)
-        lens = torch.randint(1, Lk + 1, (B,), generator=g)
-        lens[0] = Lk
-        key_mask = (torch.arange(Lk)[None] < lens[:, None]).to(torch.uint8).cuda()
-        if Lk > 4:
-            key_mask[-1, 1] = 0
-    pair_dist = affine = None
-    if gasa:
-        pair_dist = (_rand(B, Lq, Lk, seed=4).abs() * 10).contiguous()
-        affine = torch.tensor([-0.5, 0.1], device='cuda')
-    o = torch.empty((B * Lq, 768), dtype=fmt, device='cuda')
-    ops.attention_multi([dict(q=q, k=k, v=v, out=o, B=B, Lq=Lq, Lk=Lk, key_mask=key_mask, pair_dist=pair_dist, bias_affine=affine)],
-                        mask_mode=ops.MASK_NEG_INF if neg_inf else ops.MASK_ADD_NEG10000, kernel='tc')
-    ref, _ = _attn_ref(q, k, v, B, Lq, Lk, key_mask, pair_dist, affine, neg_inf)
-    assert relerr(o, ref) < (1.5e-2 if fmt == torch.bfloat16 else 2.5e-3)
-
-
-@pytest.mark.parametrize('fmt', [torch.bfloat16, torch.float16])
-def test_attention_tcgen05_multi_problem(ops, fmt):
-    """the two token streams of a row-stacked DUET activation (global 30 nodes with GASA | local 37 views) against one shared
-    85-token context, and HAMT's bidirectional pair (85 x 53 | 53 x 85), in one launch each; padding rows stay untouched"""
-    B = 16
-    for (La, Lb, Lka, Lkb, gasa) in ((30, 37, 85, 85, False), (30, 37, 30, 37, True), (85, 53, 53, 85, False)):
-        ra = (B * La + 255) // 256 * 256
-        R = ra + B * Lb
-        x = _rand(R, 2304, seed=5).to(fmt)
-        ctx = _rand(B * 85, 3072, seed=6).to(fmt)
-        out = torch.full((R, 768), 7.0, device='cuda', dtype=fmt)
-        ga, gb = torch.Generator().manual_seed(1), torch.Generator().manual_seed(2)
-        ma = (torch.arange(Lka)[None] < torch.randint(1, Lka + 1, (B,), generator=ga)[:, None]).to(torch.uint8).cuda()
-        mb = (torch.arange(Lkb)[None] < torch.randint(1, Lkb + 1, (B,), generator=gb)[:, None]).to(torch.uint8).cuda()
-        dist = (_rand(B, La, Lka, seed=7).abs() * 10).contiguous() if gasa else None
-        aff = torch.tensor([-0.3, 0.05], device='cuda') if gasa else None
-        if Lka == 85 and Lkb == 85:                          # cross-attention: both streams read the projected context
-            ka, va, kb, vb = ctx[:, :768], ctx[:, 768:1536], ctx[:, 1536:2304], ctx[:, 2304:]
-        elif gasa:                                           # self-attention inside each stream
-            ka, va, kb, vb = x[:B * La, 768:1536], x[:B * La, 1536:], x[ra:, 768:1536], x[ra:, 1536:]
-        else:                                                # HAMT: each stream attends to the other one
-            ka, va, kb, vb = x[ra:, 768:1536], x[ra:, 1536:], x[:B * La, 768:1536], x[:B * La, 1536:]
-        pa = dict(q=x[:B * La, :768], k=ka, v=va, out=out[:B * La], B=B, Lq=La, Lk=Lka, key_mask=ma, pair_dist=dist, bias_affine=aff)
-        pb = dict(q=x[ra:, :768], k=kb, v=vb, out=out[ra:], B=B, Lq=Lb, Lk=Lkb, key_mask=mb)
-        ops.attention_multi([pa, pb], kernel='tc')
-        refa, _ = _attn_ref(pa['q'], ka, va, B, La, Lka, ma, dist, aff, False)
-        refb, _ = _attn_ref(pb['q'], kb, vb, B, Lb, Lkb, mb, None, None, False)
-        tol = 1.5e-2 if fmt == torch.bfloat16 else 2.5e-3
-        assert relerr(out[:B * La], refa) < tol and relerr(out[ra:], refb) < tol
-        assert bool((out[B * La:ra].float() == 7.0).all())
-
-
-SP_ATTN_CASES = [c for c in TC_ATTN_CASES if c[2] <= 96] + [(64, 37, 85, True, False, False), (3, 50, 96, True, True, False),
-                                                            (2, 40, 81, True, True, True), (2, 17, 1, False, False, False)]
+SP_ATTN_CASES = [c for c in ATTN_EDGE_CASES if c[2] <= 96] + [(64, 37, 85, True, False, False), (3, 50, 96, True, True, False),
+                                                              (2, 40, 81, True, True, True), (2, 17, 1, False, False, False)]
 
 
 @pytest.mark.parametrize('B,Lq,Lk,masked,gasa,neg_inf', SP_ATTN_CASES)
 @pytest.mark.parametrize('fmt', [torch.bfloat16, torch.float16])
-def test_attention_single_pass(ops, B, Lq, Lk, masked, gasa, neg_inf, fmt, monkeypatch):
+def test_attention_single_pass(ops, B, Lq, Lk, masked, gasa, neg_inf, fmt):
     """attn_fwd_sp_kernel (the default for <= 96 keys without dropout / lse: exactly unrolled key blocks, one softmax pass in the
-    log2 domain) against the fp32 reference and against the generic kernel (VI_ATTN_SP=0) on the same inputs"""
+    log2 domain) against the fp32 reference and against the generic kernel (which a log-sum-exp output selects) on the same
+    inputs"""
     qkv_q = _rand(B * Lq, 2304, seed=1).to(fmt)
     qkv_k = _rand(B * Lk, 2304, seed=2).to(fmt)
     q, k, v = qkv_q[:, :768], qkv_k[:, 768:1536], qkv_k[:, 1536:]
@@ -627,9 +573,9 @@ def test_attention_single_pass(ops, B, Lq, Lk, masked, gasa, neg_inf, fmt, monke
     prob = dict(q=q, k=k, v=v, B=B, Lq=Lq, Lk=Lk, key_mask=key_mask, pair_dist=pair_dist, bias_affine=affine)
     o = torch.full((B * Lq + 3, 768), 7.0, dtype=fmt, device='cuda')
     ops.attention_multi([dict(prob, out=o[:B * Lq])], mask_mode=mode)
-    monkeypatch.setenv('VI_ATTN_SP', '0')
     o_gen = torch.empty((B * Lq, 768), dtype=fmt, device='cuda')
-    ops.attention_multi([dict(prob, out=o_gen)], mask_mode=mode)
+    lse = torch.empty((B, 12, Lq), dtype=torch.float32, device='cuda')
+    ops.attention_multi([dict(prob, out=o_gen, lse=lse)], mask_mode=mode)
     ref, _ = _attn_ref(q, k, v, B, Lq, Lk, key_mask, pair_dist, affine, neg_inf)
     tol = 1.5e-2 if fmt == torch.bfloat16 else 2.5e-3
     assert relerr(o[:B * Lq], ref) < tol

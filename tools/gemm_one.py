@@ -13,8 +13,7 @@ tile = sys.argv[4] if len(sys.argv) > 4 else 'auto'
 epi = int(sys.argv[5]) if len(sys.argv) > 5 else 0
 res = int(sys.argv[6]) if len(sys.argv) > 6 else 0
 f32 = int(sys.argv[7]) if len(sys.argv) > 7 else 0
-if tile != 'auto':
-    os.environ['VI_GEMM_TILE'] = tile
+tile = None if tile == 'auto' else int(tile.rstrip('p')) | (ops.TILE_PAIR if tile.endswith('p') else 0)
 ops.ensure_init(torch.zeros(1, device='cuda'))
 x = torch.randn(M, K, device='cuda').bfloat16()
 w = (torch.randn(N, K, device='cuda') * 0.05).bfloat16()
@@ -29,6 +28,6 @@ if fold:
     stats[:, :, 1] = 32.0
     ln = (_lib.LN_FOLD, w.float().sum(1), stats, 1e-12)
 for _ in range(5):
-    ops.gemm(x, w, b, residual=r, epilogue=epi, out=out, ln=ln)
+    ops.gemm(x, w, b, residual=r, epilogue=epi, out=out, ln=ln, tile=tile)
 torch.cuda.synchronize()
 print('ok')

@@ -42,20 +42,19 @@ for name, M, N, K, ends, epi, res, f32 in SHAPES:
     out = torch.empty(M, N, dtype=torch.float32 if f32 else torch.bfloat16, device='cuda')
     rec = {'name': name, 'M': M, 'N': N, 'K': K, 'gflop': round(2.0 * M * N * K / 1e9, 2)}
     for tile in tiles:
-        if tile == 'auto':
-            os.environ.pop('VI_GEMM_TILE', None)
-        else:
+        tv = None
+        if tile != 'auto':
             if N % int(tile.rstrip('p')):
                 continue
-            os.environ['VI_GEMM_TILE'] = tile
+            tv = int(tile.rstrip('p')) | (ops.TILE_PAIR if tile.endswith('p') else 0)
         for _ in range(3):
-            ops.gemm(x, w, b, residual=r, epilogue=epi, out=out, group_row_end=ends)
+            ops.gemm(x, w, b, residual=r, epilogue=epi, out=out, group_row_end=ends, tile=tv)
         torch.cuda.synchronize()
         torch.cuda._sleep(3_000_000)                   # let the host run ahead so launches queue back to back
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(REP):
-            ops.gemm(x, w, b, residual=r, epilogue=epi, out=out, group_row_end=ends)
+            ops.gemm(x, w, b, residual=r, epilogue=epi, out=out, group_row_end=ends, tile=tv)
         e1.record()
         torch.cuda.synchronize()
         t = e0.elapsed_time(e1) / REP

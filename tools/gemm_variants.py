@@ -53,23 +53,21 @@ for name, N, K, xin in (('proj768', 768, 768, x16), ('qkv2304', 2304, 768, x16),
     for tile in tiles:
         if tile and N % (tile & 0xFFF):
             continue
-        os.environ.pop('VI_GEMM_TILE', None)
-        if tile:
-            os.environ['VI_GEMM_TILE'] = '%d%s' % (tile & 0xFFF, 'p' if tile & 0x1000 else '')
+        tt = tile or None                                  # 0: the measured table / cost model
         t = {}
         if N == 768:
-            t['f32+res'] = timeit(lambda: ops.gemm(xin, w, b, residual=res, out=z32, group_row_end=ends))
-            t['f32+res+stats+dual'] = timeit(lambda: ops.gemm(xin, w, b, residual=res, out=z32, out16=z16, group_row_end=ends, stats_out=stats_o))
-            t['f32+lnres+stats+dual'] = timeit(lambda: ops.gemm(xin, w, b, residual=res, out=z32, out16=z16, group_row_end=ends, stats_out=stats_o,
+            t['f32+res'] = timeit(lambda: ops.gemm(xin, w, b, residual=res, out=z32, group_row_end=ends, tile=tt))
+            t['f32+res+stats+dual'] = timeit(lambda: ops.gemm(xin, w, b, residual=res, out=z32, out16=z16, group_row_end=ends, tile=tt, stats_out=stats_o))
+            t['f32+lnres+stats+dual'] = timeit(lambda: ops.gemm(xin, w, b, residual=res, out=z32, out16=z16, group_row_end=ends, tile=tt, stats_out=stats_o,
                                                               ln=(_lib.LN_RESIDUAL, gam, stats, 1e-12)))
-            t['f32+res+dual'] = timeit(lambda: ops.gemm(xin, w, b, residual=res, out=z32, out16=z16, group_row_end=ends))
+            t['f32+res+dual'] = timeit(lambda: ops.gemm(xin, w, b, residual=res, out=z32, out16=z16, group_row_end=ends, tile=tt))
         if K == 768:
             y = torch.empty(M, N, device=dev, dtype=fmt)
             epi = 1 if N == 3072 else 0
-            t['h16'] = timeit(lambda: ops.gemm(xin, w, b, epilogue=epi, out=y, group_row_end=ends))
-            t['h16+fold'] = timeit(lambda: ops.gemm(xin, w, b, epilogue=epi, out=y, group_row_end=ends, ln=(_lib.LN_FOLD, s, stats, 1e-12)))
+            t['h16'] = timeit(lambda: ops.gemm(xin, w, b, epilogue=epi, out=y, group_row_end=ends, tile=tt))
+            t['h16+fold'] = timeit(lambda: ops.gemm(xin, w, b, epilogue=epi, out=y, group_row_end=ends, tile=tt, ln=(_lib.LN_FOLD, s, stats, 1e-12)))
             if epi:
-                t['h16_noact'] = timeit(lambda: ops.gemm(xin, w, b, epilogue=0, out=y, group_row_end=ends))
+                t['h16_noact'] = timeit(lambda: ops.gemm(xin, w, b, epilogue=0, out=y, group_row_end=ends, tile=tt))
         rec[str(tile)] = {k: round(v, 2) for k, v in t.items()}
     out[name] = rec
     print(name, json.dumps(rec), flush=True)

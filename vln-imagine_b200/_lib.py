@@ -58,13 +58,9 @@ class AttnProblem(C.Structure):
 PROTOTYPES = {
     'vi_version': [],
     'vi_init': [_i],
-    'vi_gemm_bf16': [_p, _l, _p, _p, _p, _l, _p, _l, _i, _i, _i, _i, _i, _i, _ip, _p],
-    'vi_gemm_bf16_tiled': [_p, _l, _p, _p, _p, _l, _p, _l, _i, _i, _i, _i, _i, _i, _ip, _i, _p],
     'vi_gemm16': [C.POINTER(GemmArgs), _p],
     'vi_gemm_f32': [_p, _l, _p, _p, _p, _l, _p, _l, _i, _i, _i, _i, _i, _ip, _p],
-    'vi_attn_fwd': [_p, _l, _p, _l, _p, _l, _p, _l, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p],
     'vi_attn_fwd_multi': [C.POINTER(AttnProblem), _i, _i, _i, _i, _p],
-    'vi_attn_fwd_tc': [C.POINTER(AttnProblem), _i, _i, _i, _i, _p],
     'vi_add_ln': [_p, _p, _p, _p, _f, _p, _p, _i, _l, _i, _ip, _p],
     'vi_embed_compose': [C.POINTER(EmbedArgs), _p],
     'vi_ln_dot': [_p, _p, _p, _f, _p, _p, _p, _l, _i, _ip, _p],
@@ -79,18 +75,14 @@ PROTOTYPES = {
     'vi_ce_rows': [_p, _l, _p, _i, _p, _l, _p],
     'vi_kl_rows': [_p, _l, _p, _l, _i, _p, _l, _p],
     'vi_copy_rows': [_p, _l, _l, _p, _p, _i, _l, _l, _l, _i, _p],
-    'vi_cast_bf16': [_p, _p, _l, _p],
     'vi_cast_h16': [_p, _p, _i, _l, _p],
     'vi_transpose': [_p, _l, _p, _l, _i, _i, _i, _i, _p],
     'vi_colsum': [_p, _l, _i, _p, _l, _i, _p, _l, _p],
-    'vi_reduce_scratch_elems': [_l, _i, _i],
     'vi_wgrad16_splits': [_i, _i, _i, _ip],
     'vi_wgrad16_workspace': [_i, _i, _i, _ip, _i],
     'vi_wgrad16': [_p, _l, _p, _l, _i, _i, _i, _i, _ip, _p, _p, _p, _l, _i, _i, _p],
     'vi_act_fwd': [_p, _p, _l, _i, _i, _p],
     'vi_act_bwd': [_p, _p, _p, _l, _i, _i, _p],
-    'vi_add_ln_bwd': [_p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _p, _l, _i, _ip, _p, _l, _p],
-    'vi_add_ln_bwd_acc': [_p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _p, _l, _i, _ip, _p, _l, _i, _p],
     'vi_add_ln_drop': [_p, _p, _p, _p, _f, _p, _p, _i, _l, _i, _ip, _f, _p, C.c_uint32, _p],
     'vi_add_ln_drop_bwd': [_p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _p, _p, _l, _i, _ip, _p, _l, _i, _f, _p, C.c_uint32, _p],
     'vi_feat_wgrad': [_p, _p, _i, _p, _p, _l, _p, _l, _p],
@@ -112,7 +104,6 @@ for _name, _args in PROTOTYPES.items():
     _fn = getattr(lib, _name)            # AttributeError here = header/library mismatch: fail loudly
     _fn.argtypes = _args
     _fn.restype = _i
-lib.vi_reduce_scratch_elems.restype = C.c_int64
 lib.vi_wgrad16_workspace.restype = C.c_int64
 lib.vi_last_error.argtypes = []
 lib.vi_last_error.restype = C.c_char_p

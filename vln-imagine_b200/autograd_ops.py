@@ -4,9 +4,9 @@ Used when a mode is called with autograd recording (fine-tuning, BASELINE.json c
 chains the nodes and accumulates gradients at fan-out points (residual branches) and into ``.grad``; it performs
 no model arithmetic itself.  Conventions:
 
-* dense layers: ``dX = dY W`` runs the tcgen05 GEMM on the transposed bf16 weight shadow, ``dW = dY^T X`` runs it on
-  kernel-transposed copies of dY and X (contraction over the rows, zero-padded to a multiple of 64), ``db`` is a
-  fixed-order column sum; grouped (row-stacked) layers loop the weight gradient over their groups;
+* dense layers: ``dX = dY W`` runs the tcgen05 GEMM on the transposed bf16 weight shadow; ``dW = dY^T X`` and ``db`` come
+  from vi_wgrad16 on dY and X as they lie in memory (all groups of a row-stacked layer in one launch).  The fp32 check mode
+  runs the GEMM on kernel-transposed copies of dY and X and takes ``db`` as a fixed-order column sum, group by group;
 * the training forward keeps pre-activations: GELU / ReLU are their own kernels instead of GEMM epilogues;
 * LayerNorm returns the fp32 residual-stream tensor and its bf16 operand copy; its backward takes both gradients;
 * the embedding composer is decomposed into primitives (small-feature linear, LayerNorm, row gather, sum);
@@ -78,7 +78,7 @@ class _GradAcc:
     """Gradient accumulation fused into the kernels (opt-in, ``fused_grad_accumulation``).  A parameter of this path is used once
     per navigation step, so autograd ends an iteration with one small ``add`` kernel per parameter per step (~1500 launches at 6
     steps).  With the switch on, the dense-layer and LayerNorm backward nodes add their parameter gradients straight into one fp32
-    accumulator per weight pack (vi_wgrad16 / vi_add_ln_bwd_acc with accumulate = 1: TMA reduce-add or a read-modify-write with one
+    accumulator per weight pack (vi_wgrad16 / vi_add_ln_drop_bwd with accumulate = 1: TMA reduce-add or a read-modify-write with one
     writer per element, in backward order - deterministic) and hand autograd ``None``; when the backward pass ends, ONE multi-tensor
     add moves the accumulators into ``.grad`` (created if missing), which is what the optimiser / the flat all-reduce buffer see.
     Not for modules whose parameters carry autograd hooks (DistributedDataParallel): those keep the plain path."""
@@ -202,7 +202,7 @@ def to_operand(t: torch.Tensor, lowp: bool) -> torch.Tensor:
     """gradient tensor -> GEMM operand dtype of the current precision mode (contiguous)"""
     t = t.contiguous()
     if lowp and t.dtype != BF16:
-        return ops.cast_bf16(t)
+        return ops.cast_h16(t, dtype=BF16)
     if not lowp and t.dtype != F32:
         return t.float()
     return t
@@ -269,7 +269,7 @@ class CastBf16Fn(Function):
 
     @staticmethod
     def forward(ctx, x):
-        return ops.cast_bf16(x)
+        return ops.cast_h16(x, dtype=BF16)
 
     @staticmethod
     def backward(ctx, dy):
@@ -299,27 +299,8 @@ class LinearFn(Function):
         if ctx.needs_input_grad[0]:
             wt = pack.get_t(lowp, n_groups)                             # [n_groups*K, N]
             dx = ops.gemm(dyo, wt, None, out_dtype=x.dtype, group_row_end=ends)
-        if lowp and wgrad16_ok(dyo, x) and _GradAcc.enabled and dyo.shape[1] * n_groups == sum(w.shape[0] for w in pack.weights):
-            # gradient accumulation inside the kernel: autograd gets None, _acc_flush moves the sums into .grad
-            has_b = pack.biases is not None
-            bs = [b for b in pack.biases if b is not None] if has_b else []
-            e = _acc_entry(pack.weights + bs, [(n_groups * N, K)] + ([(n_groups * N,)] if has_b else []), x.device)
-            if 'slices' not in e:
-                sl, off = [], 0
-                for wsrc in pack.weights:
-                    sl.append((wsrc, e['t'][0][off:off + wsrc.shape[0]]))
-                    off += wsrc.shape[0]
-                off = 0
-                for bsrc, wsrc in zip(pack.biases or [], pack.weights):
-                    if bsrc is not None:
-                        sl.append((bsrc, e['t'][1][off:off + wsrc.shape[0]]))
-                    off += wsrc.shape[0]
-                e['slices'] = sl
-            beta = _acc_begin(e)
-            wgrad16(dyo, x, ends, has_b, out=(e['t'][0], e['t'][1] if has_b else None), accumulate=beta)
-            return (dx, dy if ctx.has_res else None, None, None, None, None, *([None] * len(pack.grad_sources())))
         if lowp and wgrad16_ok(dyo, x):
-            dW, db = wgrad16(dyo, x, ends, pack.biases is not None)
+            grads = _lin_param_grads(pack, dyo, x, ends)
         else:                                                           # fp32 check mode / odd shapes: transposed copies
             dW = torch.empty((n_groups * N, K), dtype=F32, device=x.device)
             db = torch.empty((n_groups * N,), dtype=F32, device=x.device) if pack.biases is not None else None
@@ -332,18 +313,7 @@ class LinearFn(Function):
                 ops.gemm(dyT, xT, None, out_dtype=F32, out=dW[g * N:(g + 1) * N])
                 if db is not None:
                     db[g * N:(g + 1) * N] = colsum(dyo[r0:r1])
-        grads, off = [], 0
-        for wsrc in pack.weights:
-            n = wsrc.shape[0]
-            grads.append(dW[off:off + n] if wsrc.requires_grad else None)
-            off += n
-        if pack.biases is not None:
-            off = 0
-            for bsrc, wsrc in zip(pack.biases, pack.weights):
-                n = wsrc.shape[0]
-                if bsrc is not None:
-                    grads.append(db[off:off + n] if bsrc.requires_grad else None)
-                off += n
+            grads = _lin_grads(pack, dW, db)
         return (dx, dy if ctx.has_res else None, None, None, None, None, *grads)
 
 
@@ -387,8 +357,7 @@ class LayerNormFn(Function):
         ctx.eps, ctx.ends, ctx.has_b, ctx.n_params = eps, ends, b is not None, n_params
         ctx.b_needs = b is not None and b.requires_grad
         ctx.a_needs = a.requires_grad
-        ctx.param_needs = [p.requires_grad for p in params]
-        ctx.param_srcs = list(params) if params else None
+        ctx.param_srcs = list(params)
         if y16 is None:
             y16 = a.new_empty(0)
             ctx.mark_non_differentiable(y16)
@@ -410,31 +379,14 @@ class LayerNormFn(Function):
         if dy16 is not None:
             dy16 = dy16.contiguous()
         dx = torch.empty_like(a)
-        half = ctx.n_params // 2
-        srcs = ctx.param_srcs
-        fused = _GradAcc.enabled and srcs is not None and half == n_groups
-        beta = 0
-        if fused:
-            e = _acc_entry(srcs, [(n_groups, HIDDEN), (n_groups, HIDDEN)], a.device)
-            if 'slices' not in e:
-                e['slices'] = [(srcs[i], e['t'][0][i]) for i in range(half)] + [(srcs[half + i], e['t'][1][i]) for i in range(half)]
-            beta = _acc_begin(e)
-            dg, dbt = e['t']
-        else:
-            dg = torch.empty((n_groups, HIDDEN), dtype=F32, device=a.device)
-            dbt = torch.empty((n_groups, HIDDEN), dtype=F32, device=a.device)
+        dg, dbt, acc, pg = _ln_param_grads(ctx.param_srcs, n_groups, a.device)
         stats = torch.empty((rows, 2), dtype=F32, device=a.device)
         sc = reduce_scratch(a.device, 16 * rows, HIDDEN, 2)           # the fused pass reduces chunks of 8 - 32 rows (>= RED_CHUNK / 16)
-        check(lib.vi_add_ln_bwd_acc(a.data_ptr(), _ptr(b), gamma.data_ptr(), ctx.eps, _ptr(dy32), _ptr(dy16), dx.data_ptr(), None,
-                                    dg.data_ptr(), dbt.data_ptr(), stats.data_ptr(), rows, n_groups,
-                                    _lib.int_array(list(ends)) if ends is not None else None, sc.data_ptr(), sc.numel(), beta,
-                                    _stream()), 'vi_add_ln_bwd')
+        check(lib.vi_add_ln_drop_bwd(a.data_ptr(), _ptr(b), gamma.data_ptr(), ctx.eps, _ptr(dy32), _ptr(dy16), dx.data_ptr(), None,
+                                     None, dg.data_ptr(), dbt.data_ptr(), stats.data_ptr(), rows, n_groups,
+                                     _lib.int_array(list(ends)) if ends is not None else None, sc.data_ptr(), sc.numel(), acc,
+                                     0.0, None, 0, _stream()), 'vi_add_ln_drop_bwd')
         _launched(2)
-        if fused:
-            return (dx if ctx.a_needs else None, dx if ctx.b_needs else None, None, None, None, None, None, None,
-                    *([None] * ctx.n_params))
-        pg = [dg[i] if ctx.param_needs[i] else None for i in range(half)] + \
-             [dbt[i] if ctx.param_needs[half + i] else None for i in range(half)]
         return (dx if ctx.a_needs else None, dx if ctx.b_needs else None, None, None, None, None, None, None, *pg)
 
 
@@ -484,54 +436,26 @@ class DenseResLNFn(Function):
             dy16 = None
         dy32 = dy32.contiguous() if dy32 is not None else None
         dy16 = dy16.contiguous() if dy16 is not None else None
-        lin_srcs = pack.grad_sources()
         ln_srcs = lnpack.grad_sources()
-        half = len(ln_srcs) // 2
-        fused = _GradAcc.enabled and half == n_ln
-        beta_ln = 0
-        if fused:
-            e = _acc_entry(ln_srcs, [(n_ln, HIDDEN), (n_ln, HIDDEN)], dev)
-            if 'slices' not in e:
-                e['slices'] = [(ln_srcs[i], e['t'][0][i]) for i in range(half)] + [(ln_srcs[half + i], e['t'][1][i]) for i in range(half)]
-            beta_ln = _acc_begin(e)
-            dg, dbt = e['t']
-        else:
-            dg = torch.empty((n_ln, HIDDEN), dtype=F32, device=dev)
-            dbt = torch.empty((n_ln, HIDDEN), dtype=F32, device=dev)
+        dg, dbt, acc, ln_grads = _ln_param_grads(ln_srcs, n_ln, dev)
         dres = torch.empty((rows, HIDDEN), dtype=F32, device=dev)
         da16 = torch.empty((rows, HIDDEN), dtype=x.dtype, device=dev)
         stats = torch.empty((rows, 2), dtype=F32, device=dev)
         sc = reduce_scratch(dev, 16 * rows, HIDDEN, 2)
         check(lib.vi_add_ln_drop_bwd(d.data_ptr(), res32.data_ptr() if p > 0 else None, g.data_ptr(), ctx.eps, _ptr(dy32), _ptr(dy16),
                                      dres.data_ptr(), None, da16.data_ptr(), dg.data_ptr(), dbt.data_ptr(), stats.data_ptr(), rows, n_ln,
-                                     _lib.int_array(list(ln_ends)) if ln_ends is not None else None, sc.data_ptr(), sc.numel(), beta_ln,
+                                     _lib.int_array(list(ln_ends)) if ln_ends is not None else None, sc.data_ptr(), sc.numel(), acc,
                                      float(p), dropout_seed(dev).data_ptr() if p > 0 else None, ctx.site, _stream()), 'vi_add_ln_drop_bwd')
         _launched(2)
-        # dense layer: dX = dA W, dW = dA^T X, db = colsum(dA) with dA = da16
-        M, K = x.shape
+        # dense layer: dX = dA W, dW = dA^T X, db = column sums of dA with dA = da16
+        K = x.shape[1]
         N = da16.shape[1]
         dx = None
         if ctx.needs_input_grad[0]:
             dx = ops.gemm(da16, pack.get_t(True, n_groups), None, out_dtype=x.dtype, group_row_end=ends)
-        has_b = pack.biases is not None
-        lin_grads = [None] * len(lin_srcs)
-        if wgrad16_ok(da16, x) and N * n_groups == sum(w_.shape[0] for w_ in pack.weights):
-            if _GradAcc.enabled:
-                bs = [b_ for b_ in pack.biases if b_ is not None] if has_b else []
-                e = _acc_entry(pack.weights + bs, [(n_groups * N, K)] + ([(n_groups * N,)] if has_b else []), dev)
-                if 'slices' not in e:
-                    e['slices'] = _lin_slices(pack, e['t'])
-                beta = _acc_begin(e)
-                wgrad16(da16, x, ends, has_b, out=(e['t'][0], e['t'][1] if has_b else None), accumulate=beta)
-            else:
-                dW, db = wgrad16(da16, x, ends, has_b)
-                lin_grads = _lin_grads(pack, dW, db)
-        else:
+        if not (wgrad16_ok(da16, x) and N * n_groups == sum(w_.shape[0] for w_ in pack.weights)):
             raise _lib.VlnImagineError('DenseResLNFn: the dense layer must be a multiple of 128 x 64 (got N=%d, K=%d)' % (N, K))
-        ln_grads = [None] * len(ln_srcs)
-        if not fused:
-            needs = [s_.requires_grad for s_ in ln_srcs]
-            ln_grads = [dg[i] if needs[i] else None for i in range(half)] + [dbt[i] if needs[half + i] else None for i in range(half)]
+        lin_grads = _lin_param_grads(pack, da16, x, ends)
         return (dx, dres if ctx.res_needs else None, None, None, None, None, None, None, None, *lin_grads, *ln_grads)
 
 
@@ -547,6 +471,44 @@ def _lin_slices(pack, tensors):
             sl.append((bsrc, tensors[1][off:off + wsrc.shape[0]]))
         off += wsrc.shape[0]
     return sl
+
+
+def _lin_param_grads(pack, dy16, x16, ends):
+    """weight and bias gradients of a LinearPack from the 16-bit dY and X (vi_wgrad16), in grad_sources() order.  With
+    fused_grad_accumulation on (and one accumulator covering the whole pack) they are added into the pack's accumulators and
+    autograd gets None for every parameter; otherwise they are returned per parameter."""
+    n_groups = 1 if ends is None else len(ends)
+    N, K = dy16.shape[1], x16.shape[1]
+    has_b = pack.biases is not None
+    if _GradAcc.enabled and N * n_groups == sum(w.shape[0] for w in pack.weights):
+        bs = [b for b in pack.biases if b is not None] if has_b else []
+        e = _acc_entry(pack.weights + bs, [(n_groups * N, K)] + ([(n_groups * N,)] if has_b else []), x16.device)
+        if 'slices' not in e:
+            e['slices'] = _lin_slices(pack, e['t'])
+        acc = _acc_begin(e)
+        wgrad16(dy16, x16, ends, has_b, out=(e['t'][0], e['t'][1] if has_b else None), accumulate=acc)
+        return [None] * len(pack.grad_sources())
+    dW, db = wgrad16(dy16, x16, ends, has_b)
+    return _lin_grads(pack, dW, db)
+
+
+def _ln_param_grads(srcs, n_groups: int, device):
+    """(dgamma, dbeta, accumulate, grads) for the LayerNorm parameters srcs = gammas + betas of n_groups groups, the buffers
+    and flag vi_add_ln_drop_bwd writes into.  With fused_grad_accumulation on they are the pack's accumulators and grads is all
+    None; otherwise fresh [n_groups, 768] buffers whose rows are the gradients autograd gets (grads, in srcs order)."""
+    half = len(srcs) // 2
+    if _GradAcc.enabled and half == n_groups:
+        e = _acc_entry(srcs, [(n_groups, HIDDEN), (n_groups, HIDDEN)], device)
+        if 'slices' not in e:
+            e['slices'] = [(srcs[i], e['t'][0][i]) for i in range(half)] + [(srcs[half + i], e['t'][1][i]) for i in range(half)]
+        acc = _acc_begin(e)
+        dg, dbt = e['t']
+        return dg, dbt, acc, [None] * len(srcs)
+    dg = torch.empty((n_groups, HIDDEN), dtype=F32, device=device)
+    dbt = torch.empty((n_groups, HIDDEN), dtype=F32, device=device)
+    grads = [dg[i] if srcs[i].requires_grad else None for i in range(half)] + \
+            [dbt[i] if srcs[half + i].requires_grad else None for i in range(half)]
+    return dg, dbt, 0, grads
 
 
 def _lin_grads(pack, dW, db):
@@ -863,7 +825,7 @@ class InfoNCELossFn(Function):
     @staticmethod
     def forward(ctx, proj, tgt, negs, row_ep, neg_ep, temperature, R, n_negs):
         proj = proj.contiguous()
-        loss, scratch = ops.infonce_loss_with_sims(proj, tgt, negs, row_ep, neg_ep, temperature, R, n_negs, proj.device)
+        loss, scratch = ops.infonce_loss(proj, tgt, negs, row_ep, neg_ep, temperature, R, n_negs, proj.device)
         ctx.save_for_backward(proj, tgt, scratch)
         ctx.extra = (negs, row_ep, neg_ep, float(temperature), R, n_negs)
         return loss
@@ -887,7 +849,7 @@ class MarginLossFn(Function):
     @staticmethod
     def forward(ctx, proj, tgt, negs, row_ep, neg_ep, margin, R, n_negs):
         proj = proj.contiguous()
-        loss, scratch = ops.margin_loss_with_sims(proj, tgt, negs, row_ep, neg_ep, margin, R, n_negs, proj.device)
+        loss, scratch = ops.margin_loss(proj, tgt, negs, row_ep, neg_ep, margin, R, n_negs, proj.device)
         ctx.save_for_backward(proj, tgt, scratch)
         ctx.extra = (negs, row_ep, neg_ep, float(margin), R, n_negs)
         return loss

@@ -9,7 +9,6 @@ a 128-row boundary, and go through ONE grouped launch per GEMM / LayerNorm.
 from __future__ import annotations
 
 import dataclasses
-import os
 from typing import List, Optional, Sequence
 
 import torch
@@ -54,7 +53,7 @@ def _attn_drop(device, p=None):
 
 def _dense_res_ln(x, lin: 'LinearPack', res32, ln: 'LNPack', eps, lowp, ends):
     """training: LN(dropout(x W^T + b) + res)  (BertSelfOutput / BertOutput, D/models/vilmodel.py:151-155,190-194)"""
-    if lowp and ag.dense_res_ln_ok(x, lin, ln, ends) and os.environ.get('VLN_IMAGINE_FUSED_DENSE_LN', '1') != '0':
+    if lowp and ag.dense_res_ln_ok(x, lin, ln, ends):
         y32, y16 = ag.dense_res_ln(x, res32, lin, ln, eps, ends, _Mode.p_hidden)       # one autograd node, dropout inside the LN kernels
         return Act(y32, y16)
     if _Mode.p_hidden > 0:
@@ -417,12 +416,6 @@ def _ctx_buffer(rows: int, like: torch.Tensor, streams) -> torch.Tensor:
     return ctx
 
 
-def fold_enabled() -> bool:
-    """LayerNorm folded into the neighbouring contractions (inference, 16-bit mode); VLN_IMAGINE_LN_FOLD=0 restores the
-    GEMM + row-kernel pairs (same results up to rounding)."""
-    return os.environ.get('VLN_IMAGINE_LN_FOLD', '1') != '0'
-
-
 def _call_groups(lin: 'LinearPack', ln: Optional['LNPack'], ends):
     """(n_groups, ends) of a grouped call: as many groups as the weights or the LayerNorm vectors need"""
     n = max(lin.n_groups, len(ln.g.tensors) if ln is not None else 1)
@@ -449,7 +442,7 @@ def linear_residual_ln(x, lin: 'LinearPack', res: Act, ln: LNPack, eps, lowp, en
     LayerNorm of ``res`` is applied to the residual inside the same epilogue.  fp32 check mode: GEMM + row kernel."""
     if isinstance(res, torch.Tensor):
         res = Act(res)
-    if not (lowp and fold_enabled()):
+    if not lowp:
         if res.pend is not None:
             res = materialize(res, lowp, ends)
         n, e = _call_groups(lin, ln, ends)

@@ -36,7 +36,6 @@ bool vi_pdl_enabled() {
 }
 
 int vi_attn_init();
-int vi_attn_tc_init();
 
 // ---- TMA tensor maps (driver entry point resolved once per process) -------------------------------------------------
 #include <mutex>
@@ -74,7 +73,7 @@ int vi_make_tmap_h16(CUtensorMap* map, const void* ptr, int f16, uint64_t cols, 
   return VI_OK;
 }
 
-extern "C" int vi_version(void) { return 100; }   // 0.1.0
+extern "C" int vi_version(void) { return 101; }   // 0.1.1
 
 extern "C" const char* vi_last_error(void) { return g_err; }
 
@@ -88,6 +87,5 @@ extern "C" int vi_init(int device) {
   }
   g_num_sms = prop.multiProcessorCount;
   if (int rc = vi_attn_init()) return rc;
-  if (int rc = vi_attn_tc_init()) return rc;
   return VI_OK;
 }

@@ -422,8 +422,8 @@ __device__ __forceinline__ void attn_sp_body(const AttnProblem& pr, uint32_t ks_
   }
 }
 
-template <bool F16, int MINB>
-__global__ void __launch_bounds__(128, MINB) attn_fwd_sp_kernel(const AttnParams p) {
+template <bool F16>
+__global__ void __launch_bounds__(128, 5) attn_fwd_sp_kernel(const AttnParams p) {
   pdl_enter();
   extern __shared__ __align__(16) uint8_t smem[];
   int z = blockIdx.z, pi = 0;
@@ -552,23 +552,23 @@ __global__ void __launch_bounds__(128) attn_fwd_f32_kernel(const AttnProblem p, 
 }  // namespace
 
 static int check_problem(const vi_attn_problem& a, int H, int dtype, AttnProblem& o) {
-  VI_CHECK_ARG(a.q && a.k && a.v && a.o, "vi_attn_fwd: null operand");
-  VI_CHECK_ARG(a.B > 0 && a.Lq > 0 && a.Lk > 0, "vi_attn_fwd: empty problem B=%d Lq=%d Lk=%d", a.B, a.Lq, a.Lk);
-  VI_CHECK_ARG(a.Lk <= 512, "vi_attn_fwd: Lk=%d exceeds the single-pass limit of 512 keys", a.Lk);
-  VI_CHECK_ARG(!a.pair_dist || a.bias_affine, "vi_attn_fwd: pair_dist needs bias_affine {w,b}");
+  VI_CHECK_ARG(a.q && a.k && a.v && a.o, "vi_attn_fwd_multi: null operand");
+  VI_CHECK_ARG(a.B > 0 && a.Lq > 0 && a.Lk > 0, "vi_attn_fwd_multi: empty problem B=%d Lq=%d Lk=%d", a.B, a.Lq, a.Lk);
+  VI_CHECK_ARG(a.Lk <= 512, "vi_attn_fwd_multi: Lk=%d exceeds the single-pass limit of 512 keys", a.Lk);
+  VI_CHECK_ARG(!a.pair_dist || a.bias_affine, "vi_attn_fwd_multi: pair_dist needs bias_affine {w,b}");
   const int64_t hd = (int64_t)H * DH;
-  VI_CHECK_ARG(a.ldq >= hd && a.ldk >= hd && a.ldv >= hd && a.ldo >= hd, "vi_attn_fwd: leading dimensions smaller than H*64");
+  VI_CHECK_ARG(a.ldq >= hd && a.ldk >= hd && a.ldv >= hd && a.ldo >= hd, "vi_attn_fwd_multi: leading dimensions smaller than H*64");
   if (dtype != VI_DT_F32) {
     VI_CHECK_ARG(a.ldq % 8 == 0 && a.ldk % 8 == 0 && a.ldv % 8 == 0 && a.ldo % 2 == 0,
-                 "vi_attn_fwd: bf16 leading dims must be multiples of 8");
+                 "vi_attn_fwd_multi: bf16 leading dims must be multiples of 8");
     VI_CHECK_ARG((((uintptr_t)a.q | (uintptr_t)a.k | (uintptr_t)a.v) & 15) == 0 && ((uintptr_t)a.o & 3) == 0,
-                 "vi_attn_fwd: misaligned bf16 operands");
+                 "vi_attn_fwd_multi: misaligned bf16 operands");
   }
   o.q = a.q; o.ldq = a.ldq; o.k = a.k; o.ldk = a.ldk; o.v = a.v; o.ldv = a.ldv; o.o = a.o; o.ldo = a.ldo;
   o.key_mask = a.key_mask; o.pair_dist = a.pair_dist; o.bias_affine = a.bias_affine; o.lse = a.lse;
   o.B = a.B; o.Lq = a.Lq; o.Lk = a.Lk; o.LkP = (a.Lk + 15) & ~15;
   VI_CHECK_ARG(a.drop_p >= 0.f && a.drop_p < 1.f && (a.drop_p == 0.f || (a.drop_seed && dtype != VI_DT_F32)),
-               "vi_attn_fwd: attention dropout needs 0 <= p < 1, a device seed pointer and the bf16 kernel");
+               "vi_attn_fwd_multi: attention dropout needs 0 <= p < 1, a device seed pointer and the bf16 kernel");
   o.drop_thresh = a.drop_p > 0.f ? vi_drop_threshold(a.drop_p) : 0u;
   if (a.drop_p > 0.f && o.drop_thresh == 0u) o.drop_thresh = 1u;
   o.drop_scale = a.drop_p > 0.f ? 1.0f / (1.0f - a.drop_p) : 1.0f;
@@ -576,20 +576,13 @@ static int check_problem(const vi_attn_problem& a, int H, int dtype, AttnProblem
   return VI_OK;
 }
 
-static bool vi_attn_sp_enabled() {               // read per call: tests switch between the two kernels within one process
-  const char* e = getenv("VI_ATTN_SP");
-  return !(e && e[0] == '0');
-}
-int vi_attn_tc_eligible(const vi_attn_problem* pr, int n, int H, int dtype);                                     // vi_attn_tc.cu
-int vi_attn_tc_launch(const vi_attn_problem* problems, int n_problems, int H, int dtype, int mask_mode, cudaStream_t st);
-
 extern "C" int vi_attn_fwd_multi(const vi_attn_problem* problems, int n_problems, int H, int dtype, int mask_mode,
                                  vi_stream_t stream) {
   VI_CHECK_ARG(problems && n_problems >= 1 && n_problems <= VI_ATTN_MAX_PROBLEMS, "vi_attn_fwd_multi: 1..%d problems",
                VI_ATTN_MAX_PROBLEMS);
   VI_CHECK_ARG(H > 0, "vi_attn_fwd_multi: H must be positive");
-  VI_CHECK_ARG(mask_mode == VI_MASK_ADD_NEG10000 || mask_mode == VI_MASK_NEG_INF, "vi_attn_fwd: bad mask_mode");
-  VI_CHECK_ARG(dtype == VI_DT_BF16 || dtype == VI_DT_F32 || dtype == VI_DT_F16, "vi_attn_fwd: bad dtype %d", dtype);
+  VI_CHECK_ARG(mask_mode == VI_MASK_ADD_NEG10000 || mask_mode == VI_MASK_NEG_INF, "vi_attn_fwd_multi: bad mask_mode");
+  VI_CHECK_ARG(dtype == VI_DT_BF16 || dtype == VI_DT_F32 || dtype == VI_DT_F16, "vi_attn_fwd_multi: bad dtype %d", dtype);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   AttnParams p;
   memset(&p, 0, sizeof(p));
@@ -601,27 +594,19 @@ extern "C" int vi_attn_fwd_multi(const vi_attn_problem* problems, int n_problems
     max_lq = p.pr[i].Lq > max_lq ? p.pr[i].Lq : max_lq;
     max_lkp = p.pr[i].LkP > max_lkp ? p.pr[i].LkP : max_lkp;
   }
-  // inference shapes go to the tcgen05 kernel (vi_attn_tc.cu); dropout / lse / > 256 keys stay on the mma.sync kernel below
-  if (vi_attn_tc_eligible(problems, n_problems, H, dtype)) return vi_attn_tc_launch(problems, n_problems, H, dtype, mask_mode, st);
   if (dtype != VI_DT_F32) {
     const int q_tiles = (max_lq + 15) / 16;
     const int nwarp = q_tiles < 4 ? q_tiles : 4;
     const int qrows = nwarp * 16;
     const size_t smem = (size_t)max_lkp * ROW * 2 * 2 + (size_t)qrows * ROW * 2 + (size_t)max_lkp * 4;
     dim3 grid((max_lq + qrows - 1) / qrows, H, total_b);
-    // inference shapes (<= 96 keys, no dropout, no log-sum-exp): the single-pass kernel; VI_ATTN_SP=0 keeps the generic one
-    bool sp = max_lkp <= 96 && vi_attn_sp_enabled();
+    // inference shapes (<= 96 keys, no dropout, no log-sum-exp): the single-pass kernel; training and longer key sets the generic one
+    bool sp = max_lkp <= 96;
     for (int i = 0; i < n_problems; ++i) sp = sp && p.pr[i].drop_thresh == 0 && p.pr[i].lse == nullptr;
-    if (sp) {
-      static const int minb_env = [] { const char* e = getenv("VI_ATTN_SP_MINB"); return e ? atoi(e) : 0; }();
-      const bool dense = minb_env ? minb_env == 5 : true;
-      if (dtype == VI_DT_F16) {
-        if (dense) VI_CUDA(vi_launch(attn_fwd_sp_kernel<true, 5>, dim3(grid), dim3(nwarp * 32), (size_t)(smem), st, p));
-        else VI_CUDA(vi_launch(attn_fwd_sp_kernel<true, 4>, dim3(grid), dim3(nwarp * 32), (size_t)(smem), st, p));
-      } else {
-        if (dense) VI_CUDA(vi_launch(attn_fwd_sp_kernel<false, 5>, dim3(grid), dim3(nwarp * 32), (size_t)(smem), st, p));
-        else VI_CUDA(vi_launch(attn_fwd_sp_kernel<false, 4>, dim3(grid), dim3(nwarp * 32), (size_t)(smem), st, p));
-      }
+    if (sp && dtype == VI_DT_F16) {
+      VI_CUDA(vi_launch(attn_fwd_sp_kernel<true>, dim3(grid), dim3(nwarp * 32), (size_t)(smem), st, p));
+    } else if (sp) {
+      VI_CUDA(vi_launch(attn_fwd_sp_kernel<false>, dim3(grid), dim3(nwarp * 32), (size_t)(smem), st, p));
     } else if (dtype == VI_DT_F16) {
       VI_CUDA(vi_launch(attn_fwd_bf16_kernel<true>, dim3(grid), dim3(nwarp * 32), (size_t)(smem), st, p));
     } else {
@@ -640,31 +625,15 @@ extern "C" int vi_attn_fwd_multi(const vi_attn_problem* problems, int n_problems
   return VI_OK;
 }
 
-extern "C" int vi_attn_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, void* o,
-                           int64_t ldo, int dtype, const uint8_t* key_mask, const float* pair_dist,
-                           const float* bias_affine, float* lse, int B, int H, int Lq, int Lk, int mask_mode,
-                           vi_stream_t stream) {
-  vi_attn_problem a;
-  a.q = q; a.ldq = ldq; a.k = k; a.ldk = ldk; a.v = v; a.ldv = ldv; a.o = o; a.ldo = ldo;
-  a.key_mask = key_mask; a.pair_dist = pair_dist; a.bias_affine = bias_affine; a.lse = lse;
-  a.B = B; a.Lq = Lq; a.Lk = Lk;
-  a.drop_p = 0.f; a.drop_site = 0; a.drop_seed = nullptr;
-  return vi_attn_fwd_multi(&a, 1, H, dtype, mask_mode, stream);
-}
-
 int vi_attn_init() {
   VI_CUDA(cudaFuncSetAttribute(attn_fwd_bf16_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 176 * 1024));
   VI_CUDA(cudaFuncSetAttribute(attn_fwd_bf16_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   VI_CUDA(cudaFuncSetAttribute(attn_fwd_bf16_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 176 * 1024));
   VI_CUDA(cudaFuncSetAttribute(attn_fwd_bf16_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<false, 4>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<true, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<true, 4>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<false, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<false, 5>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<true, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<true, 5>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+  VI_CUDA(cudaFuncSetAttribute(attn_fwd_sp_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   VI_CUDA(cudaFuncSetAttribute(attn_fwd_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   return VI_OK;
 }

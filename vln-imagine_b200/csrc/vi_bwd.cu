@@ -244,112 +244,10 @@ __global__ void __launch_bounds__(256) dropout_kernel(const T* x, T* __restrict_
 // ---------------------------------------------------------------------------------------------
 // LayerNorm backward.  y = LN(a [+ b]) * gamma + beta;  dy = dy32 [+ dy16].
 //   dx[r] = rstd * (g - mean(g) - xhat * mean(g * xhat)),  g = dy * gamma      (one warp per row)
-//   stats[r] = {mean, rstd} for the parameter-gradient pass
+//   dgamma[c] = sum_r dy * xhat,  dbeta[c] = sum_r dy;  stats[r] = {mean, rstd}
 // ---------------------------------------------------------------------------------------------
 
-__global__ void __launch_bounds__(128) ln_bwd_dx_kernel(const float* a, const float* b,
-                                                        const float* gamma, float eps,
-                                                        const float* dy32, const bf16* dy16,
-                                                        float* __restrict__ dx32, bf16* __restrict__ dx16,
-                                                        float* __restrict__ stats, long long rows, const RowGroups grp) {
-  pdl_enter();
-  const int lane = threadIdx.x & 31;
-  const long long row = (long long)blockIdx.x * 4 + (threadIdx.x >> 5);
-  if (row >= rows) return;
-  gamma += group_of_row(grp, row) * D;
-  float x[24], g[24];
-  float s = 0.f;
-#pragma unroll
-  for (int j = 0; j < 6; ++j) {
-    const int c = (lane + 32 * j) * 4;
-    float4 t = *reinterpret_cast<const float4*>(a + row * D + c);
-    if (b) {
-      const float4 u = *reinterpret_cast<const float4*>(b + row * D + c);
-      t.x += u.x; t.y += u.y; t.z += u.z; t.w += u.w;
-    }
-    x[4 * j] = t.x; x[4 * j + 1] = t.y; x[4 * j + 2] = t.z; x[4 * j + 3] = t.w;
-    s += t.x + t.y + t.z + t.w;
-  }
-  const float mean = warp_sum(s) * (1.0f / D);
-  float q = 0.f;
-#pragma unroll
-  for (int i = 0; i < 24; ++i) { const float d = x[i] - mean; q = fmaf(d, d, q); }
-  const float rstd = rsqrtf(warp_sum(q) * (1.0f / D) + eps);
-  float sg = 0.f, sgx = 0.f;
-#pragma unroll
-  for (int j = 0; j < 6; ++j) {
-    const int c = (lane + 32 * j) * 4;
-    float d[4] = {0.f, 0.f, 0.f, 0.f};
-    if (dy32) {
-      const float4 t = *reinterpret_cast<const float4*>(dy32 + row * D + c);
-      d[0] = t.x; d[1] = t.y; d[2] = t.z; d[3] = t.w;
-    }
-    if (dy16) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e) d[e] += __bfloat162float(dy16[row * D + c + e]);
-    }
-    const float4 gm = *reinterpret_cast<const float4*>(gamma + c);
-    const float gmv[4] = {gm.x, gm.y, gm.z, gm.w};
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const float xh = (x[4 * j + e] - mean) * rstd;
-      const float gg = d[e] * gmv[e];
-      x[4 * j + e] = xh;
-      g[4 * j + e] = gg;
-      sg += gg;
-      sgx = fmaf(gg, xh, sgx);
-    }
-  }
-  const float mg = warp_sum(sg) * (1.0f / D), mgx = warp_sum(sgx) * (1.0f / D);
-#pragma unroll
-  for (int j = 0; j < 6; ++j) {
-    const int c = (lane + 32 * j) * 4;
-    float o[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) o[e] = rstd * (g[4 * j + e] - mg - x[4 * j + e] * mgx);
-    if (dx32) *reinterpret_cast<float4*>(dx32 + row * D + c) = make_float4(o[0], o[1], o[2], o[3]);
-    if (dx16) *reinterpret_cast<uint2*>(dx16 + row * D + c) = make_uint2(pack_bf16x2(o[0], o[1]), pack_bf16x2(o[2], o[3]));
-  }
-  if (lane == 0) { stats[2 * row] = mean; stats[2 * row + 1] = rstd; }
-}
-
-// stage 1 of dgamma[c] = sum_r dy * xhat, dbeta[c] = sum_r dy: partials per 128-row chunk into part[2][n_chunks][768];
-// grid (768 / 64, n_chunks), 256 threads (stage 2: chunk_sum_kernel per row group)
-__global__ void __launch_bounds__(256) ln_bwd_param_partial_kernel(const float* a, const float* b,
-                                                                   const float* dy32, const bf16* dy16,
-                                                                   const float* stats, float* __restrict__ part,
-                                                                   long long rows, int n_chunks) {
-  pdl_enter();
-  __shared__ float2 rg[8][32], rb[8][32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int c = blockIdx.x * 64 + 2 * lane;
-  const long long r0 = (long long)blockIdx.y * RED_CHUNK;
-  const long long r1 = r0 + RED_CHUNK < rows ? r0 + RED_CHUNK : rows;
-  float2 sg = make_float2(0.f, 0.f), sb = make_float2(0.f, 0.f);
-  for (long long r = r0 + warp; r < r1; r += 8) {
-    float2 x = ld2f(a + r * D + c);
-    if (b) { const float2 u = ld2f(b + r * D + c); x.x += u.x; x.y += u.y; }
-    float2 d = make_float2(0.f, 0.f);
-    if (dy32) d = ld2f(dy32 + r * D + c);
-    if (dy16) { const float2 u = ld2f(dy16 + r * D + c); d.x += u.x; d.y += u.y; }
-    const float mean = stats[2 * r], rstd = stats[2 * r + 1];
-    sg.x = fmaf(d.x, (x.x - mean) * rstd, sg.x);
-    sg.y = fmaf(d.y, (x.y - mean) * rstd, sg.y);
-    sb.x += d.x; sb.y += d.y;
-  }
-  rg[warp][lane] = sg;
-  rb[warp][lane] = sb;
-  __syncthreads();
-  if (warp == 0) {
-    float2 t = make_float2(0.f, 0.f), u = make_float2(0.f, 0.f);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) { t.x += rg[i][lane].x; t.y += rg[i][lane].y; u.x += rb[i][lane].x; u.y += rb[i][lane].y; }
-    *reinterpret_cast<float2*>(part + (long long)blockIdx.y * D + c) = t;
-    *reinterpret_cast<float2*>(part + ((long long)n_chunks + blockIdx.y) * D + c) = u;
-  }
-}
-
-// dx AND the parameter-gradient partials in ONE pass over the rows (the two-kernel form above reads a, b and dy twice): a CTA of
+// dx AND the parameter-gradient partials in ONE pass over the rows: a CTA of
 // 8 warps owns chunk_rows = 8 / 16 / 32 consecutive rows (1 / 2 / 4 per warp), every lane keeps the dgamma / dbeta contributions of its
 // 24 columns in registers, the 8 warps are summed through shared memory in a fixed order and the chunk's partial row goes to
 // part[2][n_chunks][768]; ln_param_sum_kernel then adds the chunks of each row group (fixed order: deterministic).
@@ -357,8 +255,7 @@ __global__ void __launch_bounds__(256) ln_bwd_param_partial_kernel(const float* 
 // grid was 40 - 160 CTAs of 8 warps walking 4 dependent row round trips each on a 148-SM part.
 constexpr int LN_CHUNK_MAX = 32;
 static int ln_chunk_rows(int64_t rows, int64_t scratch_elems) {
-  static const int forced = [] { const char* e = getenv("VI_LN_CHUNK"); return e ? atoi(e) : 0; }();      // 8 / 16 / 32: A/B switch
-  int chunk = (forced == 8 || forced == 16 || forced == 32) ? forced : rows <= 296 * 8 ? 8 : rows <= 296 * 16 ? 16 : LN_CHUNK_MAX;
+  int chunk = rows <= 296 * 8 ? 8 : rows <= 296 * 16 ? 16 : LN_CHUNK_MAX;
   while (chunk < LN_CHUNK_MAX && (int64_t)2 * ((rows + chunk - 1) / chunk) * D > scratch_elems) chunk *= 2;     // caller's workspace decides
   return chunk;
 }
@@ -989,10 +886,6 @@ inline RowGroups one_group() {
   return g;
 }
 
-extern "C" int64_t vi_reduce_scratch_elems(int64_t rows, int cols, int n_out) {
-  return (int64_t)n_out * ((rows + RED_CHUNK - 1) / RED_CHUNK) * cols;
-}
-
 extern "C" int vi_colsum(const void* x, int64_t ld, int dtype, float* out, int64_t rows, int cols, float* scratch,
                          int64_t scratch_elems, vi_stream_t stream) {
   VI_CHECK_ARG(x && out && scratch && rows > 0 && cols > 0 && ld >= cols, "vi_colsum: bad operands");
@@ -1057,55 +950,35 @@ extern "C" int vi_act_bwd(const void* x, const void* dy, void* dx, int64_t n, in
   return VI_OK;
 }
 
-extern "C" int vi_add_ln_bwd(const float* a, const float* b, const float* gamma, float eps, const float* dy32, const void* dy16,
-                             float* dx32, void* dx16, float* dgamma, float* dbeta, float* stats, int64_t rows, int n_groups,
-                             const int32_t* group_row_end, float* scratch, int64_t scratch_elems, vi_stream_t stream) {
-  return vi_add_ln_bwd_acc(a, b, gamma, eps, dy32, dy16, dx32, dx16, dgamma, dbeta, stats, rows, n_groups, group_row_end, scratch,
-                           scratch_elems, 0, stream);
-}
-
-extern "C" int vi_add_ln_bwd_acc(const float* a, const float* b, const float* gamma, float eps, const float* dy32, const void* dy16,
-                                 float* dx32, void* dx16, float* dgamma, float* dbeta, float* stats, int64_t rows, int n_groups,
-                                 const int32_t* group_row_end, float* scratch, int64_t scratch_elems, int accumulate,
-                                 vi_stream_t stream) {
-  return vi_add_ln_drop_bwd(a, b, gamma, eps, dy32, dy16, dx32, dx16, nullptr, dgamma, dbeta, stats, rows, n_groups, group_row_end,
-                            scratch, scratch_elems, accumulate, 0.f, nullptr, 0u, stream);
-}
-
 extern "C" int vi_add_ln_drop_bwd(const float* a, const float* b, const float* gamma, float eps, const float* dy32, const void* dy16,
                                   float* dx32, void* dx16, void* dxa16, float* dgamma, float* dbeta, float* stats, int64_t rows,
                                   int n_groups, const int32_t* group_row_end, float* scratch, int64_t scratch_elems, int accumulate,
                                   float p, const uint32_t* seed, uint32_t site, vi_stream_t stream) {
   VI_CHECK_ARG(p >= 0.f && p < 1.f && (p == 0.f || seed), "vi_add_ln_drop_bwd: 0 <= p < 1 and a device seed pointer");
-  VI_CHECK_ARG(!dxa16 || (dgamma && dbeta && ((uintptr_t)dxa16 & 7) == 0), "vi_add_ln_drop_bwd: dxa16 needs dgamma / dbeta and 8-byte alignment");
-  VI_CHECK_ARG(p == 0.f || (dgamma && dbeta && rows * D < (1LL << 32)), "vi_add_ln_drop_bwd: dropout needs the one-pass form and < 2^32 elements");
+  VI_CHECK_ARG(((uintptr_t)dxa16 & 7) == 0, "vi_add_ln_drop_bwd: dxa16 must be 8-byte aligned");
+  VI_CHECK_ARG(p == 0.f || rows * D < (1LL << 32), "vi_add_ln_drop_bwd: dropout needs < 2^32 elements");
   DropArgs dr;
   dr.thresh = vi_drop_threshold(p); dr.scale = 1.0f / (1.0f - p); dr.seed = p > 0.f ? seed : nullptr; dr.site = site;
   dr.dxa16 = reinterpret_cast<bf16*>(dxa16);
   RowGroups grp;
-  VI_CHECK_ARG(make_groups(grp, n_groups, group_row_end), "vi_add_ln_bwd: bad row groups");
+  VI_CHECK_ARG(make_groups(grp, n_groups, group_row_end), "vi_add_ln_drop_bwd: bad row groups");
   for (int g = 0; g + 1 < n_groups; ++g)
-    VI_CHECK_ARG(group_row_end[g] % RED_CHUNK == 0, "vi_add_ln_bwd: row groups must end on multiples of %d rows", RED_CHUNK);
-  VI_CHECK_ARG(a && gamma && (dy32 || dy16) && (dx32 || dx16) && stats, "vi_add_ln_bwd: null operand");
+    VI_CHECK_ARG(group_row_end[g] % RED_CHUNK == 0, "vi_add_ln_drop_bwd: row groups must end on multiples of %d rows", RED_CHUNK);
+  VI_CHECK_ARG(a && gamma && (dy32 || dy16) && (dx32 || dx16) && dgamma && dbeta && stats, "vi_add_ln_drop_bwd: null operand");
   VI_CHECK_ARG(aligned16(a) && aligned16(b) && aligned16(gamma) && aligned16(dy32) && aligned16(dx32) &&
-                   ((uintptr_t)dx16 & 7) == 0, "vi_add_ln_bwd: misaligned operands");
+                   ((uintptr_t)dx16 & 7) == 0, "vi_add_ln_drop_bwd: misaligned operands");
   if (rows <= 0) return VI_OK;
-  if (dgamma && dbeta) {
-    // one pass: dx + per-chunk partials of dgamma / dbeta, then the fixed-order sum of the chunks of every row group
-    VI_CHECK_ARG(aligned16(dgamma) && aligned16(dbeta) && aligned16(scratch), "vi_add_ln_bwd: dgamma / dbeta / scratch must be 16-byte aligned");
-    const int chunk = scratch ? ln_chunk_rows(rows, scratch_elems) : LN_CHUNK_MAX;
-    const int nch = (int)((rows + chunk - 1) / chunk);
-    VI_CHECK_ARG(scratch && scratch_elems >= (int64_t)2 * nch * D, "vi_add_ln_bwd: scratch too small (need 2 x ceil(rows / %d) x %d floats)",
-                 LN_CHUNK_MAX, D);
-    VI_CUDA(vi_launch(ln_bwd_fused_kernel, dim3((unsigned)nch), dim3(256), 0, ST(stream), a, b, gamma, eps, dy32,
-                      reinterpret_cast<const bf16*>(dy16), dx32, reinterpret_cast<bf16*>(dx16), stats, scratch, (long long)rows, nch, chunk,
-                      grp, dr));
-    VI_CUDA(vi_launch(ln_param_sum_kernel, dim3(D / 128, n_groups, 2), dim3(256), 0, ST(stream), (const float*)scratch, dgamma, dbeta, nch,
-                      chunk, (long long)rows, grp, (int)(accumulate != 0)));
-  } else {
-    VI_CUDA(vi_launch(ln_bwd_dx_kernel, dim3((unsigned)((rows + 3) / 4)), dim3(128), 0, ST(stream), a, b, gamma, eps, dy32,
-                      reinterpret_cast<const bf16*>(dy16), dx32, reinterpret_cast<bf16*>(dx16), stats, (long long)rows, grp));
-  }
+  // one pass: dx + per-chunk partials of dgamma / dbeta, then the fixed-order sum of the chunks of every row group
+  VI_CHECK_ARG(aligned16(dgamma) && aligned16(dbeta) && aligned16(scratch), "vi_add_ln_drop_bwd: dgamma / dbeta / scratch must be 16-byte aligned");
+  const int chunk = scratch ? ln_chunk_rows(rows, scratch_elems) : LN_CHUNK_MAX;
+  const int nch = (int)((rows + chunk - 1) / chunk);
+  VI_CHECK_ARG(scratch && scratch_elems >= (int64_t)2 * nch * D, "vi_add_ln_drop_bwd: scratch too small (need 2 x ceil(rows / %d) x %d floats)",
+               LN_CHUNK_MAX, D);
+  VI_CUDA(vi_launch(ln_bwd_fused_kernel, dim3((unsigned)nch), dim3(256), 0, ST(stream), a, b, gamma, eps, dy32,
+                    reinterpret_cast<const bf16*>(dy16), dx32, reinterpret_cast<bf16*>(dx16), stats, scratch, (long long)rows, nch, chunk,
+                    grp, dr));
+  VI_CUDA(vi_launch(ln_param_sum_kernel, dim3(D / 128, n_groups, 2), dim3(256), 0, ST(stream), (const float*)scratch, dgamma, dbeta, nch,
+                    chunk, (long long)rows, grp, (int)(accumulate != 0)));
   return VI_OK;
 }
 
@@ -1161,7 +1034,7 @@ extern "C" int vi_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ld
   VI_CHECK_ARG(!pair_dist || bias_affine, "vi_attn_bwd: pair_dist needs bias_affine");
   VI_CHECK_ARG(drop_p >= 0.f && drop_p < 1.f && (drop_p == 0.f || drop_seed), "vi_attn_bwd: bad dropout arguments");
   VI_CHECK_ARG(H * 64 <= ldq && H * 64 <= ldk && H * 64 <= ldv && H * 64 <= ldo, "vi_attn_bwd: leading dimensions smaller than H*64");
-  if (dtype == VI_DT_BF16 && !getenv("VI_ATTN_BWD_SIMT")) {
+  if (dtype == VI_DT_BF16) {
     const int rc = vi_attn_bwd_tc(q, ldq, k, ldk, v, ldv, dout, ldo, dq, lddq, dk, lddk, dv, lddv, key_mask, pair_dist,
                                   bias_affine, d_affine, B, H, Lq, Lk, mask_mode, drop_p, drop_site, drop_seed, ST(stream));
     if (rc <= 0) return rc;            // launched (0) or failed (< 0); 1 = does not fit -> fp32-arithmetic kernel below

@@ -1,5 +1,5 @@
 // vi_gemm_simt.cu - the fp32 check-mode GEMM (FFMA, no tensor cores): Y = epi(X W^T + bias) + residual.
-// Same contract and grouped form as vi_gemm_bf16; used for the 1e-4 parity mode that BASELINE.json
+// Same contract and grouped form as vi_gemm16; used for the 1e-4 parity mode that BASELINE.json
 // asks for and to cross-check the tcgen05 kernel.  64x64 output tile, 16x16 threads, 4x4 micro-tile,
 // K staged through shared memory in blocks of 16.
 #include "vi_common.cuh"

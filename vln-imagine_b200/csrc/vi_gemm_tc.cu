@@ -664,12 +664,6 @@ struct Choice { int bn; bool pair; };
 // L2 -> SM operand traffic of the whole problem (about 6300 B/cycle chip-wide), plus one exposed epilogue.
 Choice pick_tile(int M, int N, int K, int nsm, bool pair_ok) {
   Choice best = {64, false};
-  if (const char* e = getenv("VI_GEMM_TILE")) {        // e.g. "192" or "256p" (tests / sweeps)
-    const int v = atoi(e);
-    const bool pr = strchr(e, 'p') != nullptr;
-    if ((v == 64 || v == 96 || v == 128 || v == 192 || v == 256) && N % v == 0 && (!pr || (pair_ok && v >= 128)))
-      return Choice{v, pr};
-  }
   double best_cost = 1e30;
   const int cands[5] = {256, 192, 128, 96, 64};
   for (int pr = 1; pr >= 0; --pr) {
@@ -696,24 +690,6 @@ Choice pick_tile(int M, int N, int K, int nsm, bool pair_ok) {
 }
 
 }  // namespace
-
-extern "C" int vi_gemm_bf16(const void* x, int64_t ldx, const void* w, const float* bias, const float* residual,
-                            int64_t ldr, void* y, int64_t ldy, int y_dtype, int M, int N, int K, int epilogue,
-                            int n_groups, const int32_t* group_row_end, vi_stream_t stream) {
-  return vi_gemm_bf16_tiled(x, ldx, w, bias, residual, ldr, y, ldy, y_dtype, M, N, K, epilogue, n_groups, group_row_end, 0,
-                            stream);
-}
-
-extern "C" int vi_gemm_bf16_tiled(const void* x, int64_t ldx, const void* w, const float* bias, const float* residual,
-                                  int64_t ldr, void* y, int64_t ldy, int y_dtype, int M, int N, int K, int epilogue,
-                                  int n_groups, const int32_t* group_row_end, int tile, vi_stream_t stream) {
-  vi_gemm_args a;
-  memset(&a, 0, sizeof(a));
-  a.x = x; a.ldx = ldx; a.w = w; a.in_dtype = VI_DT_BF16; a.bias = bias; a.residual = residual; a.ldr = ldr;
-  a.y = y; a.ldy = ldy; a.y_dtype = y_dtype; a.M = M; a.N = N; a.K = K; a.epilogue = epilogue; a.n_groups = n_groups;
-  a.group_row_end = group_row_end; a.tile = tile;
-  return vi_gemm16(&a, stream);
-}
 
 extern "C" int vi_gemm16(const vi_gemm_args* args, vi_stream_t stream) {
   VI_CHECK_ARG(args, "vi_gemm16: null args");
@@ -773,7 +749,7 @@ extern "C" int vi_gemm16(const vi_gemm_args* args, vi_stream_t stream) {
   VI_CHECK_ARG(n_groups == 1 || a.group_row_end[n_groups - 1] == M, "vi_gemm16: last group must end at M");
 
   const int nsm = vi_num_sms();
-  Choice c = pick_tile(M, N, K, nsm, pair_ok);
+  Choice c;
   if (a.tile != 0) {                     // caller-selected tile (the Python host keeps a measured table per shape)
     const int bn = a.tile & 0xFFF;
     const bool pr = (a.tile & VI_TILE_PAIR) != 0;
@@ -781,6 +757,8 @@ extern "C" int vi_gemm16(const vi_gemm_args* args, vi_stream_t stream) {
                  "vi_gemm16: tile width %d does not divide N=%d", bn, N);
     VI_CHECK_ARG(!pr || (pair_ok && bn >= 128), "vi_gemm16: CTA-pair tiles need width >= 128 and 256-row group ends");
     c = Choice{bn, pr};
+  } else {
+    c = pick_tile(M, N, K, nsm, pair_ok);
   }
   const int tm = c.pair ? 2 * BM : BM;
   p.num_m_tiles = (M + tm - 1) / tm;

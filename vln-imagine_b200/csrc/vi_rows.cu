@@ -139,61 +139,21 @@ __global__ void __launch_bounds__(128) add_ln_drop_kernel(const float* a, const 
   row_store(r, y32, y16, row, lane, f16 != 0);
 }
 
-// NR rows per warp (1 by default), 4 warps per CTA.  Everything a row needs PER COLUMN - the TRANSPOSED weight of the small
-// feature projection ([feat_dim][768], prepared by the caller once per weight version) and up to eleven 768-wide vectors
-// (LayerNorm gains / biases, the feature bias, constant rows; 33 - 76 KB in all) - is read with plain 16-byte loads through
-// the SM's L1.  The grid is ONE wave whose warps start together, so without help every warp walks the k-loop and the vectors
-// as a chain of 20 - 30 dependent L2 round trips (ncu: 29 of 36 cycles per issued instruction on the long scoreboard); the
-// kernel therefore touches every parameter line once at its top, all loads in flight, ahead of the dependency wait - measured
-// 8.5 us per navigation step (3 launches), 0.8255 -> 0.8170 ms.  The rows' own data (the row, its table row) is prefetched
-// at the top and loaded when it is needed, which keeps the live registers at one accumulator row + one operand row per row.
-// Measured and rejected: two rows per warp sharing every parameter load (VI_EMBED_NR=2: half the L1 traffic, 150 registers,
-// 0.4 % slower - the kernel is latency-, not L1-bandwidth-bound); staging the parameters in shared memory per CTA (80 KB for
-// 8 rows: the L2 -> SM traffic dominates); prefetch.global.L1 for the warm-up (CCTL.PF1: no effect).
+// One row per warp, 4 warps per CTA.  Everything a row needs PER COLUMN - the TRANSPOSED weight of the small feature
+// projection ([feat_dim][768], prepared by the caller once per weight version) and up to eleven 768-wide vectors (LayerNorm
+// gains / biases, the feature bias, constant rows; 33 - 76 KB in all) - is read with plain 16-byte loads through the SM's L1.
+// The grid is ONE wave whose warps start together, so without help every warp walks the k-loop and the vectors as a chain of
+// 20 - 30 dependent L2 round trips (ncu: 29 of 36 cycles per issued instruction on the long scoreboard); the kernel therefore
+// touches every parameter line once at its top, all loads in flight, ahead of the dependency wait - measured 8.5 us per
+// navigation step (3 launches), 0.8255 -> 0.8170 ms.  The row's own data (the row, its table row) is prefetched at the top
+// and loaded when it is needed, which keeps the live registers at one accumulator row + one operand row.
+// Measured and rejected: two rows per warp sharing every parameter load (half the L1 traffic, 150 registers, 0.4 % slower -
+// the kernel is latency-, not L1-bandwidth-bound); staging the parameters in shared memory per CTA (80 KB for 8 rows: the
+// L2 -> SM traffic dominates); prefetch.global.L1 for the warm-up (CCTL.PF1: no effect).
 constexpr int EMBED_WARPS = 4;
 
 __device__ __forceinline__ void prefetch_row_l1(const float* src, int lane) {       // 768 floats = 24 lines of 128 bytes
   if (lane < 24) asm volatile("prefetch.global.L1 [%0];" ::"l"(src + lane * 32));
-}
-// in-place LayerNorm of the warp's rows with ONE read of the gain / bias vectors
-template <int NR>
-__device__ __forceinline__ void row_layernorm_n(Row (&r)[NR], const float* gamma, const float* beta, float eps, int lane) {
-  float mean[NR], rstd[NR];
-#pragma unroll
-  for (int q = 0; q < NR; ++q) {
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < V4 * 4; ++i) s += r[q].v[i];
-    mean[q] = warp_sum(s) * (1.0f / D);
-    float v = 0.f;
-#pragma unroll
-    for (int i = 0; i < V4 * 4; ++i) { const float d = r[q].v[i] - mean[q]; v = fmaf(d, d, v); }
-    rstd[q] = rsqrtf(warp_sum(v) * (1.0f / D) + eps);
-  }
-  const float4* g4 = reinterpret_cast<const float4*>(gamma);
-  const float4* b4 = reinterpret_cast<const float4*>(beta);
-#pragma unroll
-  for (int j = 0; j < V4; ++j) {
-    const float4 g = *(g4 + lane + 32 * j), b = *(b4 + lane + 32 * j);
-#pragma unroll
-    for (int q = 0; q < NR; ++q) {
-      r[q].v[4 * j] = (r[q].v[4 * j] - mean[q]) * rstd[q] * g.x + b.x;
-      r[q].v[4 * j + 1] = (r[q].v[4 * j + 1] - mean[q]) * rstd[q] * g.y + b.y;
-      r[q].v[4 * j + 2] = (r[q].v[4 * j + 2] - mean[q]) * rstd[q] * g.z + b.z;
-      r[q].v[4 * j + 3] = (r[q].v[4 * j + 3] - mean[q]) * rstd[q] * g.w + b.w;
-    }
-  }
-}
-// r[q] += the same 768-wide vector (one read for both rows)
-template <int NR>
-__device__ __forceinline__ void rows_add_vec(Row (&r)[NR], const float* vec, int lane) {
-  const float4* s4 = reinterpret_cast<const float4*>(vec);
-#pragma unroll
-  for (int j = 0; j < V4; ++j) {
-    const float4 t = *(s4 + lane + 32 * j);
-#pragma unroll
-    for (int q = 0; q < NR; ++q) { r[q].v[4 * j] += t.x; r[q].v[4 * j + 1] += t.y; r[q].v[4 * j + 2] += t.z; r[q].v[4 * j + 3] += t.w; }
-  }
 }
 
 // Brings the 128-byte line into the SM's L1 with a real load: prefetch.global.L1 (CCTL.PF1) measured as a no-op for this
@@ -208,7 +168,6 @@ __device__ __forceinline__ void warm_sink(float warm) {
   if (warm == -1.2345678e-30f) asm volatile("nanosleep.u32 0;");
 }
 
-template <int NR>
 __global__ void __launch_bounds__(EMBED_WARPS * 32) embed_compose_kernel(const vi_embed_args p) {
   pdl_launch_dependents();
   // Warm the L1 with every PARAMETER line the rows will read (the transposed weight and the vectors), all loads in flight at
@@ -231,96 +190,63 @@ __global__ void __launch_bounds__(EMBED_WARPS * 32) embed_compose_kernel(const v
   }
   pdl_wait();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const long long row0 = ((long long)blockIdx.x * EMBED_WARPS + warp) * NR;
+  const long long row = (long long)blockIdx.x * EMBED_WARPS + warp;
   const long long end = p.rows + p.zero_rows;
-  if (row0 >= end) return;
-  // padding rows behind the stream (row-stacked activations): zeros
-#pragma unroll
-  for (int q = 0; q < NR; ++q) {
-    if (row0 + q >= p.rows && row0 + q < end) {
-      Row z;
-      row_zero(z);
-      row_store(z, p.y32, reinterpret_cast<bf16*>(p.y16), row0 + q, lane, p.y16_dtype == VI_DT_F16);
-    }
+  if (row >= end) return;
+  if (row >= p.rows) {                             // padding rows behind the stream (row-stacked activations): zeros
+    Row z;
+    row_zero(z);
+    row_store(z, p.y32, reinterpret_cast<bf16*>(p.y16), row, lane, p.y16_dtype == VI_DT_F16);
+    return;
   }
-  if (row0 >= p.rows) return;
-  long long rq[NR];                                // a warp whose second row does not exist recomputes its first one
-  bool live[NR];
-#pragma unroll
-  for (int q = 0; q < NR; ++q) { live[q] = row0 + q < p.rows; rq[q] = live[q] ? row0 + q : row0; }
 
-  // ---- the rows' own data: small loads now, the 3 KB rows prefetched into L1
-  float fv[NR];
-  long long ti[NR];
-#pragma unroll
-  for (int q = 0; q < NR; ++q) {
-    fv[q] = (p.feat && lane < p.feat_dim) ? *(p.feat + rq[q] * p.feat_dim + lane) : 0.f;
-    ti[q] = p.idx ? p.idx[rq[q]] : 0;
-    if (p.a) prefetch_row_l1(p.a + rq[q] * D, lane);
-  }
-#pragma unroll
-  for (int q = 0; q < NR; ++q)
-    if (p.idx) prefetch_row_l1(p.table + ti[q] * D, lane);
+  // ---- the row's own data: small loads now, the 3 KB rows prefetched into L1
+  const float fv = (p.feat && lane < p.feat_dim) ? *(p.feat + row * p.feat_dim + lane) : 0.f;
+  const long long ti = p.idx ? p.idx[row] : 0;
+  if (p.a) prefetch_row_l1(p.a + row * D, lane);
+  if (p.idx) prefetch_row_l1(p.table + ti * D, lane);
 
-  Row acc[NR];
-#pragma unroll
-  for (int q = 0; q < NR; ++q) row_zero(acc[q]);
-  // ---- feature projection: every weight value is loaded once and used for both rows
+  Row acc;
+  row_zero(acc);
   if (p.feat) {
-    if (p.feat_b) rows_add_vec(acc, p.feat_b, lane);
+    if (p.feat_b) row_add(acc, p.feat_b, lane);
     for (int k = 0; k < p.feat_dim; ++k) {
-      float f[NR];
-#pragma unroll
-      for (int q = 0; q < NR; ++q) f[q] = __shfl_sync(0xffffffffu, fv[q], k);
+      const float f = __shfl_sync(0xffffffffu, fv, k);
       const float4* w4 = reinterpret_cast<const float4*>(p.feat_w + (long long)k * D);       // transposed: [feat_dim][768]
 #pragma unroll
       for (int j = 0; j < V4; ++j) {
         const float4 w = *(w4 + lane + 32 * j);
-#pragma unroll
-        for (int q = 0; q < NR; ++q) {
-          acc[q].v[4 * j] = fmaf(f[q], w.x, acc[q].v[4 * j]);
-          acc[q].v[4 * j + 1] = fmaf(f[q], w.y, acc[q].v[4 * j + 1]);
-          acc[q].v[4 * j + 2] = fmaf(f[q], w.z, acc[q].v[4 * j + 2]);
-          acc[q].v[4 * j + 3] = fmaf(f[q], w.w, acc[q].v[4 * j + 3]);
-        }
+        acc.v[4 * j] = fmaf(f, w.x, acc.v[4 * j]);
+        acc.v[4 * j + 1] = fmaf(f, w.y, acc.v[4 * j + 1]);
+        acc.v[4 * j + 2] = fmaf(f, w.z, acc.v[4 * j + 2]);
+        acc.v[4 * j + 3] = fmaf(f, w.w, acc.v[4 * j + 3]);
       }
     }
-    if (p.feat_gamma) row_layernorm_n(acc, p.feat_gamma, p.feat_beta, p.eps, lane);
+    if (p.feat_gamma) row_layernorm(acc, p.feat_gamma, p.feat_beta, p.eps, lane);
   }
   if (p.a) {
-    Row a[NR];
-#pragma unroll
-    for (int q = 0; q < NR; ++q) row_load(a[q], p.a + rq[q] * D, lane);
-    if (p.a_gamma) row_layernorm_n(a, p.a_gamma, p.a_beta, p.eps, lane);
-#pragma unroll
-    for (int q = 0; q < NR; ++q) row_acc(acc[q], a[q]);
+    Row a;
+    row_load(a, p.a + row * D, lane);
+    if (p.a_gamma) row_layernorm(a, p.a_gamma, p.a_beta, p.eps, lane);
+    row_acc(acc, a);
   }
-#pragma unroll
-  for (int q = 0; q < NR; ++q) {
-    if (p.a2) row_add(acc[q], p.a2 + rq[q] * D, lane);
-    if (p.a3) row_add(acc[q], p.a3 + rq[q] * D, lane);
-    if (p.idx) row_add(acc[q], p.table + ti[q] * D, lane);
-    if (p.pos_table) row_add(acc[q], p.pos_table + (rq[q] % p.pos_period) * D, lane);
-  }
-  if (p.const_row) rows_add_vec(acc, p.const_row, lane);
-  if (p.const_row2) rows_add_vec(acc, p.const_row2, lane);
-  if (p.out_gamma) row_layernorm_n(acc, p.out_gamma, p.out_beta, p.eps, lane);
+  if (p.a2) row_add(acc, p.a2 + row * D, lane);
+  if (p.a3) row_add(acc, p.a3 + row * D, lane);
+  if (p.idx) row_add(acc, p.table + ti * D, lane);
+  if (p.pos_table) row_add(acc, p.pos_table + (row % p.pos_period) * D, lane);
+  if (p.const_row) row_add(acc, p.const_row, lane);
+  if (p.const_row2) row_add(acc, p.const_row2, lane);
+  if (p.out_gamma) row_layernorm(acc, p.out_gamma, p.out_beta, p.eps, lane);
   if (p.ln2_gamma) {
     // a second LayerNorm chained on the result (norm1 of the first panorama layer, D/models/transformer.py:171): the fp32
     // output keeps the first result (the residual stream), the 16-bit output is the operand of the next contraction
-#pragma unroll
-    for (int q = 0; q < NR; ++q)
-      if (p.y32 && live[q]) row_store(acc[q], p.y32, nullptr, rq[q], lane);
-    row_layernorm_n(acc, p.ln2_gamma, p.ln2_beta, p.ln2_eps, lane);
-#pragma unroll
-    for (int q = 0; q < NR; ++q)
-      if (live[q]) row_store(acc[q], nullptr, reinterpret_cast<bf16*>(p.y16), rq[q], lane, p.y16_dtype == VI_DT_F16);
+    if (p.y32) row_store(acc, p.y32, nullptr, row, lane);
+    row_layernorm(acc, p.ln2_gamma, p.ln2_beta, p.ln2_eps, lane);
+    row_store(acc, nullptr, reinterpret_cast<bf16*>(p.y16), row, lane, p.y16_dtype == VI_DT_F16);
     warm_sink(warm);
     return;
   }
-#pragma unroll
-  for (int q = 0; q < NR; ++q)
-    if (live[q]) row_store(acc[q], p.y32, reinterpret_cast<bf16*>(p.y16), rq[q], lane, p.y16_dtype == VI_DT_F16);
+  row_store(acc, p.y32, reinterpret_cast<bf16*>(p.y16), row, lane, p.y16_dtype == VI_DT_F16);
   warm_sink(warm);
 }
 
@@ -715,13 +641,8 @@ extern "C" int vi_embed_compose(const vi_embed_args* args, vi_stream_t stream) {
   VI_CHECK_ARG(aligned16(p.feat_b) && aligned16(p.feat_w), "vi_embed_compose: feat_b / feat_w must be 16-byte aligned");
   VI_CHECK_ARG(p.zero_rows >= 0, "vi_embed_compose: negative zero_rows");
   if (p.rows <= 0) return VI_OK;
-  static const int nr_env = [] { const char* e = getenv("VI_EMBED_NR"); return e ? atoi(e) : 0; }();      // 2: the two-rows-per-warp variant
-  const int nr = nr_env == 2 ? 2 : 1;
-  const long long blocks = (p.rows + p.zero_rows + EMBED_WARPS * nr - 1) / (EMBED_WARPS * nr);
-  if (nr == 2)
-    VI_CUDA(vi_launch(embed_compose_kernel<2>, dim3((unsigned)blocks), dim3(EMBED_WARPS * 32), (size_t)0, ST(stream), p));
-  else
-    VI_CUDA(vi_launch(embed_compose_kernel<1>, dim3((unsigned)blocks), dim3(EMBED_WARPS * 32), (size_t)0, ST(stream), p));
+  const long long blocks = (p.rows + p.zero_rows + EMBED_WARPS - 1) / EMBED_WARPS;
+  VI_CUDA(vi_launch(embed_compose_kernel, dim3((unsigned)blocks), dim3(EMBED_WARPS * 32), (size_t)0, ST(stream), p));
   VI_LAUNCH_CHECK();
   return VI_OK;
 }
@@ -856,10 +777,6 @@ extern "C" int vi_copy_rows(const float* src, int64_t src_batch_stride, int64_t 
                                                           dst_row_stride, rows, rows_per_batch));
   VI_LAUNCH_CHECK();
   return VI_OK;
-}
-
-extern "C" int vi_cast_bf16(const float* src, void* dst, int64_t n, vi_stream_t stream) {
-  return vi_cast_h16(src, dst, VI_DT_BF16, n, stream);
 }
 
 extern "C" int vi_cast_h16(const float* src, void* dst, int dst_dtype, int64_t n, vi_stream_t stream) {

@@ -562,12 +562,8 @@ int launch_wgrad_pair(const WgradMaps& m, const WgradParams& p, int pairs, cudaS
   return VI_OK;
 }
 
-// the CTA-pair form serves shapes whose N is a multiple of 256 and whose K is a multiple of 128 (VI_WGRAD_PAIR=0: never)
-bool wgrad_pair_ok(int N, int K) {
-  const char* e = getenv("VI_WGRAD_PAIR");
-  if (e && e[0] == '0') return false;
-  return N % 256 == 0 && K % 128 == 0;
-}
+// the CTA-pair form serves shapes whose N is a multiple of 256 and whose K is a multiple of 128
+bool wgrad_pair_ok(int N, int K) { return N % 256 == 0 && K % 128 == 0; }
 
 }  // namespace
 

@@ -172,14 +172,14 @@ def align_forward(model, align_txt_embeds, align_imagine_embeds, flags, noun_phr
         negs = None
         if rows.n_negs:
             negs, _ = ops.gather_mean(txt, rows.np_off, rows.np_rows, rows.n_negs, want16=False)
-        loss = ops.infonce_loss(proj, tgt, negs, rows.ep, rows.np_ep if rows.n_negs else None,
-                                float(cfg.infonce_temperature), rows.R, rows.n_negs, dev)
+        loss, _ = ops.infonce_loss(proj, tgt, negs, rows.ep, rows.np_ep if rows.n_negs else None,
+                                   float(cfg.infonce_temperature), rows.R, rows.n_negs, dev)
     elif cfg.aux_loss_type == 'constrastive-margin':          # (sic) H/r2r/parser.py:117, H/models/vilmodel_cmt.py:825-856
         negs = None
         if rows.n_negs:
             negs, _ = ops.gather_mean(txt, rows.np_off, rows.np_rows, rows.n_negs, want16=False)
-        loss = ops.margin_loss(proj, tgt, negs, rows.ep, rows.np_ep if rows.n_negs else None,
-                               float(cfg.contrastive_margin_value), rows.R, rows.n_negs, dev)
+        loss, _ = ops.margin_loss(proj, tgt, negs, rows.ep, rows.np_ep if rows.n_negs else None,
+                                  float(cfg.contrastive_margin_value), rows.R, rows.n_negs, dev)
     else:
         raise NotImplementedError('aux_loss_type %r' % cfg.aux_loss_type)
     ops.scatter_rows(proj, rows.slot, out)
@@ -395,7 +395,7 @@ class GlocalTextPathNavCMT(nn.Module):
         km = blocks.mask_u8(pano_masks)
         with blocks.grad_mode(self._recording(view_img_fts) and not self.config.fix_pano_embedding, self._drop()):
             a = blocks.linear(blocks.operand(v32, lowp), pk['img_linear'], lowp, out_dtype=F32)
-            folded = lowp and blocks.fold_enabled() and not blocks.training() and len(pk['pano']) > 0
+            folded = lowp and not blocks.training() and len(pk['pano']) > 0
             x = blocks.embed(B * V, dev, a=a, a_ln=ie.img_layer_norm, feat=_f32c(loc_fts).view(B * V, -1),
                              feat_lin=ie.loc_linear, feat_ln=ie.loc_layer_norm,
                              idx=nav_types.long().contiguous().view(-1), table=ie.nav_type_embedding.weight,
@@ -876,7 +876,7 @@ class VLNBert(nn.Module):
                 dev = m.embeddings.LayerNorm.weight.device
                 tok = graphs.weights_token(m, self._wt_cache)
                 out = self._g_pano({k: batch[k] for k in ('view_img_fts', 'loc_fts', 'nav_types', 'view_lens')}, dev,
-                                   extra_key=(m.precision, ops.h16(), blocks.fold_enabled()), weights_token=tok)
+                                   extra_key=(m.precision, ops.h16()), weights_token=tok)
                 return out['pano_embeds'], out['pano_masks']
             return m(mode, batch)
         if mode == 'navigation':
@@ -900,7 +900,7 @@ class VLNBert(nn.Module):
                 # The graph stops before the global / local fusion: the ~1700 viewpoint-id strings of a batch are
                 # interned on the host AFTER the encoder has been queued (the GPU would otherwise idle for that long),
                 # then the one fusion kernel is launched eagerly on the graph's outputs.
-                pre = self._g_nav(t, dev, extra_key=(m.precision, ops.h16(), blocks.fold_enabled(), cfg.imagine_enc_pano, cfg.concat_imagine_with if
+                pre = self._g_nav(t, dev, extra_key=(m.precision, ops.h16(), cfg.imagine_enc_pano, cfg.concat_imagine_with if
                                                      cfg.imagine_enc_pano else None), weights_token=tok,
                                   borrowed={'ctx_kv%d' % i: x for i, x in enumerate(kv)}, no_clone_prefix='_')
                 out = m.fuse_logits(pre, batch['gmap_vpids'], batch['vp_cand_vpids'], Gb, Pb)

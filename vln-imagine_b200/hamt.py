@@ -593,7 +593,7 @@ class VLNBertCMT(nn.Module):
                            hist_pano_img_feats=hist_pano_img_feats, hist_pano_ang_feats=hist_pano_ang_feats)
                 t = {k: loc[k] for k in self.HIST_TENSORS if loc[k] is not None}
                 t['ob_step_ids'] = torch.full((hist_img_feats.shape[0],), int(ob_step), dtype=torch.int64)
-                return self._g_hist(t, dev, extra_key=(m.precision, ops.h16(), blocks.fold_enabled()), weights_token=graphs.weights_token(m, self._wt_cache))['hist']
+                return self._g_hist(t, dev, extra_key=(m.precision, ops.h16()), weights_token=graphs.weights_token(m, self._wt_cache))['hist']
             return m('history', hist_img_feats=self._env_dropout(hist_img_feats), hist_ang_feats=hist_ang_feats,
                      ob_step_ids=ob_step, hist_pano_img_feats=self._env_dropout(hist_pano_img_feats),
                      hist_pano_ang_feats=hist_pano_ang_feats)
@@ -616,7 +616,7 @@ class VLNBertCMT(nn.Module):
                     dims = {'hist_embeds': {1: Tb}, 'hist_masks': {1: Tb}, 'ob_img_feats': {1: Ob}, 'ob_ang_feats': {1: Ob},
                             'ob_nav_types': {1: Ob}, 'ob_masks': {1: Ob}}
                     t = {k: (graphs.pad_to(v, dims[k], dev) if k in dims else v) for k, v in t.items()}
-                out = self._g_vis(t, dev, extra_key=(m.precision, ops.h16(), blocks.fold_enabled(), m.config.imagine_enc_pano),
+                out = self._g_vis(t, dev, extra_key=(m.precision, ops.h16(), m.config.imagine_enc_pano),
                                   weights_token=graphs.weights_token(m, self._wt_cache))
                 logits = out['act_logits'][:, :O]
                 return (logits, out['states']) if return_states else (logits,)

@@ -149,7 +149,7 @@ def autotune_enabled() -> bool:
     """Timing tile candidates on first use is OFF by default: shapes missing from tile_table.json use the library's cost
     model, so results and timings are reproducible from process to process and a rollout never stalls on a tuning pass.
     tools/tune_tiles.py (VLN_IMAGINE_AUTOTUNE=1) measures new shapes and rewrites the table."""
-    return os.environ.get('VLN_IMAGINE_AUTOTUNE', '0') == '1' and not os.environ.get('VI_GEMM_TILE')
+    return os.environ.get('VLN_IMAGINE_AUTOTUNE', '0') == '1'
 
 
 def _table_tile(key) -> int:
@@ -199,12 +199,13 @@ def gemm(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None,
          residual: Optional[torch.Tensor] = None, epilogue: int = EPI_NONE,
          out_dtype: Optional[torch.dtype] = None, group_row_end: Optional[Sequence[int]] = None,
          out: Optional[torch.Tensor] = None, out16: Optional[torch.Tensor] = None, ln=None,
-         stats_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+         stats_out: Optional[torch.Tensor] = None, tile: Optional[int] = None) -> torch.Tensor:
     """Y = epi(X W^T + bias) + residual.  x bf16 / fp16 -> tcgen05 kernel (vi_gemm16); x fp32 -> fp32 check-mode kernel.
     w is [n_groups*N, K]; group_row_end (python ints) splits the rows of x between the weight blocks.
     out16: a 16-bit tensor that receives a copy of an fp32 output.  ln = (mode, vec_a, stats, eps): LayerNorm folded into
     this contraction (_lib.LN_FOLD / LN_RESIDUAL, see include/vlnimagine.h); stats_out: float32 [N/32, M, 2] that receives
-    the per-chunk row statistics of the output."""
+    the per-chunk row statistics of the output.  tile: the output-tile shape (width | TILE_PAIR, 0 = the library's cost model)
+    instead of the measured table / autotuner; a shape the problem does not admit raises."""
     M, K, ldx = _rows2d(x, 'x')
     n_groups = 1 if group_row_end is None else len(group_row_end)
     if w.dim() != 2 or not w.is_contiguous() or w.shape[1] != K or w.shape[0] % n_groups:
@@ -244,9 +245,7 @@ def gemm(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None,
         def launch(tile):
             a.tile = tile
             check(lib.vi_gemm16(a, _stream()), 'vi_gemm16')
-        if os.environ.get('VI_GEMM_TILE'):
-            tile = 0
-        else:
+        if tile is None:
             pair_ok = ge is None or all(e % 256 == 0 for e in ge[:-1])
             tile = _tune_tile(key, launch, N, pair_ok)
         tr = _Counters.gemm_trace
@@ -277,24 +276,17 @@ def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, B: int, Lq: int
               key_mask: Optional[torch.Tensor] = None, pair_dist: Optional[torch.Tensor] = None,
               bias_affine: Optional[torch.Tensor] = None, mask_mode: int = MASK_ADD_NEG10000,
               out: Optional[torch.Tensor] = None, lse: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """q [B*Lq, >=768 view], k/v [B*Lk, view] -> o [B*Lq, 768]; 12 heads of 64."""
-    _, _, ldq = _rows2d(q, 'q')
-    _, _, ldk = _rows2d(k, 'k')
-    _, _, ldv = _rows2d(v, 'v')
+    """q [B*Lq, >=768 view], k/v [B*Lk, view] -> o [B*Lq, 768]; 12 heads of 64.  One problem of attention_multi."""
     if out is None:
         out = torch.empty((B * Lq, HIDDEN), dtype=q.dtype, device=q.device)
-    if key_mask is not None and (key_mask.dtype != torch.uint8 or not key_mask.is_contiguous()):
-        raise _lib.VlnImagineError('key_mask must be a contiguous uint8 tensor')
-    check(lib.vi_attn_fwd(q.data_ptr(), ldq, k.data_ptr(), ldk, v.data_ptr(), ldv, out.data_ptr(), out.stride(0),
-                          _DT[q.dtype], _ptr(key_mask), _ptr(pair_dist),
-                          _ptr(bias_affine), _ptr(lse), B, HEADS, Lq, Lk, mask_mode, _stream()), 'vi_attn_fwd')
-    _launched(1)
+    attention_multi([dict(q=q, k=k, v=v, out=out, B=B, Lq=Lq, Lk=Lk, key_mask=key_mask, pair_dist=pair_dist,
+                          bias_affine=bias_affine, lse=lse)], mask_mode)
     return out
 
 
-def attention_multi(problems, mask_mode: int = MASK_ADD_NEG10000, kernel: str = 'auto'):
+def attention_multi(problems, mask_mode: int = MASK_ADD_NEG10000):
     """Several attention problems in one launch.  Each problem is a dict with q, k, v (2-D row views), out,
-    B, Lq, Lk and optional key_mask (uint8 [B, Lk]), pair_dist, bias_affine, lse.  kernel='tc': the tcgen05 kernel by name."""
+    B, Lq, Lk and optional key_mask (uint8 [B, Lk]), pair_dist, bias_affine, lse."""
     n = len(problems)
     arr = (_lib.AttnProblem * n)()
     dtype = None
@@ -316,10 +308,7 @@ def attention_multi(problems, mask_mode: int = MASK_ADD_NEG10000, kernel: str = 
             dtype = q.dtype
         elif dtype != q.dtype:
             raise _lib.VlnImagineError('attention problems of one launch must share a dtype')
-    if kernel == 'tc':
-        check(lib.vi_attn_fwd_tc(arr, n, HEADS, _DT[dtype], mask_mode, _stream()), 'vi_attn_fwd_tc')
-    else:
-        check(lib.vi_attn_fwd_multi(arr, n, HEADS, _DT[dtype], mask_mode, _stream()), 'vi_attn_fwd_multi')
+    check(lib.vi_attn_fwd_multi(arr, n, HEADS, _DT[dtype], mask_mode, _stream()), 'vi_attn_fwd_multi')
     _launched(1 if is16(dtype) else n)
 
 
@@ -454,26 +443,8 @@ def cosine_loss(proj: Optional[torch.Tensor], tgt: Optional[torch.Tensor], R: in
 
 
 def infonce_loss(proj, tgt, negs, row_episode, neg_episode, temperature: float, R: int, n_negs: int, device):
-    loss = torch.empty((), dtype=F32, device=device)
-    scratch = torch.empty((max(R, 1) * (n_negs + 2),), dtype=F32, device=device)
-    check(lib.vi_infonce_loss(_ptr(proj), _ptr(tgt), _ptr(negs), _ptr(row_episode), _ptr(neg_episode), temperature,
-                              scratch.data_ptr(), loss.data_ptr(), R, n_negs, _stream()), 'vi_infonce_loss')
-    _launched(3)
-    return loss
-
-
-def margin_loss(proj, tgt, negs, row_episode, neg_episode, margin: float, R: int, n_negs: int, device):
-    loss = torch.empty((), dtype=F32, device=device)
-    scratch = torch.empty((max(R, 1) * (n_negs + 2),), dtype=F32, device=device)
-    check(lib.vi_margin_loss(_ptr(proj), _ptr(tgt), _ptr(negs), _ptr(row_episode), _ptr(neg_episode), margin,
-                             scratch.data_ptr(), loss.data_ptr(), R, n_negs, _stream()), 'vi_margin_loss')
-    _launched(3)
-    return loss
-
-
-def infonce_loss_with_sims(proj, tgt, negs, row_episode, neg_episode, temperature: float, R: int, n_negs: int, device):
-    """infonce_loss that also hands back the forward scratch (its first R * (n_negs + 1) floats are the scaled
-    similarities the backward pass needs)."""
+    """(loss, scratch): the forward scratch's first R * (n_negs + 1) floats are the scaled similarities the backward
+    pass needs"""
     loss = torch.empty((), dtype=F32, device=device)
     scratch = torch.empty((max(R, 1) * (n_negs + 2),), dtype=F32, device=device)
     check(lib.vi_infonce_loss(_ptr(proj), _ptr(tgt), _ptr(negs), _ptr(row_episode), _ptr(neg_episode), temperature,
@@ -482,8 +453,8 @@ def infonce_loss_with_sims(proj, tgt, negs, row_episode, neg_episode, temperatur
     return loss, scratch
 
 
-def margin_loss_with_sims(proj, tgt, negs, row_episode, neg_episode, margin: float, R: int, n_negs: int, device):
-    """margin_loss that also hands back the forward scratch (its first R * (n_negs + 1) floats are the cosines)."""
+def margin_loss(proj, tgt, negs, row_episode, neg_episode, margin: float, R: int, n_negs: int, device):
+    """(loss, scratch): the forward scratch's first R * (n_negs + 1) floats are the cosines the backward pass needs"""
     loss = torch.empty((), dtype=F32, device=device)
     scratch = torch.empty((max(R, 1) * (n_negs + 2),), dtype=F32, device=device)
     check(lib.vi_margin_loss(_ptr(proj), _ptr(tgt), _ptr(negs), _ptr(row_episode), _ptr(neg_episode), margin,
@@ -498,11 +469,6 @@ def copy_rows(src: torch.Tensor, src_bs: int, src_rs: int, n_batches: int, rows_
     check(lib.vi_copy_rows(src.data_ptr(), src_bs, src_rs, _ptr(dst32), _ptr(dst16), _dt16(dst16), dst_bs, dst_rs, n_batches,
                            rows_per_batch, _stream()), 'vi_copy_rows')
     _launched(1)
-
-
-def cast_bf16(src: torch.Tensor, dst: Optional[torch.Tensor] = None):
-    """fp32 -> bf16 (the training path and weight shadows of it)"""
-    return cast_h16(src, dst, BF16)
 
 
 def cast_h16(src: torch.Tensor, dst: Optional[torch.Tensor] = None, dtype=None):

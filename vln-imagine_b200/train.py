@@ -221,13 +221,8 @@ class GraphedIteration:
         from . import autograd_ops
         self._keepalive = list(autograd_ops._GradAcc.buffers.values())    # the graphs hold raw pointers to these accumulators
         self.g_update = torch.cuda.CUDAGraph()
-        import os
-        if os.environ.get('VI_TRAIN_SHARED_POOL', '0') == '1':
-            with graphs.capture(self.g_update, pool=self.g_grad.pool()):
-                update_fn()
-        else:
-            with graphs.capture(self.g_update):
-                update_fn()
+        with graphs.capture(self.g_update):
+            update_fn()
 
     def _invalidate_packs(self):
         for m in self.model.modules():
