@@ -256,6 +256,17 @@ int vi_margin_loss(const float* proj, const float* tgt, const float* negs, const
 int vi_ce_rows(const float* logits, int64_t ld, const int64_t* labels, int n_cols, float* out, int64_t rows, vi_stream_t stream);
 int vi_kl_rows(const float* logits, int64_t ld, const float* targets, int64_t ldt, int n_cols, float* out, int64_t rows,
                vi_stream_t stream);
+/* Backward of vi_ce_rows / vi_kl_rows (what torch autograd gives for the two losses above), vi_xent.cu:
+ *   dx[r, c] = dloss[r] * (softmax(logits[r, 0:n_cols])[c] * T[r] - t[r, c])   for c < n_cols
+ *   cross-entropy: t = one-hot(labels[r]), T = 1;  KL: t = targets[r], T = sum_c targets[r, c].
+ * dloss: device fp32 [rows], the incoming gradient of each row's loss.  Output rows of ld_out >= n_cols elements as fp32 (dx32)
+ * and / or 16-bit (dx16, dx16_dtype VI_DT_BF16 / VI_DT_F16: the operand of the gradient GEMMs); columns n_cols <= c < ld_out are
+ * written as exact zeros.  A -inf logit has softmax 0.  rows == 0 is a no-op.  Rows of >= 256 columns with ld % 4 == 0,
+ * ld_out % 8 == 0 and 16-byte aligned pointers take a CTA per row (16-byte loads and stores); others a warp per row. */
+int vi_ce_rows_bwd(const float* logits, int64_t ld, const int64_t* labels, int n_cols, const float* dloss, float* dx32, void* dx16,
+                   int dx16_dtype, int64_t ld_out, int64_t rows, vi_stream_t stream);
+int vi_kl_rows_bwd(const float* logits, int64_t ld, const float* targets, int64_t ldt, int n_cols, const float* dloss, float* dx32,
+                   void* dx16, int dx16_dtype, int64_t ld_out, int64_t rows, vi_stream_t stream);
 /* dst[b, r, 0:768] = src[b, r, 0:768] for n_batches x rows_per_batch rows; strides in ELEMENTS.  Writes an
  * fp32 and/or a 16-bit copy.  Builds the cross-attention context cat([txt_embeds, imagine_embeds], 1)
  * (D/models/vilmodel.py:1157, H/models/vilmodel_cmt.py:1110) and gathers the token-0 rows that feed

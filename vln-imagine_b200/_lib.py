@@ -74,6 +74,8 @@ PROTOTYPES = {
     'vi_margin_loss': [_p, _p, _p, _p, _p, _f, _p, _p, _i, _i, _p],
     'vi_ce_rows': [_p, _l, _p, _i, _p, _l, _p],
     'vi_kl_rows': [_p, _l, _p, _l, _i, _p, _l, _p],
+    'vi_ce_rows_bwd': [_p, _l, _p, _i, _p, _p, _p, _i, _l, _l, _p],
+    'vi_kl_rows_bwd': [_p, _l, _p, _l, _i, _p, _p, _p, _i, _l, _l, _p],
     'vi_copy_rows': [_p, _l, _l, _p, _p, _i, _l, _l, _l, _i, _p],
     'vi_cast_h16': [_p, _p, _i, _l, _p],
     'vi_transpose': [_p, _l, _p, _l, _i, _i, _i, _i, _p],

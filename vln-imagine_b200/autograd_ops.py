@@ -290,37 +290,109 @@ class LinearFn(Function):
     @staticmethod
     def backward(ctx, dy):
         (x,) = ctx.saved_tensors
-        pack, lowp, ends = ctx.pack, ctx.lowp, ctx.ends
-        dyo = to_operand(dy, lowp)
-        M, K = x.shape
-        n_groups = 1 if ends is None else len(ends)
-        N = dyo.shape[1]
-        dx = None
-        if ctx.needs_input_grad[0]:
-            wt = pack.get_t(lowp, n_groups)                             # [n_groups*K, N]
-            dx = ops.gemm(dyo, wt, None, out_dtype=x.dtype, group_row_end=ends)
-        if lowp and wgrad16_ok(dyo, x):
-            grads = _lin_param_grads(pack, dyo, x, ends)
-        else:                                                           # fp32 check mode / odd shapes: transposed copies
-            dW = torch.empty((n_groups * N, K), dtype=F32, device=x.device)
-            db = torch.empty((n_groups * N,), dtype=F32, device=x.device) if pack.biases is not None else None
-            bounds = [0] + (list(ends) if ends is not None else [M])
-            for g in range(n_groups):
-                r0, r1 = bounds[g], min(bounds[g + 1], M)
-                rp = pad64(r1 - r0) if lowp else r1 - r0
-                dyT = transpose(dyo[r0:r1], rp)                             # [N, rp]
-                xT = transpose(x[r0:r1], rp)                                # [K, rp]
-                ops.gemm(dyT, xT, None, out_dtype=F32, out=dW[g * N:(g + 1) * N])
-                if db is not None:
-                    db[g * N:(g + 1) * N] = colsum(dyo[r0:r1])
-            grads = _lin_grads(pack, dW, db)
+        dx, grads = _linear_bwd(ctx.pack, x, to_operand(dy, ctx.lowp), ctx.lowp, ctx.ends, ctx.needs_input_grad[0])
         return (dx, dy if ctx.has_res else None, None, None, None, None, *grads)
+
+
+def _linear_bwd(pack, x, dyo, lowp, ends, need_dx):
+    """(dX, parameter gradients in grad_sources() order) of y = x W^T + b from dY in the operand format of the precision mode.
+    ``pack`` provides get_t / weights / biases; its stacked weight may be padded with zero rows past the parameters (the
+    gradients handed back are the parameters' rows)."""
+    M, K = x.shape
+    n_groups = 1 if ends is None else len(ends)
+    N = dyo.shape[1]
+    dx = None
+    if need_dx:
+        wt = pack.get_t(lowp, n_groups)                             # [n_groups*K, N]
+        dx = ops.gemm(dyo, wt, None, out_dtype=x.dtype, group_row_end=ends)
+    if lowp and wgrad16_ok(dyo, x):
+        return dx, _lin_param_grads(pack, dyo, x, ends)
+    dW = torch.empty((n_groups * N, K), dtype=F32, device=x.device)   # fp32 check mode / odd shapes: transposed copies
+    db = torch.empty((n_groups * N,), dtype=F32, device=x.device) if pack.biases is not None else None
+    bounds = [0] + (list(ends) if ends is not None else [M])
+    for g in range(n_groups):
+        r0, r1 = bounds[g], min(bounds[g + 1], M)
+        rp = pad64(r1 - r0) if lowp else r1 - r0
+        dyT = transpose(dyo[r0:r1], rp)                             # [N, rp]
+        xT = transpose(x[r0:r1], rp)                                # [K, rp]
+        ops.gemm(dyT, xT, None, out_dtype=F32, out=dW[g * N:(g + 1) * N])
+        if db is not None:
+            db[g * N:(g + 1) * N] = colsum(dyo[r0:r1])
+    return dx, _lin_grads(pack, dW, db)
 
 
 def linear(x, pack, lowp, residual=None, out_dtype=None, ends=None):
     """differentiable dense layer (no fused activation); pack = blocks.LinearPack"""
     out_dtype = out_dtype or (BF16 if lowp else F32)
     return LinearFn.apply(x, residual, pack, lowp, out_dtype, ends, *pack.grad_sources())
+
+
+class PaddedLinearFn(Function):
+    """scores = x W^T + b of a dense layer whose output width is padded with zero weight rows (pretrain._PaddedLinear: the tied
+    MLM decoder 30522 -> 30592, the MRC classifier 1000 -> 1024; multiples of 128, the column granule of vi_wgrad16).
+    Returns (scores fp32 [M, n_pad], handle).  ``handle`` (an [M, n_pad] view of one element, in the operand format of the
+    precision mode) is where the loss node (CERowsFn / KLRowsFn) sends d scores, so the gradient reaches this node as the
+    16-bit GEMM operand its loss kernel wrote, with no cast pass.  A gradient of the fp32 scores themselves (another loss)
+    is cast to the operand format and added.  Backward: dX through the transposed shadow
+    of the padded weight, dW (first n rows: for the tied decoder autograd adds them to the embedding lookup's scatter-add)
+    and db through vi_wgrad16 (the fp32 check mode: transposed copies)."""
+
+    @staticmethod
+    def forward(ctx, x, pack, lowp, *params):
+        w, b = pack.get_train(lowp)
+        y = ops.gemm(x, w, b, out_dtype=F32)
+        ctx.save_for_backward(x)
+        ctx.pack, ctx.lowp = pack, lowp
+        ctx.set_materialize_grads(False)
+        handle = torch.zeros((), dtype=BF16 if lowp else F32, device=x.device).expand(y.shape)
+        return y, handle
+
+    @staticmethod
+    def backward(ctx, dy, dh):
+        (x,) = ctx.saved_tensors
+        g = dh.contiguous() if dh is not None else None
+        if dy is not None:
+            g = to_operand(dy, ctx.lowp) if g is None else g + to_operand(dy, ctx.lowp)
+        dx, grads = _linear_bwd(ctx.pack, x, g, ctx.lowp, None, ctx.needs_input_grad[0])
+        return (dx, None, None, *grads)
+
+
+def padded_linear(x, pack, lowp):
+    """differentiable padded dense layer -> (scores, gradient handle); see PaddedLinearFn"""
+    return PaddedLinearFn.apply(x, pack, lowp, *pack.grad_sources())
+
+
+class CERowsFn(Function):
+    """per-row cross-entropy (ops.ce_rows) over the first n_cols columns of fp32 ``logits``; the gradient w.r.t. the logits is
+    written by vi_ce_rows_bwd in the dtype of ``handle`` (bf16: the operand of the gradient GEMMs; fp32 in the check mode) and
+    returned for ``handle``, which is the logits tensor itself or PaddedLinearFn's handle."""
+
+    @staticmethod
+    def forward(ctx, logits, handle, labels, n_cols):
+        ctx.save_for_backward(logits, labels)
+        ctx.n_cols, ctx.dtype, ctx.ld_out = n_cols, handle.dtype, handle.shape[1]
+        return ops.ce_rows(logits, labels, n_cols)
+
+    @staticmethod
+    def backward(ctx, dloss):
+        logits, labels = ctx.saved_tensors
+        return None, ops.ce_rows_bwd(logits, labels, ctx.n_cols, dloss, ctx.dtype, ctx.ld_out), None, None
+
+
+class KLRowsFn(Function):
+    """per-row KL(targets || softmax(logits)) (ops.kl_rows); gradient as in CERowsFn (vi_kl_rows_bwd), none for the targets"""
+
+    @staticmethod
+    def forward(ctx, logits, handle, targets, n_cols):
+        targets = targets.contiguous()
+        ctx.save_for_backward(logits, targets)
+        ctx.n_cols, ctx.dtype, ctx.ld_out = n_cols, handle.dtype, handle.shape[1]
+        return ops.kl_rows(logits, targets, n_cols)
+
+    @staticmethod
+    def backward(ctx, dloss):
+        logits, targets = ctx.saved_tensors
+        return None, ops.kl_rows_bwd(logits, targets, ctx.n_cols, dloss, ctx.dtype, ctx.ld_out), None, None
 
 
 class ActFn(Function):

@@ -73,7 +73,7 @@ int vi_make_tmap_h16(CUtensorMap* map, const void* ptr, int f16, uint64_t cols, 
   return VI_OK;
 }
 
-extern "C" int vi_version(void) { return 101; }   // 0.1.1
+extern "C" int vi_version(void) { return 102; }   // 0.1.2
 
 extern "C" const char* vi_last_error(void) { return g_err; }
 

@@ -498,3 +498,35 @@ def kl_rows(logits: torch.Tensor, targets: torch.Tensor, n_cols: int) -> torch.T
     check(lib.vi_kl_rows(logits.data_ptr(), ld, targets.data_ptr(), ldt, n_cols, out.data_ptr(), R, _stream()), 'vi_kl_rows')
     _launched(1)
     return out
+
+
+def _xent_out(R: int, ld_out: int, dtype, device):
+    out = torch.empty((R, ld_out), dtype=dtype, device=device)
+    return (out, None) if dtype == F32 else (None, out)
+
+
+def ce_rows_bwd(logits: torch.Tensor, labels: torch.Tensor, n_cols: int, dloss: torch.Tensor, dtype=F32,
+                ld_out: Optional[int] = None) -> torch.Tensor:
+    """gradient of ce_rows w.r.t. the logits: dloss[r] * (softmax(logits[r, :n_cols]) - one_hot(labels[r])) as [R, ld_out] rows of
+    ``dtype`` (fp32, or the 16-bit operand of the gradient GEMMs); columns n_cols .. ld_out - 1 (default: the logits' width) are 0"""
+    R, W, ld = _rows2d(logits, 'logits')
+    d32, d16 = _xent_out(R, ld_out or W, dtype, logits.device)
+    dloss = dloss.float().contiguous()
+    check(lib.vi_ce_rows_bwd(logits.data_ptr(), ld, labels.long().contiguous().data_ptr(), n_cols, dloss.data_ptr(), _ptr(d32), _ptr(d16),
+                             _DT[d16.dtype] if d16 is not None else _lib.DT_BF16, ld_out or W, R, _stream()), 'vi_ce_rows_bwd')
+    _launched(1)
+    return d32 if d32 is not None else d16
+
+
+def kl_rows_bwd(logits: torch.Tensor, targets: torch.Tensor, n_cols: int, dloss: torch.Tensor, dtype=F32,
+                ld_out: Optional[int] = None) -> torch.Tensor:
+    """gradient of kl_rows w.r.t. the logits: dloss[r] * (softmax(logits[r, :n_cols]) * sum(targets[r]) - targets[r]), laid out as
+    in ce_rows_bwd"""
+    R, W, ld = _rows2d(logits, 'logits')
+    _, _, ldt = _rows2d(targets, 'targets')
+    d32, d16 = _xent_out(R, ld_out or W, dtype, logits.device)
+    dloss = dloss.float().contiguous()
+    check(lib.vi_kl_rows_bwd(logits.data_ptr(), ld, targets.data_ptr(), ldt, n_cols, dloss.data_ptr(), _ptr(d32), _ptr(d16),
+                             _DT[d16.dtype] if d16 is not None else _lib.DT_BF16, ld_out or W, R, _stream()), 'vi_kl_rows_bwd')
+    _launched(1)
+    return d32 if d32 is not None else d16

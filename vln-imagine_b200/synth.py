@@ -483,3 +483,20 @@ def duet_pretrain_batch(seed: int = 5, batch: int = 3, n_vp: int = 20, max_steps
                 gmap_lens=gmap_lens, gmap_step_ids=gmap_step_ids, gmap_pos_fts=gmap_pos_fts, gmap_pair_dists=pd,
                 gmap_vpids=gmap_vpids, vp_pos_fts=vp_pos_fts, gmap_visited_masks=gmap_visited_masks,
                 vp_view_mrc_masks=vp_view_mrc_masks, vp_view_probs=vp_view_probs)
+
+
+def duet_pretrain_sap_labels(batch: dict) -> dict:
+    """``global_act_labels`` / ``local_act_labels`` of the sap collate function (data/tasks.py) for a duet_pretrain_batch: the
+    last admissible graph node (valid, unvisited) and the last navigable candidate of the last panorama ([stop] = 0 when there
+    is none), so both targets have finite logits.  Returns the batch with the two labels added."""
+    B = len(batch['traj_step_lens'])
+    last = np.cumsum(np.asarray(batch['traj_step_lens'])) - 1
+    nav = np.asarray(batch['traj_nav_types'])[last]
+    visited = np.asarray(batch['gmap_visited_masks'])
+    gl, ll = np.zeros(B, np.int64), np.zeros(B, np.int64)
+    for b in range(B):
+        ok = [g for g in range(1, int(batch['gmap_lens'][b])) if not visited[b, g]]
+        gl[b] = ok[-1] if ok else 0
+        cand = [j + 1 for j in range(len(batch['traj_cand_vpids'][b][-1])) if nav[b, j] == 1]
+        ll[b] = cand[-1] if cand else 0
+    return dict(batch, global_act_labels=gl, local_act_labels=ll)
