@@ -5,7 +5,6 @@ duet_oracle.py (the blocks are the same classes as in map_nav_src): whole trajec
 features are aggregated from them (``_aggregate_gmap_features``), and the three proxy tasks of the R2R recipe
 (config/r2r_pretrain.json: mlm, mrc, sap) put their heads on top.  Paths below are relative to VLN-DUET/pretrain_src/.
 Pinned to the real reference by ``oracle/gen_golden.py --model duet_pretrain`` (tests/golden/duet_pretrain.npz).
-Groundwork: the product side of this row is not built yet.
 """
 from __future__ import annotations
 

@@ -556,32 +556,89 @@ class CrossPack:
         self.ln = LNPack([x.output.LayerNorm for x in xatts])
 
 
-def cross_attn(x: Act, kv: torch.Tensor, kv_col0: Sequence[int], ctx_len: int, ctx_mask, pk: CrossPack,
-               streams: List[Stream], ends, lowp: bool, eps=1e-12, defer=False) -> Act:
-    """LN(x + O(attn(Q(x), K(ctx), V(ctx)))).  kv holds the projected context [B*ctx_len, *] with this
-    stream's K at columns kv_col0[i] and V at kv_col0[i]+768.
+def cross_attn(x: Act, ctxs, pk: CrossPack, streams: List[Stream], ends, lowp: bool, eps=1e-12, defer=False) -> Act:
+    """LN(x + O(attn(Q(x), K(ctx), V(ctx)))).  ctxs[i] = (kv, col0, ctx_len, key_mask) is the context of streams[i]: the
+    projected context [B*ctx_len, *] with its K at columns col0 and V at col0+768.  Streams may share one kv tensor.
     Reference: BertXAttention, VLN-DUET/map_nav_src/models/vilmodel.py:302-364."""
     rows = x.f32.shape[0]
     if _Mode.train:
         xin = x.operand(lowp)
         q = ag.linear(xin, pk.q, lowp, ends=ends)
-        spec = [dict(q=(0, s.row0, 0), k=(1, 0, c0), v=(1, 0, c0 + HIDDEN), B=s.B, Lq=s.L, Lk=ctx_len, key_mask=ctx_mask,
-                     out_row0=s.row0, drop=_attn_drop(xin.device)) for s, c0 in zip(streams, kv_col0)]
-        ctx = ag.AttentionFn.apply(spec, rows, MASK_ADD_NEG10000, 2, q, kv)
+        kvs, spec = [], []
+        for s, (kv, c0, n, m) in zip(streams, ctxs):
+            if not any(kv is t for t in kvs):
+                kvs.append(kv)
+            bi = 1 + next(i for i, t in enumerate(kvs) if t is kv)
+            spec.append(dict(q=(0, s.row0, 0), k=(bi, 0, c0), v=(bi, 0, c0 + HIDDEN), B=s.B, Lq=s.L, Lk=n, key_mask=m,
+                             out_row0=s.row0, drop=_attn_drop(xin.device)))
+        ctx = ag.AttentionFn.apply(spec, rows, MASK_ADD_NEG10000, 1 + len(kvs), q, *kvs)
         return _dense_res_ln(ctx, pk.o, x.f32, pk.ln, eps, lowp, ends)
     q = gemm_act(x, pk.q, lowp, ends)
     ctx = _ctx_buffer(rows, q, streams)
     ops.attention_multi([dict(q=s.view(q), k=kv[:, c0:c0 + HIDDEN], v=kv[:, c0 + HIDDEN:c0 + 2 * HIDDEN], out=s.view(ctx),
-                              B=s.B, Lq=s.L, Lk=ctx_len, key_mask=ctx_mask) for s, c0 in zip(streams, kv_col0)])
+                              B=s.B, Lq=s.L, Lk=n, key_mask=m) for s, (kv, c0, n, m) in zip(streams, ctxs)])
     return linear_residual_ln(ctx, pk.o, x, pk.ln, eps, lowp, ends, defer=defer)
 
 
-def linear(x: torch.Tensor, pk: LinearPack, lowp: bool, out_dtype=None, ends=None, residual=None) -> torch.Tensor:
-    """y = x W^T + b [+ residual] for a LinearPack (no activation); differentiable in training."""
+def linear(x: torch.Tensor, pk: LinearPack, lowp: bool, out_dtype=None, ends=None, residual=None, epilogue=EPI_NONE) -> torch.Tensor:
+    """y = epi(x W^T + b) [+ residual] for a LinearPack; differentiable in training (the activation as its own node)."""
     if _Mode.train:
-        return ag.linear(x, pk, lowp, residual=residual, out_dtype=out_dtype, ends=ends)
+        y = ag.linear(x, pk, lowp, residual=residual, out_dtype=out_dtype, ends=ends)
+        return ag.ActFn.apply(y, epilogue) if epilogue != EPI_NONE else y
     w, b = pk.get(lowp)
-    return ops.gemm(x, w, b, residual=residual, out_dtype=out_dtype or (x.dtype if lowp else F32), group_row_end=ends)
+    return ops.gemm(x, w, b, residual=residual, epilogue=epilogue, out_dtype=out_dtype or (x.dtype if lowp else F32),
+                    group_row_end=ends)
+
+
+def stack_rows(parts: Sequence[torch.Tensor], row0: Sequence[int]) -> torch.Tensor:
+    """fp32 rows of several streams -> one tensor with stream i at row0[i] (stack_layout) and zero rows in the gaps
+    between streams"""
+    out, cur = [], 0
+    for p, r0 in zip(parts, row0):
+        if r0 > cur:
+            out.append(torch.zeros((r0 - cur, HIDDEN), dtype=F32, device=p.device))
+        out.append(p)
+        cur = r0 + p.shape[0]
+    return torch.cat(out, 0)
+
+
+def embed_streams(specs, row0: Sequence[int], rows: int, device, lowp: bool) -> Act:
+    """Input embeddings of several streams (one ``embed`` keyword dict per stream, with its 'rows') stacked on the
+    stack_layout boundaries.  Inference: each composer launch writes its slice of one preallocated activation and
+    zero-fills the gap behind it.  Training: one ``embed`` node per stream, stacked by stack_rows."""
+    if _Mode.train:
+        return as_act(stack_rows([embed(device=device, **kw).f32 for kw in specs], row0), lowp)
+    x32 = torch.empty((rows, HIDDEN), dtype=F32, device=device)
+    x16 = torch.empty((rows, HIDDEN), dtype=ops.h16(), device=device) if lowp else None
+    for i, kw in enumerate(specs):
+        r0, r1 = row0[i], (row0[i + 1] if i + 1 < len(row0) else rows)
+        embed(device=device, y32=x32[r0:r1], y16=x16[r0:r1] if lowp else None, zero_rows=r1 - r0 - kw['rows'], **kw)
+    return Act(x32, x16)
+
+
+def gather_rows(src: torch.Tensor, idx, n: int, lowp: Optional[bool] = None) -> torch.Tensor:
+    """rows = src[idx] (fp32); with ``lowp`` given, the GEMM operand of that precision instead.  Inference: one
+    vi_gather_mean over unit segments.  Training: GatherRowsFn (adjoint: scatter-add)."""
+    dev = src.device
+    if _Mode.train:
+        y = ag.GatherRowsFn.apply(src, torch.as_tensor(idx).to(dev, torch.int64, non_blocking=True), 0, n)
+        return y if lowp is None else operand(y, lowp)
+    unit = torch.arange(n + 1, dtype=torch.int32, device=dev)
+    idx = torch.as_tensor(idx).to(dev, torch.int32, non_blocking=True)
+    if lowp is None:
+        return ops.gather_mean(src, unit, idx, n, want16=False)[0]
+    y32, y16 = ops.gather_mean(src, unit, idx, n, want16=lowp, want32=not lowp)
+    return y16 if lowp else y32
+
+
+def segment_mean(src: torch.Tensor, offsets, rows, n: int) -> torch.Tensor:
+    """y[r] = mean of src[rows[offsets[r]:offsets[r+1]]] over ragged segments (int32 index arrays).  Inference: one
+    vi_gather_mean.  Training: RaggedMeanFn (a source row may sit in several segments)."""
+    offsets = torch.as_tensor(offsets).to(src.device)
+    rows = torch.as_tensor(rows).to(src.device)
+    if _Mode.train:
+        return ag.RaggedMeanFn.apply(src, offsets, rows, n)
+    return ops.gather_mean(src, offsets, rows, n, want16=False)[0]
 
 
 def as_act(x32: torch.Tensor, lowp: bool) -> Act:
@@ -600,12 +657,13 @@ def operand(x32: torch.Tensor, lowp: bool) -> torch.Tensor:
     return ag.CastBf16Fn.apply(x32) if _Mode.train else ops.cast_h16(x32)
 
 
-def embed(rows: int, device, *, a=None, a_ln=None, feat=None, feat_lin=None, feat_ln=None, idx=None, table=None,
+def embed(rows: int, device, *, a=None, a_ln=None, a2=None, feat=None, feat_lin=None, feat_ln=None, idx=None, table=None,
           pos_table=None, pos_period=0, const_rows=(), out_ln=None, eps=1e-12, lowp=False, y32=None, y16=None,
-          dropout=False, chain_ln=None, chain_eps=1e-5) -> Act:
-    """Input-embedding composer  LN_out([LN_a](a) + LN_f(W feat + b) + table[idx] + pos[row % period] + consts).
+          dropout=False, chain_ln=None, chain_eps=1e-5, zero_rows=0) -> Act:
+    """Input-embedding composer  LN_out([LN_a](a) + a2 + LN_f(W feat + b) + table[idx] + pos[row % period] + consts).
     *_ln are nn.LayerNorm-like parameter holders, feat_lin an nn.Linear-like holder.  Inference: ONE fused kernel
-    (vi_embed_compose).  Training: the same sum built from differentiable primitives (autograd_ops)."""
+    (vi_embed_compose), which also zero-fills ``zero_rows`` rows behind the output.  Training: the same sum built from
+    differentiable primitives (autograd_ops)."""
     ln_pair = lambda m: (m.weight, m.bias) if m is not None else None      # noqa: E731
     if not _Mode.train:
         consts = list(const_rows) + [None, None]
@@ -618,12 +676,12 @@ def embed(rows: int, device, *, a=None, a_ln=None, feat=None, feat_lin=None, fea
                                          const_row=consts[0], const_row2=consts[1], out_ln=ln_pair(out_ln), eps=eps,
                                          want16=True, want32=True, ln2=ln_pair(chain_ln), ln2_eps=chain_eps)
             return Act(o32, o16)
-        o32, o16 = ops.embed_compose(rows, device, a=a, a_ln=ln_pair(a_ln), feat=feat,
+        o32, o16 = ops.embed_compose(rows, device, a=a, a2=a2, a_ln=ln_pair(a_ln), feat=feat,
                                      feat_w=feat_lin.weight if feat_lin is not None else None,
                                      feat_b=feat_lin.bias if feat_lin is not None else None, feat_ln=ln_pair(feat_ln),
                                      idx=idx, table=table, pos_table=pos_table, pos_period=pos_period,
                                      const_row=consts[0], const_row2=consts[1], out_ln=ln_pair(out_ln), eps=eps,
-                                     y32=y32, y16=y16, want16=lowp and y16 is None and (y32 is None))
+                                     y32=y32, y16=y16, want16=lowp and y16 is None and (y32 is None), zero_rows=zero_rows)
         return Act(o32, o16)
     terms = []
     if a is not None:
@@ -632,6 +690,8 @@ def embed(rows: int, device, *, a=None, a_ln=None, feat=None, feat_lin=None, fea
             terms.append(t)
         else:
             terms.append(a)
+    if a2 is not None:
+        terms.append(a2)
     if feat is not None:
         t = ag.SmallLinearFn.apply(feat, feat_lin.weight, feat_lin.bias)
         if feat_ln is not None:

@@ -23,7 +23,7 @@ import torch.nn as nn
 
 from . import autograd_ops as ag
 from . import blocks, graphs, ops, params
-from .blocks import Act, Stream
+from .blocks import Stream
 from .config import duet_config
 from .ops import BF16, F32, HIDDEN
 
@@ -416,11 +416,10 @@ class GlocalTextPathNavCMT(nn.Module):
     def _panorama_with_objects(self, view_img_fts, obj_img_fts, loc_fts, nav_types, view_lens, obj_lens):
         """'panorama' with the REVERIE object boxes (:1096-1114): per episode the LayerNorm-ed object embeddings follow the
         LayerNorm-ed view embeddings, zero padded to the longest; everything after that is the R2R path over P = max(view_len
-        + obj_len) tokens.  The ragged concatenation is one row gather over [views ; objects ; a zero row].  Inference only."""
+        + obj_len) tokens.  The ragged concatenation is one row gather over [views ; objects ; a zero row] (adjoint in training:
+        a scatter-add)."""
         self._guard(view_img_fts)
         lowp, pk, ie = self.lowp, self._pk(), self.img_embeddings
-        if self._recording(view_img_fts, obj_img_fts) and not self.config.fix_pano_embedding:
-            return self._panorama_with_objects_train(view_img_fts, obj_img_fts, loc_fts, nav_types, view_lens, obj_lens)
         B, V, _ = view_img_fts.shape
         O = obj_img_fts.shape[1]
         dev = view_img_fts.device
@@ -429,61 +428,15 @@ class GlocalTextPathNavCMT(nn.Module):
         P = max(a + b for a, b in zip(vl, ol))
         if loc_fts.shape[1] != P or nav_types.shape[1] != P:
             raise ValueError('loc_fts / nav_types must cover max(view_len + obj_len) = %d tokens' % P)
-        v32 = _f32c(view_img_fts).view(B * V, -1)
-        o32 = _f32c(obj_img_fts).view(B * O, -1)
-        w, b = pk['img_linear'].get(lowp)
-        nv, _ = ops.add_ln(ops.gemm(ops.cast_h16(v32) if lowp else v32, w, b, out_dtype=F32), None, ie.img_layer_norm.weight,
-                           ie.img_layer_norm.bias, 1e-12, want16=False)
-        if ie.obj_linear is not None:                          # obj_feat_size != image_feat_size (:464-468)
-            w, b = pk['obj_linear'].get(lowp)
-            oln = ie.obj_layer_norm
-        else:
-            oln = ie.img_layer_norm
-        no, _ = ops.add_ln(ops.gemm(ops.cast_h16(o32) if lowp else o32, w, b, out_dtype=F32), None, oln.weight, oln.bias, 1e-12,
-                           want16=False)
-        src = torch.cat([nv, no, torch.zeros((1, HIDDEN), dtype=F32, device=dev)], 0)
-        zero_row = B * V + B * O
-        idx = np.full((B, P), zero_row, np.int32)
+        idx = np.full((B, P), B * V + B * O, np.int64)         # row B * V + B * O: the appended zero row
         for i in range(B):
             idx[i, :vl[i]] = i * V + np.arange(vl[i])
             idx[i, vl[i]:vl[i] + ol[i]] = B * V + i * O + np.arange(ol[i])
-        idx_d = torch.from_numpy(idx.reshape(-1)).to(dev, non_blocking=True)
-        unit = torch.arange(B * P + 1, dtype=torch.int32, device=dev)
-        a, _ = ops.gather_mean(src, unit, idx_d, B * P, want16=False)
         pano_lens = (view_lens + obj_lens).to(dev)
         pano_masks = torch.arange(P, device=dev)[None, :] < pano_lens[:, None]
         km = blocks.mask_u8(pano_masks)
-        with blocks.grad_mode(False, (0.0, 0.0)):
-            x32 = blocks.embed(B * P, dev, a=a, feat=_f32c(loc_fts).view(B * P, -1), feat_lin=ie.loc_linear, feat_ln=ie.loc_layer_norm,
-                               idx=nav_types.long().contiguous().view(-1), table=ie.nav_type_embedding.weight,
-                               const_rows=(self.embeddings.token_type_embeddings.weight[1],), out_ln=ie.layer_norm).f32
-            for lp in pk['pano']:
-                x32 = blocks.pano_layer(x32, lp, B, P, km, lowp)
-            y32 = blocks.layer_norm(x32, None, pk['pano_norm'], 1e-12, False).f32
-        return y32.view(B, P, HIDDEN).detach(), pano_masks
-
-    def _panorama_with_objects_train(self, view_img_fts, obj_img_fts, loc_fts, nav_types, view_lens, obj_lens):
-        """'panorama' with object boxes and autograd recording (REVERIE / SOON fine-tuning, :1096-1131): the same sequence from the
-        differentiable blocks; the ragged [views ; objects] concatenation is a row gather whose adjoint is a scatter-add."""
-        lowp, pk, ie = self.lowp, self._pk(), self.img_embeddings
-        B, V, _ = view_img_fts.shape
-        O = obj_img_fts.shape[1]
-        dev = view_img_fts.device
-        vl = [int(x) for x in view_lens.tolist()]
-        ol = [int(x) for x in obj_lens.tolist()]
-        P = max(a + b for a, b in zip(vl, ol))
-        if loc_fts.shape[1] != P or nav_types.shape[1] != P:
-            raise ValueError('loc_fts / nav_types must cover max(view_len + obj_len) = %d tokens' % P)
-        zero_row = B * V + B * O
-        idx = np.full((B, P), zero_row, np.int64)
-        for i in range(B):
-            idx[i, :vl[i]] = i * V + np.arange(vl[i])
-            idx[i, vl[i]:vl[i] + ol[i]] = B * V + i * O + np.arange(ol[i])
-        idx_d = torch.from_numpy(idx.reshape(-1)).to(dev, non_blocking=True)
-        pano_lens = (view_lens + obj_lens).to(dev)
-        pano_masks = torch.arange(P, device=dev)[None, :] < pano_lens[:, None]
-        km = blocks.mask_u8(pano_masks)
-        with blocks.grad_mode(True, self._drop()):
+        recording = self._recording(view_img_fts, obj_img_fts) and not self.config.fix_pano_embedding
+        with blocks.grad_mode(recording, self._drop()):
             v32 = _f32c(view_img_fts).view(B * V, -1)
             o32 = _f32c(obj_img_fts).view(B * O, -1)
             nv = blocks.layer_norm(blocks.linear(blocks.operand(v32, lowp), pk['img_linear'], lowp, out_dtype=F32), None,
@@ -495,101 +448,127 @@ class GlocalTextPathNavCMT(nn.Module):
             no = blocks.layer_norm(blocks.linear(blocks.operand(o32, lowp), olin, lowp, out_dtype=F32), None, blocks.LNPack([oln]),
                                    1e-12, False).f32
             src = torch.cat([nv, no, torch.zeros((1, HIDDEN), dtype=F32, device=dev)], 0)
-            a = ag.GatherRowsFn.apply(src, idx_d, 0, B * P)
+            a = blocks.gather_rows(src, idx.reshape(-1), B * P)
             x32 = blocks.embed(B * P, dev, a=a, feat=_f32c(loc_fts).view(B * P, -1), feat_lin=ie.loc_linear, feat_ln=ie.loc_layer_norm,
                                idx=nav_types.long().contiguous().view(-1), table=ie.nav_type_embedding.weight,
                                const_rows=(self.embeddings.token_type_embeddings.weight[1],), out_ln=ie.layer_norm, dropout=True).f32
             for lp in pk['pano']:
                 x32 = blocks.pano_layer(x32, lp, B, P, km, lowp)
             y32 = blocks.layer_norm(x32, None, pk['pano_norm'], 1e-12, False).f32
-        return y32.view(B, P, HIDDEN), pano_masks
+        out = y32.view(B, P, HIDDEN)
+        return (out if recording else out.detach()), pano_masks
 
     def forward_navigation_per_step(self, txt_embeds, txt_masks, gmap_img_embeds, gmap_step_ids, gmap_pos_fts,
                                     gmap_masks, gmap_pair_dists, gmap_visited_masks, gmap_vpids,
                                     vp_img_embeds, vp_pos_fts, vp_masks, vp_nav_masks, vp_obj_masks, vp_cand_vpids,
                                     imagine_embeds=None, imagine_masks=None, ctx_kv=None, defer_fuse=False):
-        """'navigation'.  :1133-1235.  ``ctx_kv`` (internal): context projections already looked up by the caller
-        (VLNBert's graph path); txt_embeds / imagine_embeds are then not read.  ``defer_fuse`` (internal): stop before the
-        global / local fusion (:1198-1217) and return its operands under '_fuse' for ``fuse_logits``."""
+        """'navigation'.  :1133-1235.  With autograd recording (fine-tuning, BASELINE.json cfg-4) every block records its
+        node.  ``ctx_kv`` (internal, inference): context projections already looked up by the caller (VLNBert's graph path);
+        txt_embeds / imagine_embeds are then not read.  ``defer_fuse`` (internal, inference): stop before the global / local
+        fusion (:1198-1217) and return its operands under '_fuse' for ``fuse_logits``."""
         if vp_obj_masks is not None and not hasattr(self, 'og_head'):
             raise ValueError('vp_obj_masks given but the model has no object-grounding head (obj_feat_size = 0)')
         self._guard(gmap_img_embeds)
-        cfg, lowp, pk = self.config, self.lowp, self._pk()
+        lowp, pk = self.lowp, self._pk()
         dev = gmap_img_embeds.device
         B, L = txt_masks.shape
         G, P = gmap_img_embeds.shape[1], vp_img_embeds.shape[1]
-        ge, le = self.global_encoder, self.local_encoder
-
-        if ctx_kv is None and self._recording(txt_embeds, gmap_img_embeds, vp_img_embeds, imagine_embeds):
-            with blocks.grad_mode(True, self._drop()):
-                return self._navigation_train(txt_embeds, txt_masks, gmap_img_embeds, gmap_step_ids, gmap_pos_fts, gmap_masks,
-                                              gmap_pair_dists, gmap_visited_masks, gmap_vpids, vp_img_embeds, vp_pos_fts,
-                                              vp_masks, vp_nav_masks, vp_cand_vpids, imagine_embeds, imagine_masks, vp_obj_masks)
-
-        # ---- input embeddings of both branches into one row-stacked activation (:1141-1152)
-        (r_g, r_l), ends, R = blocks.stack_layout([B * G, B * P])
-        x32 = torch.empty((R, HIDDEN), dtype=F32, device=dev)
-        x16 = torch.empty((R, HIDDEN), dtype=ops.h16(), device=dev) if lowp else None
-        # the padding rows between the two streams are zero-filled by the first composer launch
-        ops.embed_compose(B * G, dev, a=_f32c(gmap_img_embeds).view(B * G, HIDDEN),
-                          feat=_f32c(gmap_pos_fts).view(B * G, -1), feat_w=ge.gmap_pos_embeddings[0].weight,
-                          feat_b=ge.gmap_pos_embeddings[0].bias,
-                          feat_ln=(ge.gmap_pos_embeddings[1].weight, ge.gmap_pos_embeddings[1].bias),
-                          idx=gmap_step_ids.long().contiguous().view(-1), table=ge.gmap_step_embeddings.weight,
-                          y32=x32[r_g:ends[0]], y16=x16[r_g:ends[0]] if lowp else None, zero_rows=ends[0] - (r_g + B * G))
-        ops.embed_compose(B * P, dev, a=_f32c(vp_img_embeds).view(B * P, HIDDEN),
-                          feat=_f32c(vp_pos_fts).view(B * P, -1), feat_w=le.vp_pos_embeddings[0].weight,
-                          feat_b=le.vp_pos_embeddings[0].bias,
-                          feat_ln=(le.vp_pos_embeddings[1].weight, le.vp_pos_embeddings[1].bias),
-                          y32=x32[r_l:r_l + B * P], y16=x16[r_l:r_l + B * P] if lowp else None)
-        x = Act(x32, x16)
-
-        # ---- context = [txt ; imagine] (:1157-1158) and its K / V projections for the 4 layers: the context never
-        # changes inside an episode (use_lang2visn_attn is off), so the projections are kept per episode
-        kvs = ctx_kv if ctx_kv is not None else self.context_kv(txt_embeds, imagine_embeds)
-        ctx_mask, C = self.context_mask(txt_masks, imagine_masks)
-
-        affine = None
-        dist = None
-        if ge.sprel_linear is not None:                       # GASA bias (:1145-1149), applied inside the attention kernel
-            affine = pk['sprel'].get()
-            dist = _f32c(gmap_pair_dists)
-        streams = [Stream(r_g, B, G, blocks.mask_u8(gmap_masks), 0, dist, affine),
-                   Stream(r_l, B, P, blocks.mask_u8(vp_masks), 1)]
-
-        # ---- 4 graph-aware cross-modal layers, both branches per launch (:384-399, :444-453)
-        for cp, sp, kv in zip(pk['x_cross'], pk['x_self'], kvs):
-            x = blocks.cross_attn(x, kv, [0, 2 * HIDDEN], C, ctx_mask, cp, streams, ends, lowp, defer=True)
-            x = blocks.self_attn_ffn(x, sp, streams, ends, lowp, defer=True)
-        x = blocks.materialize(x, lowp, ends)
-
-        gmap_out = x.f32[r_g:r_g + B * G].view(B, G, HIDDEN)
-        vp_out = x.f32[r_l:r_l + B * P].view(B, P, HIDDEN)
-
-        # ---- heads (:1182-1196) and global/local fusion (:1198-1217)
-        fuse_raw = None
-        if self.sap_fuse_linear is not None:
-            cat = torch.empty((B, 2 * HIDDEN), dtype=ops.h16() if lowp else F32, device=dev)
-            c32, c16 = (None, cat) if lowp else (cat, None)
-            ops.copy_rows(x.f32[r_g:], G * HIDDEN, HIDDEN, B, 1, c32, c16, 2 * HIDDEN, HIDDEN)
-            ops.copy_rows(x.f32[r_l:], P * HIDDEN, HIDDEN, B, 1, c32[:, HIDDEN:] if c32 is not None else None,
-                          c16[:, HIDDEN:] if c16 is not None else None, 2 * HIDDEN, HIDDEN)
-            fuse_raw = blocks.cls_head(cat, pk['fuse'], lowp)
-        raw = blocks.cls_head(x.operand(lowp), pk['sap'], lowp, ends)
-        if defer_fuse:
-            return {'gmap_embeds': gmap_out, 'vp_embeds': vp_out, '_g_raw': raw[r_g:], '_l_raw': raw[r_l:], '_fuse_raw': fuse_raw,
-                    '_gmap_masks': blocks.mask_u8(gmap_masks), '_visited': blocks.mask_u8(gmap_visited_masks),
-                    '_nav_masks': blocks.mask_u8(vp_nav_masks)}
-        gmap_ids, cand_ids = self.intern_vpids(gmap_vpids, vp_cand_vpids, G, P, dev)
-        gl, ll, fl = ops.duet_fuse_logits(raw[r_g:], raw[r_l:], fuse_raw, blocks.mask_u8(gmap_masks),
-                                          blocks.mask_u8(gmap_visited_masks), blocks.mask_u8(vp_nav_masks),
-                                          gmap_ids, cand_ids, B, G, P)
-        obj_logits = None
-        if vp_obj_masks is not None:                           # object grounding logits (:1220-1225): -inf outside the object tokens
-            og_raw = blocks.cls_head(x.operand(lowp)[r_l:r_l + B * P], pk['og'], lowp)
-            obj_logits = ops.mask_logits_navtype(og_raw, vp_obj_masks.long().contiguous().view(-1)).view(B, P)
+        recording = ctx_kv is None and self._recording(txt_embeds, gmap_img_embeds, vp_img_embeds, imagine_embeds)
+        with blocks.grad_mode(recording, self._drop() if recording else (0.0, 0.0)):
+            x, row0, ends = self._branch_inputs(_f32c(gmap_img_embeds).view(B * G, HIDDEN), gmap_pos_fts, gmap_step_ids,
+                                                _f32c(vp_img_embeds).view(B * P, HIDDEN), vp_pos_fts, B, G, P)
+            r_g, r_l = row0
+            # context = [txt ; imagine] (:1157-1158).  Inference: its K / V projections for the 4 layers are kept per episode
+            # (the context never changes inside one, use_lang2visn_attn is off); training projects it in every layer
+            ctx = kvs = None
+            if recording:
+                ctx32 = _f32c(txt_embeds)
+                if self._with_imagine():
+                    if imagine_embeds is None:
+                        raise ValueError('navigation needs imagine_embeds and imagine_masks when imagine_enc_pano is set')
+                    ctx32 = torch.cat([ctx32, _f32c(imagine_embeds)], 1)
+                ctx = blocks.operand(ctx32.view(-1, HIDDEN), lowp)
+            else:
+                kvs = ctx_kv if ctx_kv is not None else self.context_kv(txt_embeds, imagine_embeds)
+            ctx_mask, C = self.context_mask(txt_masks, imagine_masks)
+            streams = self._branch_streams(B, G, P, row0, gmap_masks, vp_masks, gmap_pair_dists)
+            x = self._cross_layers(x, streams, ends, C, ctx_mask, kvs=kvs, ctx=ctx)
+            gmap_out = x.f32[r_g:r_g + B * G].view(B, G, HIDDEN)
+            vp_out = x.f32[r_l:r_l + B * P].view(B, P, HIDDEN)
+            # heads (:1182-1196) and global/local fusion (:1198-1217)
+            raw, fuse_raw = self._sap_heads(x, pk['sap'], pk.get('fuse'), B, G, P, row0, ends)
+            if defer_fuse:
+                return {'gmap_embeds': gmap_out, 'vp_embeds': vp_out, '_g_raw': raw[r_g:], '_l_raw': raw[r_l:], '_fuse_raw': fuse_raw,
+                        '_gmap_masks': blocks.mask_u8(gmap_masks), '_visited': blocks.mask_u8(gmap_visited_masks),
+                        '_nav_masks': blocks.mask_u8(vp_nav_masks)}
+            gmap_ids, cand_ids = self.intern_vpids(gmap_vpids, vp_cand_vpids, G, P, dev)
+            gl, ll, fl = self._fuse_step(raw, fuse_raw, gmap_masks, gmap_visited_masks, vp_nav_masks, gmap_ids, cand_ids,
+                                         B, G, P, row0)
+            obj_logits = None
+            if vp_obj_masks is not None:                       # object grounding logits (:1220-1225): -inf outside the object tokens
+                og_raw = blocks.cls_head(x.operand(lowp)[r_l:r_l + B * P], pk['og'], lowp)
+                if recording:
+                    obj_logits = og_raw.view(B, P).masked_fill(vp_obj_masks.logical_not(), float('-inf'))
+                else:
+                    obj_logits = ops.mask_logits_navtype(og_raw, vp_obj_masks.long().contiguous().view(-1)).view(B, P)
         return {'gmap_embeds': gmap_out, 'vp_embeds': vp_out, 'global_logits': gl, 'local_logits': ll,
                 'fused_logits': fl, 'obj_logits': obj_logits}
+
+    # -- pieces of the navigation step that pre-training (pretrain.py) runs as well --------------------------------------
+    def _branch_inputs(self, gmap_img, gmap_pos_fts, gmap_step_ids, vp_img, vp_pos_fts, B, G, P):
+        """input embeddings of both branches in one row-stacked activation (:1141-1152) -> (Act, row0, ends)"""
+        ge, le = self.global_encoder, self.local_encoder
+        row0, ends, R = blocks.stack_layout([B * G, B * P])
+        x = blocks.embed_streams([
+            dict(rows=B * G, a=gmap_img, feat=_f32c(gmap_pos_fts).view(B * G, -1), feat_lin=ge.gmap_pos_embeddings[0],
+                 feat_ln=ge.gmap_pos_embeddings[1], idx=gmap_step_ids.long().contiguous().view(-1), table=ge.gmap_step_embeddings.weight),
+            dict(rows=B * P, a=vp_img, feat=_f32c(vp_pos_fts).view(B * P, -1), feat_lin=le.vp_pos_embeddings[0],
+                 feat_ln=le.vp_pos_embeddings[1])], row0, R, gmap_img.device, self.lowp)
+        return x, row0, ends
+
+    def _branch_streams(self, B, G, P, row0, gmap_masks, vp_masks, gmap_pair_dists):
+        """the global (map) and local (panorama) streams; the global one carries the GASA bias (:1145-1149), applied inside the
+        attention kernel"""
+        sl = self.global_encoder.sprel_linear
+        dist = affine = aparams = None
+        if sl is not None:
+            dist, affine, aparams = _f32c(gmap_pair_dists), self._pk()['sprel'].get(), (sl.weight, sl.bias)
+        return [Stream(row0[0], B, G, blocks.mask_u8(gmap_masks), 0, dist, affine, aparams),
+                Stream(row0[1], B, P, blocks.mask_u8(vp_masks), 1)]
+
+    def _cross_layers(self, x, streams, ends, C, ctx_mask, kvs=None, ctx=None):
+        """the graph-aware cross-modal layers, both branches per launch (:384-399, :444-453).  The context's K_g | V_g | K_l | V_l
+        [B*C, 4*768] per layer: ``kvs`` when given, else projected from the context operand ``ctx`` in each layer."""
+        lowp, pk = self.lowp, self._pk()
+        for i, (cp, sp) in enumerate(zip(pk['x_cross'], pk['x_self'])):
+            kv = kvs[i] if kvs is not None else blocks.linear(ctx, cp.kv, lowp)
+            x = blocks.cross_attn(x, [(kv, 0, C, ctx_mask), (kv, 2 * HIDDEN, C, ctx_mask)], cp, streams, ends, lowp, defer=True)
+            x = blocks.self_attn_ffn(x, sp, streams, ends, lowp, defer=True)
+        return blocks.materialize(x, lowp, ends)
+
+    def _sap_heads(self, x, sap, fuse, B, G, P, row0, ends):
+        """(raw action logit of every token of both branches, raw fused logit of the two [stop] tokens or None) (:1182-1217)"""
+        lowp = self.lowp
+        r_g, r_l = row0
+        fuse_raw = None
+        if fuse is not None:
+            if blocks.training():
+                cat = blocks.operand(torch.cat([x.f32[r_g:r_g + B * G].view(B, G, HIDDEN)[:, 0],
+                                                x.f32[r_l:r_l + B * P].view(B, P, HIDDEN)[:, 0]], 1), lowp)
+            else:
+                cat = torch.empty((B, 2 * HIDDEN), dtype=ops.h16() if lowp else F32, device=x.f32.device)
+                c32, c16 = (None, cat) if lowp else (cat, None)
+                ops.copy_rows(x.f32[r_g:], G * HIDDEN, HIDDEN, B, 1, c32, c16, 2 * HIDDEN, HIDDEN)
+                ops.copy_rows(x.f32[r_l:], P * HIDDEN, HIDDEN, B, 1, c32[:, HIDDEN:] if c32 is not None else None,
+                              c16[:, HIDDEN:] if c16 is not None else None, 2 * HIDDEN, HIDDEN)
+            fuse_raw = blocks.cls_head(cat, fuse, lowp)
+        return blocks.cls_head(x.operand(lowp), sap, lowp, ends), fuse_raw
+
+    def _fuse_step(self, raw, fuse_raw, gmap_masks, visited, nav, gmap_ids, cand_ids, B, G, P, row0):
+        """global / local / fused action logits from the raw head outputs (:1198-1217)"""
+        args = (raw[row0[0]:row0[0] + B * G], raw[row0[1]:row0[1] + B * P], fuse_raw, blocks.mask_u8(gmap_masks),
+                blocks.mask_u8(visited), blocks.mask_u8(nav), gmap_ids, cand_ids, B, G, P)
+        return ag.FuseLogitsFn.apply(*args) if blocks.training() else ops.duet_fuse_logits(*args)
 
     def fuse_logits(self, pre: dict, gmap_vpids, vp_cand_vpids, G: int, P: int) -> dict:
         """Second half of a ``defer_fuse`` navigation call: intern the viewpoint ids (host work that then overlaps the
@@ -672,70 +651,6 @@ class GlocalTextPathNavCMT(nn.Module):
         """forget the cached context projections (new episode with recycled tensors, or to bound memory)"""
         for slot in self._ctx_slots.values():
             slot['ident'], slot['refs'] = None, None
-
-    def _navigation_train(self, txt_embeds, txt_masks, gmap_img_embeds, gmap_step_ids, gmap_pos_fts, gmap_masks,
-                          gmap_pair_dists, gmap_visited_masks, gmap_vpids, vp_img_embeds, vp_pos_fts, vp_masks,
-                          vp_nav_masks, vp_cand_vpids, imagine_embeds, imagine_masks, vp_obj_masks=None):
-        """'navigation' with autograd recording (fine-tuning, BASELINE.json cfg-4): the same layer sequence as
-        forward_navigation_per_step built from the differentiable blocks; torch only concatenates / slices rows."""
-        cfg, lowp, pk = self.config, self.lowp, self._pk()
-        dev = txt_embeds.device
-        B, L, _ = txt_embeds.shape
-        G, P = gmap_img_embeds.shape[1], vp_img_embeds.shape[1]
-        ge, le = self.global_encoder, self.local_encoder
-        (r_g, r_l), ends, R = blocks.stack_layout([B * G, B * P])
-        g_in = blocks.embed(B * G, dev, a=_f32c(gmap_img_embeds).view(B * G, HIDDEN), feat=_f32c(gmap_pos_fts).view(B * G, -1),
-                            feat_lin=ge.gmap_pos_embeddings[0], feat_ln=ge.gmap_pos_embeddings[1],
-                            idx=gmap_step_ids.long().contiguous().view(-1), table=ge.gmap_step_embeddings.weight).f32
-        l_in = blocks.embed(B * P, dev, a=_f32c(vp_img_embeds).view(B * P, HIDDEN), feat=_f32c(vp_pos_fts).view(B * P, -1),
-                            feat_lin=le.vp_pos_embeddings[0], feat_ln=le.vp_pos_embeddings[1]).f32
-        parts = [g_in]
-        if ends[0] > B * G:
-            parts.append(torch.zeros((ends[0] - B * G, HIDDEN), dtype=F32, device=dev))
-        x = blocks.as_act(torch.cat(parts + [l_in], 0), lowp)
-
-        txt = _f32c(txt_embeds)
-        if cfg.imagine_enc_pano and cfg.concat_imagine_with == 'language':
-            if imagine_embeds is None or imagine_masks is None:
-                raise ValueError('navigation needs imagine_embeds and imagine_masks when imagine_enc_pano is set')
-            C = L + imagine_embeds.shape[1]
-            ctx32 = torch.cat([txt, _f32c(imagine_embeds)], 1).view(B * C, HIDDEN)
-            ctx_mask = blocks.mask_u8(torch.cat([txt_masks.bool(), imagine_masks.bool()], 1))
-        else:
-            C = L
-            ctx32 = txt.view(B * L, HIDDEN)
-            ctx_mask = blocks.mask_u8(txt_masks)
-        ctx = blocks.operand(ctx32, lowp)
-
-        affine = dist = aparams = None
-        if ge.sprel_linear is not None:
-            affine = pk['sprel'].get()
-            dist = _f32c(gmap_pair_dists)
-            aparams = (ge.sprel_linear.weight, ge.sprel_linear.bias)
-        streams = [Stream(r_g, B, G, blocks.mask_u8(gmap_masks), 0, dist, affine, aparams),
-                   Stream(r_l, B, P, blocks.mask_u8(vp_masks), 1)]
-        for cp, sp in zip(pk['x_cross'], pk['x_self']):
-            kv = blocks.linear(ctx, cp.kv, lowp)
-            x = blocks.cross_attn(x, kv, [0, 2 * HIDDEN], C, ctx_mask, cp, streams, ends, lowp)
-            x = blocks.self_attn_ffn(x, sp, streams, ends, lowp)
-
-        gmap_out = x.f32[r_g:r_g + B * G].view(B, G, HIDDEN)
-        vp_out = x.f32[r_l:r_l + B * P].view(B, P, HIDDEN)
-        fuse_raw = None
-        if self.sap_fuse_linear is not None:
-            cat = torch.cat([gmap_out[:, 0], vp_out[:, 0]], 1)
-            fuse_raw = blocks.cls_head(blocks.operand(cat, lowp), pk['fuse'], lowp)
-        raw = blocks.cls_head(x.operand(lowp), pk['sap'], lowp, ends)
-        gmap_ids, cand_ids = self.intern_vpids(gmap_vpids, vp_cand_vpids, G, P, dev)
-        gl, ll, fl = ag.FuseLogitsFn.apply(raw[r_g:r_g + B * G], raw[r_l:r_l + B * P], fuse_raw, blocks.mask_u8(gmap_masks),
-                                           blocks.mask_u8(gmap_visited_masks), blocks.mask_u8(vp_nav_masks), gmap_ids,
-                                           cand_ids, B, G, P)
-        obj_logits = None
-        if vp_obj_masks is not None:                           # object grounding head (:1220-1225)
-            og_raw = blocks.cls_head(x.operand(lowp)[r_l:r_l + B * P], pk['og'], lowp)
-            obj_logits = og_raw.view(B, P).masked_fill(vp_obj_masks.logical_not(), float('-inf'))
-        return {'gmap_embeds': gmap_out, 'vp_embeds': vp_out, 'global_logits': gl, 'local_logits': ll,
-                'fused_logits': fl, 'obj_logits': obj_logits}
 
     def intern_vpids(self, gmap_vpids, vp_cand_vpids, G, P, dev):
         """Viewpoint-id strings -> int32 tensors on ``dev`` (gmap padding -1, candidate padding -2).  Callers that

@@ -426,10 +426,7 @@ class NavCMT(nn.Module):
             ob = ob.detach()
         lang = torch.cat([_f32c(txt_embeds), _f32c(imagine_embeds)], 1) if Il else _f32c(txt_embeds)
         visn = torch.cat([_f32c(hist_embeds), ob.view(B, O, HIDDEN)] + ([_f32c(imagine_embeds)] if Iv else []), 1)
-        parts = [lang.reshape(B * C, HIDDEN)]
-        if ends[0] > B * C:
-            parts.append(torch.zeros((ends[0] - B * C, HIDDEN), dtype=F32, device=dev))
-        x = blocks.as_act(torch.cat(parts + [visn.reshape(B * Nv, HIDDEN)], 0), lowp)
+        x = blocks.as_act(blocks.stack_rows([lang.reshape(B * C, HIDDEN), visn.reshape(B * Nv, HIDDEN)], (r_l, r_v)), lowp)
         lang_mask = blocks.mask_u8(torch.cat([txt_masks.bool(), imagine_masks.bool()], 1) if Il else txt_masks)
         visn_mask = blocks.mask_u8(torch.cat([hist_masks.bool(), ob_masks.bool()] + ([imagine_masks.bool()] if Iv else []), 1))
         streams = [Stream(r_l, B, C, lang_mask, 0), Stream(r_v, B, Nv, visn_mask, 1)]

@@ -14,12 +14,14 @@ attention, row kernels); what it adds is
 Parameter names equal the reference's (tests/golden/duet_pretrain_manifest.json).  Oracle: oracle/pretrain_oracle.py, pinned to
 the real reference.
 
-Training: with autograd recording (grad mode on, parameters that require grad) ``forward`` runs the same layer sequence from the
-differentiable blocks (``_trunk_train``, as duet._navigation_train) and returns the per-row losses; ``loss.mean().backward()`` runs
-libvlnimagine kernels only.  The padded decoder / classifier is ``autograd_ops.PaddedLinearFn`` (the tied decoder's weight gradient
-adds onto the word-embedding lookup's), the losses ``CERowsFn`` / ``KLRowsFn``, whose backward kernel (vi_ce_rows_bwd /
-vi_kl_rows_bwd) writes the bf16 operand of the decoder's gradient GEMMs directly.  Train-mode dropout: bf16 only, as the
-navigation model.  Under torch.no_grad() the inference path below runs unchanged.
+One code path serves inference and training.  Each task runs its layer sequence from the mode-switching blocks (blocks.py) and
+the navigation model's pieces (duet.GlocalTextPathNavCMT._branch_inputs / _cross_layers / _sap_heads / _fuse_step) under
+``blocks.grad_mode``: under torch.no_grad() they are plain libvlnimagine launches; with autograd recording (grad mode on,
+parameters that require grad) every step records a node whose backward is libvlnimagine kernels too, and ``forward`` returns the
+per-row losses for ``loss.mean().backward()``.  In training the padded decoder / classifier is ``autograd_ops.PaddedLinearFn``
+(the tied decoder's weight gradient adds onto the word-embedding lookup's), the losses ``CERowsFn`` / ``KLRowsFn``, whose backward
+kernel (vi_ce_rows_bwd / vi_kl_rows_bwd) writes the bf16 operand of the decoder's gradient GEMMs directly.  Train-mode dropout:
+bf16 only, as the navigation model.
 """
 from __future__ import annotations
 
@@ -215,140 +217,31 @@ class GlocalTextPathCMTPreTraining(nn.Module):
         return self._head_packs
 
     # -- shared trunk ----------------------------------------------------------------------------------------------------
-    def _trunk(self, batch, want_l2v=False):
-        """GlocalTextPathCMT.forward / forward_mlm, model/vilmodel.py:660-747 -> dict of row-stacked results"""
-        blocks, duet, ops, params = _lazy()
-        bert = self.bert
-        lowp, pk = bert.lowp, bert._pk()
-        dev = bert.embeddings.LayerNorm.weight.device
-        F32, HID = torch.float32, 768
-        to = lambda t, dt=None: torch.as_tensor(t).to(dev, dtype=dt, non_blocking=True)     # noqa: E731
-        txt_ids = to(batch['txt_ids'])
-        B, L = txt_ids.shape
-        txt_lens = [int(x) for x in batch['txt_lens']]
-        txt_masks = torch.arange(L, device=dev)[None, :] < to(batch['txt_lens'])[:, None]
-        txt = bert.forward_text(txt_ids, txt_masks)                                  # (B, L, 768) fp32
-        # every panorama of every trajectory through the panorama encoder (vilmodel.py:484-528)
-        step_lens = [int(x) for x in batch['traj_step_lens']]
-        view_lens = to(batch['traj_vp_view_lens'])
-        pano, _ = bert.forward_panorama_per_step(to(batch['traj_view_img_fts'], F32), None, to(batch['traj_loc_fts'], F32),
-                                                 to(batch['traj_nav_types']), view_lens, None)
-        N, V, _ = pano.shape
-        vl_host = [int(x) for x in batch['traj_vp_view_lens']]
-        last = np.cumsum(step_lens) - 1
-        # local branch: [stop] + the LAST panorama of each trajectory (vilmodel.py:538-553)
-        P = max(vl_host[i] for i in last) + 1
-        src = torch.cat([pano.reshape(N * V, HID), torch.zeros((1, HID), dtype=F32, device=dev)], 0)
-        zero_row = N * V
-        vp_idx = np.full((B, P), zero_row, np.int32)
-        for b, i in enumerate(last):
-            n = min(V, P - 1)
-            vp_idx[b, 1:1 + n] = i * V + np.arange(n)
-        vp_lens = torch.as_tensor([vl_host[i] + 1 for i in last], device=dev)
-        vp_masks = torch.arange(P, device=dev)[None, :] < vp_lens[:, None]
-        unit = lambda n: torch.arange(n + 1, dtype=torch.int32, device=dev)                # noqa: E731
-        vp_img, _ = ops.gather_mean(src, unit(B * P), torch.from_numpy(vp_idx.reshape(-1)).to(dev), B * P, want16=False)
-        le, ge = bert.local_encoder, bert.global_encoder
-        # global branch: the graph-node features aggregated from the trajectory (vilmodel.py:577-611) in one segment-mean launch
-        off, rows, G = gmap_aggregation_rows(step_lens, vl_host, batch['traj_vpids'], batch['traj_cand_vpids'],
-                                             batch['gmap_vpids'], V)
-        gmap_img, _ = ops.gather_mean(src, torch.from_numpy(off).to(dev), torch.from_numpy(rows).to(dev), B * G, want16=False)
-        gmap_masks = torch.arange(G, device=dev)[None, :] < to(batch['gmap_lens'])[:, None]
-        # input embeddings of both branches into one row-stacked activation (vilmodel.py:613-625, 538-553)
-        row0, ends, R = blocks.stack_layout([B * G, B * P])
-        x32 = torch.zeros((R, HID), dtype=F32, device=dev)
-        x16 = torch.zeros((R, HID), dtype=ops.h16(), device=dev) if lowp else None
-        r_l = row0[-1]
-        if True:
-            ops.embed_compose(B * G, dev, a=gmap_img, feat=to(batch['gmap_pos_fts'], F32).reshape(B * G, -1).contiguous(),
-                              feat_w=ge.gmap_pos_embeddings[0].weight, feat_b=ge.gmap_pos_embeddings[0].bias,
-                              feat_ln=(ge.gmap_pos_embeddings[1].weight, ge.gmap_pos_embeddings[1].bias),
-                              idx=to(batch['gmap_step_ids']).long().contiguous().view(-1), table=ge.gmap_step_embeddings.weight,
-                              y32=x32[0:B * G], y16=x16[0:B * G] if lowp else None)
-        ops.embed_compose(B * P, dev, a=vp_img, feat=to(batch['vp_pos_fts'], F32).reshape(B * P, -1).contiguous(),
-                          feat_w=le.vp_pos_embeddings[0].weight, feat_b=le.vp_pos_embeddings[0].bias,
-                          feat_ln=(le.vp_pos_embeddings[1].weight, le.vp_pos_embeddings[1].bias),
-                          y32=x32[r_l:r_l + B * P], y16=x16[r_l:r_l + B * P] if lowp else None)
-        out = dict(B=B, L=L, G=G, P=P, r_l=r_l, ends=ends, txt=txt, txt_masks=txt_masks, vp_masks=vp_masks, dev=dev,
-                   last=last, vl_host=vl_host, V=V)
-        x_in = blocks.Act(x32, x16)
-        tmask = blocks.mask_u8(txt_masks)
-        if want_l2v:
-            out['l2v'] = self._lang2visn(x_in, txt, tmask, B, L, G, P, r_l, blocks.mask_u8(gmap_masks), blocks.mask_u8(vp_masks))
-            return out
-        # the 4 graph-aware cross-modal layers; context = the instruction (no imagination tokens in pre-training)
-        ctx = blocks.operand(txt.reshape(B * L, HID), lowp)
-        affine = dist = None
-        if ge.sprel_linear is not None:
-            affine, dist = pk['sprel'].get(), to(batch['gmap_pair_dists'], F32).contiguous()
-        streams = [blocks.Stream(0, B, G, blocks.mask_u8(gmap_masks), 0, dist, affine),
-                   blocks.Stream(r_l, B, P, blocks.mask_u8(vp_masks), 1)]
-        x, e = x_in, ends
-        for cp, sp in zip(pk['x_cross'], pk['x_self']):
-            w, b = cp.kv.get(lowp)
-            kv = ops.gemm(ctx, w, b)                             # [B*L, 4*768] = K_g | V_g | K_l | V_l
-            x = blocks.cross_attn(x, kv, [0, 2 * HID], L, tmask, cp, streams, e, lowp, defer=True)
-            x = blocks.self_attn_ffn(x, sp, streams, e, lowp, defer=True)
-        out['x'] = blocks.materialize(x, lowp, e)
-        return out
-
-    def _lang2visn(self, x_in, txt, tmask, B, L, G, P, r_l, gmask, vmask):
-        """GraphLXRTXLayer.forward_lang2visn x 4 for both branches (vilmodel.py:400-411, 719-735): the instruction attends to
-        the (fixed) map / panorama input embeddings; two language streams (global | local weights) stacked along the rows."""
-        blocks, duet, ops, params = _lazy()
-        bert = self.bert
-        lowp, pk = bert.lowp, bert._pk()
-        HID = 768
-        dev = txt.device
-        (r0, r1), ends, R = blocks.stack_layout([B * L, B * L])
-        t32 = txt.reshape(B * L, HID).contiguous()
-        l32 = torch.zeros((R, HID), dtype=torch.float32, device=dev)
-        l32[r0:r0 + B * L] = t32
-        l32[r1:r1 + B * L] = t32
-        lang = blocks.as_act(l32, lowp)
-        streams = [blocks.Stream(r0, B, L, tmask, 0), blocks.Stream(r1, B, L, tmask, 1)]
-        vg = x_in.operand(lowp)[0:B * G]
-        vl = x_in.operand(lowp)[r_l:r_l + B * P]
-        for cp, kvp, sp in zip(pk['x_cross'], pk['l2v_kv'], pk['l2v_self']):
-            wg, bg = kvp[0].get(lowp)
-            wl, bl = kvp[1].get(lowp)
-            kv_g = ops.gemm(vg, wg, bg)                          # [B*G, 1536] = K | V of the map tokens (global weights)
-            kv_l = ops.gemm(vl, wl, bl)                          # [B*P, 1536] of the panorama tokens (local weights)
-            q = blocks.gemm_act(lang, cp.q, lowp, ends)
-            ctx = blocks._ctx_buffer(R, q, streams)
-            ops.attention_multi([
-                dict(q=streams[0].view(q), k=kv_g[:, :HID], v=kv_g[:, HID:], out=streams[0].view(ctx), B=B, Lq=L, Lk=G, key_mask=gmask),
-                dict(q=streams[1].view(q), k=kv_l[:, :HID], v=kv_l[:, HID:], out=streams[1].view(ctx), B=B, Lq=L, Lk=P, key_mask=vmask)])
-            lang = blocks.linear_residual_ln(ctx, cp.o, lang, cp.ln, 1e-12, lowp, ends, defer=True)
-            lang = blocks.self_attn_ffn(lang, sp, streams, ends, lowp, defer=True)
-        lang = blocks.materialize(lang, lowp, ends, want16=False)
-        return lang.f32[r0:r0 + B * L], lang.f32[r1:r1 + B * L]
-
-    # -- the same trunk with autograd recording (pre-training) -------------------------------------------------------------
     def _recording(self) -> bool:
         return torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
 
-    def _trunk_train(self, batch, want_l2v=False):
-        """_trunk with autograd recording: the same layer sequence from the differentiable blocks (as duet._navigation_train).
-        The gathers of the panorama rows become autograd nodes: the vp-image gather a row gather (adjoint: scatter-add), the
-        graph-node aggregation a ragged segment mean (one view row can sit in a visited and an unvisited segment)."""
+    def _trunk(self, batch, want_l2v=False):
+        """GlocalTextPathCMT.forward / forward_mlm, model/vilmodel.py:660-747 -> dict of row-stacked results.  In training the
+        gathers of the panorama rows are autograd nodes: the vp-image gather a row gather (adjoint: scatter-add), the graph-node
+        aggregation a ragged segment mean (one view row can sit in a visited and an unvisited segment)."""
         blocks, duet, ops, params = _lazy()
-        from . import autograd_ops as ag
         bert = self.bert
-        lowp, pk = bert.lowp, bert._pk()
+        lowp = bert.lowp
         dev = bert.embeddings.LayerNorm.weight.device
         F32, HID = torch.float32, 768
         to = lambda t, dt=None: torch.as_tensor(t).to(dev, dtype=dt, non_blocking=True)     # noqa: E731
         txt_ids = to(batch['txt_ids'])
         B, L = txt_ids.shape
         txt_masks = torch.arange(L, device=dev)[None, :] < to(batch['txt_lens'])[:, None]
-        txt = bert.forward_text(txt_ids, txt_masks)
+        txt = bert.forward_text(txt_ids, txt_masks)                                  # (B, L, 768) fp32
+        # every panorama of every trajectory through the panorama encoder (vilmodel.py:484-528)
         step_lens = [int(x) for x in batch['traj_step_lens']]
         pano, _ = bert.forward_panorama_per_step(to(batch['traj_view_img_fts'], F32), None, to(batch['traj_loc_fts'], F32),
                                                  to(batch['traj_nav_types']), to(batch['traj_vp_view_lens']), None)
         N, V, _ = pano.shape
         vl_host = [int(x) for x in batch['traj_vp_view_lens']]
         last = np.cumsum(step_lens) - 1
+        # local branch: [stop] + the LAST panorama of each trajectory (vilmodel.py:538-553)
         P = max(vl_host[i] for i in last) + 1
         vp_idx = np.full((B, P), N * V, np.int64)                                       # row N * V: the appended zero row
         for b, i in enumerate(last):
@@ -356,84 +249,70 @@ class GlocalTextPathCMTPreTraining(nn.Module):
             vp_idx[b, 1:1 + n] = i * V + np.arange(n)
         vp_lens = torch.as_tensor([vl_host[i] + 1 for i in last], device=dev)
         vp_masks = torch.arange(P, device=dev)[None, :] < vp_lens[:, None]
+        # global branch: the graph-node features aggregated from the trajectory (vilmodel.py:577-611) in one segment mean
         off, rows, G = gmap_aggregation_rows(step_lens, vl_host, batch['traj_vpids'], batch['traj_cand_vpids'],
                                              batch['gmap_vpids'], V)
         gmap_masks = torch.arange(G, device=dev)[None, :] < to(batch['gmap_lens'])[:, None]
-        le, ge = bert.local_encoder, bert.global_encoder
-        with blocks.grad_mode(True, bert._drop()):
-            src = torch.cat([pano.reshape(N * V, HID), torch.zeros((1, HID), dtype=F32, device=dev)], 0)
-            vp_img = ag.GatherRowsFn.apply(src, torch.from_numpy(vp_idx.reshape(-1)).to(dev), 0, B * P)
-            gmap_img = ag.RaggedMeanFn.apply(src, torch.from_numpy(off).to(dev), torch.from_numpy(rows).to(dev), B * G)
-            (r_g, r_l), ends, R = blocks.stack_layout([B * G, B * P])
-            g_in = blocks.embed(B * G, dev, a=gmap_img, feat=to(batch['gmap_pos_fts'], F32).reshape(B * G, -1).contiguous(),
-                                feat_lin=ge.gmap_pos_embeddings[0], feat_ln=ge.gmap_pos_embeddings[1],
-                                idx=to(batch['gmap_step_ids']).long().contiguous().view(-1), table=ge.gmap_step_embeddings.weight).f32
-            l_in = blocks.embed(B * P, dev, a=vp_img, feat=to(batch['vp_pos_fts'], F32).reshape(B * P, -1).contiguous(),
-                                feat_lin=le.vp_pos_embeddings[0], feat_ln=le.vp_pos_embeddings[1]).f32
-            parts = [g_in] + ([torch.zeros((r_l - B * G, HID), dtype=F32, device=dev)] if r_l > B * G else []) + [l_in]
-            x = blocks.as_act(torch.cat(parts, 0), lowp)
-            out = dict(B=B, L=L, G=G, P=P, r_l=r_l, ends=ends, dev=dev, last=last)
-            tmask = blocks.mask_u8(txt_masks)
-            if want_l2v:
-                out['l2v'] = self._lang2visn_train(x, txt, tmask, B, L, G, P, r_l, blocks.mask_u8(gmap_masks), blocks.mask_u8(vp_masks))
-                return out
-            ctx = blocks.operand(txt.reshape(B * L, HID), lowp)
-            affine = dist = aparams = None
-            if ge.sprel_linear is not None:
-                affine, dist = pk['sprel'].get(), to(batch['gmap_pair_dists'], F32).contiguous()
-                aparams = (ge.sprel_linear.weight, ge.sprel_linear.bias)
-            streams = [blocks.Stream(r_g, B, G, blocks.mask_u8(gmap_masks), 0, dist, affine, aparams),
-                       blocks.Stream(r_l, B, P, blocks.mask_u8(vp_masks), 1)]
-            for cp, sp in zip(pk['x_cross'], pk['x_self']):
-                kv = blocks.linear(ctx, cp.kv, lowp)                # [B*L, 4*768] = K_g | V_g | K_l | V_l
-                x = blocks.cross_attn(x, kv, [0, 2 * HID], L, tmask, cp, streams, ends, lowp)
-                x = blocks.self_attn_ffn(x, sp, streams, ends, lowp)
-            out['x'] = x
+        src = torch.cat([pano.reshape(N * V, HID), torch.zeros((1, HID), dtype=F32, device=dev)], 0)
+        vp_img = blocks.gather_rows(src, vp_idx.reshape(-1), B * P)
+        gmap_img = blocks.segment_mean(src, off, rows, B * G)
+        # input embeddings of both branches into one row-stacked activation (vilmodel.py:613-625, 538-553)
+        x, row0, ends = bert._branch_inputs(gmap_img, to(batch['gmap_pos_fts'], F32), to(batch['gmap_step_ids']), vp_img,
+                                            to(batch['vp_pos_fts'], F32), B, G, P)
+        out = dict(B=B, L=L, G=G, P=P, r_l=row0[1], ends=ends, dev=dev, last=last)
+        tmask = blocks.mask_u8(txt_masks)
+        if want_l2v:
+            out['l2v'] = self._lang2visn(x, txt, tmask, B, L, G, P, row0[1], blocks.mask_u8(gmap_masks), blocks.mask_u8(vp_masks))
+            return out
+        # the 4 graph-aware cross-modal layers; context = the instruction (no imagination tokens in pre-training)
+        streams = bert._branch_streams(B, G, P, row0, gmap_masks, vp_masks, to(batch['gmap_pair_dists'], F32))
+        out['x'] = bert._cross_layers(x, streams, ends, L, tmask, ctx=blocks.operand(txt.reshape(B * L, HID), lowp))
         return out
 
-    def _lang2visn_train(self, x_in, txt, tmask, B, L, G, P, r_l, gmask, vmask):
-        """_lang2visn with autograd recording.  Both language streams start from the same text rows, so their gradients sum
-        back into the text encoder; both attention problems (text -> map, text -> panorama) run as one AttentionFn node."""
+    def _lang2visn(self, x_in, txt, tmask, B, L, G, P, r_l, gmask, vmask):
+        """GraphLXRTXLayer.forward_lang2visn x 4 for both branches (vilmodel.py:400-411, 719-735): the instruction attends to
+        the (fixed) map / panorama input embeddings; two language streams (global | local weights) stacked along the rows.  In
+        training both start from the same text rows, so their gradients sum back into the text encoder."""
         blocks, duet, ops, params = _lazy()
-        from . import autograd_ops as ag
         bert = self.bert
         lowp, pk = bert.lowp, bert._pk()
-        HID = 768
-        dev = txt.device
-        (r0, r1), ends, R = blocks.stack_layout([B * L, B * L])
-        t32 = txt.reshape(B * L, HID)
-        parts = [t32] + ([torch.zeros((r1 - B * L, HID), dtype=torch.float32, device=dev)] if r1 > B * L else []) + [t32]
-        lang = blocks.as_act(torch.cat(parts, 0), lowp)
-        streams = [blocks.Stream(r0, B, L, tmask, 0), blocks.Stream(r1, B, L, tmask, 1)]
+        row0, ends, R = blocks.stack_layout([B * L, B * L])
+        t32 = txt.reshape(B * L, 768)
+        lang = blocks.as_act(blocks.stack_rows([t32, t32], row0), lowp)
+        streams = [blocks.Stream(row0[0], B, L, tmask, 0), blocks.Stream(row0[1], B, L, tmask, 1)]
         vg = x_in.operand(lowp)[0:B * G]
         vl = x_in.operand(lowp)[r_l:r_l + B * P]
         for cp, kvp, sp in zip(pk['x_cross'], pk['l2v_kv'], pk['l2v_self']):
-            kv_g = blocks.linear(vg, kvp[0], lowp)                  # [B*G, 1536] = K | V of the map tokens (global weights)
-            kv_l = blocks.linear(vl, kvp[1], lowp)                  # [B*P, 1536] of the panorama tokens (local weights)
-            q = blocks.linear(lang.operand(lowp), cp.q, lowp, ends=ends)
-            spec = [dict(q=(0, r0, 0), k=(1, 0, 0), v=(1, 0, HID), B=B, Lq=L, Lk=G, key_mask=gmask, out_row0=r0,
-                         drop=blocks._attn_drop(dev)),
-                    dict(q=(0, r1, 0), k=(2, 0, 0), v=(2, 0, HID), B=B, Lq=L, Lk=P, key_mask=vmask, out_row0=r1,
-                         drop=blocks._attn_drop(dev))]
-            ctx = ag.AttentionFn.apply(spec, R, ops.MASK_ADD_NEG10000, 3, q, kv_g, kv_l)
-            lang = blocks._dense_res_ln(ctx, cp.o, lang.f32, cp.ln, 1e-12, lowp, ends)
-            lang = blocks.self_attn_ffn(lang, sp, streams, ends, lowp)
-        return lang.f32[r0:r0 + B * L], lang.f32[r1:r1 + B * L]
+            kv_g = blocks.linear(vg, kvp[0], lowp)               # [B*G, 1536] = K | V of the map tokens (global weights)
+            kv_l = blocks.linear(vl, kvp[1], lowp)               # [B*P, 1536] of the panorama tokens (local weights)
+            lang = blocks.cross_attn(lang, [(kv_g, 0, G, gmask), (kv_l, 0, P, vmask)], cp, streams, ends, lowp, defer=True)
+            lang = blocks.self_attn_ffn(lang, sp, streams, ends, lowp, defer=True)
+        lang = blocks.materialize(lang, lowp, ends, want16=False)
+        return lang.f32[row0[0]:row0[0] + B * L], lang.f32[row0[1]:row0[1] + B * L]
 
-    def _head_train(self, h32, lin, act, ln, dec, lowp):
-        """Linear -> act -> LayerNorm(1e-12) -> padded Linear with autograd recording -> (scores, gradient handle)"""
+    def _head(self, x, lin, act, ln, dec):
+        """GEMM operand -> Linear -> act -> LayerNorm(1e-12) -> padded Linear -> (scores [rows, n_pad], gradient handle)"""
         blocks, duet, ops, params = _lazy()
-        from . import autograd_ops as ag
-        with blocks.grad_mode(True, self.bert._drop()):
-            hidden = ag.ActFn.apply(blocks.linear(blocks.operand(h32, lowp), lin, lowp, out_dtype=torch.float32), act)
-            y = blocks.layer_norm(hidden, None, ln, 1e-12, lowp)
-            return ag.padded_linear(y.operand(lowp), dec, lowp)
+        lowp = self.bert.lowp
+        y = blocks.layer_norm(blocks.linear(x, lin, lowp, out_dtype=torch.float32, epilogue=act), None, ln, 1e-12, lowp)
+        return dec(y.operand(lowp), lowp)
+
+    @staticmethod
+    def _row_loss(kl, logits, handle, target, n_cols):
+        """per-row KL (soft targets) or cross-entropy (labels) over the first n_cols columns.  Training: the loss node sends the
+        logits' gradient to ``handle`` (PaddedLinearFn's, or the logits themselves when None)."""
+        blocks, duet, ops, params = _lazy()
+        if blocks.training():
+            from . import autograd_ops as ag
+            fn = ag.KLRowsFn if kl else ag.CERowsFn
+            return fn.apply(logits, logits if handle is None else handle, target, n_cols)
+        return (ops.kl_rows if kl else ops.ce_rows)(logits, target, n_cols)
 
     # -- tasks -----------------------------------------------------------------------------------------------------------
     def forward(self, batch, task, compute_loss=True):
         """With autograd recording (parameters that require grad, grad mode on) every step records a node whose forward and
         backward are libvlnimagine kernels; ``compute_loss=True`` returns the per-row losses the reference's trainer averages.
-        Under torch.no_grad() the inference path runs."""
+        Under torch.no_grad() the same steps run as plain launches."""
         blocks, duet, ops, params = _lazy()
         with ops.half_format(self.bert.h16_format()):
             if task.startswith('mlm'):
@@ -447,87 +326,53 @@ class GlocalTextPathCMTPreTraining(nn.Module):
     def forward_mlm(self, batch, compute_loss=True):
         """pretrain_cmt.py:128-150: prediction scores [n_masked, vocab] (or the per-token cross-entropy)"""
         blocks, duet, ops, params = _lazy()
-        if self._recording():
-            return self._mlm_train(batch, compute_loss)
-        t = self._trunk(batch, want_l2v=True)
-        lowp, dev, hp = self.bert.lowp, t['dev'], self._hp()
-        gt, vt = t['l2v']
-        labels = torch.as_tensor(batch['txt_labels'])
-        pos = torch.nonzero(labels.reshape(-1) != -1).flatten()
-        n = int(pos.numel())
-        idx = pos.to(torch.int32).to(dev)
-        unit = torch.arange(n + 1, dtype=torch.int32, device=dev)
-        a, _ = ops.gather_mean(gt, unit, idx, n, want16=False)
-        b, _ = ops.gather_mean(vt, unit, idx, n, want16=False)
-        h32, h16 = ops.embed_compose(n, dev, a=a, a2=b, want16=lowp)               # (global + local) text states of the masked tokens
-        w, bias = hp['mlm_t'].get(lowp)
-        hidden = ops.gemm(h16 if lowp else h32, w, bias, epilogue=ops.EPI_GELU, out_dtype=torch.float32)
-        pr = self.mlm_head.predictions
-        y32, y16 = ops.add_ln(hidden, None, pr.transform.LayerNorm.weight, pr.transform.LayerNorm.bias, 1e-12, want16=lowp)
-        w, bias, vocab = hp['mlm_dec'].get(lowp)
-        scores = ops.gemm(y16 if lowp else y32, w, bias, out_dtype=torch.float32)   # [n, 30528]: the padded tail is never read
-        if compute_loss:
-            return ops.ce_rows(scores, labels.reshape(-1)[pos].to(dev), vocab)
-        return scores[:, :vocab]
+        with blocks.grad_mode(self._recording(), self.bert._drop()):
+            t = self._trunk(batch, want_l2v=True)
+            lowp, dev, hp = self.bert.lowp, t['dev'], self._hp()
+            gt, vt = t['l2v']
+            labels = torch.as_tensor(batch['txt_labels'])
+            pos = torch.nonzero(labels.reshape(-1) != -1).flatten()
+            n = int(pos.numel())
+            h = blocks.embed(n, dev, a=blocks.gather_rows(gt, pos, n), a2=blocks.gather_rows(vt, pos, n), lowp=lowp)
+            scores, handle = self._head(h.operand(lowp), hp['mlm_t'], ops.EPI_GELU, hp['mlm_ln'], hp['mlm_dec'])
+            vocab = hp['mlm_dec'].n                     # the padded tail columns are never read
+            if compute_loss:
+                return self._row_loss(False, scores, handle, labels.reshape(-1)[pos].to(dev), vocab)
+            return scores[:, :vocab]
 
     def forward_mrc(self, batch, compute_loss=True):
         """pretrain_cmt.py:158-204 (views only): soft-label classification of the masked views of the last panorama"""
         blocks, duet, ops, params = _lazy()
-        if self._recording():
-            return self._mrc_train(batch, compute_loss)
-        t = self._trunk(batch)          # the global branch is independent of the local one: running both changes nothing
-        lowp, dev, hp = self.bert.lowp, t['dev'], self._hp()
-        B, P, r_l = t['B'], t['P'], t['r_l']
-        masks = torch.as_tensor(batch['vp_view_mrc_masks'])
-        bi, vi = torch.nonzero(masks, as_tuple=True)
-        rows = (r_l + bi * P + 1 + vi).to(torch.int32).to(dev)                      # token 0 of every episode is [stop]
-        n = int(rows.numel())
-        unit = torch.arange(n + 1, dtype=torch.int32, device=dev)
-        h32, h16 = ops.gather_mean(t['x'].f32, unit, rows, n, want16=lowp, want32=not lowp)
-        w, bias = hp['mrc0'].get(lowp)
-        hidden = ops.gemm(h16 if lowp else h32, w, bias, epilogue=ops.EPI_RELU, out_dtype=torch.float32)
-        net = self.image_classifier.net
-        y32, y16 = ops.add_ln(hidden, None, net[2].weight, net[2].bias, 1e-12, want16=lowp)
-        w, bias, n_cls = hp['mrc3'].get(lowp)
-        logits = ops.gemm(y16 if lowp else y32, w, bias, out_dtype=torch.float32)
-        targets = torch.as_tensor(batch['vp_view_probs'])[masks].to(dev, torch.float32).contiguous()
-        if compute_loss:
-            return ops.kl_rows(logits, targets, n_cls)
-        return logits[:, :n_cls], targets
+        with blocks.grad_mode(self._recording(), self.bert._drop()):
+            t = self._trunk(batch)      # the global branch is independent of the local one: running both changes nothing
+            lowp, dev, hp = self.bert.lowp, t['dev'], self._hp()
+            P, r_l = t['P'], t['r_l']
+            masks = torch.as_tensor(batch['vp_view_mrc_masks'])
+            bi, vi = torch.nonzero(masks, as_tuple=True)
+            rows = r_l + bi * P + 1 + vi                                            # token 0 of every episode is [stop]
+            h = blocks.gather_rows(t['x'].f32, rows, int(rows.numel()), lowp=lowp)
+            logits, handle = self._head(h, hp['mrc0'], ops.EPI_RELU, hp['mrc_ln'], hp['mrc3'])
+            n_cls = hp['mrc3'].n
+            targets = torch.as_tensor(batch['vp_view_probs'])[masks].to(dev, torch.float32).contiguous()
+            if compute_loss:
+                return self._row_loss(True, logits, handle, targets, n_cls)
+            return logits[:, :n_cls], targets
 
     def forward_sap(self, batch, compute_loss=True):
         """pretrain_cmt.py:206-262: global / local / fused action logits (or the three summed cross-entropies)"""
         blocks, duet, ops, params = _lazy()
-        if self._recording():
-            return self._sap_train(batch, compute_loss)
-        t = self._trunk(batch)
-        lowp, dev, hp = self.bert.lowp, t['dev'], self._hp()
-        B, G, P, r_l, ends, x = t['B'], t['G'], t['P'], t['r_l'], t['ends'], t['x']
-        fuse_raw = None
-        if 'fuse' in hp:
-            cat = torch.empty((B, 2 * 768), dtype=ops.h16() if lowp else torch.float32, device=dev)
-            c32, c16 = (None, cat) if lowp else (cat, None)
-            ops.copy_rows(x.f32, G * 768, 768, B, 1, c32, c16, 2 * 768, 768)
-            ops.copy_rows(x.f32[r_l:], P * 768, 768, B, 1, c32[:, 768:] if c32 is not None else None,
-                          c16[:, 768:] if c16 is not None else None, 2 * 768, 768)
-            fuse_raw = blocks.cls_head(cat, hp['fuse'], lowp)
-        raw = blocks.cls_head(x.operand(lowp), hp['sap'], lowp, ends)
-        gmap_masks = torch.arange(G, device=dev)[None, :] < torch.as_tensor(batch['gmap_lens']).to(dev)[:, None]
-        visited = torch.as_tensor(batch['gmap_visited_masks']).to(dev)
-        last = t['last']
-        nav_types = torch.as_tensor(batch['traj_nav_types'])[torch.as_tensor(last)]
-        nav = torch.zeros((B, P), dtype=torch.bool)
-        nav[:, 0] = True                                        # [stop] is always admissible (pretrain_cmt.py:231-236)
-        nav[:, 1:] = nav_types[:, :P - 1] == 1
-        cand = [[None] + list(c[-1]) for c in batch['traj_cand_vpids']]
-        gmap_ids, cand_ids = self.bert.intern_vpids(batch['gmap_vpids'], cand, G, P, dev)
-        gl, ll, fl = ops.duet_fuse_logits(raw[0:], raw[r_l:], fuse_raw, blocks.mask_u8(gmap_masks), blocks.mask_u8(visited),
-                                          blocks.mask_u8(nav.to(dev)), gmap_ids, cand_ids, B, G, P)
-        if compute_loss:
-            ga = torch.as_tensor(batch['global_act_labels']).to(dev)
-            la = torch.as_tensor(batch['local_act_labels']).to(dev)
-            return ops.ce_rows(gl, ga, G) + ops.ce_rows(ll, la, P) + ops.ce_rows(fl, ga, G)
-        return gl, ll, fl
+        with blocks.grad_mode(self._recording(), self.bert._drop()):
+            t = self._trunk(batch)
+            dev, hp = t['dev'], self._hp()
+            B, G, P, row0 = t['B'], t['G'], t['P'], (0, t['r_l'])
+            raw, fuse_raw = self.bert._sap_heads(t['x'], hp['sap'], hp.get('fuse'), B, G, P, row0, t['ends'])
+            gl, ll, fl = self.bert._fuse_step(raw, fuse_raw, *self._sap_masks(batch, t), B, G, P, row0)
+            if compute_loss:
+                ga = torch.as_tensor(batch['global_act_labels']).to(dev)
+                la = torch.as_tensor(batch['local_act_labels']).to(dev)
+                return (self._row_loss(False, gl, None, ga, G) + self._row_loss(False, ll, None, la, P)
+                        + self._row_loss(False, fl, None, ga, G))
+            return gl, ll, fl
 
     def _sap_masks(self, batch, t):
         """(gmap masks, visited masks, navigable masks of the local tokens, gmap ids, candidate ids) of forward_sap"""
@@ -541,63 +386,6 @@ class GlocalTextPathCMTPreTraining(nn.Module):
         cand = [[None] + list(c[-1]) for c in batch['traj_cand_vpids']]
         gmap_ids, cand_ids = self.bert.intern_vpids(batch['gmap_vpids'], cand, G, P, dev)
         return gmap_masks, visited, nav.to(dev), gmap_ids, cand_ids
-
-    def _mlm_train(self, batch, compute_loss):
-        blocks, duet, ops, params = _lazy()
-        from . import autograd_ops as ag
-        t = self._trunk_train(batch, want_l2v=True)
-        lowp, dev, hp = self.bert.lowp, t['dev'], self._hp()
-        gt, vt = t['l2v']
-        labels = torch.as_tensor(batch['txt_labels'])
-        pos = torch.nonzero(labels.reshape(-1) != -1).flatten()
-        n = int(pos.numel())
-        idx = pos.to(dev)
-        with blocks.grad_mode(True, self.bert._drop()):
-            h = ag.SumRowsFn.apply(2, ag.GatherRowsFn.apply(gt, idx, 0, n), ag.GatherRowsFn.apply(vt, idx, 0, n))
-        scores, handle = self._head_train(h, hp['mlm_t'], ops.EPI_GELU, hp['mlm_ln'], hp['mlm_dec'], lowp)
-        vocab = hp['mlm_dec'].n
-        if compute_loss:
-            return ag.CERowsFn.apply(scores, handle, labels.reshape(-1)[pos].to(dev), vocab)
-        return scores[:, :vocab]
-
-    def _mrc_train(self, batch, compute_loss):
-        blocks, duet, ops, params = _lazy()
-        from . import autograd_ops as ag
-        t = self._trunk_train(batch)
-        lowp, dev, hp = self.bert.lowp, t['dev'], self._hp()
-        B, P, r_l = t['B'], t['P'], t['r_l']
-        masks = torch.as_tensor(batch['vp_view_mrc_masks'])
-        bi, vi = torch.nonzero(masks, as_tuple=True)
-        rows = (r_l + bi * P + 1 + vi).to(dev)
-        with blocks.grad_mode(True, self.bert._drop()):
-            h = ag.GatherRowsFn.apply(t['x'].f32, rows, 0, int(rows.numel()))
-        logits, handle = self._head_train(h, hp['mrc0'], ops.EPI_RELU, hp['mrc_ln'], hp['mrc3'], lowp)
-        n_cls = hp['mrc3'].n
-        targets = torch.as_tensor(batch['vp_view_probs'])[masks].to(dev, torch.float32).contiguous()
-        if compute_loss:
-            return ag.KLRowsFn.apply(logits, handle, targets, n_cls)
-        return logits[:, :n_cls], targets
-
-    def _sap_train(self, batch, compute_loss):
-        blocks, duet, ops, params = _lazy()
-        from . import autograd_ops as ag
-        t = self._trunk_train(batch)
-        lowp, dev, hp = self.bert.lowp, t['dev'], self._hp()
-        B, G, P, r_l, ends, x = t['B'], t['G'], t['P'], t['r_l'], t['ends'], t['x']
-        gmap_masks, visited, nav, gmap_ids, cand_ids = self._sap_masks(batch, t)
-        with blocks.grad_mode(True, self.bert._drop()):
-            fuse_raw = None
-            if 'fuse' in hp:
-                cat = torch.cat([x.f32[0:B * G].view(B, G, 768)[:, 0], x.f32[r_l:r_l + B * P].view(B, P, 768)[:, 0]], 1)
-                fuse_raw = blocks.cls_head(blocks.operand(cat, lowp), hp['fuse'], lowp)
-            raw = blocks.cls_head(x.operand(lowp), hp['sap'], lowp, ends)
-            gl, ll, fl = ag.FuseLogitsFn.apply(raw[0:B * G], raw[r_l:r_l + B * P], fuse_raw, blocks.mask_u8(gmap_masks),
-                                               blocks.mask_u8(visited), blocks.mask_u8(nav), gmap_ids, cand_ids, B, G, P)
-        if compute_loss:
-            ga = torch.as_tensor(batch['global_act_labels']).to(dev)
-            la = torch.as_tensor(batch['local_act_labels']).to(dev)
-            return ag.CERowsFn.apply(gl, gl, ga, G) + ag.CERowsFn.apply(ll, ll, la, P) + ag.CERowsFn.apply(fl, fl, ga, G)
-        return gl, ll, fl
 
 
 class _PaddedLinear:
@@ -638,10 +426,15 @@ class _PaddedLinear:
             v[key] = ops.cast_h16(v['w32'], dtype=key[1])
         return v[key], v['b']
 
-    def get(self, lowp: bool):
-        """(weight, bias, n) of the inference GEMM"""
+    def __call__(self, x, lowp: bool):
+        """x W^T + b -> (fp32 scores [rows, n_pad], gradient handle).  Training: autograd_ops.PaddedLinearFn over the
+        128-padded weight.  Inference: one GEMM over the 64-padded weight (handle None)."""
+        blocks, duet, ops, params = _lazy()
+        if blocks.training():
+            from .autograd_ops import padded_linear
+            return padded_linear(x, self, lowp)
         w, b = self._get(lowp, 64)
-        return w, b, self.n
+        return ops.gemm(x, w, b, out_dtype=torch.float32), None
 
     def get_train(self, lowp: bool):
         """(weight, bias) of the training GEMM: bf16 shadow or fp32, padded to a multiple of 128 rows"""
