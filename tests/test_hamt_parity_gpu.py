@@ -207,3 +207,17 @@ def test_hamt_action_token_variants_vs_reference_golden(lib_built, concat, tok):
             assert max_rel(outs[0], ref) < TOL[precision], (tag, precision)
             if precision == 'fp32':
                 assert torch.equal(outs[0].cpu().argmax(-1), ref.argmax(-1))
+            # the same call with autograd recording (eval(): no dropout) matches the reference too, and every parameter of the
+            # cross-modal layers, the observation embedding and the action head gets a finite gradient
+            model.zero_grad(set_to_none=True)
+            logits = model('visual', txt_embeds=txt, txt_masks=ep['txt_masks'], hist_embeds=hist_list, hist_lens=hist_lens,
+                           ob_img_feats=ep['ob_img_feats'], ob_ang_feats=ep['ob_ang_feats'], ob_nav_types=ep['ob_nav_types'],
+                           ob_masks=ep['ob_masks'], imagine_embeds=img, imagine_masks=ep['imagine_masks'])[0]
+            assert logits.requires_grad
+            assert max_rel(logits, ref) < TOL[precision], (tag, precision, 'recording')
+            logits.sum().backward()
+            trained = [(n, p) for n, p in model.vln_bert.named_parameters()
+                       if p.requires_grad and n.startswith(('encoder.x_layers.', 'img_embeddings.', 'next_action.'))]
+            assert trained
+            bad = [n for n, p in trained if p.grad is None or not bool(torch.isfinite(p.grad).all())]
+            assert not bad, (tag, precision, bad)

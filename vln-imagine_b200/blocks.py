@@ -506,33 +506,39 @@ class SelfFFNPack:
         self.ln2 = LNPack([m.LayerNorm for m in outs])
 
 
+def attn(x: Act, qkv: LinearPack, o: LinearPack, ln: LNPack, streams: List[Stream], ends, lowp: bool, eps=1e-12,
+         kv_of=None) -> Act:
+    """LN(x + O(attn(QKV(x)))) over all rows, the LayerNorm left pending in inference.  Stream i reads the keys / values of
+    streams[kv_of[i]] (default: its own, self-attention).  HAMT's cross-modal layer is kv_of = (1, 0): both directions share
+    one QKV / output projection (H/models/vilmodel_cmt.py:385-397).  Group ends reach a call only when its weights or
+    LayerNorm have per-stream groups."""
+    rows = x.f32.shape[0]
+    kvs = streams if kv_of is None else [streams[j] for j in kv_of]
+    if _Mode.train:
+        xin = x.operand(lowp)
+        t = ag.linear(xin, qkv, lowp, ends=_call_groups(qkv, None, ends)[1])
+        spec, extras = [], ()
+        for s, k in zip(streams, kvs):
+            spec.append(dict(q=(0, s.row0, 0), k=(0, k.row0, HIDDEN), v=(0, k.row0, 2 * HIDDEN), B=s.B, Lq=s.L, Lk=k.L,
+                             key_mask=k.mask, pair_dist=s.pair_dist, bias_affine=s.bias_affine, out_row0=s.row0,
+                             drop=_attn_drop(xin.device)))
+            if s.pair_dist is not None and s.affine_params is not None:
+                extras = tuple(s.affine_params)
+        ctx = ag.AttentionFn.apply(spec, rows, MASK_ADD_NEG10000, 1, t, *extras)
+        return _dense_res_ln(ctx, o, x.f32, ln, eps, lowp, _call_groups(o, ln, ends)[1])
+    t = gemm_act(x, qkv, lowp, ends)                                   # [rows, 2304]
+    ctx = _ctx_buffer(rows, t, streams)
+    ops.attention_multi([dict(q=s.view(t)[:, 0:HIDDEN], k=k.view(t)[:, HIDDEN:2 * HIDDEN], v=k.view(t)[:, 2 * HIDDEN:3 * HIDDEN],
+                              out=s.view(ctx), B=s.B, Lq=s.L, Lk=k.L, key_mask=k.mask, pair_dist=s.pair_dist,
+                              bias_affine=s.bias_affine) for s, k in zip(streams, kvs)])
+    return linear_residual_ln(ctx, o, x, ln, eps, lowp, ends, defer=True)
+
+
 def self_attn_ffn(x: Act, pk: SelfFFNPack, streams: List[Stream], ends, lowp: bool, eps=1e-12, defer=False) -> Act:
     """Post-LN BERT layer: LN(x + O(attn(QKV(x)))) then LN(y + W2 gelu(W1 y)).  ``defer``: the last LayerNorm may stay
     pending for the next block (blocks.Pending).
     Reference: BertLayer, VLN-DUET/map_nav_src/models/vilmodel.py:196-209 (and :80-194)."""
-    rows = x.f32.shape[0]
-    if _Mode.train:
-        xin = x.operand(lowp)
-        qkv = ag.linear(xin, pk.qkv, lowp, ends=ends)
-        spec, extras = [], ()
-        for s in streams:
-            spec.append(dict(q=(0, s.row0, 0), k=(0, s.row0, HIDDEN), v=(0, s.row0, 2 * HIDDEN), B=s.B, Lq=s.L, Lk=s.L,
-                             key_mask=s.mask, pair_dist=s.pair_dist, bias_affine=s.bias_affine, out_row0=s.row0,
-                             drop=_attn_drop(xin.device)))
-            if s.pair_dist is not None and s.affine_params is not None:
-                extras = tuple(s.affine_params)
-        ctx = ag.AttentionFn.apply(spec, rows, MASK_ADD_NEG10000, 1, qkv, *extras)
-        y = _dense_res_ln(ctx, pk.o, x.f32, pk.ln1, eps, lowp, ends)
-        return ffn(y, pk.w1, pk.w2, pk.ln2, ends, lowp, eps)
-    qkv = gemm_act(x, pk.qkv, lowp, ends)                              # [rows, 2304]
-    ctx = _ctx_buffer(rows, qkv, streams)
-    probs = []
-    for s in streams:
-        q = s.view(qkv)
-        probs.append(dict(q=q[:, 0:HIDDEN], k=q[:, HIDDEN:2 * HIDDEN], v=q[:, 2 * HIDDEN:3 * HIDDEN], out=s.view(ctx),
-                          B=s.B, Lq=s.L, Lk=s.L, key_mask=s.mask, pair_dist=s.pair_dist, bias_affine=s.bias_affine))
-    ops.attention_multi(probs)
-    y = linear_residual_ln(ctx, pk.o, x, pk.ln1, eps, lowp, ends, defer=True)
+    y = attn(x, pk.qkv, pk.o, pk.ln1, streams, ends, lowp, eps)
     return ffn(y, pk.w1, pk.w2, pk.ln2, ends, lowp, eps, defer=defer)
 
 
@@ -616,6 +622,61 @@ def embed_streams(specs, row0: Sequence[int], rows: int, device, lowp: bool) -> 
     return Act(x32, x16)
 
 
+def stack_segments(parts, row0: Sequence[int], lowp: bool) -> Act:
+    """Streams made of token segments: parts[i] lists the fp32 [B, n_k, 768] segments that stream i concatenates along its
+    tokens, stacked on the stack_layout boundaries.  Inference: one vi_copy_rows per segment into one preallocated
+    activation, the gap behind each stream zero-filled.  Training: torch.cat per stream, stacked by stack_rows."""
+    if _Mode.train:
+        return as_act(stack_rows([(s[0] if len(s) == 1 else torch.cat(s, 1)).reshape(-1, HIDDEN) for s in parts], row0), lowp)
+    B, dev = parts[0][0].shape[0], parts[0][0].device
+    lens = [sum(seg.shape[1] for seg in s) for s in parts]
+    rows = row0[-1] + B * lens[-1]
+    x32 = torch.empty((rows, HIDDEN), dtype=F32, device=dev)
+    x16 = torch.empty((rows, HIDDEN), dtype=ops.h16(), device=dev) if lowp else None
+    for i in range(len(parts) - 1):
+        r0, r1 = row0[i] + B * lens[i], row0[i + 1]
+        if r1 > r0:
+            x32[r0:r1].zero_()
+            if lowp:
+                x16[r0:r1].zero_()
+    for s, r0, n in zip(parts, row0, lens):
+        for seg in s:
+            k = seg.shape[1]
+            ops.copy_rows(seg, k * HIDDEN, HIDDEN, B, k, x32[r0:], x16[r0:] if lowp else None, n * HIDDEN, HIDDEN)
+            r0 += k
+    return Act(x32, x16)
+
+
+def take_rows(v: torch.Tensor, lowp: Optional[bool] = None) -> torch.Tensor:
+    """[B, n, 768] view of episode-strided fp32 rows -> contiguous [B * n, 768] rows (fp32); with ``lowp`` given, the GEMM
+    operand of that precision instead.  Inference: one vi_copy_rows reading the view in place."""
+    if _Mode.train:
+        y = v.reshape(-1, HIDDEN)
+        return y.contiguous() if lowp is None else operand(y, lowp)
+    B, n = v.shape[0], v.shape[1]
+    y32 = torch.empty((B * n, HIDDEN), dtype=F32, device=v.device) if not lowp else None
+    y16 = torch.empty((B * n, HIDDEN), dtype=ops.h16(), device=v.device) if lowp else None
+    ops.copy_rows(v, v.stride(0), HIDDEN, B, n, y32, y16, n * HIDDEN, HIDDEN)
+    return y16 if lowp else y32
+
+
+def mul_bcast(x: torch.Tensor, s: torch.Tensor, lowp: bool) -> torch.Tensor:
+    """y[b, r] = x[b, r] * s[b] for x a [B, n, 768] and s a [B, 768] view of fp32 rows -> the [B * n, 768] GEMM operand.
+    Inference: one vi_mul_bcast reading both views in place.  Training: MulBcastFn."""
+    if _Mode.train:
+        return ag.MulBcastFn.apply(x, s, lowp)
+    y32, y16 = ops.mul_bcast(x, x.stride(0), s, s.stride(0), x.shape[0], x.shape[1], want16=lowp, want32=not lowp)
+    return y16 if lowp else y32
+
+
+def mask_logits(raw: torch.Tensor, keep: torch.Tensor) -> torch.Tensor:
+    """raw logits, one per row -> logits shaped like ``keep`` with -inf where keep == 0 (padding navigation type, no object).
+    Inference: vi_mask_logits_navtype.  Training: masked_fill."""
+    if _Mode.train:
+        return raw.view(keep.shape).masked_fill(keep == 0, float('-inf'))
+    return ops.mask_logits_navtype(raw, keep.long().contiguous().view(-1)).view(keep.shape)
+
+
 def gather_rows(src: torch.Tensor, idx, n: int, lowp: Optional[bool] = None) -> torch.Tensor:
     """rows = src[idx] (fp32); with ``lowp`` given, the GEMM operand of that precision instead.  Inference: one
     vi_gather_mean over unit segments.  Training: GatherRowsFn (adjoint: scatter-add)."""
@@ -631,12 +692,15 @@ def gather_rows(src: torch.Tensor, idx, n: int, lowp: Optional[bool] = None) -> 
     return y16 if lowp else y32
 
 
-def segment_mean(src: torch.Tensor, offsets, rows, n: int) -> torch.Tensor:
+def segment_mean(src: torch.Tensor, offsets, rows, n: int, seg: Optional[int] = None) -> torch.Tensor:
     """y[r] = mean of src[rows[offsets[r]:offsets[r+1]]] over ragged segments (int32 index arrays).  Inference: one
-    vi_gather_mean.  Training: RaggedMeanFn (a source row may sit in several segments)."""
+    vi_gather_mean.  Training: RaggedMeanFn (a source row may sit in several segments); with ``seg`` given, disjoint segments
+    of ``seg`` rows each, SegmentMeanFn (its adjoint is a plain row scatter)."""
     offsets = torch.as_tensor(offsets).to(src.device)
     rows = torch.as_tensor(rows).to(src.device)
     if _Mode.train:
+        if seg is not None:
+            return ag.SegmentMeanFn.apply(src, offsets, rows, n, seg)
         return ag.RaggedMeanFn.apply(src, offsets, rows, n)
     return ops.gather_mean(src, offsets, rows, n, want16=False)[0]
 
@@ -659,11 +723,11 @@ def operand(x32: torch.Tensor, lowp: bool) -> torch.Tensor:
 
 def embed(rows: int, device, *, a=None, a_ln=None, a2=None, feat=None, feat_lin=None, feat_ln=None, idx=None, table=None,
           pos_table=None, pos_period=0, const_rows=(), out_ln=None, eps=1e-12, lowp=False, y32=None, y16=None,
-          dropout=False, chain_ln=None, chain_eps=1e-5, zero_rows=0) -> Act:
+          dropout=False, chain_ln=None, chain_eps=1e-5, zero_rows=0, want32=True) -> Act:
     """Input-embedding composer  LN_out([LN_a](a) + a2 + LN_f(W feat + b) + table[idx] + pos[row % period] + consts).
     *_ln are nn.LayerNorm-like parameter holders, feat_lin an nn.Linear-like holder.  Inference: ONE fused kernel
-    (vi_embed_compose), which also zero-fills ``zero_rows`` rows behind the output.  Training: the same sum built from
-    differentiable primitives (autograd_ops)."""
+    (vi_embed_compose), which also zero-fills ``zero_rows`` rows behind the output; ``want32=False`` skips its fp32 output
+    when the 16-bit one is all the caller reads.  Training: the same sum built from differentiable primitives (autograd_ops)."""
     ln_pair = lambda m: (m.weight, m.bias) if m is not None else None      # noqa: E731
     if not _Mode.train:
         consts = list(const_rows) + [None, None]
@@ -681,7 +745,8 @@ def embed(rows: int, device, *, a=None, a_ln=None, a2=None, feat=None, feat_lin=
                                      feat_b=feat_lin.bias if feat_lin is not None else None, feat_ln=ln_pair(feat_ln),
                                      idx=idx, table=table, pos_table=pos_table, pos_period=pos_period,
                                      const_row=consts[0], const_row2=consts[1], out_ln=ln_pair(out_ln), eps=eps,
-                                     y32=y32, y16=y16, want16=lowp and y16 is None and (y32 is None), zero_rows=zero_rows)
+                                     y32=y32, y16=y16, want16=lowp and y16 is None and (y32 is None), want32=want32,
+                                     zero_rows=zero_rows)
         return Act(o32, o16)
     terms = []
     if a is not None:

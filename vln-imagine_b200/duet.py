@@ -25,7 +25,7 @@ from . import autograd_ops as ag
 from . import blocks, graphs, ops, params
 from .blocks import Stream
 from .config import duet_config
-from .ops import BF16, F32, HIDDEN
+from .ops import F32, HIDDEN
 
 
 def _f32c(t: torch.Tensor) -> torch.Tensor:
@@ -143,7 +143,10 @@ def _align_rows(B, L, I, flags, noun_phrase_segs, dev):
 
 def align_forward(model, align_txt_embeds, align_imagine_embeds, flags, noun_phrase_segs, lowp: bool, rows: AlignRows = None):
     """Shared by DUET and HAMT.  Returns (loss 0-d tensor, imagine embeds with projected rows written back).  ``rows``: index
-    arrays already built by the caller (REVERIE) instead of the sub-instruction annotation."""
+    arrays already built by the caller (REVERIE) instead of the sub-instruction annotation.  With autograd recording the
+    projection MLP, the loss and the write-back of the projected rows (models/vilmodel.py:646) are differentiable; the
+    noun-phrase means of the negatives are constants, and the text target trains only when the text requires grad
+    (fix_lang_inside_cosine_model off, :1256-1262)."""
     cfg = model.config
     B, L, _ = align_txt_embeds.shape
     I = align_imagine_embeds.shape[1]
@@ -151,77 +154,42 @@ def align_forward(model, align_txt_embeds, align_imagine_embeds, flags, noun_phr
     rows = rows.to(dev) if rows is not None else _align_rows(B, L, I, flags, noun_phrase_segs, dev)
     txt = _f32c(align_txt_embeds).view(B * L, HIDDEN)
     img = _f32c(align_imagine_embeds).view(B * I, HIDDEN)
-    out = img.clone()
     if rows.R == 0:
         # the reference returns the python int 0 here (models/vilmodel.py:650-651); a 0-d tensor is a superset
-        return torch.zeros((), dtype=F32, device=dev), out.view(B, I, HIDDEN)
+        return torch.zeros((), dtype=F32, device=dev), img.clone().view(B, I, HIDDEN)
     pk = model._pk()['align']
-    if blocks.training():
-        return _align_forward_train(model, txt, img, rows, pk, lowp, (B, I))
-    x32, x16 = ops.gather_mean(img, rows.unit, rows.slot, rows.R, want16=lowp, want32=not lowp)
-    x = x16 if lowp else x32
+    train = blocks.training()
+    if train:
+        if txt.requires_grad and cfg.aux_loss_type != 'cosine':
+            raise NotImplementedError('training the text encoder through the %r alignment loss (fix_lang_inside_cosine_model=False) '
+                                      'is not built: only the cosine form carries gradients to the text means' % cfg.aux_loss_type)
+        if cfg.aux_loss_type not in ('cosine', 'contrastive-InfoNCE', 'constrastive-margin'):
+            raise NotImplementedError('backward of aux_loss_type %r' % cfg.aux_loss_type)
+        x = ag.GatherSlotsFn.apply(img, rows.unit, rows.slot, rows.R, lowp)
+        if model.training:
+            x = ag.dropout(x, 0.15)                           # MLPProjectionHead.dropout (models/vilmodel.py:578,585)
+    else:
+        x32, x16 = ops.gather_mean(img, rows.unit, rows.slot, rows.R, want16=lowp, want32=not lowp)
+        x = x16 if lowp else x32
     for j, lp in enumerate(pk):
-        w, _ = lp.get(lowp)
         last = j == len(pk) - 1
-        x = ops.gemm(x, w, None, epilogue=ops.EPI_NONE if last else ops.EPI_RELU, out_dtype=F32 if (last or not lowp) else x.dtype)
-    proj = x
-    tgt, _ = ops.gather_mean(txt, rows.tok_off, rows.tok_rows, rows.R, want16=False)
+        x = blocks.linear(x, lp, lowp, out_dtype=F32 if (last or not lowp) else x.dtype, epilogue=ops.EPI_NONE if last else ops.EPI_RELU)
+    tgt = blocks.segment_mean(txt, rows.tok_off, rows.tok_rows, rows.R)
+    negs, neg_ep = None, None
+    if rows.n_negs and cfg.aux_loss_type != 'cosine':         # AlignWithContrastiveLossWithNegativeSamples (:689-779)
+        negs, _ = ops.gather_mean(txt, rows.np_off, rows.np_rows, rows.n_negs, want16=False)
+        neg_ep = rows.np_ep
     if cfg.aux_loss_type == 'cosine':
-        loss, _ = ops.cosine_loss(proj, tgt, rows.R, dev)
+        loss = ag.CosineLossFn.apply(x, tgt, rows.R) if train else ops.cosine_loss(x, tgt, rows.R, dev)[0]
     elif cfg.aux_loss_type == 'contrastive-InfoNCE':
-        negs = None
-        if rows.n_negs:
-            negs, _ = ops.gather_mean(txt, rows.np_off, rows.np_rows, rows.n_negs, want16=False)
-        loss, _ = ops.infonce_loss(proj, tgt, negs, rows.ep, rows.np_ep if rows.n_negs else None,
-                                   float(cfg.infonce_temperature), rows.R, rows.n_negs, dev)
+        args = (x, tgt, negs, rows.ep, neg_ep, float(cfg.infonce_temperature), rows.R, rows.n_negs)
+        loss = ag.InfoNCELossFn.apply(*args) if train else ops.infonce_loss(*args, dev)[0]
     elif cfg.aux_loss_type == 'constrastive-margin':          # (sic) H/r2r/parser.py:117, H/models/vilmodel_cmt.py:825-856
-        negs = None
-        if rows.n_negs:
-            negs, _ = ops.gather_mean(txt, rows.np_off, rows.np_rows, rows.n_negs, want16=False)
-        loss, _ = ops.margin_loss(proj, tgt, negs, rows.ep, rows.np_ep if rows.n_negs else None,
-                                  float(cfg.contrastive_margin_value), rows.R, rows.n_negs, dev)
+        args = (x, tgt, negs, rows.ep, neg_ep, float(cfg.contrastive_margin_value), rows.R, rows.n_negs)
+        loss = ag.MarginLossFn.apply(*args) if train else ops.margin_loss(*args, dev)[0]
     else:
         raise NotImplementedError('aux_loss_type %r' % cfg.aux_loss_type)
-    ops.scatter_rows(proj, rows.slot, out)
-    return loss, out.view(B, I, HIDDEN)
-
-
-def _align_forward_train(model, txt, img, rows, pk, lowp, shape):
-    """align_forward with autograd recording: the projection MLP, the cosine loss and the write-back of the
-    projected rows (models/vilmodel.py:646) are differentiable; the noun-phrase text means are constants
-    (``fix_lang_inside_cosine_model``, :1249-1255 - the released configuration)."""
-    cfg = model.config
-    if txt.requires_grad and cfg.aux_loss_type != 'cosine':
-        raise NotImplementedError('training the text encoder through the %r alignment loss (fix_lang_inside_cosine_model=False) '
-                                  'is not built: only the cosine form carries gradients to the text means' % cfg.aux_loss_type)
-    if cfg.aux_loss_type not in ('cosine', 'contrastive-InfoNCE', 'constrastive-margin'):
-        raise NotImplementedError('backward of aux_loss_type %r' % cfg.aux_loss_type)
-    B, I = shape
-    x = ag.GatherSlotsFn.apply(img, rows.unit, rows.slot, rows.R, lowp)
-    if model.training:
-        x = ag.dropout(x, 0.15)                               # MLPProjectionHead.dropout (models/vilmodel.py:578,585)
-    for j, lp in enumerate(pk):
-        last = j == len(pk) - 1
-        x = ag.linear(x, lp, lowp, out_dtype=F32 if (last or not lowp) else BF16)
-        if not last:
-            x = ag.ActFn.apply(x, ops.EPI_RELU)
-    if txt.requires_grad:                                     # fix_lang_inside_cosine_model off (:1256-1262): the text means train too
-        tgt = ag.RaggedMeanFn.apply(txt, rows.tok_off, rows.tok_rows, rows.R)
-    else:
-        tgt, _ = ops.gather_mean(txt, rows.tok_off, rows.tok_rows, rows.R, want16=False)
-    if cfg.aux_loss_type == 'cosine':
-        loss = ag.CosineLossFn.apply(x, tgt, rows.R)
-    else:                                                     # AlignWithContrastiveLossWithNegativeSamples (:689-779)
-        negs = None
-        if rows.n_negs:
-            negs, _ = ops.gather_mean(txt, rows.np_off, rows.np_rows, rows.n_negs, want16=False)
-        if cfg.aux_loss_type == 'constrastive-margin':        # (sic) H/models/vilmodel_cmt.py:825-856
-            loss = ag.MarginLossFn.apply(x, tgt, negs, rows.ep, rows.np_ep if rows.n_negs else None,
-                                         float(cfg.contrastive_margin_value), rows.R, rows.n_negs)
-        else:
-            loss = ag.InfoNCELossFn.apply(x, tgt, negs, rows.ep, rows.np_ep if rows.n_negs else None,
-                                          float(cfg.infonce_temperature), rows.R, rows.n_negs)
-    out = ag.ScatterSlotsFn.apply(img, x, rows.slot, rows.unit)
+    out = ag.ScatterSlotsFn.apply(img, x, rows.slot, rows.unit) if train else ops.scatter_rows(x, rows.slot, img.clone())
     return loss, out.view(B, I, HIDDEN)
 
 
@@ -506,11 +474,7 @@ class GlocalTextPathNavCMT(nn.Module):
                                          B, G, P, row0)
             obj_logits = None
             if vp_obj_masks is not None:                       # object grounding logits (:1220-1225): -inf outside the object tokens
-                og_raw = blocks.cls_head(x.operand(lowp)[r_l:r_l + B * P], pk['og'], lowp)
-                if recording:
-                    obj_logits = og_raw.view(B, P).masked_fill(vp_obj_masks.logical_not(), float('-inf'))
-                else:
-                    obj_logits = ops.mask_logits_navtype(og_raw, vp_obj_masks.long().contiguous().view(-1)).view(B, P)
+                obj_logits = blocks.mask_logits(blocks.cls_head(x.operand(lowp)[r_l:r_l + B * P], pk['og'], lowp), vp_obj_masks)
         return {'gmap_embeds': gmap_out, 'vp_embeds': vp_out, 'global_logits': gl, 'local_logits': ll,
                 'fused_logits': fl, 'obj_logits': obj_logits}
 

@@ -22,7 +22,7 @@ import torch.nn as nn
 
 from . import autograd_ops as ag
 from . import blocks, graphs, ops, params
-from .blocks import Act, Stream
+from .blocks import Stream
 from .config import hamt_config
 from .duet import _f32c, align_forward
 from .ops import BF16, F32, HIDDEN
@@ -93,6 +93,7 @@ class NavCMT(nn.Module):
             pk['ob_img'] = blocks.LinearPack([self.img_embeddings.img_linear.weight], [self.img_embeddings.img_linear.bias])
             he = self.hist_embeddings
             pk['hist_img'] = blocks.LinearPack([he.img_linear.weight], [he.img_linear.bias])
+            pk['hist_ln'] = blocks.LNPack([he.layer_norm])
             if he.pano_encoder is not None:
                 pk['hist_pano_img'] = blocks.LinearPack([he.pano_img_linear.weight], [he.pano_img_linear.bias])
                 pk['hist_pano'] = [blocks.SelfFFNPack([l.attention], [l.intermediate], [l.output]) for l in he.pano_encoder.layer]
@@ -157,74 +158,32 @@ class NavCMT(nn.Module):
         out = x.f32.view(B, L, HIDDEN)
         return out.detach() if frozen else out
 
+    def _mean_rows(self, B, n, row0, per, dev):
+        """(offsets, rows) index arrays of B disjoint n-row segments, segment b = rows row0 + b * per + [0, n).  Built once per
+        layout: a captured graph replays the first eager call's arrays and must not create its own."""
+        key = (B, n, row0, per, str(dev))
+        if key not in self._mean_idx:
+            idx = row0 + torch.arange(B, device=dev)[:, None] * per + torch.arange(n, device=dev)[None, :]
+            self._mean_idx[key] = (torch.arange(0, B * n + 1, n, dtype=torch.int32, device=dev), idx.reshape(-1).to(torch.int32))
+        return self._mean_idx[key]
+
     def forward_history(self, hist_img_feats, hist_ang_feats, ob_step_ids, hist_pano_img_feats, hist_pano_ang_feats):
         """'history': HistoryEmbeddings.forward, :576-618."""
-        he = self.hist_embeddings
-        lowp = self.lowp
-        if not self.fix_hist_embedding and self._recording(hist_img_feats) and any(p.requires_grad for p in he.parameters()):
-            return self._history_train(hist_img_feats, hist_ang_feats, ob_step_ids, hist_pano_img_feats, hist_pano_ang_feats)
-        type_row = he.type_embedding.weight[0]
-        ln = (he.layer_norm.weight, he.layer_norm.bias)
-        if hist_img_feats is None:
-            ops.ensure_init(he.cls_token)
-            y32, _ = ops.embed_compose(1, he.cls_token.device, a=he.cls_token.view(1, HIDDEN), const_row=type_row, out_ln=ln)
-            return y32.detach() if self.fix_hist_embedding else y32
-        ops.ensure_init(hist_img_feats)
-        dev = hist_img_feats.device
-        B = hist_img_feats.shape[0]
-        pk = self._pk()
-        f32 = _f32c(hist_img_feats)
-        w, b = pk['hist_img'].get(lowp)
-        a = ops.gemm(ops.cast_h16(f32) if lowp else f32, w, b, out_dtype=F32)
-        # position embedding of the current step: a [B] index tensor (the same id for every episode, :597), so the
-        # step never becomes a pointer baked into a captured graph
-        if torch.is_tensor(ob_step_ids) and ob_step_ids.numel() == B:
-            step_idx = ob_step_ids.long().contiguous().view(-1)
-        else:
-            step = int(ob_step_ids.view(-1)[0]) if torch.is_tensor(ob_step_ids) else int(ob_step_ids)
-            step_idx = torch.full((B,), step, dtype=torch.int64, device=dev)
-        e32, _ = ops.embed_compose(B, dev, a=a, a_ln=(he.img_layer_norm.weight, he.img_layer_norm.bias),
-                                   feat=_f32c(hist_ang_feats), feat_w=he.ang_linear.weight, feat_b=he.ang_linear.bias,
-                                   feat_ln=(he.ang_layer_norm.weight, he.ang_layer_norm.bias),
-                                   idx=step_idx, table=he.position_embeddings.weight, const_row=type_row)
-        pano_mean = None
-        if he.pano_encoder is not None:
-            V = hist_pano_img_feats.shape[1]
-            p32 = _f32c(hist_pano_img_feats).view(B * V, -1)
-            w, b = pk['hist_pano_img'].get(lowp)
-            pa = ops.gemm(ops.cast_h16(p32) if lowp else p32, w, b, out_dtype=F32)
-            y32, y16 = ops.embed_compose(B * V, dev, a=pa, a_ln=(he.pano_img_layer_norm.weight, he.pano_img_layer_norm.bias),
-                                         feat=_f32c(hist_pano_ang_feats).view(B * V, -1), feat_w=he.pano_ang_linear.weight,
-                                         feat_b=he.pano_ang_linear.bias,
-                                         feat_ln=(he.pano_ang_layer_norm.weight, he.pano_ang_layer_norm.bias), want16=lowp)
-            x = Act(y32, y16)
-            s = [Stream(0, B, V, None)]                       # the reference's mask is all ones (:606-607)
-            for lp in pk['hist_pano']:
-                x = blocks.self_attn_ffn(x, lp, s, None, lowp)
-            key = (B, V, str(dev))
-            if key not in self._mean_idx:
-                self._mean_idx[key] = (torch.arange(0, B * V + 1, V, dtype=torch.int32, device=dev),
-                                       torch.arange(B * V, dtype=torch.int32, device=dev))
-            off, idx = self._mean_idx[key]
-            pano_mean, _ = ops.gather_mean(x.f32, off, idx, B, want16=False)
-        y32, _ = ops.add_ln(e32, pano_mean, ln[0], ln[1], 1e-12, want16=False)
-        return y32.detach() if self.fix_hist_embedding else y32
-
-    def _history_train(self, hist_img_feats, hist_ang_feats, ob_step_ids, hist_pano_img_feats, hist_pano_ang_feats):
-        """'history' with autograd recording (fix_hist_embedding=False, :576-618): the same sum from the differentiable blocks;
-        nn.Dropout after the final LayerNorm (:616)."""
         he, lowp, pk = self.hist_embeddings, self.lowp, self._pk()
+        recording = not self.fix_hist_embedding and self._recording(hist_img_feats) and any(p.requires_grad for p in he.parameters())
         type_row = he.type_embedding.weight[0]
-        with blocks.grad_mode(True, self._drop()):
+        with blocks.grad_mode(recording, self._drop() if recording else (0.0, 0.0)):
             if hist_img_feats is None:
                 ops.ensure_init(he.cls_token)
                 y = blocks.embed(1, he.cls_token.device, a=he.cls_token.view(1, HIDDEN), const_rows=(type_row,), out_ln=he.layer_norm,
-                                 dropout=True)
-                return y.f32
+                                 dropout=True).f32
+                return y.detach() if self.fix_hist_embedding else y
             ops.ensure_init(hist_img_feats)
             dev = hist_img_feats.device
             B = hist_img_feats.shape[0]
             a = blocks.linear(blocks.operand(_f32c(hist_img_feats), lowp), pk['hist_img'], lowp, out_dtype=F32)
+            # position embedding of the current step: a [B] index tensor (the same id for every episode, :597), so the
+            # step never becomes a pointer baked into a captured graph
             if torch.is_tensor(ob_step_ids) and ob_step_ids.numel() == B:
                 step_idx = ob_step_ids.long().contiguous().view(-1)
             else:
@@ -238,16 +197,15 @@ class NavCMT(nn.Module):
                 pa = blocks.linear(blocks.operand(_f32c(hist_pano_img_feats).view(B * V, -1), lowp), pk['hist_pano_img'], lowp, out_dtype=F32)
                 x = blocks.embed(B * V, dev, a=pa, a_ln=he.pano_img_layer_norm, feat=_f32c(hist_pano_ang_feats).view(B * V, -1),
                                  feat_lin=he.pano_ang_linear, feat_ln=he.pano_ang_layer_norm, lowp=lowp, dropout=True)
-                st = [Stream(0, B, V, None)]                  # the reference's mask is all ones (:606-607)
+                s = [Stream(0, B, V, None)]                   # the reference's mask is all ones (:606-607)
                 for lp in pk['hist_pano']:
-                    x = blocks.self_attn_ffn(x, lp, st, None, lowp)
-                off = torch.arange(0, B * V + 1, V, dtype=torch.int32, device=dev)
-                idx = torch.arange(B * V, dtype=torch.int32, device=dev)
-                pano_mean = ag.SegmentMeanFn.apply(x.f32, off, idx, B, V)
-            y = blocks.layer_norm(e32, pano_mean, blocks.LNPack([he.layer_norm]), 1e-12, False).f32
-            if blocks._Mode.p_hidden > 0:
+                    x = blocks.self_attn_ffn(x, lp, s, None, lowp)
+                off, idx = self._mean_rows(B, V, 0, V, dev)
+                pano_mean = blocks.segment_mean(x.f32, off, idx, B, seg=V)
+            y = blocks.layer_norm(e32, pano_mean, pk['hist_ln'], 1e-12, False).f32
+            if blocks._Mode.p_hidden > 0:                     # nn.Dropout after the final LayerNorm (:616)
                 y = ag.dropout(y, blocks._Mode.p_hidden)
-        return y
+        return y.detach() if self.fix_hist_embedding else y
 
     def forward_imagination(self, imagine_pano_img_feats, imagine_masks=None):
         """'imagine', :1040-1048: the bypass embedding (:620-631) or the ImagineEmbeddings encoder (:634-703)."""
@@ -270,34 +228,21 @@ class NavCMT(nn.Module):
         B, I, _ = feats.shape
         if I >= im.position_embeddings.weight.shape[0]:
             raise ValueError('imagination length %d out of bounds (max_imagination_len %d, :683)' % (I, im.position_embeddings.weight.shape[0]))
-        dev = feats.device
-        if self._recording(feats) and any(p.requires_grad for p in im.parameters()) and not self.fix_imagine_embeds:
-            # fine-tuning: the same sequence from the differentiable blocks; nn.Dropout after both LayerNorms (:686, :701)
-            with blocks.grad_mode(True, self._drop()):
-                x = blocks.embed(B * I, dev, a=_f32c(feats).view(B * I, -1), pos_table=im.position_embeddings.weight, pos_period=I,
-                                 const_rows=(im.type_embedding.weight[0],), lowp=lowp)
-                a = blocks.linear(x.operand(lowp), pk['imag_img'], lowp, out_dtype=F32)
-                x = blocks.layer_norm(a, None, pk['imag_ln0'], 1e-12, lowp)
-                if blocks._Mode.p_hidden > 0:
-                    x = blocks.as_act(ag.dropout(x.f32, blocks._Mode.p_hidden), lowp)
-                st = [Stream(0, B, I, blocks.mask_u8(imagine_masks))]
-                for lp in pk['imag_enc']:
-                    x = blocks.self_attn_ffn(x, lp, st, None, lowp)
-                out = blocks.layer_norm(x.f32, None, pk['imag_ln1'], 1e-12, False).f32
-                if blocks._Mode.p_hidden > 0:
-                    out = ag.dropout(out, blocks._Mode.p_hidden)
-            return out.view(B, I, HIDDEN)
-        x32, x16 = ops.embed_compose(B * I, dev, a=_f32c(feats).view(B * I, -1), pos_table=im.position_embeddings.weight, pos_period=I,
-                                     const_row=im.type_embedding.weight[0], want16=lowp, want32=not lowp)
-        w, b = pk['imag_img'].get(lowp)
-        a = ops.gemm(x16 if lowp else x32, w, b, out_dtype=F32)
-        y32, y16 = ops.add_ln(a, None, im.pano_img_layer_norm.weight, im.pano_img_layer_norm.bias, 1e-12, want16=lowp)
-        x = Act(y32, y16)
-        s = [Stream(0, B, I, blocks.mask_u8(imagine_masks))]
-        for lp in pk['imag_enc']:
-            x = blocks.self_attn_ffn(x, lp, s, None, lowp)
-        out, _ = ops.add_ln(x.f32, None, im.layer_norm.weight, im.layer_norm.bias, 1e-12, want16=False)
-        return out.view(B, I, HIDDEN).detach()
+        recording = self._recording(feats) and any(p.requires_grad for p in im.parameters()) and not self.fix_imagine_embeds
+        with blocks.grad_mode(recording, self._drop() if recording else (0.0, 0.0)):
+            x = blocks.embed(B * I, feats.device, a=_f32c(feats).view(B * I, -1), pos_table=im.position_embeddings.weight,
+                             pos_period=I, const_rows=(im.type_embedding.weight[0],), lowp=lowp, want32=not lowp)
+            a = blocks.linear(x.operand(lowp), pk['imag_img'], lowp, out_dtype=F32)
+            x = blocks.layer_norm(a, None, pk['imag_ln0'], 1e-12, lowp)
+            if blocks._Mode.p_hidden > 0:                     # nn.Dropout after both LayerNorms (:686, :701)
+                x = blocks.as_act(ag.dropout(x.f32, blocks._Mode.p_hidden), lowp)
+            s = [Stream(0, B, I, blocks.mask_u8(imagine_masks))]
+            for lp in pk['imag_enc']:
+                x = blocks.self_attn_ffn(x, lp, s, None, lowp)
+            out = blocks.layer_norm(x.f32, None, pk['imag_ln1'], 1e-12, False).f32
+            if blocks._Mode.p_hidden > 0:
+                out = ag.dropout(out, blocks._Mode.p_hidden)
+        return out.view(B, I, HIDDEN)
 
     def forward_visual(self, txt_embeds, txt_masks, hist_embeds, hist_masks, ob_img_feats, ob_ang_feats, ob_nav_types,
                        ob_masks, imagine_embeds=None, imagine_masks=None):
@@ -317,153 +262,51 @@ class NavCMT(nn.Module):
         on_visn = bool(I) and cfg.concat_imagine_with == 'visual'
         Il, Iv = (0, I) if on_visn else (I, 0)
         C, Nv = L + Il, T + O + Iv
-        if self._recording(txt_embeds, hist_embeds, ob_img_feats, imagine_embeds):
-            with blocks.grad_mode(True, self._drop()):
-                return self._visual_train(txt_embeds, txt_masks, hist_embeds, hist_masks, ob_img_feats, ob_ang_feats,
-                                          ob_nav_types, ob_masks, imagine_embeds, imagine_masks)
-        (r_l, r_v), ends, R = blocks.stack_layout([B * C, B * Nv])
-        x32 = torch.empty((R, HIDDEN), dtype=F32, device=dev)
-        x16 = torch.empty((R, HIDDEN), dtype=ops.h16(), device=dev) if lowp else None
-        if ends[0] > B * C:
-            x32[B * C:ends[0]].zero_()
-            if lowp:
-                x16[B * C:ends[0]].zero_()
-        lang32, lang16 = x32[r_l:], (x16[r_l:] if lowp else None)
-        visn32, visn16 = x32[r_v:], (x16[r_v:] if lowp else None)
-        # language stream = [txt ; imagine]  (:1110)
-        ops.copy_rows(_f32c(txt_embeds), L * HIDDEN, HIDDEN, B, L, lang32, lang16, C * HIDDEN, HIDDEN)
-        if Il:
-            ops.copy_rows(_f32c(imagine_embeds), I * HIDDEN, HIDDEN, B, I, lang32[L:], lang16[L:] if lowp else None,
-                          C * HIDDEN, HIDDEN)
-        # vision stream = [hist ; ob]  (:1087); observation embedding :521-544, :1073-1077
-        ops.copy_rows(_f32c(hist_embeds), T * HIDDEN, HIDDEN, B, T, visn32, visn16, Nv * HIDDEN, HIDDEN)
-        ie = self.img_embeddings
-        o32 = _f32c(ob_img_feats).view(B * O, -1)
-        w, b = pk['ob_img'].get(lowp)
-        a = ops.gemm(ops.cast_h16(o32) if lowp else o32, w, b, out_dtype=F32)
-        ob32, _ = ops.embed_compose(B * O, dev, a=a, a_ln=(ie.img_layer_norm.weight, ie.img_layer_norm.bias),
-                                    feat=_f32c(ob_ang_feats).view(B * O, -1), feat_w=ie.ang_linear.weight, feat_b=ie.ang_linear.bias,
-                                    feat_ln=(ie.ang_layer_norm.weight, ie.ang_layer_norm.bias),
-                                    idx=ob_nav_types.long().contiguous().view(-1), table=ie.nav_type_embedding.weight,
-                                    const_row=self.embeddings.token_type_embeddings.weight[1],
-                                    out_ln=(ie.layer_norm.weight, ie.layer_norm.bias))
-        ops.copy_rows(ob32, O * HIDDEN, HIDDEN, B, O, visn32[T:], visn16[T:] if lowp else None, Nv * HIDDEN, HIDDEN)
-        if Iv:
-            ops.copy_rows(_f32c(imagine_embeds), I * HIDDEN, HIDDEN, B, I, visn32[T + O:], visn16[T + O:] if lowp else None,
-                          Nv * HIDDEN, HIDDEN)
-        x = Act(x32, x16)
+        (r_l, r_v), ends, _ = blocks.stack_layout([B * C, B * Nv])
+        recording = self._recording(txt_embeds, hist_embeds, ob_img_feats, imagine_embeds)
+        with blocks.grad_mode(recording, self._drop() if recording else (0.0, 0.0)):
+            # observation embedding :521-544, :1073-1077
+            ie = self.img_embeddings
+            a = blocks.linear(blocks.operand(_f32c(ob_img_feats).view(B * O, -1), lowp), pk['ob_img'], lowp, out_dtype=F32)
+            ob = blocks.embed(B * O, dev, a=a, a_ln=ie.img_layer_norm, feat=_f32c(ob_ang_feats).view(B * O, -1), feat_lin=ie.ang_linear,
+                              feat_ln=ie.ang_layer_norm, idx=ob_nav_types.long().contiguous().view(-1), table=ie.nav_type_embedding.weight,
+                              const_rows=(self.embeddings.token_type_embeddings.weight[1],), out_ln=ie.layer_norm, dropout=True).f32
+            if self.fix_obs_embedding:
+                ob = ob.detach()
+            # language stream = [txt ; imagine] (:1110), vision stream = [hist ; ob] (:1087) [; imagine] (:1106-1108)
+            imag = [_f32c(imagine_embeds)] if I else []
+            x = blocks.stack_segments([[_f32c(txt_embeds)] + (imag if Il else []),
+                                       [_f32c(hist_embeds), ob.view(B, O, HIDDEN)] + (imag if Iv else [])], (r_l, r_v), lowp)
+            lang_mask = blocks.mask_u8(torch.cat([txt_masks.bool(), imagine_masks.bool()], 1) if Il else txt_masks)
+            visn_mask = blocks.mask_u8(torch.cat([hist_masks.bool(), ob_masks.bool()] + ([imagine_masks.bool()] if Iv else []), 1))
+            streams = [Stream(r_l, B, C, lang_mask, 0), Stream(r_v, B, Nv, visn_mask, 1)]
+            for cp, sp in zip(pk['x_cross'], pk['x_self']):
+                # bidirectional cross-attention with shared weights, both directions read the layer inputs (:385-397)
+                x = blocks.attn(x, cp['qkv'], cp['o'], cp['ln'], streams, ends, lowp, kv_of=(1, 0))
+                x = blocks.self_attn_ffn(x, sp, streams, ends, lowp, defer=True)
+            x = blocks.materialize(x, lowp, ends, want16=False)
 
-        lang_mask = blocks.mask_u8(torch.cat([txt_masks.bool(), imagine_masks.bool()], 1) if Il else txt_masks)
-        visn_mask = blocks.mask_u8(torch.cat([hist_masks.bool(), ob_masks.bool()] + ([imagine_masks.bool()] if Iv else []), 1))
-        streams = [Stream(r_l, B, C, lang_mask, 0), Stream(r_v, B, Nv, visn_mask, 1)]
-
-        for cp, sp in zip(pk['x_cross'], pk['x_self']):
-            # bidirectional cross-attention with shared weights, both directions read the layer inputs (:385-397)
-            qkv = blocks.gemm_act(x, cp['qkv'], lowp, ends)    # all rows: Q | K | V
-            ctx = blocks._ctx_buffer(R, qkv, streams)
-            ql, qv = qkv[r_l:r_l + B * C], qkv[r_v:r_v + B * Nv]
-            ops.attention_multi([
-                dict(q=ql[:, :HIDDEN], k=qv[:, HIDDEN:2 * HIDDEN], v=qv[:, 2 * HIDDEN:], out=ctx[r_l:r_l + B * C],
-                     B=B, Lq=C, Lk=Nv, key_mask=visn_mask),
-                dict(q=qv[:, :HIDDEN], k=ql[:, HIDDEN:2 * HIDDEN], v=ql[:, 2 * HIDDEN:], out=ctx[r_v:r_v + B * Nv],
-                     B=B, Lq=Nv, Lk=C, key_mask=lang_mask)])
-            x = blocks.linear_residual_ln(ctx, cp['o'], x, cp['ln'], 1e-12, lowp, ends, defer=True)
-            x = blocks.self_attn_ffn(x, sp, streams, ends, lowp, defer=True)
-        x = blocks.materialize(x, lowp, ends, want16=False)
-
-        lang_out = x.f32[r_l:r_l + B * C].view(B, C, HIDDEN)
-        visn_out = x.f32[r_v:r_v + B * Nv].view(B, Nv, HIDDEN)
-        txt_out, hist_out, ob_out = lang_out[:, :L], visn_out[:, :T], visn_out[:, T:T + O]      # :1173-1182
-        tok = cfg.act_pred_token                               # :1189-1199
-        if tok == 'ob_txt':
-            h32, h16 = ops.mul_bcast(ob_out, Nv * HIDDEN, lang_out, C * HIDDEN, B, O, want16=lowp, want32=not lowp)
-        elif tok == 'ob_hist':                                 # ob * hist[:, :1]: token 0 of the vision stream
-            h32, h16 = ops.mul_bcast(ob_out, Nv * HIDDEN, visn_out, Nv * HIDDEN, B, O, want16=lowp, want32=not lowp)
-        elif tok in ('ob_txt_hist', 'ob_imagine_text'):        # ob * (txt[:, :1] + hist[:, :1] | mean over the imagination tokens)
-            t0 = torch.empty((B, HIDDEN), dtype=F32, device=dev)
-            ops.copy_rows(lang_out, C * HIDDEN, HIDDEN, B, 1, t0, None, HIDDEN, HIDDEN)
-            if tok == 'ob_txt_hist':
-                other = torch.empty((B, HIDDEN), dtype=F32, device=dev)
-                ops.copy_rows(visn_out, Nv * HIDDEN, HIDDEN, B, 1, other, None, HIDDEN, HIDDEN)
-            else:                                              # torch.mean(imagine_embeds, 1): all I output tokens, unmasked
-                row0, per = (r_v + T + O, Nv) if on_visn else (r_l + L, C)
-                key = ('imag', B, I, row0, per, str(dev))
-                if key not in self._mean_idx:
-                    idx = (row0 + torch.arange(B, device=dev)[:, None] * per + torch.arange(I, device=dev)[None, :]).reshape(-1)
-                    self._mean_idx[key] = (torch.arange(0, B * I + 1, I, dtype=torch.int32, device=dev), idx.to(torch.int32))
-                off, idx = self._mean_idx[key]
-                other, _ = ops.gather_mean(x.f32, off, idx, B, want16=False)
-            gate, _ = ops.embed_compose(B, dev, a=t0, a2=other)
-            h32, h16 = ops.mul_bcast(ob_out, Nv * HIDDEN, gate, HIDDEN, B, O, want16=lowp, want32=not lowp)
-        else:                                                  # 'ob'
-            h32 = torch.empty((B * O, HIDDEN), dtype=F32, device=dev) if not lowp else None
-            h16 = torch.empty((B * O, HIDDEN), dtype=ops.h16(), device=dev) if lowp else None
-            ops.copy_rows(ob_out, Nv * HIDDEN, HIDDEN, B, O, h32, h16, O * HIDDEN, HIDDEN)
-        raw = blocks.cls_head(h16 if lowp else h32, pk['act'], lowp)
-        act_logits = ops.mask_logits_navtype(raw, ob_nav_types.long().contiguous().view(-1)).view(B, O)
-        return act_logits, txt_out, hist_out, ob_out
-
-    def _visual_train(self, txt_embeds, txt_masks, hist_embeds, hist_masks, ob_img_feats, ob_ang_feats, ob_nav_types,
-                      ob_masks, imagine_embeds, imagine_masks):
-        """'visual' with autograd recording: the same layer sequence as forward_visual from the differentiable blocks
-        (torch only concatenates / slices rows).  :1056-1205."""
-        cfg, lowp, pk = self.config, self.lowp, self._pk()
-        dev = txt_embeds.device
-        B, L, _ = txt_embeds.shape
-        T, O = hist_embeds.shape[1], ob_img_feats.shape[1]
-        I = imagine_embeds.shape[1] if cfg.imagine_enc_pano else 0
-        on_visn = bool(I) and cfg.concat_imagine_with == 'visual'      # :1106-1112
-        Il, Iv = (0, I) if on_visn else (I, 0)
-        C, Nv = L + Il, T + O + Iv
-        (r_l, r_v), ends, R = blocks.stack_layout([B * C, B * Nv])
-        ie = self.img_embeddings
-        o32 = _f32c(ob_img_feats).view(B * O, -1)
-        a = blocks.linear(blocks.operand(o32, lowp), pk['ob_img'], lowp, out_dtype=F32)
-        ob = blocks.embed(B * O, dev, a=a, a_ln=ie.img_layer_norm, feat=_f32c(ob_ang_feats).view(B * O, -1), feat_lin=ie.ang_linear,
-                          feat_ln=ie.ang_layer_norm, idx=ob_nav_types.long().contiguous().view(-1), table=ie.nav_type_embedding.weight,
-                          const_rows=(self.embeddings.token_type_embeddings.weight[1],), out_ln=ie.layer_norm, dropout=True).f32
-        if self.fix_obs_embedding:
-            ob = ob.detach()
-        lang = torch.cat([_f32c(txt_embeds), _f32c(imagine_embeds)], 1) if Il else _f32c(txt_embeds)
-        visn = torch.cat([_f32c(hist_embeds), ob.view(B, O, HIDDEN)] + ([_f32c(imagine_embeds)] if Iv else []), 1)
-        x = blocks.as_act(blocks.stack_rows([lang.reshape(B * C, HIDDEN), visn.reshape(B * Nv, HIDDEN)], (r_l, r_v)), lowp)
-        lang_mask = blocks.mask_u8(torch.cat([txt_masks.bool(), imagine_masks.bool()], 1) if Il else txt_masks)
-        visn_mask = blocks.mask_u8(torch.cat([hist_masks.bool(), ob_masks.bool()] + ([imagine_masks.bool()] if Iv else []), 1))
-        streams = [Stream(r_l, B, C, lang_mask, 0), Stream(r_v, B, Nv, visn_mask, 1)]
-        for cp, sp in zip(pk['x_cross'], pk['x_self']):
-            # bidirectional cross-attention with shared weights, both directions read the layer inputs (:385-397)
-            qkv = ag.linear(x.operand(lowp), cp['qkv'], lowp)
-            spec = [dict(q=(0, r_l, 0), k=(0, r_v, HIDDEN), v=(0, r_v, 2 * HIDDEN), B=B, Lq=C, Lk=Nv, key_mask=visn_mask, out_row0=r_l,
-                         drop=blocks._attn_drop(dev)),
-                    dict(q=(0, r_v, 0), k=(0, r_l, HIDDEN), v=(0, r_l, 2 * HIDDEN), B=B, Lq=Nv, Lk=C, key_mask=lang_mask, out_row0=r_v,
-                         drop=blocks._attn_drop(dev))]
-            ctx = ag.AttentionFn.apply(spec, R, blocks.MASK_ADD_NEG10000, 1, qkv)
-            x = blocks._dense_res_ln(ctx, cp['o'], x.f32, cp['ln'], 1e-12, lowp, None)
-            x = blocks.self_attn_ffn(x, sp, streams, ends, lowp)
-        lang_out = x.f32[r_l:r_l + B * C].view(B, C, HIDDEN)
-        visn_out = x.f32[r_v:r_v + B * Nv].view(B, Nv, HIDDEN)
-        txt_out, hist_out, ob_out = lang_out[:, :L], visn_out[:, :T], visn_out[:, T:T + O]      # :1173-1182
-        tok = cfg.act_pred_token                               # :1189-1199
-        if tok == 'ob':
-            h = blocks.operand(ob_out.reshape(B * O, HIDDEN), lowp)
-        else:
-            if tok == 'ob_txt':
-                gate = lang_out[:, 0]
-            elif tok == 'ob_hist':
-                gate = visn_out[:, 0]
-            elif tok == 'ob_txt_hist':
-                gate = ag.SumRowsFn.apply(2, lang_out[:, 0].contiguous(), visn_out[:, 0].contiguous())
-            elif tok == 'ob_imagine_text':                     # txt[:, :1] + mean over ALL imagination output tokens (unmasked)
-                row0, per = (r_v + T + O, Nv) if on_visn else (r_l + L, C)
-                idx = (row0 + torch.arange(B, device=dev)[:, None] * per + torch.arange(I, device=dev)[None, :]).reshape(-1).to(torch.int32)
-                off = torch.arange(0, B * I + 1, I, dtype=torch.int32, device=dev)
-                mean = ag.SegmentMeanFn.apply(x.f32, off, idx, B, I)
-                gate = ag.SumRowsFn.apply(2, lang_out[:, 0].contiguous(), mean)
+            lang_out = x.f32[r_l:r_l + B * C].view(B, C, HIDDEN)
+            visn_out = x.f32[r_v:r_v + B * Nv].view(B, Nv, HIDDEN)
+            txt_out, hist_out, ob_out = lang_out[:, :L], visn_out[:, :T], visn_out[:, T:T + O]      # :1173-1182
+            tok = cfg.act_pred_token                           # :1189-1199
+            if tok == 'ob':
+                h = blocks.take_rows(ob_out, lowp)
             else:
-                raise NotImplementedError('act_pred_token %r' % tok)
-            h = ag.MulBcastFn.apply(ob_out, gate, lowp)
-        raw = blocks.cls_head(h, pk['act'], lowp)
-        act_logits = raw.view(B, O).masked_fill(ob_nav_types.view(B, O) == 0, float('-inf'))
+                if tok == 'ob_txt':
+                    gate = lang_out[:, 0]
+                elif tok == 'ob_hist':                         # ob * hist[:, :1]: token 0 of the vision stream
+                    gate = visn_out[:, 0]
+                else:                                          # ob * (txt[:, :1] + hist[:, :1] | mean over the imagination tokens)
+                    t0 = blocks.take_rows(lang_out[:, :1])
+                    if tok == 'ob_txt_hist':
+                        other = blocks.take_rows(visn_out[:, :1])
+                    else:                                      # torch.mean(imagine_embeds, 1): all I output tokens, unmasked
+                        off, idx = self._mean_rows(B, I, *((r_v + T + O, Nv) if on_visn else (r_l + L, C)), dev)
+                        other = blocks.segment_mean(x.f32, off, idx, B, seg=I)
+                    gate = blocks.embed(B, dev, a=t0, a2=other).f32
+                h = blocks.mul_bcast(ob_out, gate, lowp)
+            act_logits = blocks.mask_logits(blocks.cls_head(h, pk['act'], lowp), ob_nav_types)
         return act_logits, txt_out, hist_out, ob_out
 
     def h16_format(self):
