@@ -351,16 +351,22 @@ int vi_mul_bcast_bwd_s(const float* dy, const float* x, float* ds, int64_t n_bat
 /* adjoint of vi_cosine_loss: dloss is the device scalar gradient of the mean; dproj / dtgt may be NULL */
 int vi_cosine_loss_bwd(const float* proj, const float* tgt, const float* dloss, float* dproj, float* dtgt, int R,
                        vi_stream_t stream);
-/* adjoint of vi_infonce_loss w.r.t. proj (the noun-phrase means are constants under fix_lang_inside_cosine_model,
- * D/models/vilmodel.py:1249-1255); `sims` = the first R * (n_negs + 1) floats the forward call left in its loss_rows scratch */
+/* adjoint of vi_infonce_loss w.r.t. proj, and w.r.t. the text operands tgt / negs when the text encoder trains through the
+ * loss (fix_lang_inside_cosine_model off, D/models/vilmodel.py:1249-1262); `sims` = the first R * (n_negs + 1) floats the forward
+ * call left in its loss_rows scratch.  dproj is required; dtgt [R, 768] and dnegs [n_negs, 768] may be NULL.  With g_rc =
+ * dloss / dcos(proj[r], column c) (column 0 = tgt[r], column c >= 1 = negs[c - 1], zero for a negative of the row's own episode):
+ *   dtgt[r]  = g_r0 (p_r / (|p_r| |t_r|) - cos_r0 t_r / |t_r|^2)                      (written by the dproj launch)
+ *   dnegs[n] = sum_r g_rn (p_r / (|p_r| |t_n|) - cos_rn t_n / |t_n|^2)                 (a second launch, fixed summation order)
+ * dnegs needs `scratch`, R * (n_negs + 1) floats (g_rc of the negative columns and 1 / |p_r|), and 16-byte aligned proj / negs /
+ * dnegs.  With dtgt and dnegs NULL the call is the proj-only adjoint: one launch, same dproj bits. */
 int vi_infonce_loss_bwd(const float* proj, const float* tgt, const float* negs, const int32_t* row_episode,
                         const int32_t* neg_episode, float temperature, const float* sims, const float* dloss,
-                        float* dproj, int R, int n_negs, vi_stream_t stream);
-/* adjoint of vi_margin_loss w.r.t. proj (H/models/vilmodel_cmt.py:825-856); `sims` = the cosines the forward call left in its
- * loss_rows scratch */
+                        float* dproj, float* dtgt, float* dnegs, float* scratch, int R, int n_negs, vi_stream_t stream);
+/* adjoint of vi_margin_loss (H/models/vilmodel_cmt.py:825-856); `sims` = the cosines the forward call left in its loss_rows
+ * scratch; dtgt / dnegs / scratch as in vi_infonce_loss_bwd */
 int vi_margin_loss_bwd(const float* proj, const float* tgt, const float* negs, const int32_t* row_episode,
                        const int32_t* neg_episode, float margin, const float* sims, const float* dloss,
-                       float* dproj, int R, int n_negs, vi_stream_t stream);
+                       float* dproj, float* dtgt, float* dnegs, float* scratch, int R, int n_negs, vi_stream_t stream);
 
 /* Dropout (training only): y = x * keep / (1 - p) with keep(i) = hash(i, *seed, site) >= p * 2^32; the backward pass is the
  * same call on the gradient.  `seed` is a device pointer (the host module advances it once per optimiser step, also inside

@@ -95,8 +95,8 @@ PROTOTYPES = {
     'vi_duet_fuse_logits_bwd': [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p],
     'vi_mul_bcast_bwd_s': [_p, _p, _p, _l, _i, _p],
     'vi_cosine_loss_bwd': [_p, _p, _p, _p, _p, _i, _p],
-    'vi_infonce_loss_bwd': [_p, _p, _p, _p, _p, _f, _p, _p, _p, _i, _i, _p],
-    'vi_margin_loss_bwd': [_p, _p, _p, _p, _p, _f, _p, _p, _p, _i, _i, _p],
+    'vi_infonce_loss_bwd': [_p, _p, _p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _i, _i, _p],
+    'vi_margin_loss_bwd': [_p, _p, _p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _i, _i, _p],
     'vi_graph_init': [_p, _p, _p, _p, _i, _i, _p],
     'vi_graph_update': [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _i, _p, _p],
     'vi_graph_embed_step': [_p, _p, _i, _i, _i, _p, _p, _i, _p, _p, _p, _i, _p, _i, _p, _p, _p],

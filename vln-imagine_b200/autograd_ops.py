@@ -891,12 +891,31 @@ class CosineLossFn(Function):
         return dp, dt, None
 
 
+def _contrastive_loss_bwd(ctx, dloss, fn, name):
+    """shared backward of InfoNCELossFn / MarginLossFn: dproj always, dtgt / dnegs only when autograd asks for them (the text
+    encoder trains through the loss); otherwise NULL, and the call is the one-launch proj-only adjoint"""
+    proj, tgt, scratch = ctx.saved_tensors
+    negs, row_ep, neg_ep, param, R, n_negs = ctx.extra
+    dloss = dloss.contiguous().float().view(1)
+    dp = torch.empty_like(proj)
+    dt = torch.empty_like(tgt) if ctx.needs_input_grad[1] else None
+    want_negs = negs is not None and ctx.needs_input_grad[2]
+    dn = torch.empty_like(negs) if want_negs else None
+    work = torch.empty(R * (n_negs + 1), dtype=F32, device=proj.device) if want_negs and n_negs else None
+    check(fn(proj.data_ptr(), tgt.data_ptr(), _ptr(negs), row_ep.data_ptr(), _ptr(neg_ep), param, scratch.data_ptr(),
+             dloss.data_ptr(), dp.data_ptr(), _ptr(dt), _ptr(dn), _ptr(work), R, n_negs, _stream()), name)
+    _launched(2 if work is not None else 1)
+    return dp, dt, dn, None, None, None, None, None
+
+
 class InfoNCELossFn(Function):
-    """compute_contrastive_loss_infonce (models/vilmodel.py:657-687) with constant noun-phrase means; grad w.r.t. proj"""
+    """compute_contrastive_loss_infonce (models/vilmodel.py:657-687); grad w.r.t. proj, and w.r.t. the noun-phrase means of the
+    positive (tgt) and of the negatives (negs) when they require grad"""
 
     @staticmethod
     def forward(ctx, proj, tgt, negs, row_ep, neg_ep, temperature, R, n_negs):
-        proj = proj.contiguous()
+        proj, tgt = proj.contiguous(), tgt.contiguous()
+        negs = negs.contiguous() if negs is not None else None
         loss, scratch = ops.infonce_loss(proj, tgt, negs, row_ep, neg_ep, temperature, R, n_negs, proj.device)
         ctx.save_for_backward(proj, tgt, scratch)
         ctx.extra = (negs, row_ep, neg_ep, float(temperature), R, n_negs)
@@ -904,23 +923,17 @@ class InfoNCELossFn(Function):
 
     @staticmethod
     def backward(ctx, dloss):
-        proj, tgt, scratch = ctx.saved_tensors
-        negs, row_ep, neg_ep, temperature, R, n_negs = ctx.extra
-        dloss = dloss.contiguous().float().view(1)
-        dp = torch.empty_like(proj)
-        check(lib.vi_infonce_loss_bwd(proj.data_ptr(), tgt.data_ptr(), _ptr(negs), row_ep.data_ptr(), _ptr(neg_ep), temperature,
-                                      scratch.data_ptr(), dloss.data_ptr(), dp.data_ptr(), R, n_negs, _stream()),
-              'vi_infonce_loss_bwd')
-        _launched(1)
-        return dp, None, None, None, None, None, None, None
+        return _contrastive_loss_bwd(ctx, dloss, lib.vi_infonce_loss_bwd, 'vi_infonce_loss_bwd')
 
 
 class MarginLossFn(Function):
-    """compute_contrastive_loss_margin (H/models/vilmodel_cmt.py:825-856) with constant noun-phrase means; grad w.r.t. proj"""
+    """compute_contrastive_loss_margin (H/models/vilmodel_cmt.py:825-856); grad w.r.t. proj, and w.r.t. the noun-phrase means of
+    the positive (tgt) and of the negatives (negs) when they require grad"""
 
     @staticmethod
     def forward(ctx, proj, tgt, negs, row_ep, neg_ep, margin, R, n_negs):
-        proj = proj.contiguous()
+        proj, tgt = proj.contiguous(), tgt.contiguous()
+        negs = negs.contiguous() if negs is not None else None
         loss, scratch = ops.margin_loss(proj, tgt, negs, row_ep, neg_ep, margin, R, n_negs, proj.device)
         ctx.save_for_backward(proj, tgt, scratch)
         ctx.extra = (negs, row_ep, neg_ep, float(margin), R, n_negs)
@@ -928,15 +941,7 @@ class MarginLossFn(Function):
 
     @staticmethod
     def backward(ctx, dloss):
-        proj, tgt, scratch = ctx.saved_tensors
-        negs, row_ep, neg_ep, margin, R, n_negs = ctx.extra
-        dloss = dloss.contiguous().float().view(1)
-        dp = torch.empty_like(proj)
-        check(lib.vi_margin_loss_bwd(proj.data_ptr(), tgt.data_ptr(), _ptr(negs), row_ep.data_ptr(), _ptr(neg_ep), margin,
-                                     scratch.data_ptr(), dloss.data_ptr(), dp.data_ptr(), R, n_negs, _stream()),
-              'vi_margin_loss_bwd')
-        _launched(1)
-        return dp, None, None, None, None, None, None, None
+        return _contrastive_loss_bwd(ctx, dloss, lib.vi_margin_loss_bwd, 'vi_margin_loss_bwd')
 
 
 class MulBcastFn(Function):

@@ -778,14 +778,18 @@ __global__ void __launch_bounds__(128) cosine_loss_bwd_kernel(const float* proj,
 
 // InfoNCE alignment loss adjoint (vilmodel.py:657-687):  loss = mean_r [ logsumexp_{c valid} s_rc - s_r0 ],
 // s_rc = cos(p_r, t_c) / tau with t_0 = the row's own noun-phrase mean and t_c (c >= 1) the noun-phrase means of OTHER
-// episodes.  With w_rc = softmax_c(s_rc) - [c == 0]:
-//     dp_r = (dloss / (R tau)) * sum_c w_rc ( t_c / (|p_r| |t_c|) - cos_rc p_r / |p_r|^2 )
+// episodes.  With w_rc = softmax_c(s_rc) - [c == 0] and g_rc = dloss w_rc / (R tau) = dloss / dcos_rc:
+//     dp_r = sum_c g_rc ( t_c / (|p_r| |t_c|) - cos_rc p_r / |p_r|^2 )
+//     dt_r = g_r0 ( p_r / (|p_r| |t_r|) - cos_r0 t_r / |t_r|^2 )                       (dtgt, optional)
+// With `gneg` given, g_rc of every negative column (0 for the row's own episode) goes to gneg[r, c - 1] and 1 / |p_r| to
+// inv_np[r]: the operands of contrastive_negs_bwd_kernel.  dproj does not depend on either option.
 // `sims` is what the forward pass left in its scratch (s_rc for every column, valid or not).  One warp per row.
 __global__ void __launch_bounds__(128) infonce_loss_bwd_kernel(const float* proj, const float* tgt, const float* negs,
                                                                const int32_t* row_ep, const int32_t* neg_ep, float inv_t,
                                                                const float* sims, const float* dloss,
-                                                               float* __restrict__ dproj, int R, int n_negs, int margin_mode,
-                                                               float margin) {
+                                                               float* __restrict__ dproj, float* __restrict__ dtgt,
+                                                               float* __restrict__ gneg, float* __restrict__ inv_np,
+                                                               int R, int n_negs, int margin_mode, float margin) {
   pdl_enter();
   const int lane = threadIdx.x & 31;
   const long long row = (long long)blockIdx.x * 4 + (threadIdx.x >> 5);
@@ -816,6 +820,7 @@ __global__ void __launch_bounds__(128) infonce_loss_bwd_kernel(const float* proj
   for (int i = 0; i < 24; ++i) { a[i] = proj[row * D + lane + 32 * i]; aa = fmaf(a[i], a[i], aa); acc[i] = 0.f; }
   aa = warp_sum(aa);
   const float na = fmaxf(sqrtf(aa), 1e-8f);
+  const float scale = dloss[0] * inv_t / (float)R;
   float wcos = 0.f;                                    // sum_c w_rc cos_rc
   for (int c = 0; c < cols; ++c) {
     if (c > 0 && neg_ep[c - 1] == ep) continue;        // warp-uniform
@@ -836,11 +841,86 @@ __global__ void __launch_bounds__(128) infonce_loss_bwd_kernel(const float* proj
 #pragma unroll
     for (int i = 0; i < 24; ++i) acc[i] = fmaf(k, tv[i], acc[i]);
     wcos = fmaf(w, s[c], wcos);                        // s = cos / tau
+    if (c == 0 && dtgt) {
+      const float nt = fmaxf(sqrtf(bb), 1e-8f), g0 = scale * w, cos0 = s[0] / inv_t;
+#pragma unroll
+      for (int i = 0; i < 24; ++i) dtgt[row * D + lane + 32 * i] = g0 * (a[i] / (na * nt) - cos0 * tv[i] / (nt * nt));
+    }
   }
   wcos /= inv_t;
-  const float scale = dloss[0] * inv_t / (float)R;
 #pragma unroll
   for (int i = 0; i < 24; ++i) dproj[row * D + lane + 32 * i] = scale * (acc[i] / na - wcos * a[i] / (na * na));
+  if (gneg) {
+    for (int c = 1 + lane; c < cols; c += 32) {
+      float w = 0.f;
+      if (neg_ep[c - 1] != ep)
+        w = margin_mode ? ((margin + s[c] - s[0] > 0.f) ? 1.f / cnt : 0.f) : expf(s[c] - mx) * inv_sum;
+      gneg[row * n_negs + c - 1] = scale * w;
+    }
+    if (lane == 0) inv_np[row] = 1.0f / na;
+  }
+}
+
+// Adjoint of the alignment losses w.r.t. the negatives (the noun-phrase means of the other episodes):
+//     dneg_n = (1 / |t_n|) sum_r g_rn p_r / |p_r|  -  (sum_r g_rn cos_rn / |t_n|^2) t_n
+// with g_rn = gneg[r, n] and 1 / |p_r| = inv_np[r] from infonce_loss_bwd_kernel, cos_rn = cos_scale * sims[r, 1 + n].  The sum
+// over rows is G^T P-hat ([n_negs, R] x [R, 768]): a CTA owns NEG_TILE negatives x 256 columns, each thread 4 columns of all
+// NEG_TILE negatives, so every row of proj is read once per NEG_TILE negatives.  Rows are summed in a fixed order and every
+// output element has one writer: two calls are bit-identical.
+constexpr int NEG_TILE = 8, NEG_ROWS = 32;
+__global__ void __launch_bounds__(64) contrastive_negs_bwd_kernel(const float* proj, const float* negs, const float* sims,
+                                                                  const float* gneg, const float* inv_np, float cos_scale,
+                                                                  float* __restrict__ dnegs, int R, int n_negs) {
+  pdl_enter();
+  __shared__ __align__(16) float wt[NEG_ROWS][NEG_TILE];
+  __shared__ float nrm[NEG_TILE], gcos[NEG_TILE];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int n0 = blockIdx.x * NEG_TILE;
+  const int col = blockIdx.y * 256 + tid * 4;
+  const long long cols = n_negs + 1;
+  // per negative: |t_n| and sum_r g_rn cos_rn (lane-strided partial sums, then the butterfly: a fixed order)
+  for (int k = warp; k < NEG_TILE; k += 2) {
+    const int n = n0 + k;
+    float tt = 0.f, gc = 0.f;
+    if (n < n_negs) {
+      for (int i = lane; i < D; i += 32) { const float t = negs[(long long)n * D + i]; tt = fmaf(t, t, tt); }
+      for (int r = lane; r < R; r += 32) gc = fmaf(gneg[(long long)r * n_negs + n], sims[r * cols + 1 + n], gc);
+    }
+    tt = warp_sum(tt); gc = warp_sum(gc);
+    if (lane == 0) { nrm[k] = fmaxf(sqrtf(tt), 1e-8f); gcos[k] = gc * cos_scale; }
+  }
+  float4 acc[NEG_TILE];
+#pragma unroll
+  for (int k = 0; k < NEG_TILE; ++k) acc[k] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int r0 = 0; r0 < R; r0 += NEG_ROWS) {
+    __syncthreads();                                   // the previous tile is consumed
+    for (int e = tid; e < NEG_ROWS * NEG_TILE; e += 64) {
+      const int j = e / NEG_TILE, k = e % NEG_TILE, r = r0 + j, n = n0 + k;
+      wt[j][k] = (r < R && n < n_negs) ? gneg[(long long)r * n_negs + n] * inv_np[r] : 0.f;
+    }
+    __syncthreads();
+    const int rows = min(NEG_ROWS, R - r0);
+#pragma unroll 4
+    for (int j = 0; j < rows; ++j) {
+      const float4 p = *reinterpret_cast<const float4*>(proj + (long long)(r0 + j) * D + col);
+#pragma unroll
+      for (int k = 0; k < NEG_TILE; ++k) {
+        const float w = wt[j][k];
+        acc[k].x = fmaf(w, p.x, acc[k].x); acc[k].y = fmaf(w, p.y, acc[k].y);
+        acc[k].z = fmaf(w, p.z, acc[k].z); acc[k].w = fmaf(w, p.w, acc[k].w);
+      }
+    }
+  }
+  __syncthreads();                                     // nrm / gcos
+#pragma unroll
+  for (int k = 0; k < NEG_TILE; ++k) {
+    const int n = n0 + k;
+    if (n >= n_negs) break;
+    const float inv = 1.0f / nrm[k], coef = gcos[k] * inv * inv;
+    const float4 t = *reinterpret_cast<const float4*>(negs + (long long)n * D + col);
+    *reinterpret_cast<float4*>(dnegs + (long long)n * D + col) =
+        make_float4(acc[k].x * inv - coef * t.x, acc[k].y * inv - coef * t.y, acc[k].z * inv - coef * t.z, acc[k].w * inv - coef * t.w);
+  }
 }
 
 inline bool make_groups(RowGroups& g, int n_groups, const int32_t* ends) {
@@ -1087,25 +1167,40 @@ extern "C" int vi_cosine_loss_bwd(const float* proj, const float* tgt, const flo
   return VI_OK;
 }
 
+// the two contrastive loss adjoints: one launch for dproj (and dtgt), a second one for dnegs when it is asked for
+static int contrastive_loss_bwd(const char* name, const float* proj, const float* tgt, const float* negs,
+                                const int32_t* row_episode, const int32_t* neg_episode, float inv_t, const float* sims,
+                                const float* dloss, float* dproj, float* dtgt, float* dnegs, float* scratch, int R, int n_negs,
+                                int margin_mode, float margin, vi_stream_t stream) {
+  VI_CHECK_ARG(proj && tgt && row_episode && sims && dloss && dproj, "%s: null operand", name);
+  VI_CHECK_ARG(n_negs == 0 || (negs && neg_episode), "%s: negatives missing", name);
+  const bool want_negs = dnegs && n_negs > 0;
+  VI_CHECK_ARG(!want_negs || scratch, "%s: dnegs needs the R * (n_negs + 1) float scratch", name);
+  VI_CHECK_ARG(!want_negs || (aligned16(proj) && aligned16(negs) && aligned16(dnegs)), "%s: misaligned operands", name);
+  if (R <= 0) return VI_OK;
+  float* gneg = want_negs ? scratch : nullptr;
+  float* inv_np = want_negs ? scratch + (long long)R * n_negs : nullptr;
+  VI_CUDA(vi_launch(infonce_loss_bwd_kernel, dim3((unsigned)((R + 3) / 4)), dim3(128), 0, ST(stream), proj, tgt, negs, row_episode,
+                    neg_episode, inv_t, sims, dloss, dproj, dtgt, gneg, inv_np, R, n_negs, margin_mode, margin));
+  if (want_negs)
+    VI_CUDA(vi_launch(contrastive_negs_bwd_kernel, dim3((unsigned)((n_negs + NEG_TILE - 1) / NEG_TILE), D / 256), dim3(64), 0,
+                      ST(stream), proj, negs, sims, (const float*)gneg, (const float*)inv_np, 1.0f / inv_t, dnegs, R, n_negs));
+  return VI_OK;
+}
+
 extern "C" int vi_infonce_loss_bwd(const float* proj, const float* tgt, const float* negs, const int32_t* row_episode,
                                    const int32_t* neg_episode, float temperature, const float* sims, const float* dloss,
-                                   float* dproj, int R, int n_negs, vi_stream_t stream) {
-  VI_CHECK_ARG(proj && tgt && row_episode && sims && dloss && dproj, "vi_infonce_loss_bwd: null operand");
-  VI_CHECK_ARG(n_negs == 0 || (negs && neg_episode), "vi_infonce_loss_bwd: negatives missing");
+                                   float* dproj, float* dtgt, float* dnegs, float* scratch, int R, int n_negs,
+                                   vi_stream_t stream) {
   VI_CHECK_ARG(temperature > 0.f, "vi_infonce_loss_bwd: temperature must be positive");
-  if (R <= 0) return VI_OK;
-  VI_CUDA(vi_launch(infonce_loss_bwd_kernel, dim3((unsigned)((R + 3) / 4)), dim3(128), 0, ST(stream), proj, tgt, negs, row_episode,
-                    neg_episode, 1.0f / temperature, sims, dloss, dproj, R, n_negs, 0, 0.f));
-  return VI_OK;
+  return contrastive_loss_bwd("vi_infonce_loss_bwd", proj, tgt, negs, row_episode, neg_episode, 1.0f / temperature, sims, dloss,
+                              dproj, dtgt, dnegs, scratch, R, n_negs, 0, 0.f, stream);
 }
 
 extern "C" int vi_margin_loss_bwd(const float* proj, const float* tgt, const float* negs, const int32_t* row_episode,
                                   const int32_t* neg_episode, float margin, const float* sims, const float* dloss,
-                                  float* dproj, int R, int n_negs, vi_stream_t stream) {
-  VI_CHECK_ARG(proj && tgt && row_episode && sims && dloss && dproj, "vi_margin_loss_bwd: null operand");
-  VI_CHECK_ARG(n_negs == 0 || (negs && neg_episode), "vi_margin_loss_bwd: negatives missing");
-  if (R <= 0) return VI_OK;
-  VI_CUDA(vi_launch(infonce_loss_bwd_kernel, dim3((unsigned)((R + 3) / 4)), dim3(128), 0, ST(stream), proj, tgt, negs, row_episode,
-                    neg_episode, 1.0f, sims, dloss, dproj, R, n_negs, 1, margin));
-  return VI_OK;
+                                  float* dproj, float* dtgt, float* dnegs, float* scratch, int R, int n_negs,
+                                  vi_stream_t stream) {
+  return contrastive_loss_bwd("vi_margin_loss_bwd", proj, tgt, negs, row_episode, neg_episode, 1.0f, sims, dloss, dproj, dtgt,
+                              dnegs, scratch, R, n_negs, 1, margin, stream);
 }

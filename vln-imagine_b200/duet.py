@@ -144,9 +144,9 @@ def _align_rows(B, L, I, flags, noun_phrase_segs, dev):
 def align_forward(model, align_txt_embeds, align_imagine_embeds, flags, noun_phrase_segs, lowp: bool, rows: AlignRows = None):
     """Shared by DUET and HAMT.  Returns (loss 0-d tensor, imagine embeds with projected rows written back).  ``rows``: index
     arrays already built by the caller (REVERIE) instead of the sub-instruction annotation.  With autograd recording the
-    projection MLP, the loss and the write-back of the projected rows (models/vilmodel.py:646) are differentiable; the
-    noun-phrase means of the negatives are constants, and the text target trains only when the text requires grad
-    (fix_lang_inside_cosine_model off, :1256-1262)."""
+    projection MLP, the loss and the write-back of the projected rows (models/vilmodel.py:646) are differentiable; the text
+    operands of the loss - the positive noun-phrase means and, for the contrastive forms, the noun-phrase means of the negatives,
+    both built from ``align_txt_embeds`` - train when the text requires grad (fix_lang_inside_cosine_model off, :1256-1262)."""
     cfg = model.config
     B, L, _ = align_txt_embeds.shape
     I = align_imagine_embeds.shape[1]
@@ -160,9 +160,6 @@ def align_forward(model, align_txt_embeds, align_imagine_embeds, flags, noun_phr
     pk = model._pk()['align']
     train = blocks.training()
     if train:
-        if txt.requires_grad and cfg.aux_loss_type != 'cosine':
-            raise NotImplementedError('training the text encoder through the %r alignment loss (fix_lang_inside_cosine_model=False) '
-                                      'is not built: only the cosine form carries gradients to the text means' % cfg.aux_loss_type)
         if cfg.aux_loss_type not in ('cosine', 'contrastive-InfoNCE', 'constrastive-margin'):
             raise NotImplementedError('backward of aux_loss_type %r' % cfg.aux_loss_type)
         x = ag.GatherSlotsFn.apply(img, rows.unit, rows.slot, rows.R, lowp)
@@ -177,7 +174,7 @@ def align_forward(model, align_txt_embeds, align_imagine_embeds, flags, noun_phr
     tgt = blocks.segment_mean(txt, rows.tok_off, rows.tok_rows, rows.R)
     negs, neg_ep = None, None
     if rows.n_negs and cfg.aux_loss_type != 'cosine':         # AlignWithContrastiveLossWithNegativeSamples (:689-779)
-        negs, _ = ops.gather_mean(txt, rows.np_off, rows.np_rows, rows.n_negs, want16=False)
+        negs = blocks.segment_mean(txt, rows.np_off, rows.np_rows, rows.n_negs)
         neg_ep = rows.np_ep
     if cfg.aux_loss_type == 'cosine':
         loss = ag.CosineLossFn.apply(x, tgt, rows.R) if train else ops.cosine_loss(x, tgt, rows.R, dev)[0]
