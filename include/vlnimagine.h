@@ -13,7 +13,8 @@
  *  - activations are row-major [rows, ld] with ld in ELEMENTS; hidden size is 768, 12 heads of 64;
  *  - return value: VI_OK or a negative VI_ERR_*; vi_last_error() gives the thread-local message;
  *    nothing throws or exits across the ABI;
- *  - re-entrant; no global mutable state besides per-process immutable driver entry points.
+ *  - re-entrant; no global mutable state besides per-process immutable driver entry points and
+ *    the launch counter below.
  */
 #ifndef VLNIMAGINE_H_
 #define VLNIMAGINE_H_
@@ -42,6 +43,8 @@ typedef void* vi_stream_t; /* cudaStream_t */
 
 int vi_version(void);
 const char* vi_last_error(void);
+/* Kernels the library has launched successfully in this process, over all devices and threads. */
+int64_t vi_launch_count(void);
 /* Select the device, resolve cuTensorMapEncodeTiled, raise the dynamic shared-memory limits. */
 int vi_init(int device);
 

@@ -21,6 +21,12 @@ def ag(lib_built):
 
 
 @pytest.fixture(scope='module')
+def ops(ag):
+    import importlib
+    return importlib.import_module('vln_imagine_b200.ops')
+
+
+@pytest.fixture(scope='module')
 def blocks(ag):
     import importlib
     return importlib.import_module('vln_imagine_b200.blocks')
@@ -52,15 +58,15 @@ class _LN:
 
 @pytest.mark.parametrize('dtype', [torch.float32, torch.bfloat16])
 @pytest.mark.parametrize('rows,cols,pad', [(37, 768, 64), (300, 2304, 320), (64, 64, 64), (1000, 14, 1000)])
-def test_transpose_and_colsum(ag, dtype, rows, cols, pad):
+def test_transpose_and_colsum(ops, dtype, rows, cols, pad):
     x = _rand(rows, cols, seed=1).to(dtype)
-    t = ag.transpose(x, pad)
+    t = ops.transpose(x, pad)
     assert t.shape == (cols, pad)
     assert torch.equal(t[:, :rows], x.t())
     assert float(t[:, rows:].float().abs().sum()) == 0.0
     view = _rand(rows, cols + 24, seed=2).to(dtype)[:, 8:8 + cols]         # strided source
-    assert torch.equal(ag.transpose(view, pad)[:, :rows], view.t())
-    cs = ag.colsum(x)
+    assert torch.equal(ops.transpose(view, pad)[:, :rows], view.t())
+    cs = ops.colsum(x)
     assert relerr(cs, x.float().sum(0)) < 1e-5
 
 
@@ -332,14 +338,14 @@ def test_infonce_loss_bwd(ag, T):
     (520, 512, 768, None),                # projection head
     (1000, 256, 192, [256, 1000]),        # 64-wide tiles, uneven groups
 ])
-def test_wgrad16_vs_torch(ag, M, N, K, ends, dtype):
+def test_wgrad16_vs_torch(ops, M, N, K, ends, dtype):
     """vi_wgrad16 (MN-major tcgen05 operands, split rows, ones-tile bias gradient) against dY^T X / dY.sum(0) in fp32 of the
     same 16-bit values; two calls are bit-identical (fixed-order reduction of the split partials)"""
     dy = (_rand(M, N, seed=51) * 0.5).to(dtype)
     x = _rand(M, K, seed=52).to(dtype)
-    assert ag.wgrad16_ok(dy, x)
-    dW, db = ag.wgrad16(dy, x, ends, True)
-    dW2, db2 = ag.wgrad16(dy, x, ends, True)
+    assert ops.wgrad16_ok(dy, x)
+    dW, db = ops.wgrad16(dy, x, ends, True)
+    dW2, db2 = ops.wgrad16(dy, x, ends, True)
     torch.cuda.synchronize()
     assert torch.equal(dW, dW2) and torch.equal(db, db2)
     bounds = [0] + (ends or [M])
@@ -349,7 +355,7 @@ def test_wgrad16_vs_torch(ag, M, N, K, ends, dtype):
         ref_b = dy[r0:r1].float().sum(0)
         assert relerr(dW[g * N:(g + 1) * N], ref_w) < 2e-3, (g, relerr(dW[g * N:(g + 1) * N], ref_w))
         assert relerr(db[g * N:(g + 1) * N], ref_b) < 2e-3, (g, relerr(db[g * N:(g + 1) * N], ref_b))
-    dW3, db3 = ag.wgrad16(dy, x, ends, False)
+    dW3, db3 = ops.wgrad16(dy, x, ends, False)
     assert db3 is None and torch.equal(dW3, dW)
 
 

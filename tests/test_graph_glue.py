@@ -99,7 +99,6 @@ def test_device_graph_maps_host_bookkeeping_without_a_gpu(monkeypatch):
     monkeypatch.setattr(gm_mod, 'lib', FakeLib())
     monkeypatch.setattr(ops, 'ensure_init', lambda t: None)
     monkeypatch.setattr(ops, '_stream', lambda: 0)
-    monkeypatch.setattr(ops, '_launched', lambda n: None)
     monkeypatch.setattr(torch.Tensor, 'pin_memory', lambda self: self)
     packed = {}
     real_pack = gm_mod._pack

@@ -39,6 +39,7 @@ def test_ctypes_prototypes_cover_the_header(lib_built):
     _lib = importlib.import_module('vln_imagine_b200._lib')
     declared = set(header_symbols()) - {'vi_last_error'}
     assert declared == set(_lib.PROTOTYPES), declared ^ set(_lib.PROTOTYPES)
+    assert _lib.QUERIES <= declared | {'vi_last_error'}
 
 
 def test_library_contains_blackwell_tensor_core_and_tma_code(lib_built):

@@ -10,7 +10,6 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from vln_imagine_b200 import _lib, ops  # noqa: E402
-from vln_imagine_b200 import autograd_ops as ag  # noqa: E402
 from vln_imagine_b200._lib import check, lib  # noqa: E402
 
 dev = torch.device('cuda')
@@ -63,7 +62,7 @@ for name, M, ends, N, K in (('nav proj 768x768', 4416, [2048, 4416], 768, 768), 
         parts.append((dy[lo:b], x[lo:b]))
         lo = b
     rec['cublas bf16 (no bias grad)'] = round(timeit(lambda: [a.t() @ c for a, c in parts]), 2)
-    rec['old: 2 transposes + gemm + colsum'] = round(timeit(lambda: [(ops.gemm(ag.transpose(a, ag.pad64(a.shape[0])), ag.transpose(c, ag.pad64(a.shape[0])),
-                                                                       None, out_dtype=torch.float32), ag.colsum(a)) for a, c in parts]), 2)
+    rec['old: 2 transposes + gemm + colsum'] = round(timeit(lambda: [(ops.gemm(ops.transpose(a, ops.pad64(a.shape[0])), ops.transpose(c, ops.pad64(a.shape[0])),
+                                                                       None, out_dtype=torch.float32), ops.colsum(a)) for a, c in parts]), 2)
     rec['TF/s'] = round(rec['gflop'] / rec['wgrad16 S=%d' % S0] * 1e3, 1)
     print(name, json.dumps(rec), flush=True)

@@ -57,6 +57,7 @@ class AttnProblem(C.Structure):
 # name -> argtypes; every entry of include/vlnimagine.h must appear here (tests check the header against it)
 PROTOTYPES = {
     'vi_version': [],
+    'vi_launch_count': [],
     'vi_init': [_i],
     'vi_gemm16': [C.POINTER(GemmArgs), _p],
     'vi_gemm_f32': [_p, _l, _p, _p, _p, _l, _p, _l, _i, _i, _i, _i, _i, _ip, _p],
@@ -102,11 +103,14 @@ PROTOTYPES = {
     'vi_graph_embed_step': [_p, _p, _i, _i, _i, _p, _p, _i, _p, _p, _p, _i, _p, _i, _p, _p, _p],
     'vi_graph_features': [_p, _p, _p, _i, _i, _p, _p, _p, _p, _p, _i, _p, _p, _p, _i, _p, _i, _p, _p],
 }
+# entry points that return a value rather than a VI_OK / VI_ERR_* status (ops.lib passes their result through unchecked)
+QUERIES = {'vi_version', 'vi_wgrad16_splits', 'vi_wgrad16_workspace', 'vi_launch_count', 'vi_last_error'}
 for _name, _args in PROTOTYPES.items():
     _fn = getattr(lib, _name)            # AttributeError here = header/library mismatch: fail loudly
     _fn.argtypes = _args
     _fn.restype = _i
 lib.vi_wgrad16_workspace.restype = C.c_int64
+lib.vi_launch_count.restype = C.c_int64
 lib.vi_last_error.argtypes = []
 lib.vi_last_error.restype = C.c_char_p
 
@@ -115,19 +119,13 @@ class VlnImagineError(RuntimeError):
     pass
 
 
+def failure(rc: int, what: str = '') -> VlnImagineError:
+    return VlnImagineError('%s failed (%d): %s' % (what or 'libvlnimagine call', rc, lib.vi_last_error().decode()))
+
+
 def check(rc: int, what: str = ''):
     if rc != VI_OK:
-        raise VlnImagineError('%s failed (%d): %s' % (what or 'libvlnimagine call', rc, lib.vi_last_error().decode()))
-
-
-_initialised = set()
-
-
-def init(device_index: int):
-    """vi_init once per device (selects it, checks sm_100, raises shared-memory limits)."""
-    if device_index not in _initialised:
-        check(lib.vi_init(device_index), 'vi_init')
-        _initialised.add(device_index)
+        raise failure(rc, what)
 
 
 def int_array(values):

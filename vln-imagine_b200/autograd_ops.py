@@ -2,7 +2,7 @@
 
 Used when a mode is called with autograd recording (fine-tuning, BASELINE.json cfg-4).  The autograd engine only
 chains the nodes and accumulates gradients at fan-out points (residual branches) and into ``.grad``; it performs
-no model arithmetic itself.  Conventions:
+no model arithmetic itself, and the nodes launch every kernel through an ``ops`` function.  Conventions:
 
 * dense layers: ``dX = dY W`` runs the tcgen05 GEMM on the transposed bf16 weight shadow; ``dW = dY^T X`` and ``db`` come
   from vi_wgrad16 on dY and X as they lie in memory (all groups of a row-stacked layer in one launch).  The fp32 check mode
@@ -14,64 +14,15 @@ no model arithmetic itself.  Conventions:
 """
 from __future__ import annotations
 
-from typing import List, Optional, Sequence
-
 import torch
 from torch.autograd import Function
 
 from . import _lib, ops
-from .ops import BF16, F32, HIDDEN, EPI_GELU, EPI_NONE, EPI_RELU, MASK_ADD_NEG10000, _ptr, _stream, check, lib, _launched
+from .ops import BF16, F32, HIDDEN, EPI_GELU, EPI_NONE, EPI_RELU, MASK_ADD_NEG10000, colsum, pad64, transpose, wgrad16, wgrad16_ok
 
 
 def needs_grad(*tensors) -> bool:
     return torch.is_grad_enabled() and any(t is not None and torch.is_tensor(t) and t.requires_grad for t in tensors)
-
-
-def pad64(n: int) -> int:
-    return (n + 63) // 64 * 64
-
-
-def _dt(t: torch.Tensor) -> int:
-    return _lib.DT_BF16 if t.dtype == BF16 else _lib.DT_F32
-
-
-def transpose(src: torch.Tensor, pad_rows: Optional[int] = None) -> torch.Tensor:
-    """[rows, cols] view -> [cols, pad_rows] (zero padded columns)"""
-    rows, cols = src.shape
-    pr = pad_rows or rows
-    dst = torch.empty((cols, pr), dtype=src.dtype, device=src.device)
-    check(lib.vi_transpose(src.data_ptr(), src.stride(0), dst.data_ptr(), dst.stride(0), rows, cols, pr, _dt(src), _stream()),
-          'vi_transpose')
-    _launched(1)
-    return dst
-
-
-_SCRATCH = {}
-RED_CHUNK = 128
-
-
-def reduce_scratch(device, rows: int, cols: int, n_out: int) -> torch.Tensor:
-    """fp32 workspace of the two-stage column reductions (caller-owned, one per device, grown on demand; launches
-    that share it are ordered by the stream they run on)"""
-    need = n_out * ((rows + RED_CHUNK - 1) // RED_CHUNK) * cols
-    t = _SCRATCH.get(device)
-    if t is None or t.numel() < need:
-        t = torch.empty((max(need, 1 << 22),), dtype=F32, device=device)
-        _SCRATCH[device] = t
-    return t
-
-
-def colsum(x: torch.Tensor) -> torch.Tensor:
-    rows, cols = x.shape
-    out = torch.empty((cols,), dtype=F32, device=x.device)
-    sc = reduce_scratch(x.device, rows, cols, 1)
-    check(lib.vi_colsum(x.data_ptr(), x.stride(0), _dt(x), out.data_ptr(), rows, cols, sc.data_ptr(), sc.numel(), _stream()),
-          'vi_colsum')
-    _launched(2)
-    return out
-
-
-_WGRAD_WS = {}
 
 
 class _GradAcc:
@@ -153,49 +104,7 @@ def _acc_flush():
     _GradAcc.queued = False
     if dsts:
         torch._foreach_add_(dsts, srcs)
-        _launched(1)
-
-
-def wgrad16(dy16: torch.Tensor, x16: torch.Tensor, ends, want_db: bool, out=None, accumulate: int = 0):
-    """(dW [n_groups * N, K] fp32, db [n_groups * N] fp32 or None) of a (grouped) dense layer from the 16-bit row-major dY [M, N]
-    and X [M, K] as they are (vi_wgrad16: MN-major tcgen05 operands, no transposed copies, bias gradient on the tensor cores).
-    out = (dW, db) preallocated; accumulate = 1 adds to them."""
-    M, N = dy16.shape
-    K = x16.shape[1]
-    bounds = [min(int(e), M) for e in ends] if ends is not None else [M]
-    G = len(bounds)
-    rows = _lib.int_array([b - (bounds[i - 1] if i else 0) for i, b in enumerate(bounds)])
-    S = int(_lib.lib.vi_wgrad16_splits(N, K, G, rows))               # host-side queries: not launches
-    need = int(_lib.lib.vi_wgrad16_workspace(N, K, G, rows, S))
-    ws = None
-    if need > 0:
-        ws = _WGRAD_WS.get(dy16.device)
-        if ws is None or ws.numel() < need:
-            ws = torch.empty((max(need, 1 << 23),), dtype=F32, device=dy16.device)
-            _WGRAD_WS[dy16.device] = ws
-    if out is not None:
-        dW, db = out
-    else:
-        dW = torch.empty((G * N, K), dtype=F32, device=dy16.device)
-        db = torch.empty((G * N,), dtype=F32, device=dy16.device) if want_db else None
-    tr = ops._Counters.gemm_trace                                    # bench.py: tensor-core launches with their FLOPs
-    if tr is not None:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-    check(lib.vi_wgrad16(dy16.data_ptr(), dy16.stride(0), x16.data_ptr(), x16.stride(0), ops._DT[dy16.dtype], N, K, G,
-                         _lib.int_array(bounds), dW.data_ptr(), _ptr(db), _ptr(ws), ws.numel() if ws is not None else 0, S,
-                         int(accumulate), _stream()), 'vi_wgrad16')
-    if tr is not None:
-        e1.record()
-        tr.append((bounds[-1], N, K, e0, e1))
-    _launched(2 if S > 1 else 1)
-    return dW, db
-
-
-def wgrad16_ok(dy16: torch.Tensor, x16: torch.Tensor) -> bool:
-    return (ops.is16(dy16.dtype) and x16.dtype == dy16.dtype and dy16.shape[1] % 128 == 0 and x16.shape[1] % 64 == 0
-            and dy16.stride(1) == 1 and x16.stride(1) == 1 and dy16.stride(0) % 8 == 0 and x16.stride(0) % 8 == 0
-            and dy16.data_ptr() % 16 == 0 and x16.data_ptr() % 16 == 0)
+        ops._Counters.other_launches += 1
 
 
 def to_operand(t: torch.Tensor, lowp: bool) -> torch.Tensor:
@@ -237,12 +146,7 @@ def next_site() -> int:
 
 def dropout_raw(x: torch.Tensor, p: float, site: int) -> torch.Tensor:
     """y = x * keep / (1 - p) (no autograd); the same call on a gradient is the backward pass"""
-    x = x.contiguous()
-    y = torch.empty_like(x)
-    check(lib.vi_dropout(x.data_ptr(), y.data_ptr(), x.numel(), float(p), dropout_seed(x.device).data_ptr(), site, _dt(x), _stream()),
-          'vi_dropout')
-    _launched(1)
-    return y
+    return ops.dropout(x, p, dropout_seed(x.device), site)
 
 
 class DropoutFn(Function):
@@ -399,12 +303,9 @@ class ActFn(Function):
     @staticmethod
     def forward(ctx, x, act):
         x = x.contiguous()
-        y = torch.empty_like(x)
-        check(lib.vi_act_fwd(x.data_ptr(), y.data_ptr(), x.numel(), act, _dt(x), _stream()), 'vi_act_fwd')
-        _launched(1)
         ctx.save_for_backward(x)
         ctx.act = act
-        return y
+        return ops.act_fwd(x, act)
 
     @staticmethod
     def backward(ctx, dy):
@@ -412,10 +313,7 @@ class ActFn(Function):
         dy = dy.contiguous()
         if dy.dtype != x.dtype:
             dy = dy.to(x.dtype)
-        dx = torch.empty_like(x)
-        check(lib.vi_act_bwd(x.data_ptr(), dy.data_ptr(), dx.data_ptr(), x.numel(), ctx.act, _dt(x), _stream()), 'vi_act_bwd')
-        _launched(1)
-        return dx, None
+        return ops.act_bwd(x, dy, ctx.act), None
 
 
 class LayerNormFn(Function):
@@ -439,7 +337,6 @@ class LayerNormFn(Function):
     def backward(ctx, dy32, dy16):
         a, b, gamma = ctx.saved_tensors
         b = b if ctx.has_b else None
-        rows = a.shape[0]
         ends = ctx.ends
         n_groups = 1 if ends is None else len(ends)
         if dy16 is not None and dy16.numel() == 0:
@@ -450,15 +347,8 @@ class LayerNormFn(Function):
             dy32 = dy32.contiguous()
         if dy16 is not None:
             dy16 = dy16.contiguous()
-        dx = torch.empty_like(a)
         dg, dbt, acc, pg = _ln_param_grads(ctx.param_srcs, n_groups, a.device)
-        stats = torch.empty((rows, 2), dtype=F32, device=a.device)
-        sc = reduce_scratch(a.device, 16 * rows, HIDDEN, 2)           # the fused pass reduces chunks of 8 - 32 rows (>= RED_CHUNK / 16)
-        check(lib.vi_add_ln_drop_bwd(a.data_ptr(), _ptr(b), gamma.data_ptr(), ctx.eps, _ptr(dy32), _ptr(dy16), dx.data_ptr(), None,
-                                     None, dg.data_ptr(), dbt.data_ptr(), stats.data_ptr(), rows, n_groups,
-                                     _lib.int_array(list(ends)) if ends is not None else None, sc.data_ptr(), sc.numel(), acc,
-                                     0.0, None, 0, _stream()), 'vi_add_ln_drop_bwd')
-        _launched(2)
+        dx, _ = ops.add_ln_drop_bwd(a, b, gamma, ctx.eps, dy32, dy16, dg, dbt, acc, ends)
         return (dx if ctx.a_needs else None, dx if ctx.b_needs else None, None, None, None, None, None, None, *pg)
 
 
@@ -474,18 +364,10 @@ class DenseResLNFn(Function):
     def forward(ctx, x, res32, pack, lnpack, eps, ends, p, site, n_lin, *params):
         w, b = pack.get(True)
         g, be = lnpack.get()
-        rows = x.shape[0]
-        n_groups = 1 if ends is None else len(ends)
         ln_ends = ends if len(lnpack.g.tensors) > 1 else None
-        earr = _lib.int_array(list(ln_ends)) if ln_ends is not None else None
         if p > 0:
-            y32 = torch.empty((rows, HIDDEN), dtype=F32, device=x.device)
-            y16 = torch.empty((rows, HIDDEN), dtype=x.dtype, device=x.device)
             d = ops.gemm(x, w, b, out_dtype=F32, group_row_end=ends)
-            check(lib.vi_add_ln_drop(d.data_ptr(), res32.data_ptr(), g.data_ptr(), be.data_ptr(), eps, y32.data_ptr(), y16.data_ptr(),
-                                     ops._DT[y16.dtype], rows, 1 if ln_ends is None else len(ln_ends), earr, float(p),
-                                     dropout_seed(x.device).data_ptr(), site, _stream()), 'vi_add_ln_drop')
-            _launched(1)
+            y32, y16 = ops.add_ln_drop(d, res32, g, be, eps, x.dtype, p, dropout_seed(x.device), site, ln_ends)
             ctx.save_for_backward(x, d, res32, g)
         else:
             d = ops.gemm(x, w, b, residual=res32, out_dtype=F32, group_row_end=ends)
@@ -500,7 +382,6 @@ class DenseResLNFn(Function):
     def backward(ctx, dy32, dy16):
         x, d, res32, g = ctx.saved_tensors
         pack, lnpack, ends, ln_ends, p = ctx.pack, ctx.lnpack, ctx.ends, ctx.ln_ends, ctx.p
-        rows = d.shape[0]
         dev = d.device
         n_groups = 1 if ends is None else len(ends)
         n_ln = 1 if ln_ends is None else len(ln_ends)
@@ -510,15 +391,8 @@ class DenseResLNFn(Function):
         dy16 = dy16.contiguous() if dy16 is not None else None
         ln_srcs = lnpack.grad_sources()
         dg, dbt, acc, ln_grads = _ln_param_grads(ln_srcs, n_ln, dev)
-        dres = torch.empty((rows, HIDDEN), dtype=F32, device=dev)
-        da16 = torch.empty((rows, HIDDEN), dtype=x.dtype, device=dev)
-        stats = torch.empty((rows, 2), dtype=F32, device=dev)
-        sc = reduce_scratch(dev, 16 * rows, HIDDEN, 2)
-        check(lib.vi_add_ln_drop_bwd(d.data_ptr(), res32.data_ptr() if p > 0 else None, g.data_ptr(), ctx.eps, _ptr(dy32), _ptr(dy16),
-                                     dres.data_ptr(), None, da16.data_ptr(), dg.data_ptr(), dbt.data_ptr(), stats.data_ptr(), rows, n_ln,
-                                     _lib.int_array(list(ln_ends)) if ln_ends is not None else None, sc.data_ptr(), sc.numel(), acc,
-                                     float(p), dropout_seed(dev).data_ptr() if p > 0 else None, ctx.site, _stream()), 'vi_add_ln_drop_bwd')
-        _launched(2)
+        dres, da16 = ops.add_ln_drop_bwd(d, res32 if p > 0 else None, g, ctx.eps, dy32, dy16, dg, dbt, acc, ln_ends, x.dtype,
+                                         (p, dropout_seed(dev), ctx.site) if p > 0 else None)
         # dense layer: dX = dA W, dW = dA^T X, db = column sums of dA with dA = da16
         K = x.shape[1]
         N = da16.shape[1]
@@ -672,14 +546,8 @@ class AttentionFn(Function):
             if s.get('pair_dist') is not None and d_affine is None:
                 d_affine = torch.zeros((2,), dtype=F32, device=q.device)
             drop = s.get('drop') if (s.get('drop') is not None and s['drop'][0] > 0) else None
-            check(lib.vi_attn_bwd(q.data_ptr(), q.stride(0), k.data_ptr(), k.stride(0), v.data_ptr(), v.stride(0), do.data_ptr(),
-                                  do.stride(0), dq.data_ptr(), dq.stride(0), dk.data_ptr(), dk.stride(0), dv.data_ptr(),
-                                  dv.stride(0), _dt(q), _ptr(s.get('key_mask')), _ptr(s.get('pair_dist')),
-                                  _ptr(s.get('bias_affine')), _ptr(d_affine) if s.get('pair_dist') is not None else None,
-                                  s['B'], ops.HEADS, s['Lq'], s['Lk'], ctx.mask_mode,
-                                  float(drop[0]) if drop else 0.0, (int(drop[1]) & 0xFFFFFFFF) if drop else 0,
-                                  drop[2].data_ptr() if drop else None, _stream()), 'vi_attn_bwd')
-            _launched(1)
+            ops.attention_bwd(q, k, v, do, dq, dk, dv, s['B'], s['Lq'], s['Lk'], ctx.mask_mode, s.get('key_mask'), s.get('pair_dist'),
+                              s.get('bias_affine'), d_affine, drop)
         extra = [None] * ctx.n_extra
         if ctx.n_extra == 2 and d_affine is not None:                   # sprel_linear.weight [1,1], .bias [1]
             extra = [d_affine[0:1].view(1, 1), d_affine[1:2]]
@@ -700,14 +568,7 @@ class SmallLinearFn(Function):
     @staticmethod
     def backward(ctx, dt):
         (feat,) = ctx.saved_tensors
-        dt = dt.contiguous()
-        fd = feat.shape[1]
-        dW = torch.empty(ctx.wshape, dtype=F32, device=dt.device)
-        db = torch.empty((HIDDEN,), dtype=F32, device=dt.device) if ctx.has_b else None
-        sc = reduce_scratch(dt.device, dt.shape[0], HIDDEN, 17)
-        check(lib.vi_feat_wgrad(dt.data_ptr(), feat.data_ptr(), fd, dW.data_ptr(), _ptr(db), dt.shape[0], sc.data_ptr(), sc.numel(),
-                                _stream()), 'vi_feat_wgrad')
-        _launched(2)
+        dW, db = ops.feat_wgrad(dt.contiguous(), feat, ctx.wshape, ctx.has_b)
         return None, dW, db
 
 
@@ -730,9 +591,7 @@ class GatherRowsFn(Function):
         (idx,) = ctx.saved_tensors
         dy = dy.contiguous()
         dt = torch.zeros(ctx.tshape, dtype=F32, device=dy.device)
-        check(lib.vi_scatter_add_rows(dy.data_ptr(), idx.data_ptr() if ctx.has_idx else None, ctx.period or 1, dt.data_ptr(),
-                                      dy.shape[0], _stream()), 'vi_scatter_add_rows')
-        _launched(1)
+        ops.scatter_add_rows(dy, idx if ctx.has_idx else None, dt, ctx.period or 1)
         return dt, None, None, None
 
 
@@ -774,13 +633,8 @@ class RowDotFn(Function):
     @staticmethod
     def forward(ctx, x, wstack, bstack, ends, n_heads, *params):
         x = x.contiguous()
-        rows = x.shape[0]
-        out = torch.empty((rows,), dtype=F32, device=x.device)
-        # the dot-product tail of vi_ln_dot without its LayerNorm (gamma = beta = NULL): one warp per row, all groups in one launch
-        n_groups = 1 if ends is None else len(ends)
-        check(lib.vi_ln_dot(x.data_ptr(), None, None, 0.0, wstack.data_ptr(), bstack.data_ptr(), out.data_ptr(), rows, n_groups,
-                            _lib.int_array([min(int(e), rows) for e in ends]) if ends is not None else None, _stream()), 'vi_ln_dot')
-        _launched(1)
+        # the dot-product tail of vi_ln_dot without its LayerNorm (gamma = beta = None): one warp per row, all groups in one launch
+        out = ops.ln_dot(x, None, None, 0.0, wstack, bstack, [min(int(e), x.shape[0]) for e in ends] if ends is not None else None)
         ctx.save_for_backward(x, wstack)
         ctx.ends, ctx.n_heads = ends, n_heads
         return out
@@ -788,18 +642,7 @@ class RowDotFn(Function):
     @staticmethod
     def backward(ctx, dout):
         x, wstack = ctx.saved_tensors
-        dout = dout.contiguous()
-        rows = x.shape[0]
-        ends = ctx.ends
-        n_groups = 1 if ends is None else len(ends)
-        dx = torch.empty_like(x)
-        dw = torch.empty((n_groups, HIDDEN), dtype=F32, device=x.device)
-        db = torch.empty((n_groups, HIDDEN), dtype=F32, device=x.device)       # the sum replicated over the columns
-        sc = reduce_scratch(x.device, rows, HIDDEN, 2)
-        check(lib.vi_rowdot_bwd(dout.data_ptr(), x.data_ptr(), wstack.data_ptr(), dx.data_ptr(), dw.data_ptr(), db.data_ptr(), rows,
-                                n_groups, _lib.int_array(list(ends)) if ends is not None else None, sc.data_ptr(), sc.numel(),
-                                _stream()), 'vi_rowdot_bwd')
-        _launched(4)
+        dx, dw, db = ops.rowdot_bwd(dout.contiguous(), x, wstack, ctx.ends)
         pg = [dw[i].view(1, HIDDEN) for i in range(ctx.n_heads)] + [db[i, 0:1] for i in range(ctx.n_heads)]
         return (dx, None, None, None, None, *pg)
 
@@ -818,15 +661,8 @@ class FuseLogitsFn(Function):
         g_raw, l_raw, fuse_raw, gm, gv, nav, gids, cids = ctx.saved_tensors
         B, G, P = ctx.dims
         c = lambda t: t.contiguous() if t is not None else None      # noqa: E731
-        dgl, dll, dfl = c(dgl), c(dll), c(dfl)
-        dg = torch.empty_like(g_raw)
-        dl = torch.empty_like(l_raw)
-        df = torch.empty((B,), dtype=F32, device=g_raw.device) if ctx.has_fuse else None
-        check(lib.vi_duet_fuse_logits_bwd(g_raw.data_ptr(), l_raw.data_ptr(), fuse_raw.data_ptr() if ctx.has_fuse else None,
-                                          gm.data_ptr(), gv.data_ptr(), nav.data_ptr(), gids.data_ptr(), cids.data_ptr(),
-                                          _ptr(dgl), _ptr(dll), _ptr(dfl), dg.data_ptr(), dl.data_ptr(), _ptr(df), B, G, P,
-                                          _stream()), 'vi_duet_fuse_logits_bwd')
-        _launched(1)
+        dg, dl, df = ops.duet_fuse_logits_bwd(g_raw, l_raw, fuse_raw if ctx.has_fuse else None, gm, gv, nav, gids, cids,
+                                              c(dgl), c(dll), c(dfl), B, G, P)
         return dg, dl, df, None, None, None, None, None, None, None, None
 
 
@@ -882,29 +718,17 @@ class CosineLossFn(Function):
     @staticmethod
     def backward(ctx, dloss):
         proj, tgt = ctx.saved_tensors
-        dloss = dloss.contiguous().float().view(1)
-        dp = torch.empty_like(proj) if ctx.needs[0] else None
-        dt = torch.empty_like(tgt) if ctx.needs[1] else None
-        check(lib.vi_cosine_loss_bwd(proj.data_ptr(), tgt.data_ptr(), dloss.data_ptr(), _ptr(dp), _ptr(dt), ctx.R, _stream()),
-              'vi_cosine_loss_bwd')
-        _launched(1)
+        dp, dt = ops.cosine_loss_bwd(proj, tgt, dloss.contiguous().float().view(1), ctx.R, *ctx.needs)
         return dp, dt, None
 
 
-def _contrastive_loss_bwd(ctx, dloss, fn, name):
+def _contrastive_loss_bwd(ctx, dloss, form):
     """shared backward of InfoNCELossFn / MarginLossFn: dproj always, dtgt / dnegs only when autograd asks for them (the text
-    encoder trains through the loss); otherwise NULL, and the call is the one-launch proj-only adjoint"""
+    encoder trains through the loss)"""
     proj, tgt, scratch = ctx.saved_tensors
     negs, row_ep, neg_ep, param, R, n_negs = ctx.extra
-    dloss = dloss.contiguous().float().view(1)
-    dp = torch.empty_like(proj)
-    dt = torch.empty_like(tgt) if ctx.needs_input_grad[1] else None
-    want_negs = negs is not None and ctx.needs_input_grad[2]
-    dn = torch.empty_like(negs) if want_negs else None
-    work = torch.empty(R * (n_negs + 1), dtype=F32, device=proj.device) if want_negs and n_negs else None
-    check(fn(proj.data_ptr(), tgt.data_ptr(), _ptr(negs), row_ep.data_ptr(), _ptr(neg_ep), param, scratch.data_ptr(),
-             dloss.data_ptr(), dp.data_ptr(), _ptr(dt), _ptr(dn), _ptr(work), R, n_negs, _stream()), name)
-    _launched(2 if work is not None else 1)
+    dp, dt, dn = ops.contrastive_loss_bwd(form, proj, tgt, negs, row_ep, neg_ep, param, scratch, dloss.contiguous().float().view(1), R,
+                                          n_negs, ctx.needs_input_grad[1], negs is not None and ctx.needs_input_grad[2])
     return dp, dt, dn, None, None, None, None, None
 
 
@@ -923,7 +747,7 @@ class InfoNCELossFn(Function):
 
     @staticmethod
     def backward(ctx, dloss):
-        return _contrastive_loss_bwd(ctx, dloss, lib.vi_infonce_loss_bwd, 'vi_infonce_loss_bwd')
+        return _contrastive_loss_bwd(ctx, dloss, 'infonce')
 
 
 class MarginLossFn(Function):
@@ -941,7 +765,7 @@ class MarginLossFn(Function):
 
     @staticmethod
     def backward(ctx, dloss):
-        return _contrastive_loss_bwd(ctx, dloss, lib.vi_margin_loss_bwd, 'vi_margin_loss_bwd')
+        return _contrastive_loss_bwd(ctx, dloss, 'margin')
 
 
 class MulBcastFn(Function):
@@ -961,10 +785,7 @@ class MulBcastFn(Function):
         B, R, _ = x.shape
         dy = dy.float().contiguous().view(B, R, HIDDEN)
         dx, _ = ops.mul_bcast(dy, R * HIDDEN, s, HIDDEN, B, R, want16=False)
-        ds = torch.empty_like(s)
-        check(lib.vi_mul_bcast_bwd_s(dy.data_ptr(), x.data_ptr(), ds.data_ptr(), B, R, _stream()), 'vi_mul_bcast_bwd_s')
-        _launched(1)
-        return dx.view(B, R, HIDDEN), ds, None
+        return dx.view(B, R, HIDDEN), ops.mul_bcast_bwd_s(dy, x, B, R), None
 
 
 class RaggedMeanFn(Function):
@@ -993,9 +814,7 @@ class RaggedMeanFn(Function):
         seg_of = torch.repeat_interleave(torch.arange(R, device=dev, dtype=torch.int64), lens, output_size=n)
         rows, _ = ops.embed_compose(n, dev, idx=seg_of, table=g)                       # one scaled copy per member row
         d = torch.zeros(ctx.shape, dtype=F32, device=dev)
-        check(lib.vi_scatter_add_rows(rows.data_ptr(), row_idx.long().data_ptr(), 1, d.data_ptr(), n, _stream()), 'vi_scatter_add_rows')
-        _launched(1)
-        return d, None, None, None
+        return ops.scatter_add_rows(rows, row_idx.long(), d), None, None, None
 
 
 class SegmentMeanFn(Function):

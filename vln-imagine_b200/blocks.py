@@ -253,7 +253,7 @@ class LinearPack:
             w = self._w16(v, BF16) if lowp else v['w32']
             n = w.shape[0] // n_groups
             with torch.no_grad():
-                v[key] = torch.cat([ag.transpose(w[g * n:(g + 1) * n]) for g in range(n_groups)], 0).contiguous()
+                v[key] = torch.cat([ops.transpose(w[g * n:(g + 1) * n]) for g in range(n_groups)], 0).contiguous()
         return v[key]
 
     def grad_sources(self):

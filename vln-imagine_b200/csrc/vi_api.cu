@@ -1,8 +1,9 @@
-// vi_api.cu - library-level entry points: init, version, thread-local error string.
+// vi_api.cu - library-level entry points: init, version, thread-local error string, launch counter.
 #include "vi_common.cuh"
 
 #include <stdarg.h>
 #include <stdlib.h>
+#include <atomic>
 
 static thread_local char g_err[512] = "";
 static int g_num_sms = 0;
@@ -73,7 +74,13 @@ int vi_make_tmap_h16(CUtensorMap* map, const void* ptr, int f16, uint64_t cols, 
   return VI_OK;
 }
 
-extern "C" int vi_version(void) { return 103; }   // 0.1.3
+static std::atomic<int64_t> g_launches{0};
+
+void vi_count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
+
+extern "C" int64_t vi_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
+
+extern "C" int vi_version(void) { return 104; }   // 0.1.4
 
 extern "C" const char* vi_last_error(void) { return g_err; }
 

@@ -45,24 +45,44 @@ int vi_num_sms();
 // 2-D row-major TMA tensor map over bf16 / fp16 elements, 128-byte swizzle, boxes of 64 columns x box_rows rows (vi_api.cu)
 int vi_make_tmap_h16(CUtensorMap* map, const void* ptr, int f16, uint64_t cols, uint64_t rows, uint64_t ld_elems, uint32_t box_rows);
 bool vi_pdl_enabled();      // programmatic dependent launch on every kernel of the library (VI_PDL=0 disables)
+void vi_count_launch();     // one more kernel launched by the library (vi_launch_count)
 
 // Launch with the programmatic-stream-serialization attribute: the kernel may start (and run its prologue) while
-// its predecessor in the stream is still draining; it calls pdl_wait() before touching global memory.
+// its predecessor in the stream is still draining; it calls pdl_wait() before touching global memory.  cluster > 1
+// groups that many consecutive CTAs into a cluster (the CTA-pair kernels).  Every kernel of the library is launched here.
 #ifdef __CUDACC__
 template <typename... KArgs, typename... Args>
-inline cudaError_t vi_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
+inline cudaError_t vi_launch_cluster(void (*kern)(KArgs...), unsigned cluster, dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                     Args... args) {
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchAttribute attr[2];
+  unsigned nattr = 0;
+  if (vi_pdl_enabled()) {
+    attr[nattr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[nattr].val.programmaticStreamSerializationAllowed = 1;
+    ++nattr;
+  }
+  if (cluster > 1) {
+    attr[nattr].id = cudaLaunchAttributeClusterDimension;
+    attr[nattr].val.clusterDim.x = cluster;
+    attr[nattr].val.clusterDim.y = 1;
+    attr[nattr].val.clusterDim.z = 1;
+    ++nattr;
+  }
   cfg.attrs = attr;
-  cfg.numAttrs = vi_pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+  cfg.numAttrs = nattr;
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+  if (e == cudaSuccess) vi_count_launch();
+  return e;
+}
+template <typename... KArgs, typename... Args>
+inline cudaError_t vi_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
+  return vi_launch_cluster(kern, 1, grid, block, smem, st, args...);
 }
 #endif
 

@@ -632,29 +632,8 @@ int launch(const Maps& m, const GemmParams& p, int grid, cudaStream_t st) {
     VI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes<BN, STAGES, PAIR, OUTMODE>()));
     attr_set = true;
   }
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(NUM_THREADS);
-  cfg.dynamicSmemBytes = smem_bytes<BN, STAGES, PAIR, OUTMODE>();
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  int nattr = 0;
-  if (vi_pdl_enabled()) {
-    attr[nattr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[nattr].val.programmaticStreamSerializationAllowed = 1;
-    ++nattr;
-  }
-  if (PAIR) {
-    attr[nattr].id = cudaLaunchAttributeClusterDimension;
-    attr[nattr].val.clusterDim.x = 2;
-    attr[nattr].val.clusterDim.y = 1;
-    attr[nattr].val.clusterDim.z = 1;
-    ++nattr;
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = nattr;
-  VI_CUDA(cudaLaunchKernelEx(&cfg, kern, m.a, m.b, m.y, m.r, m.y2, p));
+  VI_CUDA(vi_launch_cluster(kern, PAIR ? 2 : 1, dim3((unsigned)grid), dim3(NUM_THREADS),
+                            (size_t)smem_bytes<BN, STAGES, PAIR, OUTMODE>(), st, m.a, m.b, m.y, m.r, m.y2, p));
   return VI_OK;
 }
 

@@ -537,27 +537,7 @@ int launch_wgrad_pair(const WgradMaps& m, const WgradParams& p, int pairs, cudaS
     VI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, wgrad_pair_smem<BN, STAGES>()));
     attr_set = true;
   }
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)(2 * pairs));
-  cfg.blockDim = dim3(NUM_THREADS);
-  cfg.dynamicSmemBytes = wgrad_pair_smem<BN, STAGES>();
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  int nattr = 0;
-  if (vi_pdl_enabled()) {
-    attr[nattr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[nattr].val.programmaticStreamSerializationAllowed = 1;
-    ++nattr;
-  }
-  attr[nattr].id = cudaLaunchAttributeClusterDimension;
-  attr[nattr].val.clusterDim.x = 2;
-  attr[nattr].val.clusterDim.y = 1;
-  attr[nattr].val.clusterDim.z = 1;
-  ++nattr;
-  cfg.attrs = attr;
-  cfg.numAttrs = nattr;
-  VI_CUDA(cudaLaunchKernelEx(&cfg, kern, m, p));
+  VI_CUDA(vi_launch_cluster(kern, 2, dim3((unsigned)(2 * pairs)), dim3(NUM_THREADS), (size_t)wgrad_pair_smem<BN, STAGES>(), st, m, p));
   VI_LAUNCH_CHECK();
   return VI_OK;
 }

@@ -17,19 +17,16 @@ No CPU path: every array below is computed on the GPU; the oracle (oracle/graph_
 from __future__ import annotations
 
 import collections.abc
-from typing import Dict, List, Optional, Sequence
+from typing import Dict, List, Sequence
 
 import numpy as np
 import torch
 
 from . import _lib, ops
-from ._lib import check, lib
+
+lib = ops.lib           # checked and traced like every library call
 
 MAX_NODES = 128
-
-
-def _ptr(t: Optional[torch.Tensor]):
-    return None if t is None else t.data_ptr()
 
 
 class _Staging:
@@ -132,9 +129,8 @@ class DeviceGraphMaps:
         self.visited_dev = torch.empty((B, N), dtype=torch.uint8, device=self.device)
         self.esum = torch.zeros((B, N, hidden), dtype=torch.float32, device=self.device)
         self.ecnt = torch.empty((B, N), dtype=torch.float32, device=self.device)
-        check(lib.vi_graph_init(self.dis.data_ptr(), self.point.data_ptr(), self.visited_dev.data_ptr(), self.ecnt.data_ptr(),
-                                B, N, ops._stream()), 'vi_graph_init')
-        ops._launched(1)
+        lib.vi_graph_init(self.dis.data_ptr(), self.point.data_ptr(), self.visited_dev.data_ptr(), self.ecnt.data_ptr(),
+                          B, N, ops._stream())
         # host mirror of what only needs strings / small ints
         self.start_vps = [ob['viewpoint'] for ob in obs]            # GraphMap.start_vp
         self.index: List[Dict[str, int]] = [dict() for _ in obs]    # viewpoint id -> node index (node_positions order)
@@ -181,10 +177,9 @@ class DeviceGraphMaps:
         self.visited[act, cur[act]] = True
         n_nodes = self.n_nodes.copy()
         d = _pack(self._staging, self.device, dict(cur_pos=cur_pos, cand_pos=cand_pos, cur=cur, cand=cand, n_nodes=n_nodes))
-        check(lib.vi_graph_update(self.pos.data_ptr(), self.dis.data_ptr(), self.point.data_ptr(), self.visited_dev.data_ptr(),
-                                  B, self.N, d['cur'].data_ptr(), d['cur_pos'].data_ptr(), d['cand'].data_ptr(),
-                                  d['cand_pos'].data_ptr(), C, d['n_nodes'].data_ptr(), ops._stream()), 'vi_graph_update')
-        ops._launched(1)
+        lib.vi_graph_update(self.pos.data_ptr(), self.dis.data_ptr(), self.point.data_ptr(), self.visited_dev.data_ptr(),
+                            B, self.N, d['cur'].data_ptr(), d['cur_pos'].data_ptr(), d['cand'].data_ptr(),
+                            d['cand_pos'].data_ptr(), C, d['n_nodes'].data_ptr(), ops._stream())
 
     def set_step_ids(self, obs: Sequence[dict], t: int, ended):
         for b, ob in enumerate(obs):                                 # agent.py:461-464
@@ -243,19 +238,16 @@ class DeviceGraphMaps:
         dev = self.device
         gmap_img = torch.empty((B, G, H), dtype=torch.float32, device=dev)
         vp_img = torch.empty((B, V + 1, H), dtype=torch.float32, device=dev)
-        check(lib.vi_graph_embed_step(pano_embeds.data_ptr(), pm.data_ptr(), B, V, H, d['cur'].data_ptr(), d['cand'].data_ptr(), C,
-                                      self.visited_dev.data_ptr(), self.esum.data_ptr(), self.ecnt.data_ptr(), self.N,
-                                      d['gnode'].data_ptr(), G, gmap_img.data_ptr(), vp_img.data_ptr(), ops._stream()),
-              'vi_graph_embed_step')
+        lib.vi_graph_embed_step(pano_embeds.data_ptr(), pm.data_ptr(), B, V, H, d['cur'].data_ptr(), d['cand'].data_ptr(), C,
+                                self.visited_dev.data_ptr(), self.esum.data_ptr(), self.ecnt.data_ptr(), self.N,
+                                d['gnode'].data_ptr(), G, gmap_img.data_ptr(), vp_img.data_ptr(), ops._stream())
         gmap_pos = torch.empty((B, G, 7), dtype=torch.float32, device=dev)
         pair = torch.empty((B, G, G), dtype=torch.float32, device=dev)
         vp_pos = torch.empty((B, V + 1, 14), dtype=torch.float32, device=dev)
-        check(lib.vi_graph_features(self.pos.data_ptr(), self.dis.data_ptr(), self.point.data_ptr(), B, self.N,
-                                    d['cur_all'].data_ptr(), d['heading'].data_ptr(), d['elevation'].data_ptr(),
-                                    d['gnode'].data_ptr(), d['lens'].data_ptr(), G, gmap_pos.data_ptr(), pair.data_ptr(),
-                                    d['cand'].data_ptr(), C, d['start'].data_ptr(), V + 1, vp_pos.data_ptr(), ops._stream()),
-              'vi_graph_features')
-        ops._launched(2)
+        lib.vi_graph_features(self.pos.data_ptr(), self.dis.data_ptr(), self.point.data_ptr(), B, self.N,
+                              d['cur_all'].data_ptr(), d['heading'].data_ptr(), d['elevation'].data_ptr(),
+                              d['gnode'].data_ptr(), d['lens'].data_ptr(), G, gmap_pos.data_ptr(), pair.data_ptr(),
+                              d['cand'].data_ptr(), C, d['start'].data_ptr(), V + 1, vp_pos.data_ptr(), ops._stream())
         view_lens = pano_inputs['view_lens']
         nav_types = pano_inputs['nav_types']
         ar = torch.arange(max(G, V + 1), device=dev)

@@ -443,12 +443,12 @@ class _PaddedLinear:
 
     def get_t(self, lowp: bool, n_groups: int = 1):
         """the transposed training weight [768, n_pad] (B operand of the input-gradient GEMM), cached with the pack"""
-        from .autograd_ops import transpose
+        blocks, duet, ops, params = _lazy()
         v = self._padded(self._pack.get(), 128)
         key = ('t', lowp)
         if key not in v:
             with torch.no_grad():
-                v[key] = transpose(self.get_train(lowp)[0])
+                v[key] = ops.transpose(self.get_train(lowp)[0])
         return v[key]
 
     def grad_sources(self):
