@@ -381,6 +381,18 @@ int vi_dropout(const void* x, void* y, int64_t n, float p, const uint32_t* seed,
 /* fp32 -> bf16 or fp16 (saturating at +-65504): 16-bit shadow copies of weights and activations */
 int vi_cast_h16(const float* src, void* dst, int dst_dtype, int64_t n, vi_stream_t stream);
 
+/* Rows of a device-resident image feature store (ImageFeaturesDB / ImaginationImageFeaturesDB held in HBM):
+ *   dst[r, 0:F] = dropout(store[idx[r], 0:F])      r < n_rows, dense outputs of F elements per row
+ * store: [n_store_rows, ld_store] of store_dtype (VI_DT_F32, VI_DT_F16 or VI_DT_BF16); an index outside [0, n_store_rows) - the
+ * padding value -1 included - gives a zero row and reads nothing.  Outputs: dst32 (fp32) and / or dst16 (dst16_dtype
+ * VI_DT_BF16 / VI_DT_F16: the operand of the first GEMM).  The result is bit for bit what the dense path computes from
+ * store[idx].float(): vi_dropout's mask and product at (drop_seed, drop_site) for the [n_rows, F] tensor (element id r * F + c;
+ * drop_p == 0: none, drop_seed may be NULL), then one rounding as in vi_cast_h16.  F and ld_store multiples of 8, pointers
+ * 16-byte aligned. */
+int vi_gather_rows(const void* store, int store_dtype, int64_t ld_store, int64_t n_store_rows, const int32_t* idx, int64_t n_rows,
+                   int F, float* dst32, void* dst16, int dst16_dtype, float drop_p, const uint32_t* drop_seed, uint32_t drop_site,
+                   vi_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Per-step graph glue of a DUET rollout (SURVEY.md section 8(f), rows N1 / N2).  Replaces the Python GraphMap /
  * FloydGraph objects (D/models/graph_utils.py:42-148) and the agent's per-step collate loops

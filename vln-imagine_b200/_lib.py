@@ -79,6 +79,7 @@ PROTOTYPES = {
     'vi_kl_rows_bwd': [_p, _l, _p, _l, _i, _p, _p, _p, _i, _l, _l, _p],
     'vi_copy_rows': [_p, _l, _l, _p, _p, _i, _l, _l, _l, _i, _p],
     'vi_cast_h16': [_p, _p, _i, _l, _p],
+    'vi_gather_rows': [_p, _i, _l, _l, _p, _l, _i, _p, _p, _i, _f, _p, C.c_uint32, _p],
     'vi_transpose': [_p, _l, _p, _l, _i, _i, _i, _i, _p],
     'vi_colsum': [_p, _l, _i, _p, _l, _i, _p, _l, _p],
     'vi_wgrad16_splits': [_i, _i, _i, _ip],

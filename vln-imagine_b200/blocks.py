@@ -15,6 +15,7 @@ import torch
 
 from . import autograd_ops as ag
 from . import ops
+from .feature_store import FeatureRows
 from .ops import BF16, F32, HIDDEN, EPI_GELU, EPI_NONE, EPI_RELU, MASK_ADD_NEG10000, MASK_NEG_INF  # noqa: F401
 
 
@@ -719,6 +720,16 @@ def operand(x32: torch.Tensor, lowp: bool) -> torch.Tensor:
     if not lowp:
         return x32
     return ag.CastBf16Fn.apply(x32) if _Mode.train else ops.cast_h16(x32)
+
+
+def feature_operand(x, lowp: bool) -> torch.Tensor:
+    """image features (dense [..., F] or feature_store.FeatureRows) -> the [rows, F] operand of their first GEMM (fp32 rows when
+    not ``lowp``).  Dense: the cast of ``operand``.  FeatureRows: one vi_gather_rows from the store, with the environment
+    dropout the host module attached (same mask and values as dropout on the dense tensor followed by the cast)."""
+    if isinstance(x, FeatureRows):
+        dtype = (BF16 if _Mode.train else ops.h16()) if lowp else F32
+        return x.gather(dtype, ag.dropout_seed(x.device) if x.drop is not None else None)
+    return operand(x.float().reshape(-1, x.shape[-1]), lowp)
 
 
 def embed(rows: int, device, *, a=None, a_ln=None, a2=None, feat=None, feat_lin=None, feat_ln=None, idx=None, table=None,

@@ -5,6 +5,7 @@
 // VLN-DUET/map_nav_src/models/vilmodel.py and VLN-HAMT/finetune_src/models/vilmodel_cmt.py; each
 // entry point cites its reference lines in include/vlnimagine.h.
 #include "vi_common.cuh"
+#include <cuda_fp16.h>
 
 namespace {
 
@@ -506,6 +507,88 @@ __global__ void cast_bf16_kernel(const float* src, bf16* dst, int f16, long long
       reinterpret_cast<uint16_t*>(dst)[j] = (uint16_t)(pack_h16x2(src[j], 0.f, f16 != 0) & 0xFFFFu);
 }
 
+// dst[r, :] = dropout(store[idx[r], 0:F]) for a device-resident feature store: 8 elements (16 bytes of a 16-bit store, two
+// float4 of an fp32 one) per thread.  Values, mask and rounding are those of the dense path store[idx].float() ->
+// vi_dropout (element id r * F + c) -> vi_cast_h16; an index outside [0, n_store) gives a zero row and reads nothing.
+template <typename T> struct StoreVec;
+template <> struct StoreVec<float> {
+  static __device__ __forceinline__ void load(const float* p, float (&f)[8]) {
+    const float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + 4);
+    f[0] = a.x; f[1] = a.y; f[2] = a.z; f[3] = a.w; f[4] = b.x; f[5] = b.y; f[6] = b.z; f[7] = b.w;
+  }
+};
+template <> struct StoreVec<bf16> {
+  static __device__ __forceinline__ void load(const bf16* p, float (&f)[8]) {
+    const uint4 u = *reinterpret_cast<const uint4*>(p);
+    const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      f[2 * j] = __uint_as_float(w[j] << 16);
+      f[2 * j + 1] = __uint_as_float(w[j] & 0xFFFF0000u);
+    }
+  }
+};
+template <> struct StoreVec<__half> {
+  static __device__ __forceinline__ void load(const __half* p, float (&f)[8]) {
+    const uint4 u = *reinterpret_cast<const uint4*>(p);
+    const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float2 t = __half22float2(*reinterpret_cast<const __half2*>(&w[j]));
+      f[2 * j] = t.x;
+      f[2 * j + 1] = t.y;
+    }
+  }
+};
+
+// One warp per output row, 8 rows per CTA: the row index is read once, then every 16-byte load of the row is issued before the
+// first store (up to 4 per lane), so a row costs two dependent memory round trips (index, then data); a thread per 8 elements
+// would repeat the index load and a 64-bit division for every 16 bytes.
+constexpr int GATHER_UNROLL = 4;
+template <typename T>
+__global__ void __launch_bounds__(256) gather_rows_kernel(const T* store, long long ld_store, long long n_store, const int32_t* idx,
+                                                          long long n_rows, int F, float* dst32, bf16* dst16, int f16,
+                                                          uint32_t thresh, float scale, const uint32_t* seed, uint32_t site) {
+  pdl_enter();
+  const int lane = threadIdx.x & 31;
+  const long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (r >= n_rows) return;
+  const long long s = idx[r];
+  const bool ok = s >= 0 && s < n_store;
+  const T* src = store + (ok ? s : 0LL) * ld_store;
+  const uint32_t key = seed ? vi_drop_key(seed, site) : 0u;
+  for (int c0 = lane * 8; c0 < F; c0 += 256 * GATHER_UNROLL) {
+    float f[GATHER_UNROLL][8];
+#pragma unroll
+    for (int u = 0; u < GATHER_UNROLL; ++u) {
+      const int c = c0 + u * 256;
+      if (ok && c < F) {
+        StoreVec<T>::load(src + c, f[u]);
+      } else {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) f[u][j] = 0.f;
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < GATHER_UNROLL; ++u) {
+      const int c = c0 + u * 256;
+      if (c >= F) break;
+      const long long o = r * F + c;
+      if (seed) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) f[u][j] = vi_hash32((uint32_t)(o + j), key) >= thresh ? f[u][j] * scale : 0.f;
+      }
+      if (dst32) {
+        float4* d = reinterpret_cast<float4*>(dst32 + o);
+        d[0] = make_float4(f[u][0], f[u][1], f[u][2], f[u][3]);
+        d[1] = make_float4(f[u][4], f[u][5], f[u][6], f[u][7]);
+      }
+      if (dst16)
+        *reinterpret_cast<uint4*>(dst16 + o) = make_uint4(pack_h16x2(f[u][0], f[u][1], f16 != 0), pack_h16x2(f[u][2], f[u][3], f16 != 0),
+                                                          pack_h16x2(f[u][4], f[u][5], f16 != 0), pack_h16x2(f[u][6], f[u][7], f16 != 0));
+    }
+  }
+}
 
 // dst[b, r, :] = src[b, r, :] for nb batches of `rpb` 768-wide rows with independent batch / row strides
 // (token concatenation [txt; imagine], token-0 gathers, fp32 -> bf16 operand copies)
@@ -787,6 +870,36 @@ extern "C" int vi_cast_h16(const float* src, void* dst, int dst_dtype, int64_t n
   const long long n4 = n / 4;
   const long long threads = n4 > 0 ? n4 : 1;
   VI_CUDA(vi_launch(cast_bf16_kernel, dim3((unsigned)((threads + 255) / 256)), dim3(256), (size_t)(0), ST(stream), src, reinterpret_cast<bf16*>(dst), (int)(dst_dtype == VI_DT_F16), n4, n));
+  VI_LAUNCH_CHECK();
+  return VI_OK;
+}
+
+extern "C" int vi_gather_rows(const void* store, int store_dtype, int64_t ld_store, int64_t n_store_rows, const int32_t* idx,
+                              int64_t n_rows, int F, float* dst32, void* dst16, int dst16_dtype, float drop_p,
+                              const uint32_t* drop_seed, uint32_t drop_site, vi_stream_t stream) {
+  VI_CHECK_ARG(store_dtype == VI_DT_F32 || dt16_ok(store_dtype), "vi_gather_rows: store_dtype must be VI_DT_F32, VI_DT_F16 or VI_DT_BF16");
+  VI_CHECK_ARG(!dst16 || dt16_ok(dst16_dtype), "vi_gather_rows: dst16_dtype must be VI_DT_BF16 or VI_DT_F16");
+  if (n_rows <= 0) return VI_OK;                  // an empty selection (e.g. imagination slots of width 0) has no pointers
+  VI_CHECK_ARG((store || n_store_rows == 0) && idx && (dst32 || dst16), "vi_gather_rows: null operand");
+  VI_CHECK_ARG(F > 0 && F % 8 == 0 && ld_store >= F && ld_store % 8 == 0 && n_store_rows >= 0,
+               "vi_gather_rows: F=%d must be a positive multiple of 8, ld_store a multiple of 8 >= F", F);
+  VI_CHECK_ARG(aligned16(store) && aligned16(dst32) && aligned16(dst16), "vi_gather_rows: operands must be 16-byte aligned");
+  VI_CHECK_ARG(drop_p >= 0.f && drop_p < 1.f && (drop_p == 0.f || drop_seed), "vi_gather_rows: 0 <= drop_p < 1, with a device seed");
+  const uint32_t thresh = vi_drop_threshold(drop_p);
+  const float scale = 1.0f / (1.0f - drop_p);
+  const uint32_t* seed = drop_p > 0.f ? drop_seed : nullptr;
+  const dim3 grid((unsigned)((n_rows + 7) / 8));
+  bf16* d16 = reinterpret_cast<bf16*>(dst16);
+  const int f16 = dst16_dtype == VI_DT_F16;
+  if (store_dtype == VI_DT_F32)
+    VI_CUDA(vi_launch(gather_rows_kernel<float>, grid, dim3(256), (size_t)0, ST(stream), reinterpret_cast<const float*>(store),
+                      (long long)ld_store, (long long)n_store_rows, idx, (long long)n_rows, F, dst32, d16, f16, thresh, scale, seed, drop_site));
+  else if (store_dtype == VI_DT_F16)
+    VI_CUDA(vi_launch(gather_rows_kernel<__half>, grid, dim3(256), (size_t)0, ST(stream), reinterpret_cast<const __half*>(store),
+                      (long long)ld_store, (long long)n_store_rows, idx, (long long)n_rows, F, dst32, d16, f16, thresh, scale, seed, drop_site));
+  else
+    VI_CUDA(vi_launch(gather_rows_kernel<bf16>, grid, dim3(256), (size_t)0, ST(stream), reinterpret_cast<const bf16*>(store),
+                      (long long)ld_store, (long long)n_store_rows, idx, (long long)n_rows, F, dst32, d16, f16, thresh, scale, seed, drop_site));
   VI_LAUNCH_CHECK();
   return VI_OK;
 }

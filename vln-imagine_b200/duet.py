@@ -22,8 +22,9 @@ import torch
 import torch.nn as nn
 
 from . import autograd_ops as ag
-from . import blocks, graphs, ops, params
+from . import blocks, feature_store, graphs, ops, params
 from .blocks import Stream
+from .feature_store import FeatureRows
 from .config import duet_config
 from .ops import F32, HIDDEN
 
@@ -341,7 +342,7 @@ class GlocalTextPathNavCMT(nn.Module):
         self._guard(imagine_feats)
         B, I, _ = imagine_feats.shape
         with blocks.grad_mode(self._recording(imagine_feats), self._drop()):
-            y = blocks.embed(B * I, imagine_feats.device, a=_f32c(imagine_feats).view(B * I, HIDDEN),
+            y = blocks.embed(B * I, imagine_feats.device, a=blocks.feature_operand(imagine_feats, False),
                              const_rows=(self.imagine_embeddings.type_embedding.weight[0],))
         return y.f32.view(B, I, HIDDEN)
 
@@ -351,15 +352,14 @@ class GlocalTextPathNavCMT(nn.Module):
             return self._panorama_with_objects(view_img_fts, obj_img_fts, loc_fts, nav_types, view_lens, obj_lens)
         self._guard(view_img_fts)
         lowp = self.lowp
-        B, V, Fd = view_img_fts.shape
+        B, V, _ = view_img_fts.shape
         dev = view_img_fts.device
         pk = self._pk()
         ie = self.img_embeddings
-        v32 = _f32c(view_img_fts).view(B * V, Fd)
         pano_masks = _arange(V, dev)[None, :] < view_lens.to(dev)[:, None]                  # ops.py:36-44
         km = blocks.mask_u8(pano_masks)
         with blocks.grad_mode(self._recording(view_img_fts) and not self.config.fix_pano_embedding, self._drop()):
-            a = blocks.linear(blocks.operand(v32, lowp), pk['img_linear'], lowp, out_dtype=F32)
+            a = blocks.linear(blocks.feature_operand(view_img_fts, lowp), pk['img_linear'], lowp, out_dtype=F32)
             folded = lowp and not blocks.training() and len(pk['pano']) > 0
             x = blocks.embed(B * V, dev, a=a, a_ln=ie.img_layer_norm, feat=_f32c(loc_fts).view(B * V, -1),
                              feat_lin=ie.loc_linear, feat_ln=ie.loc_layer_norm,
@@ -402,9 +402,8 @@ class GlocalTextPathNavCMT(nn.Module):
         km = blocks.mask_u8(pano_masks)
         recording = self._recording(view_img_fts, obj_img_fts) and not self.config.fix_pano_embedding
         with blocks.grad_mode(recording, self._drop()):
-            v32 = _f32c(view_img_fts).view(B * V, -1)
             o32 = _f32c(obj_img_fts).view(B * O, -1)
-            nv = blocks.layer_norm(blocks.linear(blocks.operand(v32, lowp), pk['img_linear'], lowp, out_dtype=F32), None,
+            nv = blocks.layer_norm(blocks.linear(blocks.feature_operand(view_img_fts, lowp), pk['img_linear'], lowp, out_dtype=F32), None,
                                    blocks.LNPack([ie.img_layer_norm]), 1e-12, False).f32
             if ie.obj_linear is not None:                      # obj_feat_size != image_feat_size (:464-468)
                 olin, oln = pk['obj_linear'], ie.obj_layer_norm
@@ -720,7 +719,7 @@ class VLNBert(nn.Module):
 
     # pure launch sequences over dicts of device tensors (what the graphs capture)
     def _pano_fn(self, t):
-        e, m = self.vln_bert.forward_panorama_per_step(t['view_img_fts'], None, t['loc_fts'], t['nav_types'], t['view_lens'], None)
+        e, m = self.vln_bert.forward_panorama_per_step(feature_store.from_graph(t, 'view_img_fts'), None, t['loc_fts'], t['nav_types'], t['view_lens'], None)
         return {'pano_embeds': e, 'pano_masks': m}
 
     def _nav_fn(self, t):
@@ -744,15 +743,19 @@ class VLNBert(nn.Module):
             if self.training and self.drop_env.p > 0:                      # models/model.py:27: nn.Dropout on the view features
                 batch = dict(batch)
                 feats = batch['view_img_fts']
-                feats = feats if feats.is_cuda else feats.to(m.embeddings.LayerNorm.weight.device, non_blocking=True)
-                ops.ensure_init(feats)
-                batch['view_img_fts'] = ag.dropout(feats.float(), float(self.drop_env.p))
+                if isinstance(feats, FeatureRows):                         # applied by the gather, at the same dropout site
+                    batch['view_img_fts'] = feats.with_dropout(self.drop_env.p, ag.next_site())
+                else:
+                    feats = feats if feats.is_cuda else feats.to(m.embeddings.LayerNorm.weight.device, non_blocking=True)
+                    ops.ensure_init(feats)
+                    batch['view_img_fts'] = ag.dropout(feats.float(), float(self.drop_env.p))
                 batch = collections.defaultdict(lambda: None, batch)
             if self._graphable() and batch['obj_img_fts'] is None:
                 dev = m.embeddings.LayerNorm.weight.device
                 tok = graphs.weights_token(m, self._wt_cache)
-                out = self._g_pano({k: batch[k] for k in ('view_img_fts', 'loc_fts', 'nav_types', 'view_lens')}, dev,
-                                   extra_key=(m.precision, ops.h16()), weights_token=tok)
+                t, borrowed = feature_store.graph_args('view_img_fts', batch['view_img_fts'])
+                t.update({k: batch[k] for k in ('loc_fts', 'nav_types', 'view_lens')})
+                out = self._g_pano(t, dev, extra_key=(m.precision, ops.h16()), weights_token=tok, borrowed=borrowed)
                 return out['pano_embeds'], out['pano_masks']
             return m(mode, batch)
         if mode == 'navigation':

@@ -42,15 +42,16 @@ def round_up(n: int, m: int) -> int:
     return (n + m - 1) // m * m
 
 
-def pad_to(x, sizes: Dict[int, int], device):
-    """x zero-/False-padded along the dimensions of ``sizes`` ({dim: new size}); host tensors are moved to ``device`` first"""
+def pad_to(x, sizes: Dict[int, int], device, fill=0):
+    """x padded with ``fill`` (default zero / False) along the dimensions of ``sizes`` ({dim: new size}); host tensors are moved
+    to ``device`` first"""
     if x is None or all(x.shape[d] == n for d, n in sizes.items()):
         return x
     x = x if x.is_cuda else x.to(device, non_blocking=True)
     shape = list(x.shape)
     for d, n in sizes.items():
         shape[d] = n
-    out = x.new_zeros(shape)
+    out = x.new_full(shape, fill)
     out[tuple(slice(0, k) for k in x.shape)] = x
     return out
 

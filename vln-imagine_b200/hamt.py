@@ -21,8 +21,9 @@ import torch
 import torch.nn as nn
 
 from . import autograd_ops as ag
-from . import blocks, graphs, ops, params
+from . import blocks, feature_store, graphs, ops, params
 from .blocks import Stream
+from .feature_store import FeatureRows
 from .config import hamt_config
 from .duet import _f32c, align_forward
 from .ops import BF16, F32, HIDDEN
@@ -181,7 +182,7 @@ class NavCMT(nn.Module):
             ops.ensure_init(hist_img_feats)
             dev = hist_img_feats.device
             B = hist_img_feats.shape[0]
-            a = blocks.linear(blocks.operand(_f32c(hist_img_feats), lowp), pk['hist_img'], lowp, out_dtype=F32)
+            a = blocks.linear(blocks.feature_operand(hist_img_feats, lowp), pk['hist_img'], lowp, out_dtype=F32)
             # position embedding of the current step: a [B] index tensor (the same id for every episode, :597), so the
             # step never becomes a pointer baked into a captured graph
             if torch.is_tensor(ob_step_ids) and ob_step_ids.numel() == B:
@@ -194,7 +195,7 @@ class NavCMT(nn.Module):
             pano_mean = None
             if he.pano_encoder is not None:
                 V = hist_pano_img_feats.shape[1]
-                pa = blocks.linear(blocks.operand(_f32c(hist_pano_img_feats).view(B * V, -1), lowp), pk['hist_pano_img'], lowp, out_dtype=F32)
+                pa = blocks.linear(blocks.feature_operand(hist_pano_img_feats, lowp), pk['hist_pano_img'], lowp, out_dtype=F32)
                 x = blocks.embed(B * V, dev, a=pa, a_ln=he.pano_img_layer_norm, feat=_f32c(hist_pano_ang_feats).view(B * V, -1),
                                  feat_lin=he.pano_ang_linear, feat_ln=he.pano_ang_layer_norm, lowp=lowp, dropout=True)
                 s = [Stream(0, B, V, None)]                   # the reference's mask is all ones (:606-607)
@@ -214,7 +215,7 @@ class NavCMT(nn.Module):
         if not self.config.bypass_imag_encoder:
             return self._imagination_encoder(imagine_pano_img_feats, imagine_masks)
         with blocks.grad_mode(self._recording(imagine_pano_img_feats) and not self.fix_imagine_embeds):
-            y = blocks.embed(B * I, imagine_pano_img_feats.device, a=_f32c(imagine_pano_img_feats).view(B * I, HIDDEN),
+            y = blocks.embed(B * I, imagine_pano_img_feats.device, a=blocks.feature_operand(imagine_pano_img_feats, False),
                              const_rows=(self.imagine_embeddings.type_embedding.weight[0],))
         out = y.f32.view(B, I, HIDDEN)
         return out.detach() if self.fix_imagine_embeds else out
@@ -230,7 +231,7 @@ class NavCMT(nn.Module):
             raise ValueError('imagination length %d out of bounds (max_imagination_len %d, :683)' % (I, im.position_embeddings.weight.shape[0]))
         recording = self._recording(feats) and any(p.requires_grad for p in im.parameters()) and not self.fix_imagine_embeds
         with blocks.grad_mode(recording, self._drop() if recording else (0.0, 0.0)):
-            x = blocks.embed(B * I, feats.device, a=_f32c(feats).view(B * I, -1), pos_table=im.position_embeddings.weight,
+            x = blocks.embed(B * I, feats.device, a=blocks.feature_operand(feats, False), pos_table=im.position_embeddings.weight,
                              pos_period=I, const_rows=(im.type_embedding.weight[0],), lowp=lowp, want32=not lowp)
             a = blocks.linear(x.operand(lowp), pk['imag_img'], lowp, out_dtype=F32)
             x = blocks.layer_norm(a, None, pk['imag_ln0'], 1e-12, lowp)
@@ -267,7 +268,7 @@ class NavCMT(nn.Module):
         with blocks.grad_mode(recording, self._drop() if recording else (0.0, 0.0)):
             # observation embedding :521-544, :1073-1077
             ie = self.img_embeddings
-            a = blocks.linear(blocks.operand(_f32c(ob_img_feats).view(B * O, -1), lowp), pk['ob_img'], lowp, out_dtype=F32)
+            a = blocks.linear(blocks.feature_operand(ob_img_feats, lowp), pk['ob_img'], lowp, out_dtype=F32)
             ob = blocks.embed(B * O, dev, a=a, a_ln=ie.img_layer_norm, feat=_f32c(ob_ang_feats).view(B * O, -1), feat_lin=ie.ang_linear,
                               feat_ln=ie.ang_layer_norm, idx=ob_nav_types.long().contiguous().view(-1), table=ie.nav_type_embedding.weight,
                               const_rows=(self.embeddings.token_type_embeddings.weight[1],), out_ln=ie.layer_norm, dropout=True).f32
@@ -387,6 +388,8 @@ class VLNBertCMT(nn.Module):
     def _env_dropout(self, x):
         """models/model_HAMT.py: nn.Dropout(feat_dropout) on image features in train() mode"""
         if x is not None and self.training and self.drop_env.p > 0:
+            if isinstance(x, FeatureRows):                    # applied by the gather, at the same dropout site
+                return x.with_dropout(self.drop_env.p, ag.next_site())
             dev = self.vln_bert.embeddings.LayerNorm.weight.device
             x = x if x.is_cuda else x.to(dev, non_blocking=True)
             ops.ensure_init(x)
@@ -395,14 +398,14 @@ class VLNBertCMT(nn.Module):
 
     def _vis_fn(self, t):
         logits, txt_o, hist_o, ob_o = self.vln_bert.forward_visual(
-            t['txt_embeds'], t['txt_masks'], t['hist_embeds'], t['hist_masks'], t['ob_img_feats'], t['ob_ang_feats'],
+            t['txt_embeds'], t['txt_masks'], t['hist_embeds'], t['hist_masks'], feature_store.from_graph(t, 'ob_img_feats'), t['ob_ang_feats'],
             t['ob_nav_types'], t['ob_masks'], t.get('imagine_embeds'), t.get('imagine_masks'))
         states = hist_o[:, 0] if self.args.no_lang_ca else self._states(txt_o, hist_o)
         return {'act_logits': logits, 'states': states}
 
     def _hist_fn(self, t):
-        return {'hist': self.vln_bert.forward_history(t['hist_img_feats'], t['hist_ang_feats'], t['ob_step_ids'],
-                                                      t.get('hist_pano_img_feats'), t.get('hist_pano_ang_feats'))}
+        return {'hist': self.vln_bert.forward_history(feature_store.from_graph(t, 'hist_img_feats'), t['hist_ang_feats'], t['ob_step_ids'],
+                                                      feature_store.from_graph(t, 'hist_pano_img_feats'), t.get('hist_pano_ang_feats'))}
 
     def _graphable(self):
         return self.use_cuda_graphs and not self.training and not torch.is_grad_enabled()
@@ -431,9 +434,14 @@ class VLNBertCMT(nn.Module):
                 dev = m.embeddings.LayerNorm.weight.device
                 loc = dict(hist_img_feats=hist_img_feats, hist_ang_feats=hist_ang_feats,
                            hist_pano_img_feats=hist_pano_img_feats, hist_pano_ang_feats=hist_pano_ang_feats)
-                t = {k: loc[k] for k in self.HIST_TENSORS if loc[k] is not None}
+                t, borrowed = {}, {}
+                for k in self.HIST_TENSORS:
+                    ti, tb = feature_store.graph_args(k, loc[k])
+                    t.update(ti)
+                    borrowed.update(tb)
                 t['ob_step_ids'] = torch.full((hist_img_feats.shape[0],), int(ob_step), dtype=torch.int64)
-                return self._g_hist(t, dev, extra_key=(m.precision, ops.h16()), weights_token=graphs.weights_token(m, self._wt_cache))['hist']
+                return self._g_hist(t, dev, extra_key=(m.precision, ops.h16()), weights_token=graphs.weights_token(m, self._wt_cache),
+                                    borrowed=borrowed)['hist']
             return m('history', hist_img_feats=self._env_dropout(hist_img_feats), hist_ang_feats=hist_ang_feats,
                      ob_step_ids=ob_step, hist_pano_img_feats=self._env_dropout(hist_pano_img_feats),
                      hist_pano_ang_feats=hist_pano_ang_feats)
@@ -445,7 +453,11 @@ class VLNBertCMT(nn.Module):
                 dev = m.embeddings.LayerNorm.weight.device
                 loc = dict(txt_embeds=txt_embeds, txt_masks=txt_masks, ob_img_feats=ob_img_feats, ob_ang_feats=ob_ang_feats,
                            ob_nav_types=ob_nav_types, ob_masks=ob_masks, imagine_embeds=imagine_embeds, imagine_masks=imagine_masks)
-                t = {k: loc[k] for k in self.VIS_TENSORS if loc[k] is not None}
+                t, borrowed = {}, {}
+                for k in self.VIS_TENSORS:
+                    ti, tb = feature_store.graph_args(k, loc[k])
+                    t.update(ti)
+                    borrowed.update(tb)
                 t['hist_embeds'] = hist
                 t['hist_masks'] = length2mask(hist_lens, hist.size(1), 'cpu').logical_not()
                 T, O = hist.size(1), ob_img_feats.shape[1]
@@ -454,10 +466,12 @@ class VLNBertCMT(nn.Module):
                     # O to multiples of 8 (masked like the reference's batch padding) so that a few captured graphs serve a rollout
                     Tb, Ob = self._buckets.up(T, 4), self._buckets.up(O, 8)
                     dims = {'hist_embeds': {1: Tb}, 'hist_masks': {1: Tb}, 'ob_img_feats': {1: Ob}, 'ob_ang_feats': {1: Ob},
-                            'ob_nav_types': {1: Ob}, 'ob_masks': {1: Ob}}
-                    t = {k: (graphs.pad_to(v, dims[k], dev) if k in dims else v) for k, v in t.items()}
+                            'ob_nav_types': {1: Ob}, 'ob_masks': {1: Ob}, 'ob_img_feats:idx': {1: Ob}}
+                    # padded feature rows are -1 (zero rows), as the zero padding of the dense features
+                    t = {k: (graphs.pad_to(v, dims[k], dev, fill=-1 if k.endswith(':idx') else 0) if k in dims else v)
+                         for k, v in t.items()}
                 out = self._g_vis(t, dev, extra_key=(m.precision, ops.h16(), m.config.imagine_enc_pano),
-                                  weights_token=graphs.weights_token(m, self._wt_cache))
+                                  weights_token=graphs.weights_token(m, self._wt_cache), borrowed=borrowed)
                 logits = out['act_logits'][:, :O]
                 return (logits, out['states']) if return_states else (logits,)
             hist_masks = length2mask(hist_lens, hist.size(1), hist.device).logical_not()

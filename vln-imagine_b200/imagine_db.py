@@ -16,6 +16,20 @@ from typing import Dict, List, Mapping, Sequence, Tuple
 import numpy as np
 
 
+def open_source(src) -> Mapping:
+    """a mapping ``key -> array`` for a dict (returned as is), an .npz path or an HDF5 path (needs h5py); the caller closes
+    what it opened"""
+    if isinstance(src, Mapping):
+        return src
+    if isinstance(src, str) and src.endswith('.npz'):
+        return np.load(src)
+    try:
+        import h5py
+    except ImportError as e:                                      # pragma: no cover
+        raise ImportError('reading %r needs h5py; pass a dict or an .npz archive instead' % (src,)) from e
+    return h5py.File(src, 'r')
+
+
 class ImaginationImageFeaturesDB(object):
     def __init__(self, img_ft_file, image_feat_size: int):
         self.image_feat_size = image_feat_size
@@ -23,16 +37,7 @@ class ImaginationImageFeaturesDB(object):
         self._feature_store: Dict[str, np.ndarray] = {}
 
     def _open(self) -> Mapping:
-        src = self.img_ft_file
-        if isinstance(src, Mapping):
-            return src
-        if isinstance(src, str) and src.endswith('.npz'):
-            return np.load(src)
-        try:
-            import h5py
-        except ImportError as e:                                  # pragma: no cover
-            raise ImportError('reading %r needs h5py; pass a dict or an .npz archive instead' % (src,)) from e
-        return h5py.File(src, 'r')
+        return open_source(self.img_ft_file)
 
     def get_image_feature(self, path_id_instr_idx: str) -> np.ndarray:
         key = path_id_instr_idx

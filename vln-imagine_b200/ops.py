@@ -526,6 +526,22 @@ def cast_h16(src: torch.Tensor, dst: Optional[torch.Tensor] = None, dtype=None):
     return dst
 
 
+def gather_rows(store: torch.Tensor, idx: torch.Tensor, dtype, drop=None) -> torch.Tensor:
+    """rows of a device feature store: out[r] = store[idx[r]] (zero row for an index outside the store) as a dense
+    [idx.numel(), F] tensor of ``dtype`` (fp32, or a 16-bit GEMM operand format); drop = (p, seed tensor, site): the mask and
+    product of ``dropout`` on the dense fp32 rows (vi_gather_rows)"""
+    n_store, F, ld = _rows2d(store, 'store')
+    if idx.dtype != torch.int32:
+        raise _lib.VlnImagineError('feature row indices must be int32 (got %s)' % idx.dtype)
+    idx = idx.to(store.device, non_blocking=True).contiguous()
+    out = torch.empty((idx.numel(), F), dtype=dtype, device=store.device)
+    d32, d16 = (out, None) if dtype == F32 else (None, out)
+    p, seed, site = drop if drop is not None else (0.0, None, 0)
+    lib.vi_gather_rows(store.data_ptr(), _DT[store.dtype], ld, n_store, idx.data_ptr(), idx.numel(), F, _ptr(d32), _ptr(d16),
+                       _dt16(d16), float(p), _ptr(seed), int(site) & 0xFFFFFFFF, _stream())
+    return out
+
+
 def ce_rows(logits: torch.Tensor, labels: torch.Tensor, n_cols: int) -> torch.Tensor:
     """per-row cross-entropy over the first n_cols columns of fp32 logits [R, ld] (F.cross_entropy, reduction='none')"""
     R, _, ld = _rows2d(logits, 'logits')
