@@ -394,6 +394,46 @@ int vi_gather_rows(const void* store, int store_dtype, int64_t ld_store, int64_t
                    vi_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * HAMT fine-tuning by imitation + A2C (H/r2r/agent_cmt.py:544-577 sampling, :661-744 loss; H/models/model_HAMT.py:289-300 Critic),
+ * vi_rl.cu.  Fixed-order reductions, no atomics: two calls give identical bits.
+ *
+ * vi_policy_sample: per episode b < B (one warp each), over the O fp32 logits of row b (-inf = not admissible):
+ *   p = softmax, entropy[b] = -sum p log p (masked entries add 0), actions[b] = an inverse-CDF sample with u in [0, 1) from the
+ *   counter-based dropout hash of (episode b, *seed, site) - a masked entry is never drawn, rounding falls back to the last
+ *   admissible token; logp[b] = log p[actions[b]]; step_mask[b] = !ended[b] (before this step); then ended[b] |= actions[b] ==
+ *   stop_idx[b].  A row with no admissible token gives action -1, logp = entropy = 0. */
+int vi_policy_sample(const float* logits, int64_t ld, int O, int B, const int64_t* stop_idx, const uint32_t* seed, uint32_t site,
+                     int64_t* actions, float* logp, float* entropy, uint8_t* ended, float* step_mask, vi_stream_t stream);
+/* adjoint of (logp, entropy) of vi_policy_sample for the given actions, the softmax recomputed from the logits:
+ *   dlogits[b, j] = g_logp[b] (1[j = a_b] - p_j) - g_entropy[b] p_j (log p_j + H_b), exact 0 at masked entries and for action -1.
+ * g_logp / g_entropy may be NULL (zero). */
+int vi_policy_bwd(const float* logits, int64_t ld, int O, int B, const int64_t* actions, const float* g_logp, const float* g_entropy,
+                  float* dlogits, int64_t ldd, vi_stream_t stream);
+/* A2C loss over T steps of B episodes ([T, B] row-major inputs; boot [B] is a constant, NULL = 0):
+ *   R_T = ended[b] ? 0 : boot[b];  R_t = gamma R_{t+1} + rewards[t, b];  A = R_t - values[t, b] (no gradient through A)
+ *   out[1] = sum m (-logp A) / N,  out[2] = sum m 0.5 (R - v)^2 / N,  out[3] = sum m (-entropy_weight entropy) / N,
+ *   out[0] = out[1] + out[2] + out[3];  N = max(sum m, 1) (VI_A2C_NORM_TOTAL), B (BATCH) or 1 (NONE).  One CTA. */
+#define VI_A2C_NORM_NONE 0
+#define VI_A2C_NORM_BATCH 1
+#define VI_A2C_NORM_TOTAL 2
+int vi_a2c_loss(const float* values, const float* logp, const float* entropy, const float* masks, const float* rewards,
+                const float* boot, const uint8_t* ended, int T, int B, float gamma, float entropy_weight, int norm, float* out,
+                vi_stream_t stream);
+/* its adjoint from gout[4] = d out[0..3]: dvalues, dlogp, dentropy [T, B] (each may be NULL) */
+int vi_a2c_loss_bwd(const float* values, const float* logp, const float* entropy, const float* masks, const float* rewards,
+                    const float* boot, const uint8_t* ended, int T, int B, float gamma, float entropy_weight, int norm,
+                    const float* gout, float* dvalues, float* dlogp, float* dentropy, vi_stream_t stream);
+/* the critic's last layer over 512-wide fp32 rows: v[r] = dropout(h[r]) . w2 + b2[0], the dropout mask of element r * 512 + c at
+ * (drop_seed, drop_site) as in vi_dropout (drop_p == 0: none).  One warp per row. */
+int vi_value_head(const float* h, int64_t rows, const float* w2, const float* b2, float drop_p, const uint32_t* drop_seed,
+                  uint32_t drop_site, float* v, vi_stream_t stream);
+/* its adjoint, h being the ReLU output of the first layer: dh[r, c] = dv[r] w2[c] keep(r, c) / (1 - p) 1[h[r, c] > 0] to dh32 (fp32)
+ * and / or dh16 (the 16-bit operand of the first layer's gradient GEMMs), dw2[c] = sum_r dv[r] dropout(h)[r, c], db2 = sum_r dv[r]
+ * (may be NULL). */
+int vi_value_head_bwd(const float* dv, const float* h, int64_t rows, const float* w2, float drop_p, const uint32_t* drop_seed,
+                      uint32_t drop_site, float* dh32, void* dh16, int dh16_dtype, float* dw2, float* db2, vi_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Per-step graph glue of a DUET rollout (SURVEY.md section 8(f), rows N1 / N2).  Replaces the Python GraphMap /
  * FloydGraph objects (D/models/graph_utils.py:42-148) and the agent's per-step collate loops
  * (D/r2r/agent.py:98-207, 466-479) by dense per-episode arrays in HBM, caller-owned:

@@ -23,6 +23,7 @@ DT_BF16, DT_F32, DT_F16 = 0, 1, 2
 LN_NONE, LN_FOLD, LN_RESIDUAL = 0, 1, 2
 EPI_NONE, EPI_GELU, EPI_RELU = 0, 1, 2
 MASK_ADD_NEG10000, MASK_NEG_INF = 0, 1
+A2C_NORM = {'none': 0, 'batch': 1, 'total': 2}
 
 _p, _i, _l, _f = C.c_void_p, C.c_int, C.c_int64, C.c_float
 _ip = C.POINTER(C.c_int32)
@@ -99,6 +100,12 @@ PROTOTYPES = {
     'vi_cosine_loss_bwd': [_p, _p, _p, _p, _p, _i, _p],
     'vi_infonce_loss_bwd': [_p, _p, _p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _i, _i, _p],
     'vi_margin_loss_bwd': [_p, _p, _p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _i, _i, _p],
+    'vi_policy_sample': [_p, _l, _i, _i, _p, _p, C.c_uint32, _p, _p, _p, _p, _p, _p],
+    'vi_policy_bwd': [_p, _l, _i, _i, _p, _p, _p, _p, _l, _p],
+    'vi_a2c_loss': [_p, _p, _p, _p, _p, _p, _p, _i, _i, _f, _f, _i, _p, _p],
+    'vi_a2c_loss_bwd': [_p, _p, _p, _p, _p, _p, _p, _i, _i, _f, _f, _i, _p, _p, _p, _p, _p],
+    'vi_value_head': [_p, _l, _p, _p, _f, _p, C.c_uint32, _p, _p],
+    'vi_value_head_bwd': [_p, _p, _l, _p, _f, _p, C.c_uint32, _p, _p, _i, _p, _p, _p],
     'vi_graph_init': [_p, _p, _p, _p, _i, _i, _p],
     'vi_graph_update': [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _i, _p, _p],
     'vi_graph_embed_step': [_p, _p, _i, _i, _i, _p, _p, _i, _p, _p, _p, _i, _p, _i, _p, _p, _p],

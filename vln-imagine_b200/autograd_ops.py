@@ -843,3 +843,77 @@ class SegmentMeanFn(Function):
         d = torch.zeros(ctx.shape, dtype=F32, device=dev)
         ops.scatter_rows(rows, row_idx, d)
         return d, None, None, None, None
+
+
+class PolicySampleFn(Function):
+    """(log p[a], entropy) of one sampled step (ops.policy_sample) as differentiable outputs, plus the actions and the step mask
+    (non-differentiable); ``ended`` is updated in place.  Backward: vi_policy_bwd recomputes the softmax from the logits."""
+
+    @staticmethod
+    def forward(ctx, logits, stop_idx, ended, site):
+        logits = logits.contiguous()
+        actions, logp, ent, mask = ops.policy_sample(logits, stop_idx, dropout_seed(logits.device), site, ended)
+        ctx.save_for_backward(logits, actions)
+        ctx.mark_non_differentiable(actions, mask)
+        return logp, ent, actions, mask
+
+    @staticmethod
+    def backward(ctx, g_logp, g_ent, _ga, _gm):
+        logits, actions = ctx.saved_tensors
+        return ops.policy_bwd(logits, actions, g_logp, g_ent), None, None, None
+
+
+def policy_sample(logits, stop_idx, ended):
+    """one step of the sampled rollout: (actions, log p[a], entropy, step mask) from a fresh site of the device seed"""
+    logp, ent, actions, mask = PolicySampleFn.apply(logits, stop_idx, ended, next_site())
+    return actions, logp, ent, mask
+
+
+class A2CLossFn(Function):
+    """(total, policy, critic, entropy) A2C loss [4] of [T, B] values / log-probs / entropies (ops.a2c_loss); the masks, rewards,
+    bootstrap value and ended flags are constants"""
+
+    @staticmethod
+    def forward(ctx, values, logp, ent, masks, rewards, boot, ended, gamma, entropy_weight, normalize):
+        ctx.save_for_backward(values, logp, ent, masks, rewards, boot, ended)
+        ctx.cfg = (gamma, entropy_weight, normalize)
+        return ops.a2c_loss(values, logp, ent, masks, rewards, boot, ended, gamma, entropy_weight, normalize)
+
+    @staticmethod
+    def backward(ctx, gout):
+        dv, dlp, de = ops.a2c_loss_bwd(*ctx.saved_tensors, *ctx.cfg, gout)
+        return dv, dlp, de, None, None, None, None, None, None, None
+
+
+class CriticFn(Function):
+    """Critic.state2value: v = dropout(relu(x W1^T + b1)) . w2 + b2 for fp32 states x [rows, 768].  The first layer runs on the
+    operand of the precision mode (a bf16 copy of x, or x itself in the fp32 check mode) with the ReLU epilogue (vi_gemm16 /
+    vi_gemm_f32); the second is vi_value_head with the dropout mask inside.  Backward: vi_value_head_bwd writes dh with the ReLU and
+    dropout masks applied as the operand of the first layer's gradient GEMMs; dx comes back in fp32."""
+
+    @staticmethod
+    def forward(ctx, x32, pack, lowp, p, site, w2, b2, *params):
+        x = ops.cast_h16(x32, dtype=BF16) if lowp else x32.contiguous()
+        w, b = pack.get(lowp)
+        h = ops.gemm(x, w, b, epilogue=EPI_RELU, out_dtype=F32)
+        drop = (p, dropout_seed(x.device), site) if p > 0 else None
+        v = ops.value_head(h, w2.detach(), b2.detach(), drop)
+        ctx.save_for_backward(x, h, w2)
+        ctx.pack, ctx.lowp, ctx.drop = pack, lowp, drop
+        return v
+
+    @staticmethod
+    def backward(ctx, dv):
+        x, h, w2 = ctx.saved_tensors
+        dh, dw2, db2 = ops.value_head_bwd(dv, h, w2.detach(), x.dtype, ctx.drop)
+        dx = None
+        if ctx.needs_input_grad[0]:
+            dx = ops.gemm(dh, ctx.pack.get_t(ctx.lowp, 1), None, out_dtype=F32)
+        _, grads = _linear_bwd(ctx.pack, x, dh, ctx.lowp, None, False)
+        return (dx, None, None, None, None, dw2.view(w2.shape), db2, *grads)
+
+
+def critic(x, pack, lowp, p, w2, b2):
+    """differentiable critic head on fp32 states ``x`` (see CriticFn)"""
+    site = next_site() if p > 0 else 0
+    return CriticFn.apply(x, pack, lowp, float(p), site, w2, b2, *pack.grad_sources())

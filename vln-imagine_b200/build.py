@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libvlnimagine.so')
-SOURCES = ['vi_api.cu', 'vi_gemm_tc.cu', 'vi_gemm_simt.cu', 'vi_attn.cu', 'vi_rows.cu', 'vi_bwd.cu', 'vi_wgrad.cu', 'vi_attn_bwd.cu', 'vi_graph.cu', 'vi_xent.cu']
+SOURCES = ['vi_api.cu', 'vi_gemm_tc.cu', 'vi_gemm_simt.cu', 'vi_attn.cu', 'vi_rows.cu', 'vi_bwd.cu', 'vi_wgrad.cu', 'vi_attn_bwd.cu', 'vi_graph.cu', 'vi_xent.cu', 'vi_rl.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-shared', '-lcudart']
 

@@ -80,7 +80,7 @@ void vi_count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
 extern "C" int64_t vi_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 
-extern "C" int vi_version(void) { return 104; }   // 0.1.4
+extern "C" int vi_version(void) { return 105; }   // 0.1.5
 
 extern "C" const char* vi_last_error(void) { return g_err; }
 

@@ -487,7 +487,45 @@ class VLNBertCMT(nn.Module):
 
     def _states(self, txt_o, hist_o):
         """states = txt_embeds[:, 0] * hist_embeds[:, 0]  (model_HAMT.py:86): one mul_bcast launch with
-        one row per episode."""
+        one row per episode.  While autograd records, the same kernel as a MulBcastFn node, so that the critic's value loss
+        reaches the cross-modal layers (agent_cmt.py:661-744)."""
         B = txt_o.shape[0]
+        if ag.needs_grad(txt_o, hist_o):
+            return ag.MulBcastFn.apply(hist_o[:, :1], txt_o[:, 0], False)
         y32, _ = ops.mul_bcast(hist_o, hist_o.stride(0), txt_o, txt_o.stride(0), B, 1, want16=False)
         return y32
+
+
+class Critic(nn.Module):
+    """models/model_HAMT.py:289-300: state2value = Linear(768, 512) -> ReLU -> Dropout(args.dropout) -> Linear(512, 1), forward
+    returns state2value(state).squeeze().  Same parameter names (state2value.0.*, state2value.3.*), so the agent's checkpoints
+    ('critic') load unchanged.  The first layer runs on vi_gemm16 with the ReLU epilogue (vi_gemm_f32 in the fp32 check mode), the
+    dropout and the 512 -> 1 layer in one vi_value_head launch; autograd_ops.CriticFn holds the backward pass."""
+
+    def __init__(self, args):
+        super().__init__()
+        self.state2value = nn.Sequential(nn.Linear(HIDDEN, 512), nn.ReLU(), nn.Dropout(p=args.dropout), nn.Linear(512, 1))
+        self.precision = os.environ.get('VLN_IMAGINE_PRECISION', 'bf16')
+        self._packs = None
+
+    def _apply(self, fn, *a, **k):
+        self._packs = None
+        return super()._apply(fn, *a, **k)
+
+    def _pk(self):
+        if self._packs is None:
+            l1 = self.state2value[0]
+            self._packs = blocks.LinearPack([l1.weight], [l1.bias])
+        return self._packs
+
+    def forward(self, state):
+        ops.ensure_init(state)
+        if self.precision not in ('bf16', 'fp32'):
+            raise ValueError("precision must be 'bf16' or 'fp32'")
+        lowp = self.precision == 'bf16'
+        x = _f32c(state).view(-1, HIDDEN)
+        p = float(self.state2value[2].p) if self.training else 0.0
+        l2 = self.state2value[3]
+        with ops.half_format(BF16):
+            v = ag.critic(x, self._pk(), lowp, p, l2.weight, l2.bias)
+        return v.squeeze()

@@ -736,3 +736,89 @@ def mul_bcast_bwd_s(dy: torch.Tensor, x: torch.Tensor, B: int, R: int) -> torch.
     ds = torch.empty((B, HIDDEN), dtype=F32, device=x.device)
     lib.vi_mul_bcast_bwd_s(dy.data_ptr(), x.data_ptr(), ds.data_ptr(), B, R, _stream())
     return ds
+
+
+# ----------------------------------------------------------------------------------------------
+# imitation + A2C fine-tuning of HAMT (vi_rl.cu)
+def policy_sample(logits: torch.Tensor, stop_idx: torch.Tensor, seed: torch.Tensor, site: int, ended: torch.Tensor):
+    """one sampling step of the agent over fp32 logits [B, O] (-inf = not admissible): (actions int64 [B], log p[a] [B], entropy [B],
+    step mask [B] = not ended before this step); ``ended`` (uint8 [B]) is updated in place with actions == stop_idx"""
+    B, O, ld = _rows2d(logits, 'logits')
+    if ended.dtype != torch.uint8 or not ended.is_contiguous() or stop_idx.dtype != torch.int64:
+        raise _lib.VlnImagineError('policy_sample: ended must be contiguous uint8 and stop_idx int64')
+    dev = logits.device
+    actions = torch.empty((B,), dtype=torch.int64, device=dev)
+    logp, ent, mask = (torch.empty((B,), dtype=F32, device=dev) for _ in range(3))
+    lib.vi_policy_sample(logits.data_ptr(), ld, O, B, stop_idx.contiguous().data_ptr(), seed.data_ptr(), int(site) & 0xFFFFFFFF,
+                         actions.data_ptr(), logp.data_ptr(), ent.data_ptr(), ended.data_ptr(), mask.data_ptr(), _stream())
+    return actions, logp, ent, mask
+
+
+def policy_bwd(logits: torch.Tensor, actions: torch.Tensor, g_logp: Optional[torch.Tensor], g_ent: Optional[torch.Tensor]):
+    """d logits [B, O] of g_logp . log p[a] + g_ent . entropy (policy_sample's outputs for the given actions)"""
+    B, O, ld = _rows2d(logits, 'logits')
+    d = torch.empty((B, O), dtype=F32, device=logits.device)
+    c = lambda t: t.float().contiguous() if t is not None else None      # noqa: E731
+    g_logp, g_ent = c(g_logp), c(g_ent)
+    lib.vi_policy_bwd(logits.data_ptr(), ld, O, B, actions.data_ptr(), _ptr(g_logp), _ptr(g_ent), d.data_ptr(), O, _stream())
+    return d
+
+
+def _a2c_operands(values, logp, ent, masks, rewards):
+    ts = [t.float().contiguous() for t in (values, logp, ent, masks, rewards)]
+    if any(t.shape != ts[0].shape or t.dim() != 2 for t in ts):
+        raise _lib.VlnImagineError('a2c_loss: values, logp, entropy, masks and rewards must all be [T, B]')
+    return ts
+
+
+def a2c_loss(values, logp, ent, masks, rewards, boot: Optional[torch.Tensor], ended: Optional[torch.Tensor], gamma: float,
+             entropy_weight: float, normalize: str) -> torch.Tensor:
+    """fp32 [4]: (total, policy, critic, entropy) A2C loss of [T, B] inputs (vi_a2c_loss); boot [B] is a constant (None = 0),
+    ended (uint8 [B]) the flags after the last step"""
+    v, lp, e, m, r = _a2c_operands(values, logp, ent, masks, rewards)
+    T, B = v.shape
+    out = torch.empty((4,), dtype=F32, device=v.device)
+    boot = boot.float().contiguous() if boot is not None else None
+    lib.vi_a2c_loss(v.data_ptr(), lp.data_ptr(), e.data_ptr(), m.data_ptr(), r.data_ptr(), _ptr(boot), _ptr(ended), T, B, float(gamma),
+                    float(entropy_weight), _lib.A2C_NORM[normalize], out.data_ptr(), _stream())
+    return out
+
+
+def a2c_loss_bwd(values, logp, ent, masks, rewards, boot, ended, gamma: float, entropy_weight: float, normalize: str,
+                 gout: torch.Tensor):
+    """(dvalues, dlogp, dentropy) [T, B] of a2c_loss from gout = d(total, policy, critic, entropy)"""
+    v, lp, e, m, r = _a2c_operands(values, logp, ent, masks, rewards)
+    T, B = v.shape
+    dv, dlp, de = (torch.empty((T, B), dtype=F32, device=v.device) for _ in range(3))
+    boot = boot.float().contiguous() if boot is not None else None
+    gout = gout.float().contiguous()
+    lib.vi_a2c_loss_bwd(v.data_ptr(), lp.data_ptr(), e.data_ptr(), m.data_ptr(), r.data_ptr(), _ptr(boot), _ptr(ended), T, B,
+                        float(gamma), float(entropy_weight), _lib.A2C_NORM[normalize], gout.data_ptr(), dv.data_ptr(), dlp.data_ptr(),
+                        de.data_ptr(), _stream())
+    return dv, dlp, de
+
+
+def value_head(h: torch.Tensor, w2: torch.Tensor, b2: torch.Tensor, drop=None) -> torch.Tensor:
+    """v [rows] = dropout(h) . w2 + b2 over contiguous fp32 [rows, 512] (vi_value_head); drop = (p, seed tensor, site)"""
+    rows = h.shape[0]
+    if h.dtype != F32 or not h.is_contiguous() or h.shape[1] != 512:
+        raise _lib.VlnImagineError('value_head: h must be contiguous fp32 [rows, 512]')
+    p, seed, site = drop if drop is not None else (0.0, None, 0)
+    v = torch.empty((rows,), dtype=F32, device=h.device)
+    lib.vi_value_head(h.data_ptr(), rows, w2.data_ptr(), b2.data_ptr(), float(p), _ptr(seed), int(site) & 0xFFFFFFFF, v.data_ptr(),
+                      _stream())
+    return v
+
+
+def value_head_bwd(dv: torch.Tensor, h: torch.Tensor, w2: torch.Tensor, dtype, drop=None):
+    """(dh [rows, 512] of ``dtype`` - fp32, or the 16-bit operand of the first layer's gradient GEMMs -, dw2 [512], db2 [1])"""
+    rows = h.shape[0]
+    p, seed, site = drop if drop is not None else (0.0, None, 0)
+    dh = torch.empty((rows, 512), dtype=dtype, device=h.device)
+    d32, d16 = (dh, None) if dtype == F32 else (None, dh)
+    dw2 = torch.empty((512,), dtype=F32, device=h.device)
+    db2 = torch.empty((1,), dtype=F32, device=h.device)
+    dv = dv.float().contiguous()
+    lib.vi_value_head_bwd(dv.data_ptr(), h.data_ptr(), rows, w2.data_ptr(), float(p), _ptr(seed), int(site) & 0xFFFFFFFF, _ptr(d32),
+                          _ptr(d16), _dt16(d16), dw2.data_ptr(), db2.data_ptr(), _stream())
+    return dh, dw2, db2

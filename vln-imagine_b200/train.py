@@ -158,6 +158,95 @@ def duet_finetune_iteration(model, ep: dict, n_steps: int = 1, cosine_weight: fl
     return loss, ce / B, aux, nav
 
 
+def hamt_stop_tokens(ob_nav_types: torch.Tensor) -> torch.Tensor:
+    """Index of the [stop] observation token per episode: the last admissible one (nav_type != 0), which is where HAMT's agent
+    places it after the candidates (ob_cand_lens - 1, r2r/agent_cmt.py).  Also the synthetic teacher action of the IL rollout,
+    standing in for _teacher_action (which needs the simulator), as in the gradient fixtures."""
+    ok = ob_nav_types != 0
+    idx = torch.arange(ok.shape[1], device=ok.device)[None, :].expand_as(ok)
+    return torch.where(ok, idx, torch.zeros_like(idx)).max(1).values
+
+
+def _hamt_rollout(model, ep: dict, n_steps: int, step):
+    """language + imagine + align once, then ``n_steps`` calls of 'visual' followed by 'history' with the history growing by one
+    token per step (r2r/agent_cmt.py:371-605); ``step(t, txt, img2, hist_embeds, hist_lens)`` runs the 'visual' call and whatever
+    the rollout does with it.  Returns (aux, the last step's inputs for a bootstrap call)."""
+    B = ep['txt_ids'].shape[0]
+    dev = ep['txt_ids'].device
+    txt = model('language', txt_ids=ep['txt_ids'], txt_masks=ep['txt_masks'])
+    img = model('imagine', imagine_pano_img_feats=ep['imagine_feats'], imagine_masks=None)
+    aux, img2 = model('align_with_contrastive_loss', align_txt_embeds=txt, txt_masks=ep['txt_masks'], align_imagine_embeds=img,
+                      imagine_masks=ep['imagine_masks'], sub_instr_segs=ep['sub_instr_segs'],
+                      sub_instr_imag_flag=ep['sub_instr_imag_flag'], noun_phrase_segs=ep['noun_phrase_segs'],
+                      obs_instr_ids=ep['obs_instr_ids'])
+    hist = [model('history').expand(B, -1)]
+    for t in range(n_steps):
+        step(txt, img2, hist, torch.full((B,), t + 1, dtype=torch.int64, device=dev))
+        hist.append(model('history', hist_img_feats=ep['hist_img_feats'], hist_ang_feats=ep['hist_ang_feats'], ob_step=t,
+                          hist_pano_img_feats=ep['hist_pano_img_feats'], hist_pano_ang_feats=ep['hist_pano_ang_feats']))
+    return aux, (txt, img2, hist, torch.full((B,), n_steps + 1, dtype=torch.int64, device=dev))
+
+
+def _hamt_visual(model, ep, txt, img2, hist, lens, return_states=False):
+    return model('visual', txt_embeds=txt, txt_masks=ep['txt_masks'], hist_embeds=hist, hist_lens=lens, ob_img_feats=ep['ob_img_feats'],
+                 ob_ang_feats=ep['ob_ang_feats'], ob_nav_types=ep['ob_nav_types'], ob_masks=ep['ob_masks'], imagine_embeds=img2,
+                 imagine_masks=ep['imagine_masks'], return_states=return_states)
+
+
+def hamt_finetune_iteration(model, critic, ep: dict, n_steps: int, rewards: torch.Tensor, ml_weight: float = 0.2, gamma: float = 0.9,
+                            entropy_weight: float = 0.01, normalize: str = 'total', aux_weight: float = 0.5, backward: bool = True,
+                            fused_accumulation: bool = False):
+    """One IL + A2C iteration of HAMT's agent (Seq2SeqCMTAgent.train with feedback 'sample', r2r/agent_cmt.py) on a batch of episodes:
+
+    * teacher-forced rollout (skipped when ``ml_weight`` is 0): cross-entropy of every step's logits on the teacher action
+      (hamt_stop_tokens), scaled by ml_weight / B, plus aux_weight x the alignment loss;
+    * sampled rollout: 'visual' with return_states=True, one vi_policy_sample per step (actions stay on the device, the device seed
+      keys the draw), then one extra 'visual' call for the bootstrap state; the critic runs ONCE over all T + 1 steps' states and the
+      A2C node (vi_a2c_loss) takes the first T values, the last one detached (r2r/agent_cmt.py:661-744).
+
+    ``model`` is hamt.VLNBertCMT, ``critic`` hamt.Critic, ``ep`` device tensors of synth.hamt_episode, ``rewards`` fp32 [n_steps, B]
+    (the simulator's distance reward is agent code).  No host synchronisation: a GraphedIteration over a container of both modules
+    (torch.nn.ModuleList([model, critic])) replays the whole iteration.  Returns (loss, parts, actions [n_steps, B]) with parts =
+    dict(ce, aux, rl, policy, critic, entropy)."""
+    B = ep['txt_ids'].shape[0]
+    dev = ep['txt_ids'].device
+    parts = {}
+    loss = None
+    if ml_weight != 0:
+        tgt = hamt_stop_tokens(ep['ob_nav_types'])
+        ces = []
+
+        def teacher_step(txt, img2, hist, lens):
+            logits = _hamt_visual(model, ep, txt, img2, hist, lens)[0]
+            ces.append(torch.nn.functional.cross_entropy(logits, tgt, reduction='sum'))
+        aux, _ = _hamt_rollout(model, ep, n_steps, teacher_step)
+        ce = torch.stack(ces).sum()
+        loss = ce * (ml_weight / B) + aux_weight * aux
+        parts.update(ce=ce / B, aux=aux)
+
+    from . import autograd_ops as ag
+    stop = hamt_stop_tokens(ep['ob_nav_types'])
+    ended = torch.zeros((B,), dtype=torch.uint8, device=dev)
+    states, logps, ents, masks, actions = [], [], [], [], []
+
+    def sample_step(txt, img2, hist, lens):
+        logits, h = _hamt_visual(model, ep, txt, img2, hist, lens, return_states=True)
+        a, lp, e, m = ag.policy_sample(logits, stop, ended)
+        for lst, v in ((states, h), (logps, lp), (ents, e), (masks, m), (actions, a)):
+            lst.append(v)
+    _, last = _hamt_rollout(model, ep, n_steps, sample_step)
+    states.append(_hamt_visual(model, ep, *last, return_states=True)[1])        # bootstrap state s_T
+    values = critic(torch.cat(states, 0)).view(n_steps + 1, B)
+    rl = ag.A2CLossFn.apply(values[:n_steps], torch.stack(logps), torch.stack(ents), torch.stack(masks), rewards.float(),
+                            values[n_steps].detach(), ended, float(gamma), float(entropy_weight), normalize)
+    parts.update(rl=rl[0], policy=rl[1], critic=rl[2], entropy=rl[3])
+    loss = rl[0] if loss is None else loss + rl[0]
+    if backward:
+        with ag.fused_grad_accumulation(fused_accumulation):
+            loss.backward()
+    return loss, parts, torch.stack(actions)
+
+
 class GraphedIteration:
     """A whole fine-tuning iteration replayed from CUDA graphs over static inputs: an iteration is ~4000 kernel launches
     whose host cost (ctypes, autograd bookkeeping) exceeds their device time at batch 64.  Two graphs bracket the one
