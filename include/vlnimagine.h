@@ -336,12 +336,22 @@ int vi_scatter_add_rows(const float* src, const int64_t* idx, int period, float*
 int vi_rowdot_bwd(const float* dout, const float* x, const float* w, float* dx, float* dw, float* db_cols, int64_t rows,
                   int n_groups, const int32_t* group_row_end, float* scratch, int64_t scratch_elems, vi_stream_t stream);
 /* attention backward for one token stream (same operand conventions as one vi_attn_problem); d_affine -> device {dw, db}
- * of the GASA affine, accumulated (+=); dq / dk / dv have the dtype of q / k / v. */
+ * of the GASA affine, accumulated (+=); dq / dk / dv have the dtype of q / k / v.  drop_p / drop_site / drop_seed repeat the
+ * forward's attention dropout (bf16 only): the mask is rebuilt from the same element ids.
+ * Every problem the forward runs, Lk <= 512:
+ *   bf16, <= 128 keys and <= 256 queries: one CTA per (episode, head), GASA gradient by atomics;
+ *   other bf16 problems: two key-blocked tensor-core launches that recompute the softmax statistics (deterministic);
+ *   fp32 (check mode), <= 201 keys: one CTA per (episode, head) with K, V, dK, dV in shared memory;
+ *   fp32, 202 .. 380 keys (the fp32 forward's own limit): two FFMA launches through the workspace (deterministic).
+ * workspace: fp32 device scratch of at least vi_attn_bwd_workspace(B, H, Lq, Lk, dtype) floats, 16-byte aligned (NULL when
+ * that is 0); a shorter one is an error (VI_ERR_ARG).  Calls on one stream may share it.  vi_attn_bwd_workspace returns 0 for
+ * a problem vi_attn_bwd rejects (more than 512 keys; fp32 beyond 380). */
+int64_t vi_attn_bwd_workspace(int B, int H, int Lq, int Lk, int dtype);
 int vi_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
                 const void* dout, int64_t ldo, void* dq, int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv,
                 int dtype, const uint8_t* key_mask, const float* pair_dist, const float* bias_affine, float* d_affine,
                 int B, int H, int Lq, int Lk, int mask_mode, float drop_p, uint32_t drop_site, const uint32_t* drop_seed,
-                vi_stream_t stream);
+                float* workspace, int64_t workspace_floats, vi_stream_t stream);
 /* adjoint of vi_duet_fuse_logits; any of d_global / d_local / d_fused may be NULL (treated as zero) */
 int vi_duet_fuse_logits_bwd(const float* g_raw, const float* l_raw, const float* fuse_raw,
                             const uint8_t* gmap_masks, const uint8_t* gmap_visited, const uint8_t* vp_nav_masks,

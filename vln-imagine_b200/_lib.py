@@ -93,7 +93,9 @@ PROTOTYPES = {
     'vi_feat_wgrad': [_p, _p, _i, _p, _p, _l, _p, _l, _p],
     'vi_scatter_add_rows': [_p, _p, _i, _p, _l, _p],
     'vi_rowdot_bwd': [_p, _p, _p, _p, _p, _p, _l, _i, _ip, _p, _l, _p],
-    'vi_attn_bwd': [_p, _l, _p, _l, _p, _l, _p, _l, _p, _l, _p, _l, _p, _l, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _f, C.c_uint32, _p, _p],
+    'vi_attn_bwd_workspace': [_i, _i, _i, _i, _i],
+    'vi_attn_bwd': [_p, _l, _p, _l, _p, _l, _p, _l, _p, _l, _p, _l, _p, _l, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _f, C.c_uint32, _p,
+                    _p, _l, _p],
     'vi_dropout': [_p, _p, _l, _f, _p, C.c_uint32, _i, _p],
     'vi_duet_fuse_logits_bwd': [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p],
     'vi_mul_bcast_bwd_s': [_p, _p, _p, _l, _i, _p],
@@ -112,12 +114,13 @@ PROTOTYPES = {
     'vi_graph_features': [_p, _p, _p, _i, _i, _p, _p, _p, _p, _p, _i, _p, _p, _p, _i, _p, _i, _p, _p],
 }
 # entry points that return a value rather than a VI_OK / VI_ERR_* status (ops.lib passes their result through unchecked)
-QUERIES = {'vi_version', 'vi_wgrad16_splits', 'vi_wgrad16_workspace', 'vi_launch_count', 'vi_last_error'}
+QUERIES = {'vi_version', 'vi_wgrad16_splits', 'vi_wgrad16_workspace', 'vi_attn_bwd_workspace', 'vi_launch_count', 'vi_last_error'}
 for _name, _args in PROTOTYPES.items():
     _fn = getattr(lib, _name)            # AttributeError here = header/library mismatch: fail loudly
     _fn.argtypes = _args
     _fn.restype = _i
 lib.vi_wgrad16_workspace.restype = C.c_int64
+lib.vi_attn_bwd_workspace.restype = C.c_int64
 lib.vi_launch_count.restype = C.c_int64
 lib.vi_last_error.argtypes = []
 lib.vi_last_error.restype = C.c_char_p

@@ -37,6 +37,8 @@ bool vi_pdl_enabled() {
 }
 
 int vi_attn_init();
+int vi_attn_bwd_init();       // vi_attn_bwd.cu
+int vi_attn_bwd_f32_init();   // vi_bwd.cu
 
 // ---- TMA tensor maps (driver entry point resolved once per process) -------------------------------------------------
 #include <mutex>
@@ -80,7 +82,7 @@ void vi_count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
 extern "C" int64_t vi_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 
-extern "C" int vi_version(void) { return 105; }   // 0.1.5
+extern "C" int vi_version(void) { return 106; }   // 0.1.6
 
 extern "C" const char* vi_last_error(void) { return g_err; }
 
@@ -94,5 +96,7 @@ extern "C" int vi_init(int device) {
   }
   g_num_sms = prop.multiProcessorCount;
   if (int rc = vi_attn_init()) return rc;
+  if (int rc = vi_attn_bwd_init()) return rc;
+  if (int rc = vi_attn_bwd_f32_init()) return rc;
   return VI_OK;
 }

@@ -515,7 +515,8 @@ __global__ void __launch_bounds__(256) rowdot_bwd_w_partial_kernel(const float* 
 }
 
 // ---------------------------------------------------------------------------------------------
-// attention backward, one CTA (8 warps) per (episode, head); fp32 arithmetic on fp32 or bf16 tensors.
+// attention backward, one CTA (8 warps) per (episode, head); fp32 arithmetic (the fp32 check mode, up to 201 keys; bf16 tensors
+// take the tensor-core kernels of vi_attn_bwd.cu).
 //   S = Q K^T / 8 + mask + (w dist + b);  P = softmax(S);  dP = dO V^T;  Dr = rowsum(dO o O);
 //   dS = P o (dP - Dr);  dQ = dS K / 8;  dK = dS^T Q / 8;  dV = P^T dO;
 //   GASA:  dw += sum dS dist,  db += sum dS  (two fp32 atomics per CTA).
@@ -650,6 +651,146 @@ __global__ void __launch_bounds__(256) attn_bwd_kernel(const AttnBwdParams p) {
     dkg[(long long)key * p.lddk + d] = from_f32<T>(dKs[e]);
     dvg[(long long)key * p.lddv + d] = from_f32<T>(dVs[e]);
   }
+}
+
+// ---------------------------------------------------------------------------------------------
+// fp32 check mode beyond attn_bwd_kernel's shared memory (202 .. 380 keys; 380 is where the fp32 forward kernel's
+// (134 Lk + 256) * 4 bytes reach its 200 KB): FFMA in two launches, one writer per output element, fixed-order sums.
+//   rows kernel, one CTA (4 warps) per (episode, head), K and V staged: per query row P and dS go to the workspace
+//               ([B * H][Lq][Lk] each) and dQ = dS K / 8 is written; GASA partials per CTA;
+//   keys kernel, thread (key, d): dK = dS^T Q / 8 and dV = P^T dO from the workspace rows; its first CTA adds the GASA
+//               partials to d_affine.
+// ---------------------------------------------------------------------------------------------
+constexpr int ATTN_BWD_F32_MAX_KEYS = 380;
+
+__global__ void __launch_bounds__(128) attn_bwd_f32_rows_kernel(const AttnBwdParams p, float* ws_p, float* ws_s, float* aff_part) {
+  pdl_enter();
+  extern __shared__ __align__(16) float sm[];
+  const int Lk = p.Lk;
+  float* Ks = sm;                        // [Lk][65]
+  float* Vs = Ks + (size_t)Lk * 65;      // [Lk][65]
+  float* madd = Vs + (size_t)Lk * 65;    // [Lk]
+  float* wbuf = madd + Lk;               // per warp: q[64], do[64]
+  float* red = wbuf + 4 * 128;           // [4][2]
+  const int b = blockIdx.y, h = blockIdx.x;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const float* kg = reinterpret_cast<const float*>(p.k) + (long long)b * Lk * p.ldk + h * 64;
+  const float* vg = reinterpret_cast<const float*>(p.v) + (long long)b * Lk * p.ldv + h * 64;
+  for (int e = tid; e < Lk * 64; e += 128) {
+    const int key = e >> 6, d = e & 63;
+    Ks[(size_t)key * 65 + d] = kg[(long long)key * p.ldk + d];
+    Vs[(size_t)key * 65 + d] = vg[(long long)key * p.ldv + d];
+  }
+  for (int key = tid; key < Lk; key += 128) {
+    float m = 0.f;
+    if (p.key_mask && !p.key_mask[(long long)b * Lk + key]) m = (p.mask_mode == VI_MASK_NEG_INF) ? -INFINITY : -10000.0f;
+    madd[key] = m;
+  }
+  __syncthreads();
+  float bw = 0.f, bb = 0.f;
+  if (p.pair_dist) { bw = p.bias_affine[0]; bb = p.bias_affine[1]; }
+  float* myq = wbuf + (size_t)warp * 128;
+  float* mydo = myq + 64;
+  const long long bh = (long long)b * p.H + h;
+  const float* qg = reinterpret_cast<const float*>(p.q) + (long long)b * p.Lq * p.ldq + h * 64;
+  const float* dog = reinterpret_cast<const float*>(p.dout) + (long long)b * p.Lq * p.ldo + h * 64;
+  float* dqg = reinterpret_cast<float*>(p.dq) + (long long)b * p.Lq * p.lddq + h * 64;
+  float aw = 0.f, ab = 0.f;
+  for (int r = warp; r < p.Lq; r += 4) {
+    myq[lane] = qg[(long long)r * p.ldq + lane];
+    myq[lane + 32] = qg[(long long)r * p.ldq + lane + 32];
+    mydo[lane] = dog[(long long)r * p.ldo + lane];
+    mydo[lane + 32] = dog[(long long)r * p.ldo + lane + 32];
+    __syncwarp();
+    float* prow = ws_p + (bh * p.Lq + r) * Lk;
+    float* srow = ws_s + (bh * p.Lq + r) * Lk;
+    const float* pd = p.pair_dist ? p.pair_dist + ((long long)b * p.Lq + r) * Lk : nullptr;
+    float mx = -INFINITY;
+    for (int key = lane; key < Lk; key += 32) {
+      float dot = 0.f, dp = 0.f;
+#pragma unroll 16
+      for (int d = 0; d < 64; ++d) {
+        dot = fmaf(myq[d], Ks[(size_t)key * 65 + d], dot);
+        dp = fmaf(mydo[d], Vs[(size_t)key * 65 + d], dp);
+      }
+      float add = madd[key];
+      if (pd) add += fmaf(bw, pd[key], bb);
+      const float s = dot * 0.125f + add;
+      prow[key] = s;
+      srow[key] = dp;
+      mx = fmaxf(mx, s);
+    }
+    mx = warp_max(mx);
+    const float mu = (mx == -INFINITY) ? 0.f : mx;
+    float sum = 0.f;
+    for (int key = lane; key < Lk; key += 32) {
+      const float e = expf(prow[key] - mu);
+      prow[key] = e;
+      sum += e;
+    }
+    sum = warp_sum(sum);
+    const float inv = sum > 0.f ? 1.0f / sum : 0.f;
+    float dr = 0.f;
+    for (int key = lane; key < Lk; key += 32) {
+      const float pj = prow[key] * inv;
+      prow[key] = pj;
+      dr = fmaf(pj, srow[key], dr);
+    }
+    dr = warp_sum(dr);
+    for (int key = lane; key < Lk; key += 32) {
+      const float g = prow[key] * (srow[key] - dr);
+      srow[key] = g;
+      if (pd) { aw = fmaf(g, pd[key], aw); ab += g; }
+    }
+    __syncwarp();
+    float q0 = 0.f, q1 = 0.f;
+    for (int key = 0; key < Lk; ++key) {
+      const float g = srow[key];
+      q0 = fmaf(g, Ks[(size_t)key * 65 + lane], q0);
+      q1 = fmaf(g, Ks[(size_t)key * 65 + lane + 32], q1);
+    }
+    dqg[(long long)r * p.lddq + lane] = q0 * 0.125f;
+    dqg[(long long)r * p.lddq + lane + 32] = q1 * 0.125f;
+    __syncwarp();
+  }
+  if (p.pair_dist && p.d_affine) {
+    aw = warp_sum(aw);
+    ab = warp_sum(ab);
+    if (lane == 0) { red[2 * warp] = aw; red[2 * warp + 1] = ab; }
+    __syncthreads();
+    if (tid == 0) {
+      aff_part[2 * bh] = (red[0] + red[2]) + (red[4] + red[6]);
+      aff_part[2 * bh + 1] = (red[1] + red[3]) + (red[5] + red[7]);
+    }
+  }
+}
+
+// grid (ceil(Lk / 4), H, B), 256 threads: thread (key 4 * blockIdx.x + tid / 64, column tid % 64)
+__global__ void __launch_bounds__(256) attn_bwd_f32_keys_kernel(const AttnBwdParams p, const float* ws_p, const float* ws_s,
+                                                                const float* aff_part) {
+  pdl_enter();
+  const int b = blockIdx.z, h = blockIdx.y, tid = threadIdx.x;
+  if (p.pair_dist && p.d_affine && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && tid < 32) {
+    float sw = 0.f, sb = 0.f;
+    for (int i = tid; i < p.B * p.H; i += 32) { sw += aff_part[2 * i]; sb += aff_part[2 * i + 1]; }
+    sw = warp_sum(sw);
+    sb = warp_sum(sb);
+    if (tid == 0) { p.d_affine[0] += sw; p.d_affine[1] += sb; }
+  }
+  const int key = blockIdx.x * 4 + (tid >> 6), d = tid & 63;
+  if (key >= p.Lk) return;
+  const long long bh = (long long)b * p.H + h;
+  const float* pc = ws_p + bh * p.Lq * p.Lk + key;
+  const float* sc = ws_s + bh * p.Lq * p.Lk + key;
+  const float* qg = reinterpret_cast<const float*>(p.q) + (long long)b * p.Lq * p.ldq + h * 64 + d;
+  const float* og = reinterpret_cast<const float*>(p.dout) + (long long)b * p.Lq * p.ldo + h * 64 + d;
+  float dk = 0.f, dv = 0.f;
+  for (int r = 0; r < p.Lq; ++r) {
+    dv = fmaf(pc[(long long)r * p.Lk], og[(long long)r * p.ldo], dv);
+    dk = fmaf(sc[(long long)r * p.Lk], qg[(long long)r * p.ldq], dk);
+  }
+  reinterpret_cast<float*>(p.dk)[((long long)b * p.Lk + key) * p.lddk + h * 64 + d] = dk * 0.125f;
+  reinterpret_cast<float*>(p.dv)[((long long)b * p.Lk + key) * p.lddv + h * 64 + d] = dv;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -944,6 +1085,13 @@ int vi_attn_bwd_tc(const void* q, int64_t ldq, const void* k, int64_t ldk, const
                    int64_t ldo, void* dq, int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv,
                    const uint8_t* key_mask, const float* pair_dist, const float* bias_affine, float* d_affine, int B, int H,
                    int Lq, int Lk, int mask_mode, float drop_p, uint32_t drop_site, const uint32_t* drop_seed, cudaStream_t st);
+// vi_attn_bwd.cu: key-blocked tensor-core kernels for the other bf16 problems (up to 512 keys) and their workspace
+int vi_attn_bwd_long(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, const void* dout,
+                     int64_t ldo, void* dq, int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv,
+                     const uint8_t* key_mask, const float* pair_dist, const float* bias_affine, float* d_affine, int B, int H,
+                     int Lq, int Lk, int mask_mode, float drop_p, uint32_t drop_site, const uint32_t* drop_seed, float* workspace,
+                     int64_t workspace_floats, cudaStream_t st);
+int64_t vi_attn_bwd_long_floats(int B, int H, int Lq);
 
 extern "C" int vi_transpose(const void* src, int64_t ld, void* dst, int64_t ldd, int rows, int cols, int pad_rows, int dtype,
                             vi_stream_t stream) {
@@ -1102,39 +1250,70 @@ extern "C" int vi_rowdot_bwd(const float* dout, const float* x, const float* w, 
   return VI_OK;
 }
 
+// per device (vi_init): the dynamic shared memory of the fp32 rows kernel (up to 195 KB at 380 keys)
+int vi_attn_bwd_f32_init() {
+  VI_CUDA(cudaFuncSetAttribute(attn_bwd_f32_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  return VI_OK;
+}
+
+// shared memory of attn_bwd_kernel<float>; the problems it fits (<= 220 KB: up to 201 keys) keep that kernel
+static size_t attn_bwd_f32_smem(int Lk) { return ((size_t)Lk * (65 * 2 + 64 * 2 + 1) + 8 * (size_t)(128 + 2 * Lk)) * sizeof(float); }
+
+// 0 for problems vi_attn_bwd does not accept, so that a call bound to fail does not first grow the caller's scratch
+extern "C" int64_t vi_attn_bwd_workspace(int B, int H, int Lq, int Lk, int dtype) {
+  if (B <= 0 || H <= 0 || Lq <= 0 || Lk <= 0 || Lk > 512) return 0;
+  if (dtype == VI_DT_F32) {
+    if (attn_bwd_f32_smem(Lk) <= 220 * 1024 || Lk > ATTN_BWD_F32_MAX_KEYS) return 0;
+    return 2 * (int64_t)B * H * Lq * Lk + 2 * (int64_t)B * H;
+  }
+  return dtype == VI_DT_BF16 ? vi_attn_bwd_long_floats(B, H, Lq) : 0;
+}
+
 extern "C" int vi_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, const void* dout,
                            int64_t ldo, void* dq, int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv, int dtype,
                            const uint8_t* key_mask, const float* pair_dist, const float* bias_affine, float* d_affine, int B,
                            int H, int Lq, int Lk, int mask_mode, float drop_p, uint32_t drop_site, const uint32_t* drop_seed,
-                           vi_stream_t stream) {
+                           float* workspace, int64_t workspace_floats, vi_stream_t stream) {
   VI_CHECK_ARG(q && k && v && dout && dq && dk && dv, "vi_attn_bwd: null operand");
   VI_CHECK_ARG(B > 0 && H > 0 && Lq > 0 && Lk > 0, "vi_attn_bwd: bad sizes B=%d H=%d Lq=%d Lk=%d", B, H, Lq, Lk);
-  VI_CHECK_ARG(((size_t)Lk * (65 * 2 + 64 * 2 + 1) + 8 * (size_t)(128 + 2 * Lk)) * sizeof(float) <= 220 * 1024,
-               "vi_attn_bwd: Lk=%d keys do not fit the 220 KB shared-memory tile", Lk);
+  VI_CHECK_ARG(dtype == VI_DT_BF16 || dtype == VI_DT_F32, "vi_attn_bwd: dtype %d is neither bf16 nor fp32", dtype);
+  VI_CHECK_ARG(Lk <= 512, "vi_attn_bwd: Lk=%d exceeds the 512 keys of the attention kernels", Lk);
   VI_CHECK_ARG(!pair_dist || bias_affine, "vi_attn_bwd: pair_dist needs bias_affine");
   VI_CHECK_ARG(drop_p >= 0.f && drop_p < 1.f && (drop_p == 0.f || drop_seed), "vi_attn_bwd: bad dropout arguments");
   VI_CHECK_ARG(H * 64 <= ldq && H * 64 <= ldk && H * 64 <= ldv && H * 64 <= ldo, "vi_attn_bwd: leading dimensions smaller than H*64");
   if (dtype == VI_DT_BF16) {
     const int rc = vi_attn_bwd_tc(q, ldq, k, ldk, v, ldv, dout, ldo, dq, lddq, dk, lddk, dv, lddv, key_mask, pair_dist,
                                   bias_affine, d_affine, B, H, Lq, Lk, mask_mode, drop_p, drop_site, drop_seed, ST(stream));
-    if (rc <= 0) return rc;            // launched (0) or failed (< 0); 1 = does not fit -> fp32-arithmetic kernel below
+    if (rc <= 0) return rc;            // launched (0) or failed (< 0); 1 = does not fit -> the key-blocked kernels
+    return vi_attn_bwd_long(q, ldq, k, ldk, v, ldv, dout, ldo, dq, lddq, dk, lddk, dv, lddv, key_mask, pair_dist, bias_affine,
+                            d_affine, B, H, Lq, Lk, mask_mode, drop_p, drop_site, drop_seed, workspace, workspace_floats,
+                            ST(stream));
   }
-  VI_CHECK_ARG(drop_p == 0.f, "vi_attn_bwd: attention dropout is implemented by the bf16 tensor-core kernel only");
+  VI_CHECK_ARG(drop_p == 0.f, "vi_attn_bwd: attention dropout needs bf16 operands (the fp32 check mode runs without it)");
   AttnBwdParams p;
   p.q = q; p.ldq = ldq; p.k = k; p.ldk = ldk; p.v = v; p.ldv = ldv; p.dout = dout; p.ldo = ldo;
   p.dq = dq; p.lddq = lddq; p.dk = dk; p.lddk = lddk; p.dv = dv; p.lddv = lddv;
   p.key_mask = key_mask; p.pair_dist = pair_dist; p.bias_affine = bias_affine; p.d_affine = d_affine;
   p.B = B; p.H = H; p.Lq = Lq; p.Lk = Lk; p.mask_mode = mask_mode;
-  const size_t smem = ((size_t)Lk * (65 * 2 + 64 * 2 + 1) + 8 * (size_t)(128 + 2 * Lk)) * sizeof(float);
-  if (dtype == VI_DT_BF16) {
-    static bool set = false;
-    if (!set) { VI_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)); set = true; }
-    VI_CUDA(vi_launch(attn_bwd_kernel<bf16>, dim3(H, B), dim3(256), smem, ST(stream), p));
-  } else {
+  const size_t smem = attn_bwd_f32_smem(Lk);
+  if (smem <= 220 * 1024) {
     static bool set = false;
     if (!set) { VI_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)); set = true; }
     VI_CUDA(vi_launch(attn_bwd_kernel<float>, dim3(H, B), dim3(256), smem, ST(stream), p));
+    return VI_OK;
   }
+  VI_CHECK_ARG(Lk <= ATTN_BWD_F32_MAX_KEYS, "vi_attn_bwd: Lk=%d exceeds the %d keys of the fp32 check mode", Lk,
+               ATTN_BWD_F32_MAX_KEYS);
+  const int64_t need = vi_attn_bwd_workspace(B, H, Lq, Lk, dtype);
+  VI_CHECK_ARG(workspace && workspace_floats >= need, "vi_attn_bwd: the workspace has %lld floats where %lld are needed (vi_attn_bwd_workspace)",
+               (long long)(workspace ? workspace_floats : 0), (long long)need);
+  float* ws_p = workspace;
+  float* ws_s = workspace + (int64_t)B * H * Lq * Lk;
+  float* aff = ws_s + (int64_t)B * H * Lq * Lk;
+  const size_t smem_rows = ((size_t)Lk * (2 * 65 + 1) + 4 * 128 + 8) * sizeof(float);
+  VI_CUDA(vi_launch(attn_bwd_f32_rows_kernel, dim3(H, B), dim3(128), smem_rows, ST(stream), p, ws_p, ws_s, aff));
+  VI_CUDA(vi_launch(attn_bwd_f32_keys_kernel, dim3((Lk + 3) / 4, H, B), dim3(256), 0, ST(stream), p, (const float*)ws_p,
+                    (const float*)ws_s, (const float*)aff));
   return VI_OK;
 }
 

@@ -659,12 +659,14 @@ def act_bwd(x: torch.Tensor, dy: torch.Tensor, act: int) -> torch.Tensor:
 def attention_bwd(q, k, v, do, dq, dk, dv, B: int, Lq: int, Lk: int, mask_mode: int, key_mask=None, pair_dist=None,
                   bias_affine=None, d_affine=None, drop=None):
     """adjoint of one attention problem into the row views dq / dk / dv; d_affine (fp32 [2]) accumulates the gradient of the GASA
-    affine when pair_dist is given; drop = (p, site, seed tensor) of the forward dropout"""
+    affine when pair_dist is given; drop = (p, site, seed tensor) of the forward dropout.  The long-sequence kernels keep their
+    softmax statistics (or, in the fp32 check mode, the P / dS rows) in the shared workspace."""
+    ws = workspace(q.device, lib.vi_attn_bwd_workspace(B, HEADS, Lq, Lk, _DT[q.dtype]))
     lib.vi_attn_bwd(q.data_ptr(), q.stride(0), k.data_ptr(), k.stride(0), v.data_ptr(), v.stride(0), do.data_ptr(), do.stride(0),
                     dq.data_ptr(), dq.stride(0), dk.data_ptr(), dk.stride(0), dv.data_ptr(), dv.stride(0), _DT[q.dtype], _ptr(key_mask),
                     _ptr(pair_dist), _ptr(bias_affine), _ptr(d_affine) if pair_dist is not None else None, B, HEADS, Lq, Lk, mask_mode,
                     float(drop[0]) if drop else 0.0, (int(drop[1]) & 0xFFFFFFFF) if drop else 0, drop[2].data_ptr() if drop else None,
-                    _stream())
+                    ws.data_ptr(), ws.numel(), _stream())
 
 
 def feat_wgrad(dt: torch.Tensor, feat: torch.Tensor, w_shape, want_db: bool):
